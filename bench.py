@@ -2,6 +2,7 @@
 """bench.py — sub-system Newton solves/sec on B200 (BASELINE.json metric).
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
+  python bench.py --gpus 1 --steps K --dump-outputs DIR    # + the outputs of the last timed step as DIR/*.npy
   python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path, host cores
 
 Workload of the line (config.workload): BASELINE.json configs[1] — 2^20 independent synthetic
@@ -76,7 +77,16 @@ def parse():
     ap.add_argument("--workload", default="configs1", choices=["configs1", "multistart8", "sweep64m"],
                     help="configs1 = the bench line (BASELINE configs[1], with the other configs under `configs`); "
                          "multistart8 / sweep64m: that config alone as the line")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the line's timed path returned in its last step as DIR/<name>.npy "
+                         "(float64 coordinates, float32 roots / update counts / flags; rank 0's batches; at most 64 MB, a fixed "
+                         "seeded sample of instances beyond that), so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "configs1"):
+        ap.error("--dump-outputs writes the outputs of the configs1 line of the b200 arm")
+    return args
 
 
 def load_peaks():
@@ -176,6 +186,38 @@ def make_batches(synth, n, rank):
     half = n // 2
     first = rank * half
     return [synth.make_pp(half, first=first), synth.make_ang(half, first=first)]
+
+
+DUMP_LIMIT = 60 * 10**6  # bytes of array data: with the .npy headers a dump stays under 64 MB
+OUT_NAMES = {1: ("x", "y"), 5: ("p1x", "p1y", "p2x", "p2y")}  # include/gcs_b200.h: point kinds x,y; line kinds p1, p2
+
+
+def dump_outputs(path, dbs):
+    """Writes the outputs of the device batches `dbs` as path/k<kind>_<name>.npy: the solved coordinates
+    (float64), the chosen root and, per seed, the update count and the convergence flag (float32, [n_seeds][n]).
+    Where all of it would exceed DUMP_LIMIT, every array of a kind keeps the same fixed seeded sample of
+    instances, whose indices are written as k<kind>_index.npy (float64)."""
+    total = sum(d.n * (8 * len(d.out) + 4 + 8 * d.n_seeds) for d in dbs)
+    # the share of every kind's instances kept, the 8-byte index of each kept instance included
+    keep = DUMP_LIMIT / (total + 8 * sum(d.n for d in dbs)) if total > DUMP_LIMIT else None
+    os.makedirs(path, exist_ok=True)
+    written = 0
+    for d in dbs:
+        idx = None
+        if keep is not None:
+            idx = np.sort(np.random.default_rng(d.kind).choice(d.n, int(d.n * keep), replace=False))
+        arrays = {name: col.cpu().numpy() for name, col in zip(OUT_NAMES[d.kind], d.out)}
+        arrays["root_index"] = d.root_index.cpu().numpy().astype(np.float32)
+        arrays["iters"] = d.iters.cpu().numpy().astype(np.float32)
+        arrays["converged"] = d.converged.cpu().numpy().astype(np.float32)
+        for name, a in arrays.items():
+            a = a if idx is None else a[..., idx]
+            np.save(os.path.join(path, f"k{d.kind}_{name}.npy"), np.ascontiguousarray(a))
+            written += a.nbytes
+        if idx is not None:
+            np.save(os.path.join(path, f"k{d.kind}_index.npy"), idx.astype(np.float64))
+            written += 8 * idx.size
+    assert written <= DUMP_LIMIT, written
 
 
 def base_config(args):
@@ -325,7 +367,7 @@ def run_reference(args, rank):
     for b in bs:
         b.want_cand = False
     ts = []
-    for i in range(args.warmup + max(args.steps, 1)):
+    for i in range(args.warmup + args.steps):
         t0 = time.perf_counter()
         for b in bs:
             solve(b, threads)
@@ -857,6 +899,11 @@ def main():
         }
         if violation is None:
             del devb0
+
+    # devb are the batches `value` was timed on, holding the outputs of their last timed launch (every
+    # timed launch of a batch recomputes the same outputs from the same inputs)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, devb)
 
     # ---- iteration histogram -> algorithmic work of the dominant kernel ----
     it1 = devb[0].iters.cpu().numpy()

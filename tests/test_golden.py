@@ -7,7 +7,7 @@ import numpy as np
 import pytest
 
 import oracle_lib as O
-from util import bits
+from util import bits, digest
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
@@ -94,19 +94,17 @@ def test_golden_contains_the_known_answers(gcs):
 
 
 def test_reference_build_agrees_with_oracle_at_scale(gcs, built):
-    """Where oracle/_ref exists (build container, GPU box): 20k instances per kind, live."""
-    import ref_lib as R
-    if not R.available():
-        pytest.skip("oracle/_ref/libgcs_ref.so not built here")
+    """20k instances per kind against what the reference build returned for them (digests in
+    tests/golden/ref_loops.npz, oracle/make_golden_ref_loops.py): candidates bit for bit, iteration counts
+    where below the reference's cap, chosen roots."""
+    ref = np.load(os.path.join(GOLD, "ref_loops.npz"))
     for kind in (1, 2, 3, 4, 5):
         a = O.solve(gcs.synth.make(kind, 20000, seed=77 + kind).alloc_outputs())
-        b = R.solve_batch(gcs.synth.make(kind, 20000, seed=77 + kind).alloc_outputs(), count_iters=True)
-        same = (bits(a.cand) == bits(b.cand)) | (np.isnan(a.cand) & np.isnan(b.cand))
-        assert same.all(), kind
-        capped = b.iters >= 999
-        assert np.array_equal(a.iters[~capped], b.iters[~capped])
-        seen = b.root_index != 2
-        assert np.array_equal(a.root_index[seen], b.root_index[seen])
+        cand, iters, root = ref[f"scale_k{kind}_sha256"]
+        assert digest(a.cand) == cand, kind
+        # the reference's count cannot tell i=999 from the cap (see ref_driver.cpp)
+        assert digest(np.minimum(a.iters, 999)) == iters, kind
+        assert digest(a.root_index) == root, kind
 
 
 def test_components_fixture_is_complete():

@@ -13,8 +13,28 @@ import host_lib as H
 import oracle_lib as O
 import sketch_gen as S
 from test_host_packer import GOLD, same_pos
+from util import digest, positions
 
 pytestmark = pytest.mark.gpu
+WHOLE_SKETCHES = [(31, 1, 3000), (32, 2, 3000), (33, 3, 3000)]
+
+
+def _ref_loops():
+    """What the reference build's sequential loop left in the elements of the sketches below
+    (oracle/make_golden_ref_loops.py)."""
+    return np.load(os.path.join(GOLD, "ref_loops.npz"))
+
+
+def _assert_same_elements(got, ref, name):
+    """Solved flags equal, every position bit for bit (NaN with NaN) through the stored digest."""
+    pos, is_set = positions(got)
+    assert np.array_equal(is_set, ref[f"{name}_set"]), np.nonzero(is_set != ref[f"{name}_set"])[0][:8]
+    assert digest(pos) == str(ref[f"{name}_pos_sha256"]), f"{name}: solved positions differ from the reference loop"
+
+
+def config4_sample(n):
+    """The fixed sample of the 100k-point linkage whose coordinates are stored beside their digest."""
+    return np.sort(np.random.default_rng(4).choice(n, 4096, replace=False))
 
 
 @pytest.fixture(scope="module")
@@ -186,36 +206,11 @@ def test_an_exception_mid_list_stops_the_loop_like_the_reference(host):
     assert sum(e["is_set"] for e in bat["elements"]) == 32  # leaves 0..29 only
 
 
-def _leaf_dicts(el, edges, leaves):
-    """Leaf list (dicts) of a decomposition given as element-index triples: the two constraints of
-    the new element + a virtual edge between its parents; the base keeps its real edges."""
-    by_pair = {(min(e["a"], e["b"]), max(e["a"], e["b"])): e for e in edges}
-    placed = set(leaves[0])
-    out = []
-    for k, lf in enumerate(leaves):
-        new = None if k == 0 else [i for i in lf if i not in placed][0]
-        es = []
-        for a, b in ((lf[0], lf[1]), (lf[0], lf[2]), (lf[1], lf[2])):
-            e = by_pair.get((min(a, b), max(a, b)))
-            if k == 0:
-                if e:
-                    es.append(e)
-            elif new in (a, b):
-                es.append(e)
-            else:
-                es.append({"a": a, "b": b, "type": 2})
-        if new is not None:
-            placed.add(new)
-        out.append({"elems": list(lf), "edges": es})
-    return out
-
-
-@pytest.mark.parametrize("seed,first,n", [(31, 1, 3000), (32, 2, 3000), (33, 3, 3000)])
+@pytest.mark.parametrize("seed,first,n", WHOLE_SKETCHES)
 def test_whole_sketch_pipeline_equals_reference_loop_on_the_same_leaves(host, seed, first, n):
     """GeometricConstraintSystem::solveGeometricConstraintSystem on a whole sketch (check ->
-    peel decomposition -> batched solveGcs on the GPU) against the reference build's sequential
-    loop over the same leaves (oracle/_ref), bit for bit."""
-    import ref_lib as R
+    peel decomposition -> batched solveGcs on the GPU) against what the reference build's sequential
+    loop over the same leaves left (tests/golden/ref_loops.npz), bit for bit."""
     el, lv = S.make_sketch(n, seed=seed, first_shape=first)
     edges = S.sketch_graph(el, lv)
     rc, got, stats = H.system_solve_ex(el, edges)
@@ -223,13 +218,8 @@ def test_whole_sketch_pipeline_equals_reference_loop_on_the_same_leaves(host, se
     assert stats["leaves"] == len(el) - 2 and stats["solved"] == stats["leaves"]
     assert stats["launches"] <= 5 * stats["waves"] and stats["waves"] < 0.2 * stats["leaves"]
     assert all(e["is_set"] for e in got)
-    if not R.available():
-        pytest.skip("oracle/_ref not present on this box")
-    nl, leaves, _, _ = H.decompose(el, edges)
-    rc, status, exp = R.leaves_solve(el, _leaf_dicts(el, edges, leaves))
-    assert rc == 0 and set(status) == {0}
-    for g, e in zip(got, exp):
-        assert g["is_set"] == e["is_set"] and same_pos(g["pos"], e["pos"])
+    ref = _ref_loops()
+    _assert_same_elements(got, ref, f"sketch{seed}")
 
 
 def test_config4_linkage_100k_points(host):
@@ -237,7 +227,8 @@ def test_config4_linkage_100k_points(host):
     the public entry point (check -> decomposition -> wave-batched solveGcs on the GPU).  The sketch
     is one the reference itself solves consistently (sketch_gen.make_linkage), so (i) EVERY distance
     constraint holds in the result to 1e-6 and (ii) every solved position equals, bit for bit, what
-    the reference build's sequential loop (oracle/_ref) leaves in the same elements."""
+    the reference build's sequential loop leaves in the same elements (stored as a digest of all of them
+    and a fixed sample, tests/golden/ref_loops.npz)."""
     el, edges = S.make_linkage(100000, seed=4)
     rc, got, stats = H.system_solve_ex(el, edges)
     assert rc == 0, H.last_error()
@@ -249,33 +240,24 @@ def test_config4_linkage_100k_points(host):
     d = np.hypot(*(xy[ea[:, 0].astype(int)] - xy[ea[:, 1].astype(int)]).T)
     resid = np.abs(d - ea[:, 2]) / np.maximum(1.0, ea[:, 2])
     assert (resid < 1e-6).all(), f"{int((resid >= 1e-6).sum())} of {len(edges)} distances do not hold, worst {resid.max():.3e}"
-    import ref_lib as R
-    if not R.available():
-        pytest.skip("oracle/_ref not present on this box")
-    nl, leaves, _, _ = H.decompose(el, edges)
-    rc, status, exp = R.leaves_solve(el, _leaf_dicts(el, edges, leaves))
-    assert rc == 0 and set(status) == {0}
-    exp_xy = np.array([e["pos"] for e in exp])
-    assert np.array_equal(xy.view(np.uint64), exp_xy.view(np.uint64)), \
-        f"{int((xy.view(np.uint64) != exp_xy.view(np.uint64)).any(axis=1).sum())} of 100000 points differ from the reference loop"
+    ref = _ref_loops()
+    idx = config4_sample(len(xy))
+    sample = ref["config4_xy_sample"]
+    assert np.array_equal(xy[idx].view(np.uint64), sample.view(np.uint64)), \
+        f"{int((xy[idx].view(np.uint64) != sample.view(np.uint64)).any(axis=1).sum())} of {len(idx)} sampled points differ from the reference loop"
+    assert digest(xy) == str(ref["config4_xy_sha256"]), "the points outside the stored sample differ from the reference loop"
 
 
 def test_unchecked_linkage_runs_into_the_cap_like_the_reference(host):
     """The stress case: a linkage drawn without regard for the reference's unchecked candidate-1 pick
     (heuristics.hpp:56).  Some leaf returns the mirrored root, the circles below it no longer meet
     and those runs spin to the iteration cap - in the reference and here alike, bit for bit."""
-    import ref_lib as R
     el, edges = S.make_linkage_unchecked(6000, seed=4)
     rc, got, stats = H.system_solve_ex(el, edges)
     assert rc == 0, H.last_error()
     assert stats["solved"] == stats["leaves"] == 5998
-    if not R.available():
-        pytest.skip("oracle/_ref not present on this box")
-    nl, leaves, _, _ = H.decompose(el, edges)
-    rc, status, exp = R.leaves_solve(el, _leaf_dicts(el, edges, leaves))
-    assert rc == 0
-    for g, e in zip(got, exp):
-        assert same_pos(g["pos"], e["pos"])
+    ref = _ref_loops()
+    _assert_same_elements(got, ref, "unchecked")
 
 
 def test_one_sketch_over_several_devices_equals_one_device(host, gcs):

@@ -14,7 +14,7 @@ import pytest
 
 import host_lib as H
 import oracle_lib as O
-from util import bits
+from util import bits, digest
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "merge3.npz")
 CASES = [1, 2, 3, 4]
@@ -123,31 +123,42 @@ def test_cuda_single_call_functions_match_the_reference(gpu, host, gold, kase):
     assert same(out[exp_ok == 1], exp[exp_ok == 1]).all()
 
 
-@pytest.mark.gpu
-def test_cuda_batch_equals_reference_build_on_fresh_rows(gpu, host):
-    """Beyond the committed fixtures: new random rows against the reference build where it travelled."""
-    import ref_lib as R
-    if not R.available():
-        pytest.skip("oracle/_ref not built on this box")
+def _ref_loops():
+    """What the reference build returned for the fresh rows and the PPP merges below (oracle/make_golden_ref_loops.py)."""
+    return np.load(os.path.join(os.path.dirname(GOLD), "ref_loops.npz"))
+
+
+def fresh_rows():
+    """Seeded rows beyond merge3.npz, per case, from the fixture's own generators (oracle/make_golden_merge3.py).
+    Case 4 leaves out the rows the host refuses: the documented difference, a fixed line shorter than 1e-9 that the
+    reference still solves (no intersection frame -> nearest-to-canvas on arbitrary candidates)."""
     import importlib.util
     spec = importlib.util.spec_from_file_location("mg3", os.path.join(os.path.dirname(GOLD), "..", "..", "oracle", "make_golden_merge3.py"))
     mg = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mg)
     mg.N = 2048
     rng = np.random.default_rng(77)
+    out = []
     for kase, gen in ((1, mg.rows_pp), (2, mg.rows_line), (3, mg.rows_pl), (4, mg.rows_ll)):
         rows = gen(rng)
-        exp, exp_ok = R.m3_solve(kase, rows)
         if kase == 4:
-            # the documented difference: a fixed line shorter than 1e-9 that the reference still
-            # solves (no intersection frame -> nearest-to-canvas on arbitrary candidates) is refused
-            tiny = (np.hypot(rows[:, 2] - rows[:, 0], rows[:, 3] - rows[:, 1]) < 1e-9) & (exp_ok == 1)
-            assert tiny.sum() < 0.01 * len(rows)
-            rows, exp, exp_ok = rows[~tiny], exp[~tiny], exp_ok[~tiny]
+            tiny = np.nonzero(np.hypot(rows[:, 2] - rows[:, 0], rows[:, 3] - rows[:, 1]) < 1e-9)[0]
+            refused = [i for i in tiny if H.m3_pack(4, rows[i:i + 1])[0] != 0]
+            assert len(refused) < 0.01 * len(rows)
+            rows = np.delete(rows, refused, axis=0)
+        out.append((kase, rows))
+    return out
+
+
+@pytest.mark.gpu
+def test_cuda_batch_equals_reference_build_on_fresh_rows(gpu, host):
+    """Beyond merge3.npz: 2048 more seeded rows per case against what the reference build returned for them."""
+    ref = _ref_loops()
+    for kase, rows in fresh_rows():
         rc, out, ok, launches = H.m3_solve(kase, rows, mode=1)
         assert rc == 0 and launches == 1
-        assert np.array_equal(ok, exp_ok)
-        assert same(out[exp_ok == 1], exp[exp_ok == 1]).all(), kase
+        assert np.array_equal(ok, ref[f"m3fresh_k{kase}_ok"])
+        assert digest(out[ok == 1]) == str(ref[f"m3fresh_k{kase}_out_sha256"]), kase
 
 
 def _ppp_scenario(rng, n_ref_only=1, n_shared_ra=2, n_shared_rb=2, n_free=2, n_a_only=1, n_b_only=1, lines=True, coincide=False):
@@ -202,42 +213,37 @@ def _ppp_scenario(rng, n_ref_only=1, n_shared_ra=2, n_shared_rb=2, n_free=2, n_a
     return types, canvas4, clusters
 
 
+PPP_SHAPES = [dict(), dict(n_shared_ra=3, n_shared_rb=2, n_free=3), dict(n_shared_ra=1, n_shared_rb=1, n_free=1, lines=False),
+              dict(n_free=0), dict(n_shared_rb=0), dict(coincide=True), dict(n_shared_ra=3, n_shared_rb=3, n_free=4, n_ref_only=3)]
+
+
+def ppp_scenarios():
+    rng = np.random.default_rng(77)
+    return [_ppp_scenario(rng, **kw) for rep in range(6) for kw in PPP_SHAPES]
+
+
 @pytest.mark.gpu
 def test_ppp_merge_enumeration_loop_equals_the_reference_solver(gpu, host):
     """The reference's real candidate enumeration (Merge3PppSolver::solve, merge3_ppp_solver.cpp:18-214:
     reference cluster x shared fixed points x free candidates, one solve2D + pickByTriangleOrientation
     per candidate, two-point anchor placement, merge, score, first best wins) against its batched form
     Gcs::B200::solveMerge3Ppp, which collects every candidate of a merge in a Merge3Batch and solves
-    them with ONE kernel launch: the merged pose must come out bit for bit, over scenarios with
-    8..72 candidates, lines riding along, a coincident candidate the loop skips, and merges without
-    any candidate."""
-    import ref_lib as R
-    if not R.available() or not hasattr(R.load(), "gcs_ref_m3_ppp_merge"):
-        pytest.skip("oracle/_ref (with the reference's merge3_ppp_solver.cpp) not present on this box")
-    rng = np.random.default_rng(77)
-    shapes = [dict(), dict(n_shared_ra=3, n_shared_rb=2, n_free=3), dict(n_shared_ra=1, n_shared_rb=1, n_free=1, lines=False),
-              dict(n_free=0), dict(n_shared_rb=0), dict(coincide=True), dict(n_shared_ra=3, n_shared_rb=3, n_free=4, n_ref_only=3)]
-    total = 0
-    devnull = os.open(os.devnull, os.O_WRONLY)
-    saved = os.dup(2)
-    os.dup2(devnull, 2)  # the reference prints a line per candidate
-    try:
-        for rep in range(6):
-            for kw in shapes:
-                types, canvas4, clusters = _ppp_scenario(rng, **kw)
-                n_ref, ids_ref, pose_ref = R.m3_ppp_merge(types, canvas4, clusters)
-                n, ids, pose, score, (cands, scored, launches) = H.m3_ppp_merge(types, canvas4, clusters)
-                assert n >= 0, H.last_error()
-                assert n == n_ref and np.array_equal(ids, ids_ref), (kw, n, n_ref)
-                assert same(pose, pose_ref).all(), (kw, pose, pose_ref)
-                assert launches == (1 if cands else 0), "every candidate of a merge goes through one launch"
-                if kw.get("n_free") == 0 or kw.get("n_shared_rb") == 0:
-                    assert cands == 0 or n >= 0
-                total += cands
-    finally:
-        os.dup2(saved, 2)
-        os.close(devnull)
-        os.close(saved)
+    them with ONE kernel launch: the merged pose must come out as the reference's solver returned it
+    (tests/golden/ref_loops.npz), bit for bit, over scenarios with 8..72 candidates, lines riding along,
+    a coincident candidate the loop skips, and merges without any candidate."""
+    ref = _ref_loops()
+    scenarios = ppp_scenarios()
+    assert len(scenarios) == len(ref["ppp_n"])
+    total, at = 0, 0
+    for (types, canvas4, clusters), n_ref in zip(scenarios, ref["ppp_n"]):
+        ids_ref, pose_ref = ref["ppp_ids"][at:at + n_ref], ref["ppp_pose4"][at:at + n_ref]
+        at += n_ref
+        n, ids, pose, score, (cands, scored, launches) = H.m3_ppp_merge(types, canvas4, clusters)
+        assert n >= 0, H.last_error()
+        assert n == n_ref and np.array_equal(ids, ids_ref), (n, n_ref)
+        assert same(pose, pose_ref).all(), (pose, pose_ref)
+        assert launches == (1 if cands else 0), "every candidate of a merge goes through one launch"
+        total += cands
     assert total > 500
 
 
@@ -323,35 +329,25 @@ def _quiet_stderr():
     return cm()
 
 
-def _need_ref_merge():
-    import ref_lib as R
-    if not R.available() or not hasattr(R.load(), "gcs_ref_m3_merge"):
-        pytest.skip("oracle/_ref (with the reference's Merge3 solver classes) not present on this box")
-    return R
-
-
 @pytest.mark.gpu
 @pytest.mark.parametrize("case", ["pll", "lpp", "llp"])
 def test_line_case_enumeration_loops_equal_the_reference_solvers(gpu, host, case):
     """Merge3PllSolver / Merge3LppSolver / Merge3LlpSolver::solve (merge3_pll_solver.cpp:15-189,
     merge3_lpp_solver.cpp:15-208, merge3_llp_solver.cpp:15-190) against their batched forms: every candidate
-    of a merge through ONE kernel launch of its kind (K2 / K3 / K4), the merged pose bit for bit - over merges
-    with 1..36 candidates, passengers of both types, and merges without any candidate."""
-    R = _need_ref_merge()
-    rng = np.random.default_rng(90 + len(case) + ord(case[0]))
+    of a merge through ONE kernel launch of its kind (K2 / K3 / K4), the merged pose bit for bit - over the
+    committed merges of every M3_SHAPES shape (1..36 candidates, passengers of both types, merges without any
+    candidate) and what the reference's classes returned for them."""
+    scenarios = [g for g in _golden_nodes() if g[0] == case]
+    assert len(scenarios) >= 15
     total = 0
-    with _quiet_stderr():
-        for rep in range(6):
-            for spec in M3_SHAPES[case]:
-                types, canvas4, clusters = _m3_scenario(rng, spec)
-                n_ref, ids_ref, pose_ref, _ = R.m3_merge(case, types, canvas4, clusters)
-                n, ids, pose, score, (cands, scored, launches, by) = H.m3_merge(case, types, canvas4, clusters)
-                assert n >= 0, H.last_error()
-                assert n == n_ref and np.array_equal(ids, ids_ref), (case, spec, n, n_ref)
-                assert same(pose, pose_ref).all(), (case, spec, pose, pose_ref)
-                assert launches == (1 if cands else 0), "every candidate of a merge goes through one launch"
-                total += cands
-    assert total > 150
+    for _, types, canvas4, clusters, n_ref, ids_ref, pose_ref, _ in scenarios:
+        n, ids, pose, score, (cands, scored, launches, by) = H.m3_merge(case, types, canvas4, clusters)
+        assert n >= 0, H.last_error()
+        assert n == n_ref and np.array_equal(ids, ids_ref), (case, n, n_ref)
+        assert same(pose, pose_ref).all(), (case, pose, pose_ref)
+        assert launches == (1 if cands else 0), "every candidate of a merge goes through one launch"
+        total += cands
+    assert total > 5 * len(scenarios)
 
 
 M3_NODE_SHAPES = [
@@ -371,87 +367,79 @@ M3_NODE_SHAPES = [
 ]
 
 
+def _golden_merge_nodes():
+    """The committed merge-node scenarios as (case the shape is built for, scenario): the fixture holds
+    M3_NODE_SHAPES in order, repeated."""
+    nodes = [g for g in _golden_nodes() if g[0] == "node"]
+    return [(M3_NODE_SHAPES[k % len(M3_NODE_SHAPES)][0], g) for k, g in enumerate(nodes)]
+
+
 @pytest.mark.gpu
 def test_merge_node_case_order_equals_the_reference(gpu, host):
     """What a Merge3 plan node does (bottom_up_plan_solver.cpp:393-431): PPP, PLL, LPP, LLP in that order, the LLL
     detector, the rigid fallback.  Gcs::B200::solveMerge3Node (PPP with its own launch; the three line cases
-    enumerated into ONE batch, at most a launch per kind) against the same sequence over the reference's own
-    classes: the same case decides and the merged pose is the same bit for bit."""
-    R = _need_ref_merge()
+    enumerated into ONE batch, at most a launch per kind) against what the same sequence over the reference's own
+    classes returned for the committed merge nodes: the same case decides and the merged pose is the same bit for bit."""
     names = {0: "ppp", 1: "pll", 2: "lpp", 3: "llp", 4: "fallback", 5: "unsolvable"}
-    rng = np.random.default_rng(4711)
     seen = set()
-    with _quiet_stderr():
-        for rep in range(5):
-            for expect, spec in M3_NODE_SHAPES:
-                types, canvas4, clusters = _m3_scenario(rng, spec, permute=(expect != "fallback"))
-                n_ref, ids_ref, pose_ref, by_ref = R.m3_merge("node", types, canvas4, clusters)
-                n, ids, pose, score, (cands, scored, launches, by) = H.m3_merge("node", types, canvas4, clusters)
-                assert n >= 0, H.last_error()
-                assert names[by] == names[by_ref] == expect, (expect, spec, names[by], names[by_ref])
-                assert n == n_ref and np.array_equal(ids, ids_ref), (expect, spec, n, n_ref)
-                assert same(pose, pose_ref).all(), (expect, spec)
-                assert launches <= 4
-                seen.add(expect)
+    for expect, (_, types, canvas4, clusters, n_ref, ids_ref, pose_ref, by_ref) in _golden_merge_nodes():
+        n, ids, pose, score, (cands, scored, launches, by) = H.m3_merge("node", types, canvas4, clusters)
+        assert n >= 0, H.last_error()
+        assert names[by] == names[by_ref] == expect, (expect, names[by], names[by_ref])
+        assert n == n_ref and np.array_equal(ids, ids_ref), (expect, n, n_ref)
+        assert same(pose, pose_ref).all(), expect
+        assert launches <= 4
+        seen.add(expect)
     assert seen == {"ppp", "pll", "llp", "fallback", "unsolvable"}  # LPP is shadowed by PLL in this order (see the shapes)
 
 
 @pytest.mark.gpu
 def test_a_level_of_merge_nodes_shares_one_batch(gpu, host):
-    """Gcs::B200::solveMerge3Level: every merge node of a plan-tree level - all shapes mixed, 40 nodes - through ONE
-    Merge3Batch, at most one launch per equation-pair kind for the whole level; node by node the result is the
-    reference's case order over its own classes, bit for bit."""
-    R = _need_ref_merge()
-    rng = np.random.default_rng(2718)
-    shapes = [M3_NODE_SHAPES[k % len(M3_NODE_SHAPES)] for k in range(40)]
-    nodes = [_m3_scenario(rng, spec, permute=(expect != "fallback")) for expect, spec in shapes]
+    """Gcs::B200::solveMerge3Level: every merge node of a plan-tree level - all shapes mixed, the committed merge
+    nodes - through ONE Merge3Batch, at most one launch per equation-pair kind for the whole level; node by node the
+    result is what the reference's case order over its own classes returned, bit for bit."""
+    golden = [g for _, g in _golden_merge_nodes()]
+    nodes = [(types, canvas4, clusters) for _, types, canvas4, clusters, *_ in golden]
     rc, got, (n_nodes, cands, launches) = H.m3_level(nodes)
     assert rc == 0, H.last_error()
-    assert n_nodes == 40 and cands > 100
+    assert n_nodes == len(nodes) >= 33 and cands > 2.5 * len(nodes)
     assert launches <= 4, "one launch per kind for the whole level"
-    with _quiet_stderr():
-        for (types, canvas4, clusters), (n, ids, pose, by) in zip(nodes, got):
-            n_ref, ids_ref, pose_ref, by_ref = R.m3_merge("node", types, canvas4, clusters)
-            assert by == by_ref and n == n_ref and np.array_equal(ids, ids_ref)
-            assert same(pose, pose_ref).all()
+    for (_, _, _, _, n_ref, ids_ref, pose_ref, by_ref), (n, ids, pose, by) in zip(golden, got):
+        assert by == by_ref and n == n_ref and np.array_equal(ids, ids_ref)
+        assert same(pose, pose_ref).all()
 
 
 def test_fallback_merge_equals_the_reference(host):
     """Merge3FallbackSolver::solve (merge3_fallback_solver.cpp:61-78): child 1, then child 2, fitted onto child 0
-    over the elements they share - host arithmetic only, so this one runs without a device."""
-    R = _need_ref_merge()
-    rng = np.random.default_rng(31)
+    over the elements they share - host arithmetic only, so this one runs without a device.  Over the committed
+    fallback merges and the committed merge nodes the fallback decides (their result is the fallback's)."""
+    scenarios = [g for g in _golden_nodes() if g[0] == "fallback"] + [g for e, g in _golden_merge_nodes() if e == "fallback"]
+    assert len(scenarios) >= 12
     hits = 0
-    for rep in range(20):
-        for spec in (dict(ra=(2, 0), rb=(2, 0), a=(1, 1)), dict(ra=(1, 1), rb=(0, 2), r=(1, 0), b=(2, 0)), dict(ra=(3, 0), rb=(0, 0), f=(2, 0)),
-                     dict(r=(1, 0), a=(1, 0), b=(1, 0)), dict(ra=(0, 1), rb=(0, 1), f=(0, 1))):
-            types, canvas4, clusters = _m3_scenario(rng, spec, permute=bool(rep % 2))
-            n_ref, ids_ref, pose_ref, _ = R.m3_merge("fallback", types, canvas4, clusters)
-            n, ids, pose, score, stats = H.m3_merge("fallback", types, canvas4, clusters)
-            assert n >= 0, H.last_error()
-            assert n == n_ref and np.array_equal(ids, ids_ref), (spec, n, n_ref)
-            assert same(pose, pose_ref).all(), spec
-            assert stats[2] == 0  # no kernel launch
-            hits += n > 0
-    assert hits > 20
+    for _, types, canvas4, clusters, n_ref, ids_ref, pose_ref, _ in scenarios:
+        n, ids, pose, score, stats = H.m3_merge("fallback", types, canvas4, clusters)
+        assert n >= 0, H.last_error()
+        assert n == n_ref and np.array_equal(ids, ids_ref), (n, n_ref)
+        assert same(pose, pose_ref).all()
+        assert stats[2] == 0  # no kernel launch
+        hits += n > 0
+    assert hits > 0.2 * len(scenarios)
 
 
 def test_a_level_without_candidates_needs_no_device(host):
     """solveMerge3Level on nodes that no enumeration has a candidate for (the fallback's and the unsolvable shapes,
     and no node at all): nothing is packed, nothing is launched - so this runs without a device - and every node
     is the reference's outcome."""
-    R = _need_ref_merge()
     rc, got, stats = H.m3_level([])
     assert rc == 0 and got == [] and stats == (0, 0, 0)
-    rng = np.random.default_rng(99)
-    shapes = [(e, s) for e, s in M3_NODE_SHAPES if e in ("fallback", "unsolvable")] * 5
-    nodes = [_m3_scenario(rng, spec, permute=(expect != "fallback")) for expect, spec in shapes]
+    chosen = [(e, g) for e, g in _golden_merge_nodes() if e in ("fallback", "unsolvable")]
+    assert len(chosen) >= 9
+    nodes = [(types, canvas4, clusters) for _, (_, types, canvas4, clusters, *_) in chosen]
     rc, got, (n_nodes, cands, launches) = H.m3_level(nodes)
     assert rc == 0, H.last_error()
     assert (n_nodes, cands, launches) == (len(nodes), 0, 0)
     names = {4: "fallback", 5: "unsolvable"}
-    for (expect, _), (types, canvas4, clusters), (n, ids, pose, by) in zip(shapes, nodes, got):
-        n_ref, ids_ref, pose_ref, by_ref = R.m3_merge("node", types, canvas4, clusters)
+    for (expect, (_, _, _, _, n_ref, ids_ref, pose_ref, by_ref)), (n, ids, pose, by) in zip(chosen, got):
         assert names[by] == names[by_ref] == expect
         assert n == n_ref and np.array_equal(ids, ids_ref) and same(pose, pose_ref).all()
 

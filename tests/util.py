@@ -1,9 +1,28 @@
 """Shared helpers for the parity tests."""
+import hashlib
+
 import numpy as np
 
 
 def bits(a):
     return np.ascontiguousarray(a, dtype=np.float64).view(np.uint64)
+
+
+def digest(a):
+    """sha256 of an array's bytes, every NaN made the same NaN: a stored fingerprint of an output too large for
+    tests/golden/ that still compares bit for bit, NaN with NaN."""
+    a = np.ascontiguousarray(a)
+    if a.dtype.kind == "f":
+        a = np.where(np.isnan(a), np.nan, a)
+    return hashlib.sha256(a.tobytes()).hexdigest()
+
+
+def positions(elements):
+    """[n][4] solved positions of host_lib element dicts (NaN past a point's two coordinates) and [n] is_set."""
+    pos = np.full((len(elements), 4), np.nan)
+    for i, e in enumerate(elements):
+        pos[i, :len(e["pos"])] = e["pos"]
+    return pos, np.array([e["is_set"] for e in elements], dtype=np.uint8)
 
 
 def assert_batches_identical(got, ref, what=""):
