@@ -71,6 +71,34 @@ class CBatch(C.Structure):
     ]
 
 
+class CProgramRow(C.Structure):
+    """gcs_b200_program_row: one leaf of a sketch program."""
+    _fields_ = [
+        ("solver", C.c_int32),
+        ("elem", C.c_int32 * 3),
+        ("value", C.c_int32 * 3),
+        ("code", C.c_int32),
+        ("sign", C.c_double * 3),
+        ("canvas", C.c_double * 9),
+    ]
+
+
+class CProgramDesc(C.Structure):
+    """gcs_b200_program_desc."""
+    _fields_ = [
+        ("n_waves", C.c_int32),
+        ("n_slots", C.c_int32),
+        ("n_values", C.c_int32),
+        ("reserved", C.c_int32),
+        ("n_rows", C.c_int64),
+        ("rows", C.POINTER(CProgramRow)),
+        ("offsets", C.POINTER(C.c_int64)),
+        ("slot_is_line", C.POINTER(C.c_uint8)),
+        ("initial", C.POINTER(C.c_double)),
+        ("value_is_angle", C.POINTER(C.c_uint8)),
+    ]
+
+
 _PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 # GCS_B200_LIB: developer override to A/B an experimental build of the same library
 LIB_PATH = os.environ.get("GCS_B200_LIB") or os.path.join(_PKG_DIR, "libgcs_b200.so")
@@ -84,6 +112,7 @@ EXPORTS = [
     "gcs_b200_contracted_stats", "gcs_b200_contracted_stats_ex", "gcs_b200_column_may_be_null", "gcs_b200_host_alloc_ex",
     "gcs_b200_solve_host_range_async", "gcs_b200_pcie_probe", "gcs_b200_solve_many",
     "gcs_b200_debug_path_buffer", "gcs_b200_resolve_variant",
+    "gcs_b200_program_create", "gcs_b200_program_run", "gcs_b200_program_run_host", "gcs_b200_program_destroy",
 ]
 
 
@@ -129,6 +158,11 @@ def load():
     lib.gcs_b200_selftest.argtypes = [C.c_int, C.c_uint64, C.c_int64, C.POINTER(C.c_uint64)]
     lib.gcs_b200_synth_pp.argtypes = [C.c_int, C.c_void_p, C.c_uint64, C.c_int64, C.c_int64,
                                       C.c_int, C.POINTER(C.c_void_p), C.c_void_p]
+    lib.gcs_b200_program_create.argtypes = [C.POINTER(CProgramDesc), C.c_int, C.POINTER(C.c_void_p)]
+    lib.gcs_b200_program_run.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
+    lib.gcs_b200_program_run_host.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
+                                              C.POINTER(C.c_float)]
+    lib.gcs_b200_program_destroy.argtypes = [C.c_void_p]
     _lib = lib
     return lib
 

@@ -156,6 +156,12 @@ int prepare_device(DeviceState* d)
 
 }  // namespace
 
+// for the other translation units of the library (sketch_program.cu)
+namespace gcsk {
+int api_fail(int code, const char* msg) { return fail(code, "%s", msg); }
+void api_count_launch() { g_launches.fetch_add(1); }
+}  // namespace gcsk
+
 extern "C" int gcs_b200_column_may_be_null(int kind, int c)
 {
     // columns that are identically zero in the anchored shapes of the zero-fixed solvers:

@@ -1,0 +1,467 @@
+// sketch_program.cu — sketch programs (include/gcs_b200.h, "sketch programs"): the wave plan of a
+// decomposed sketch kept on the device and run for K instances of its constraint values.
+//
+// Device layout.  The caller's tables are instance-major (values [K][n_values], positions
+// [K][n_slots][4]).  The kind batches of a wave put the K instances of one row next to each other
+// (sub-system (row r, instance j) at index r*K + j of its kind's batch), so the threads of a warp
+// share a row recipe and write consecutive column entries.  The gather kernel is the device copy of
+// the numeric half of the host packer (Gcs::B200 packNumeric, host/src/b200/leaf_batch.cpp): same
+// reads, same operations in the same order, built with --fmad=false like every kernel of the
+// library, so the columns it writes are the host's bit for bit.
+#include <cuda_runtime.h>
+
+#include <cstdarg>
+#include <cstdio>
+#include <cstring>
+#include <vector>
+
+#include "../../include/gcs_b200.h"
+
+namespace gcsk {
+int api_fail(int code, const char* msg);  // gcs_b200_api.cu: sets gcs_b200_last_error()
+void api_count_launch();
+}  // namespace gcsk
+
+namespace {
+
+int failf(int code, const char* fmt, ...)
+{
+    char buf[400];
+    va_list ap;
+    va_start(ap, fmt);
+    vsnprintf(buf, sizeof(buf), fmt, ap);
+    va_end(ap);
+    return gcsk::api_fail(code, buf);
+}
+
+#define PROG_TRY(expr)                                                                                    \
+    do {                                                                                                  \
+        cudaError_t e_ = (expr);                                                                          \
+        if (e_ != cudaSuccess) return failf(GCS_E_CUDA, "%s -> %s (%s:%d)", #expr, cudaGetErrorString(e_), \
+            __FILE__, __LINE__);                                                                          \
+    } while (0)
+
+constexpr int kKinds = GCS_KIND_COUNT;
+constexpr int kThreads = 256;
+
+// Gcs::B200::kindOf / the roles' element types / the values each solver reads, by solver id
+constexpr int kKindOfSolver[9] = { 0, GCS_KIND_PP, GCS_KIND_SDD, GCS_KIND_ANG, GCS_KIND_PP, GCS_KIND_SDD, GCS_KIND_PPL,
+    GCS_KIND_PLL, GCS_KIND_ANG };
+constexpr bool kRoleIsLine[9][3] = { {}, { 0, 0, 0 }, { 0, 0, 1 }, { 1, 0, 1 }, { 0, 0, 0 }, { 0, 0, 1 }, { 0, 1, 0 },
+    { 1, 1, 0 }, { 1, 0, 1 } };
+constexpr bool kReads[9][3] = { {}, { 1, 1, 1 }, { 1, 1, 1 }, { 1, 1, 1 }, { 0, 1, 1 }, { 0, 1, 1 }, { 0, 1, 1 },
+    { 0, 1, 1 }, { 1, 0, 1 } };
+constexpr int kInCols[kKinds + 1] = { 0, 6, 9, 10, 12, 13 };
+constexpr int kOutCols[kKinds + 1] = { 0, 2, 4, 2, 2, 4 };
+
+// one wave: rows [seg[0], seg[5]) of the program relative to `rows`, kind k + 1 at [seg[k], seg[k+1])
+struct WaveArgs {
+    const gcs_b200_program_row* rows;
+    long long seg[kKinds + 1];
+    long long K;
+    double* cols[kKinds];      // kind batch: input columns, then output columns, `cap` apart
+    long long cap[kKinds];
+    uint8_t* code[kKinds];
+    uint8_t* root[kKinds];
+    uint8_t* conv[kKinds];     // [2][n] of the launch
+    double* pos;               // [K][n_slots][4]
+    const double* val;         // [K][n_values]
+    long long n_slots, n_values;
+    uint32_t* nonconverged;    // [K] or null
+};
+
+struct Where {
+    long long r, j, i;  // row (relative to the wave), instance, index in the kind batch
+    int k;              // kind - 1
+};
+
+__device__ __forceinline__ bool locate(const WaveArgs& w, Where& at)
+{
+    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= w.seg[kKinds] * w.K) return false;
+    at.r = t / w.K;
+    at.j = t - at.r * w.K;
+    int k = 0;
+    while (at.r >= w.seg[k + 1]) ++k;
+    at.k = k;
+    at.i = (at.r - w.seg[k]) * w.K + at.j;
+    return true;
+}
+
+__global__ void __launch_bounds__(kThreads) program_gather_kernel(const WaveArgs w)
+{
+    Where at;
+    if (!locate(w, at)) return;
+    const gcs_b200_program_row& row = w.rows[at.r];
+    double* const pos = w.pos + at.j * w.n_slots * 4;
+    const double* const val = w.val + at.j * w.n_values;
+    double* const c = w.cols[at.k];
+    const long long cap = w.cap[at.k], i = at.i;
+    auto in = [&](int col, double v) { c[col * cap + i] = v; };
+    double* const pa = pos + 4 * (long long)row.elem[0];
+    double* const pb = pos + 4 * (long long)row.elem[1];
+    const double v0 = row.value[0] >= 0 ? val[row.value[0]] : 0.0;
+    const double v1 = row.value[1] >= 0 ? val[row.value[1]] : 0.0;
+    const double v2 = row.value[2] >= 0 ? val[row.value[2]] : 0.0;
+    const double* const cst = row.canvas;
+    w.code[at.k][i] = (uint8_t)row.code;
+    switch (row.solver) {
+    case 1:  // ZeroFixedPointsTriangle: P1 -> (0, 0), P2 -> (d12, 0)
+        pa[0] = 0.0, pa[1] = 0.0, pb[0] = v0, pb[1] = 0.0;
+        in(0, 0.0), in(1, 0.0), in(2, v1), in(3, v0), in(4, 0.0), in(5, v2);
+        break;
+    case 4:  // TwoFixedPointsDistance
+        in(0, pa[0]), in(1, pa[1]), in(2, v1), in(3, pb[0]), in(4, pb[1]), in(5, v2);
+        break;
+    case 2:  // ZeroFixedPPLTriangle
+        pa[0] = 0.0, pa[1] = 0.0, pb[0] = v0, pb[1] = 0.0;
+        in(0, 0.0), in(1, 0.0), in(2, v0), in(3, 0.0);
+        in(4, row.sign[1] * v1), in(5, row.sign[2] * v2), in(6, cst[0]), in(7, cst[1]), in(8, cst[2]);
+        break;
+    case 5:  // TwoFixedPointsLine
+        in(0, pa[0]), in(1, pa[1]), in(2, pb[0]), in(3, pb[1]);
+        in(4, row.sign[1] * v1), in(5, row.sign[2] * v2), in(6, cst[0]), in(7, cst[1]), in(8, cst[2]);
+        break;
+    case 6:  // FixedPointAndLineFreePoint: a point, b line
+        in(0, pa[0]), in(1, pa[1]), in(2, v1), in(3, pb[0]), in(4, pb[1]), in(5, pb[2]), in(6, pb[3]);
+        in(7, row.sign[2] * v2), in(8, cst[0]), in(9, cst[1]);
+        break;
+    case 7:  // TwoFixedLinesFreePoint
+        in(0, pa[0]), in(1, pa[1]), in(2, pa[2]), in(3, pa[3]), in(4, row.sign[1] * v1);
+        in(5, pb[0]), in(6, pb[1]), in(7, pb[2]), in(8, pb[3]), in(9, row.sign[2] * v2);
+        in(10, cst[0]), in(11, cst[1]);
+        break;
+    case 3: {  // ZeroFixedLLPAngleTriangle: line1 -> (x1, 0)-(x2, 0), point -> (0, sign * d(P, line1)); v0 holds cos(angle)
+        const double sd1 = row.sign[1] * v1;
+        pa[0] = cst[7], pa[1] = 0.0, pa[2] = cst[8], pa[3] = 0.0;
+        pb[0] = 0.0, pb[1] = sd1;
+        in(0, cst[5]), in(1, cst[6]), in(2, v0), in(3, cst[0]), in(4, cst[1]), in(5, cst[2]), in(6, cst[3]);
+        in(7, 0.0), in(8, sd1), in(9, row.sign[2] * v2), in(10, 0.0), in(11, 0.0), in(12, cst[4]);
+        break;
+    }
+    case 8: {  // FixedLineAndPointFreeLine: a fixed line, b point; v0 holds cos(angle)
+        const double p1x = pa[0], p1y = pa[1], p2x = pa[2], p2y = pa[3];
+        in(0, p2x - p1x), in(1, p2y - p1y), in(2, v0), in(3, cst[0]), in(4, cst[1]), in(5, cst[2]), in(6, cst[3]);
+        in(7, pb[0]), in(8, pb[1]), in(9, row.sign[2] * v2), in(10, (p1x + p2x) / 2.0), in(11, (p1y + p2y) / 2.0);
+        in(12, cst[4]);
+        break;
+    }
+    }
+}
+
+__global__ void __launch_bounds__(kThreads) program_scatter_kernel(const WaveArgs w)
+{
+    Where at;
+    if (!locate(w, at)) return;
+    const gcs_b200_program_row& row = w.rows[at.r];
+    const int kind = at.k + 1;
+    const int nin = kind == 1 ? 6 : kind == 2 ? 9 : kind == 3 ? 10 : kind == 4 ? 12 : 13;
+    const int nout = (kind == GCS_KIND_SDD || kind == GCS_KIND_ANG) ? 4 : 2;
+    const double* const c = w.cols[at.k];
+    const long long cap = w.cap[at.k], i = at.i;
+    double* const dst = w.pos + at.j * w.n_slots * 4 + 4 * (long long)row.elem[2];
+    for (int q = 0; q < nout; ++q) dst[q] = c[(nin + q) * cap + i];
+    if (w.nonconverged) {
+        const long long n = (w.seg[at.k + 1] - w.seg[at.k]) * w.K;
+        const unsigned root = w.root[at.k][i];
+        if (root >= 2 || !w.conv[at.k][root * n + i]) atomicAdd(w.nonconverged + at.j, 1u);
+    }
+}
+
+int validate_desc(const gcs_b200_program_desc* d)
+{
+    if (!d) return failf(GCS_E_INVALID, "null program descriptor");
+    if (d->n_waves < 0 || d->n_slots < 0 || d->n_values < 0 || d->n_rows < 0)
+        return failf(GCS_E_INVALID, "negative count in the program descriptor");
+    if (!d->offsets) return failf(GCS_E_INVALID, "null offsets");
+    if ((d->n_rows > 0 && !d->rows) || (d->n_slots > 0 && (!d->slot_is_line || !d->initial)) || (d->n_values > 0 && !d->value_is_angle))
+        return failf(GCS_E_INVALID, "null table in the program descriptor");
+    const long long nseg = (long long)d->n_waves * kKinds;
+    if (d->offsets[0] != 0) return failf(GCS_E_INVALID, "offsets[0] is %lld, not 0", (long long)d->offsets[0]);
+    for (long long s = 0; s < nseg; ++s)
+        if (d->offsets[s + 1] < d->offsets[s])
+            return failf(GCS_E_INVALID, "offsets decrease at segment %lld (%lld after %lld)", s, (long long)d->offsets[s + 1], (long long)d->offsets[s]);
+    if (d->offsets[nseg] != d->n_rows)
+        return failf(GCS_E_INVALID, "offsets end at %lld, not at n_rows = %lld", (long long)d->offsets[nseg], (long long)d->n_rows);
+    for (int s = 0; s < d->n_slots; ++s)
+        if (d->slot_is_line[s] > 1) return failf(GCS_E_INVALID, "slot %d: type %d is neither point (0) nor line (1)", s, d->slot_is_line[s]);
+    for (long long s = 0; s < nseg; ++s) {
+        const int kind = (int)(s % kKinds) + 1;
+        for (long long r = d->offsets[s]; r < d->offsets[s + 1]; ++r) {
+            const gcs_b200_program_row& row = d->rows[r];
+            if (row.solver < 1 || row.solver > 8) return failf(GCS_E_INVALID, "row %lld: unknown solver id %d", r, row.solver);
+            if (kKindOfSolver[row.solver] != kind)
+                return failf(GCS_E_INVALID, "row %lld: solver %d (kind %d) in a kind-%d segment", r, row.solver, kKindOfSolver[row.solver], kind);
+            if (row.code < 0 || row.code > 255) return failf(GCS_E_INVALID, "row %lld: code %d out of range", r, row.code);
+            for (int q = 0; q < 3; ++q) {
+                const int e = row.elem[q];
+                if (e < 0 || e >= d->n_slots) return failf(GCS_E_INVALID, "row %lld: element slot %d out of range (%d slots)", r, e, d->n_slots);
+                if ((d->slot_is_line[e] != 0) != kRoleIsLine[row.solver][q])
+                    return failf(GCS_E_INVALID, "row %lld: slot %d of role %c has the wrong element type for solver %d", r, e, 'a' + q, row.solver);
+                const int v = row.value[q];
+                if (!kReads[row.solver][q]) {
+                    if (v != -1) return failf(GCS_E_INVALID, "row %lld: solver %d reads no v%d, value slot must be -1 (got %d)", r, row.solver, q, v);
+                    continue;
+                }
+                if (v < 0 || v >= d->n_values) return failf(GCS_E_INVALID, "row %lld: value slot %d out of range (%d values)", r, v, d->n_values);
+                const bool cosine = q == 0 && (row.solver == 3 || row.solver == 8);
+                if ((d->value_is_angle[v] != 0) != cosine)
+                    return failf(GCS_E_INVALID, "row %lld: value slot %d is %s an angle slot, v%d of solver %d needs %s", r, v,
+                        d->value_is_angle[v] ? "" : "not", q, row.solver, cosine ? "one" : "a distance");
+            }
+            if (row.elem[0] == row.elem[1] || row.elem[0] == row.elem[2] || row.elem[1] == row.elem[2])
+                return failf(GCS_E_INVALID, "row %lld: the three roles need three distinct slots", r);
+        }
+    }
+    return GCS_OK;
+}
+
+}  // namespace
+
+struct gcs_b200_program {
+    int device = 0;
+    int n_waves = 0, n_slots = 0, n_values = 0;
+    long long n_rows = 0;
+    std::vector<long long> offsets;
+    long long max_rows[kKinds] = {};  // most rows of a kind in one wave
+    gcs_b200_program_row* rows = nullptr;
+    double* initial = nullptr;
+    cudaStream_t stream = nullptr;  // uploads and gcs_b200_program_run_host
+    // kind batches, sized for `scratch_k` instances
+    unsigned char* scratch = nullptr;
+    long long scratch_k = 0;
+    size_t scratch_bytes = 0;
+    // tables of gcs_b200_program_run_host, sized for `tables_k` instances
+    double* values = nullptr;
+    double* positions = nullptr;
+    uint32_t* counts = nullptr;
+    long long tables_k = 0;
+    cudaEvent_t ev[4] = {};
+};
+
+namespace {
+
+size_t align256(size_t v) { return (v + 255) / 256 * 256; }
+
+// sub-systems a kind's columns are spaced for: K instances of the kind's largest wave, in multiples
+// of 32 so that every column starts 256-byte aligned like the library's other device batches
+long long kind_cap(const gcs_b200_program* p, int kind, long long K) { return (p->max_rows[kind - 1] * K + 31) / 32 * 32; }
+
+size_t kind_bytes(int kind, long long cap)
+{
+    return align256((size_t)(kInCols[kind] + kOutCols[kind]) * cap * sizeof(double)) + 4 * align256((size_t)cap);
+}
+
+// device current; makes the kind batches hold K instances of the largest wave
+int ensure_scratch(gcs_b200_program* p, long long K, cudaStream_t st)
+{
+    if (K <= p->scratch_k) return GCS_OK;
+    size_t bytes = 0;
+    for (int k = 1; k <= kKinds; ++k) bytes += kind_bytes(k, kind_cap(p, k, K));
+    if (p->scratch) {
+        PROG_TRY(cudaStreamSynchronize(st));  // a run still in flight may use them
+        PROG_TRY(cudaFree(p->scratch));
+        p->scratch = nullptr, p->scratch_k = 0, p->scratch_bytes = 0;
+    }
+    if (bytes && cudaMalloc(&p->scratch, bytes) != cudaSuccess) {
+        cudaGetLastError();
+        return failf(GCS_E_NOMEM, "cudaMalloc(%zu) for the kind batches of %lld instances failed", bytes, K);
+    }
+    p->scratch_k = K, p->scratch_bytes = bytes;
+    return GCS_OK;
+}
+
+struct CurrentDevice {
+    int prev = -1;
+    explicit CurrentDevice(int dev)
+    {
+        if (cudaGetDevice(&prev) != cudaSuccess) cudaGetLastError(), prev = -1;
+        if (prev != dev) cudaSetDevice(dev);
+    }
+    ~CurrentDevice()
+    {
+        if (prev >= 0) cudaSetDevice(prev);
+    }
+};
+
+int run_on(gcs_b200_program* p, long long K, const double* values, double* positions, uint32_t* nonconverged, int variant,
+    cudaStream_t st)
+{
+    int rc = ensure_scratch(p, K, st);
+    if (rc != GCS_OK) return rc;
+    // every instance starts from the initial positions: one copy, then doubling copies
+    const size_t table = (size_t)p->n_slots * 4 * sizeof(double);
+    if (table) {
+        PROG_TRY(cudaMemcpyAsync(positions, p->initial, table, cudaMemcpyDeviceToDevice, st));
+        for (long long have = 1; have < K;) {
+            const long long n = have < K - have ? have : K - have;
+            PROG_TRY(cudaMemcpyAsync(reinterpret_cast<unsigned char*>(positions) + (size_t)have * table, positions, (size_t)n * table,
+                cudaMemcpyDeviceToDevice, st));
+            have += n;
+        }
+    }
+    if (nonconverged) PROG_TRY(cudaMemsetAsync(nonconverged, 0, (size_t)K * sizeof(uint32_t), st));
+    WaveArgs w;
+    memset(&w, 0, sizeof(w));
+    w.K = K;
+    w.pos = positions, w.val = values, w.n_slots = p->n_slots, w.n_values = p->n_values;
+    w.nonconverged = nonconverged;
+    {
+        unsigned char* at = p->scratch;
+        for (int k = 1; k <= kKinds; ++k) {
+            const long long cap = kind_cap(p, k, K);
+            w.cols[k - 1] = reinterpret_cast<double*>(at);
+            w.cap[k - 1] = cap;
+            unsigned char* flags = at + align256((size_t)(kInCols[k] + kOutCols[k]) * cap * sizeof(double));
+            w.code[k - 1] = flags, w.root[k - 1] = flags + align256((size_t)cap), w.conv[k - 1] = flags + 2 * align256((size_t)cap);
+            at += kind_bytes(k, cap);
+        }
+    }
+    for (int wave = 0; wave < p->n_waves; ++wave) {
+        const long long* off = p->offsets.data() + (size_t)wave * kKinds;
+        w.rows = p->rows + off[0];
+        for (int k = 0; k <= kKinds; ++k) w.seg[k] = off[k] - off[0];
+        const long long threads = w.seg[kKinds] * K;
+        if (threads == 0) continue;
+        const long long grid = (threads + kThreads - 1) / kThreads;
+        if (grid > 0x7fffffffLL) return failf(GCS_E_INVALID, "wave %d: %lld sub-systems are too many for one launch", wave, threads);
+        program_gather_kernel<<<(unsigned)grid, kThreads, 0, st>>>(w);
+        gcsk::api_count_launch();
+        PROG_TRY(cudaGetLastError());
+        gcs_b200_batch batch[kKinds];
+        const gcs_b200_batch* list[kKinds];
+        int count = 0;
+        for (int k = 1; k <= kKinds; ++k) {
+            const long long n = (w.seg[k] - w.seg[k - 1]) * K;
+            if (n == 0) continue;
+            gcs_b200_batch& b = batch[count];
+            memset(&b, 0, sizeof(b));
+            b.kind = k, b.n_seeds = 2, b.n = n, b.mem = GCS_MEM_DEVICE, b.variant = variant;
+            const long long cap = w.cap[k - 1];
+            for (int c = 0; c < kInCols[k]; ++c) b.in[c] = w.cols[k - 1] + c * cap;
+            for (int c = 0; c < kOutCols[k]; ++c) b.out[c] = w.cols[k - 1] + (kInCols[k] + c) * cap;
+            b.code = w.code[k - 1], b.root_index = w.root[k - 1], b.converged = w.conv[k - 1];
+            list[count++] = &b;
+        }
+        rc = gcs_b200_solve_many(list, count, p->device, st);
+        if (rc != GCS_OK) return rc;
+        program_scatter_kernel<<<(unsigned)grid, kThreads, 0, st>>>(w);
+        gcsk::api_count_launch();
+        PROG_TRY(cudaGetLastError());
+    }
+    return GCS_OK;
+}
+
+int check_run(const gcs_b200_program* p, long long K, const double* values, const double* positions, int variant)
+{
+    if (!p) return failf(GCS_E_INVALID, "null program");
+    if (K < 1) return failf(GCS_E_INVALID, "n_instances must be >= 1 (got %lld)", K);
+    if ((p->n_values > 0 && !values) || (p->n_slots > 0 && !positions)) return failf(GCS_E_INVALID, "null value or position table");
+    if (variant < GCS_VARIANT_DEFAULT || variant > GCS_VARIANT_CONTRACTED_LINEAR) return failf(GCS_E_INVALID, "unknown variant %d", variant);
+    return GCS_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int gcs_b200_program_create(const gcs_b200_program_desc* d, int device, gcs_b200_program** out)
+{
+    if (!out) return failf(GCS_E_INVALID, "null output handle");
+    *out = nullptr;
+    int rc = validate_desc(d);
+    if (rc != GCS_OK) return rc;
+    const int ndev = gcs_b200_device_count();
+    if (ndev <= 0) return failf(GCS_E_NO_DEVICE, "no CUDA device; this library has no CPU fallback");
+    if (device < 0 || device >= ndev) return failf(GCS_E_NO_DEVICE, "device %d out of range (%d present)", device, ndev);
+    CurrentDevice cur(device);
+    auto* p = new gcs_b200_program();
+    p->device = device, p->n_waves = d->n_waves, p->n_slots = d->n_slots, p->n_values = d->n_values, p->n_rows = d->n_rows;
+    p->offsets.assign(d->offsets, d->offsets + (size_t)d->n_waves * kKinds + 1);
+    for (int w = 0; w < d->n_waves; ++w)
+        for (int k = 0; k < kKinds; ++k) {
+            const long long rows = p->offsets[(size_t)w * kKinds + k + 1] - p->offsets[(size_t)w * kKinds + k];
+            if (rows > p->max_rows[k]) p->max_rows[k] = rows;
+        }
+    auto bail = [&](int code) {
+        gcs_b200_program_destroy(p);
+        return code;
+    };
+    if (cudaStreamCreateWithFlags(&p->stream, cudaStreamNonBlocking) != cudaSuccess) return bail(failf(GCS_E_CUDA, "stream creation failed"));
+    for (auto& e : p->ev)
+        if (cudaEventCreate(&e) != cudaSuccess) return bail(failf(GCS_E_CUDA, "event creation failed"));
+    const size_t row_bytes = (size_t)d->n_rows * sizeof(gcs_b200_program_row), init_bytes = (size_t)d->n_slots * 4 * sizeof(double);
+    if ((row_bytes && cudaMalloc(&p->rows, row_bytes) != cudaSuccess) || (init_bytes && cudaMalloc(&p->initial, init_bytes) != cudaSuccess)) {
+        cudaGetLastError();
+        return bail(failf(GCS_E_NOMEM, "cudaMalloc for a program of %lld rows and %d slots failed", (long long)d->n_rows, d->n_slots));
+    }
+    if ((row_bytes && cudaMemcpyAsync(p->rows, d->rows, row_bytes, cudaMemcpyHostToDevice, p->stream) != cudaSuccess)
+        || (init_bytes && cudaMemcpyAsync(p->initial, d->initial, init_bytes, cudaMemcpyHostToDevice, p->stream) != cudaSuccess)
+        || cudaStreamSynchronize(p->stream) != cudaSuccess)
+        return bail(failf(GCS_E_CUDA, "program upload failed: %s", cudaGetErrorString(cudaGetLastError())));
+    *out = p;
+    return GCS_OK;
+}
+
+int gcs_b200_program_run(gcs_b200_program* p, int64_t K, const double* values, double* positions, uint32_t* nonconverged, int variant,
+    void* stream)
+{
+    int rc = check_run(p, K, values, positions, variant);
+    if (rc != GCS_OK) return rc;
+    CurrentDevice cur(p->device);
+    return run_on(p, K, values, positions, nonconverged, variant, static_cast<cudaStream_t>(stream));
+}
+
+int gcs_b200_program_run_host(gcs_b200_program* p, int64_t K, const double* values, double* positions, uint32_t* nonconverged,
+    int variant, float ms[3])
+{
+    int rc = check_run(p, K, values, positions, variant);
+    if (rc != GCS_OK) return rc;
+    CurrentDevice cur(p->device);
+    const size_t vbytes = (size_t)K * p->n_values * sizeof(double), pbytes = (size_t)K * p->n_slots * 4 * sizeof(double);
+    if (K > p->tables_k) {
+        PROG_TRY(cudaStreamSynchronize(p->stream));
+        cudaFree(p->values), cudaFree(p->positions), cudaFree(p->counts);
+        p->values = p->positions = nullptr, p->counts = nullptr, p->tables_k = 0;
+        if ((vbytes && cudaMalloc(&p->values, vbytes) != cudaSuccess) || (pbytes && cudaMalloc(&p->positions, pbytes) != cudaSuccess)
+            || cudaMalloc(&p->counts, (size_t)K * sizeof(uint32_t)) != cudaSuccess) {
+            cudaGetLastError();
+            return failf(GCS_E_NOMEM, "cudaMalloc for the tables of %lld instances (%zu + %zu bytes) failed", (long long)K, vbytes, pbytes);
+        }
+        p->tables_k = K;
+    }
+    cudaStream_t st = p->stream;
+    PROG_TRY(cudaEventRecord(p->ev[0], st));
+    if (vbytes) PROG_TRY(cudaMemcpyAsync(p->values, values, vbytes, cudaMemcpyHostToDevice, st));
+    PROG_TRY(cudaEventRecord(p->ev[1], st));
+    rc = run_on(p, K, p->values, p->positions, nonconverged ? p->counts : nullptr, variant, st);
+    if (rc != GCS_OK) {
+        cudaStreamSynchronize(st);
+        return rc;
+    }
+    PROG_TRY(cudaEventRecord(p->ev[2], st));
+    if (pbytes) PROG_TRY(cudaMemcpyAsync(positions, p->positions, pbytes, cudaMemcpyDeviceToHost, st));
+    if (nonconverged) PROG_TRY(cudaMemcpyAsync(nonconverged, p->counts, (size_t)K * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    PROG_TRY(cudaEventRecord(p->ev[3], st));
+    PROG_TRY(cudaStreamSynchronize(st));
+    if (ms)
+        for (int q = 0; q < 3; ++q) PROG_TRY(cudaEventElapsedTime(&ms[q], p->ev[q], p->ev[q + 1]));
+    return GCS_OK;
+}
+
+void gcs_b200_program_destroy(gcs_b200_program* p)
+{
+    if (!p) return;
+    {
+        CurrentDevice cur(p->device);
+        if (p->stream) cudaStreamSynchronize(p->stream), cudaStreamDestroy(p->stream);
+        for (auto e : p->ev)
+            if (e) cudaEventDestroy(e);
+        cudaFree(p->rows), cudaFree(p->initial), cudaFree(p->scratch);
+        cudaFree(p->values), cudaFree(p->positions), cudaFree(p->counts);
+        cudaGetLastError();
+    }
+    delete p;
+}
+
+}  // extern "C"

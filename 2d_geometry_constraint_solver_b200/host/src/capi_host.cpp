@@ -16,6 +16,7 @@
 
 #include <gcs/b200/canvas_transform.hpp>
 #include <gcs/b200/leaf_batch.hpp>
+#include <gcs/b200/sketch_program.hpp>
 #include <gcs/decomposition/top_down/stree_top_down_strategy.hpp>
 #include <gcs/model/constraints.hpp>
 #include <gcs/model/elements.hpp>
@@ -81,8 +82,9 @@ void readBack(const Gcs::Element& el, gcs_host_element& e)
 }
 
 // one leaf graph over (a subset of) shared elements; `local[i]` = index into `elems` of node i
+// `made` (may be null) receives the constraints of the real edges, in edge order
 Gcs::ConstraintGraph makeLeaf(const std::vector<std::shared_ptr<Gcs::Element>>& elems, const int32_t* local, int n_local,
-    const gcs_host_edge* edges, int n_edges)
+    const gcs_host_edge* edges, int n_edges, std::vector<std::shared_ptr<Gcs::Constraint>>* made = nullptr)
 {
     Gcs::ConstraintGraph g;
     std::vector<Gcs::ConstraintGraph::NodeIdType> nodes;
@@ -105,10 +107,39 @@ Gcs::ConstraintGraph makeLeaf(const std::vector<std::shared_ptr<Gcs::Element>>& 
             continue;
         }
         const auto eid = g.getGraph().addEdge(nodeOf(ed.a), nodeOf(ed.b)).value();
-        if (ed.type == 0)
-            g.addConstraint(eid, std::make_shared<Gcs::Constraint>(Gcs::DistanceConstraint(ed.value)));
-        else
-            g.addConstraint(eid, std::make_shared<Gcs::Constraint>(Gcs::AngleConstraint(ed.value, ed.flip != 0)));
+        auto con = ed.type == 0 ? std::make_shared<Gcs::Constraint>(Gcs::DistanceConstraint(ed.value))
+                                : std::make_shared<Gcs::Constraint>(Gcs::AngleConstraint(ed.value, ed.flip != 0));
+        if (made) made->push_back(con);
+        g.addConstraint(eid, std::move(con));
+    }
+    return g;
+}
+
+// A whole sketch as one graph over new elements; `made` (may be null) receives the constraints of
+// the real edges, in edge order.
+Gcs::ConstraintGraph makeSketch(std::vector<std::shared_ptr<Gcs::Element>>& elems, int n_el, const gcs_host_element* el, int n_edges,
+    const gcs_host_edge* edges, std::vector<std::shared_ptr<Gcs::Constraint>>* made = nullptr)
+{
+    Gcs::ConstraintGraph g;
+    std::vector<Gcs::ConstraintGraph::NodeIdType> nodes;
+    elems.reserve(static_cast<std::size_t>(n_el));
+    for (int i = 0; i < n_el; ++i) {
+        elems.push_back(makeElement(el[i]));
+        nodes.push_back(g.getGraph().addNode());
+        g.addElement(nodes.back(), elems.back());
+    }
+    for (int k = 0; k < n_edges; ++k) {
+        const auto& ed = edges[k];
+        const auto a = nodes.at(static_cast<std::size_t>(ed.a)), b = nodes.at(static_cast<std::size_t>(ed.b));
+        if (ed.type == 2) {
+            g.addVirtualEdge(a, b);
+            continue;
+        }
+        const auto eid = g.getGraph().addEdge(a, b).value();
+        auto con = ed.type == 0 ? std::make_shared<Gcs::Constraint>(Gcs::DistanceConstraint(ed.value))
+                                : std::make_shared<Gcs::Constraint>(Gcs::AngleConstraint(ed.value, ed.flip != 0));
+        if (made) made->push_back(con);
+        g.addConstraint(eid, std::move(con));
     }
     return g;
 }
@@ -343,27 +374,7 @@ GCS_API int gcs_host_system_solve_ex(int n_el, gcs_host_element* el, int n_edges
 {
     try {
         std::vector<std::shared_ptr<Gcs::Element>> elems;
-        Gcs::ConstraintGraph g;
-        std::vector<Gcs::ConstraintGraph::NodeIdType> nodes;
-        elems.reserve(static_cast<std::size_t>(n_el));
-        for (int i = 0; i < n_el; ++i) {
-            elems.push_back(makeElement(el[i]));
-            nodes.push_back(g.getGraph().addNode());
-            g.addElement(nodes.back(), elems.back());
-        }
-        for (int k = 0; k < n_edges; ++k) {
-            const auto& ed = edges[k];
-            const auto a = nodes.at(static_cast<std::size_t>(ed.a)), b = nodes.at(static_cast<std::size_t>(ed.b));
-            if (ed.type == 2) {
-                g.addVirtualEdge(a, b);
-                continue;
-            }
-            const auto eid = g.getGraph().addEdge(a, b).value();
-            if (ed.type == 0)
-                g.addConstraint(eid, std::make_shared<Gcs::Constraint>(Gcs::DistanceConstraint(ed.value)));
-            else
-                g.addConstraint(eid, std::make_shared<Gcs::Constraint>(Gcs::AngleConstraint(ed.value, ed.flip != 0)));
-        }
+        Gcs::ConstraintGraph g = makeSketch(elems, n_el, el, n_edges, edges);
         // the three steps of GeometricConstraintSystem::solveGeometricConstraintSystem, timed apart
         auto strategy = std::make_unique<Gcs::DeficitStreeBasedTopDownStrategy>();
         Gcs::DeficitStreeBasedTopDownStrategy* st = strategy.get();
@@ -785,5 +796,124 @@ GCS_API int gcs_host_canvas_transform(int n_el, gcs_host_element* el)
         return fail(ex);
     }
 }
+
+
+// ---- sketch programs (gcs/b200/sketch_program.hpp) ----
+// A handle holds the sketch's elements and constraints and the program compiled from them.  Values
+// are indexed by the order of the real (non-virtual) edges in `edges`.
+struct gcs_host_program {
+    std::vector<std::shared_ptr<Gcs::Element>> elems;
+    std::vector<std::shared_ptr<Gcs::Constraint>> cons;
+    std::unique_ptr<Gcs::B200::SketchProgram> prog;
+};
+
+// Check, decompose and compile a whole sketch (no device).  Returns 0 or -1.
+GCS_API int gcs_host_program_create(int n_el, const gcs_host_element* el, int n_edges, const gcs_host_edge* edges, gcs_host_program** out)
+{
+    try {
+        auto h = std::make_unique<gcs_host_program>();
+        Gcs::ConstraintGraph g = makeSketch(h->elems, n_el, el, n_edges, edges, &h->cons);
+        Gcs::DeficitStreeBasedTopDownStrategy st;
+        if (st.checkConstraintGraphConstrainedness(g) != Gcs::Constrainedness::WELL_CONSTRAINED && !st.resolve(g))
+            throw std::runtime_error("Gcs is not well-constrained, current algorithms do not support such inputs");
+        const auto leaves = st.decomposeConstraintGraph(g);
+        h->prog = std::make_unique<Gcs::B200::SketchProgram>(Gcs::B200::SketchProgram::compile(leaves, h->elems, h->cons));
+        *out = h.release();
+        return 0;
+    } catch (const std::exception& ex) {
+        return fail(ex);
+    }
+}
+
+// Compile a given leaf list (the records of gcs_host_leaves_solve; no device).  Returns 0 or -1.
+GCS_API int gcs_host_program_create_leaves(int n_el, const gcs_host_element* el, int n_leaves, const int32_t* leaf_elems,
+    const int32_t* edge_offsets, const gcs_host_edge* edges, gcs_host_program** out)
+{
+    try {
+        auto h = std::make_unique<gcs_host_program>();
+        for (int i = 0; i < n_el; ++i) h->elems.push_back(makeElement(el[i]));
+        std::vector<Gcs::ConstraintGraph> leaves;
+        for (int l = 0; l < n_leaves; ++l)
+            leaves.push_back(makeLeaf(h->elems, leaf_elems + 3 * l, 3, edges + edge_offsets[l], edge_offsets[l + 1] - edge_offsets[l], &h->cons));
+        h->prog = std::make_unique<Gcs::B200::SketchProgram>(Gcs::B200::SketchProgram::compile(leaves, h->elems, h->cons));
+        *out = h.release();
+        return 0;
+    } catch (const std::exception& ex) {
+        return fail(ex);
+    }
+}
+
+// counts[6] = waves, rows, slots, values, leaves, unsupported leaves.  Every other array may be NULL:
+// offsets [waves * 5 + 1] (rows of wave w, kind k: offsets[5w + k-1] .. offsets[5w + k]); per row
+// solver, leaf, elems [3] (slots of roles a, b, c), values [3] (value slots of v0..v2, -1 = none), code;
+// per slot solved_after (solved flag after a run); per leaf solver and level (-1 = not run).
+GCS_API int gcs_host_program_describe(const gcs_host_program* h, int64_t* counts, int64_t* offsets, int32_t* row_solver, int64_t* row_leaf,
+    int32_t* row_elems, int32_t* row_values, uint8_t* row_code, uint8_t* solved_after, int32_t* leaf_solver, int32_t* leaf_level)
+{
+    const auto& p = *h->prog;
+    const auto& rows = p.rows();
+    const auto& rep = p.report();
+    if (counts) {
+        counts[0] = static_cast<int64_t>(p.waves()), counts[1] = static_cast<int64_t>(rows.size());
+        counts[2] = static_cast<int64_t>(p.nSlots()), counts[3] = static_cast<int64_t>(p.nValues());
+        counts[4] = static_cast<int64_t>(rep.leaves), counts[5] = static_cast<int64_t>(rep.unsupported);
+    }
+    if (offsets) std::memcpy(offsets, p.offsets().data(), p.offsets().size() * sizeof(int64_t));
+    for (std::size_t r = 0; r < rows.size(); ++r) {
+        if (row_solver) row_solver[r] = rows[r].solver;
+        if (row_leaf) row_leaf[r] = p.rowLeaf()[r];
+        if (row_code) row_code[r] = static_cast<uint8_t>(rows[r].code);
+        for (int q = 0; q < 3; ++q) {
+            if (row_elems) row_elems[3 * r + static_cast<std::size_t>(q)] = rows[r].elem[q];
+            if (row_values) row_values[3 * r + static_cast<std::size_t>(q)] = rows[r].value[q];
+        }
+    }
+    if (solved_after) std::memcpy(solved_after, p.solvedAfter().data(), p.solvedAfter().size());
+    for (std::size_t l = 0; l < rep.leaves; ++l) {
+        if (leaf_solver) leaf_solver[l] = static_cast<int32_t>(rep.solver[l]);
+        if (leaf_level) leaf_level[l] = rep.level[l];
+    }
+    return 0;
+}
+
+// K instances: values [K][n_values] (angles in radians), positions out [K][n_slots][4], nonconverged
+// [K] (may be NULL).  stats (may be NULL) holds 7 values: launches, compile us, upload us, device us,
+// download us (device time), run us (host clock), devices used.  Returns 0 or -1.
+GCS_API int gcs_host_program_run(gcs_host_program* h, int64_t K, const double* values, double* positions, uint32_t* nonconverged,
+    int n_devices, int64_t* stats)
+{
+    try {
+        const auto st = h->prog->run(values, K, positions, nonconverged, n_devices);
+        if (stats) {
+            stats[0] = st.launches, stats[1] = static_cast<int64_t>(h->prog->compileSeconds() * 1e6);
+            stats[2] = static_cast<int64_t>(st.uploadMs * 1e3), stats[3] = static_cast<int64_t>(st.deviceMs * 1e3);
+            stats[4] = static_cast<int64_t>(st.downloadMs * 1e3), stats[5] = static_cast<int64_t>(st.seconds * 1e6);
+            stats[6] = n_devices;
+        }
+        return 0;
+    } catch (const std::exception& ex) {
+        return fail(ex);
+    }
+}
+
+// The edit loop: values (may be NULL: keep the current ones) become the constraints' values, then
+// SketchProgram::solve(); el receives every element's solved flag and position.  Returns 0 or -1.
+GCS_API int gcs_host_program_solve(gcs_host_program* h, const double* values, gcs_host_element* el)
+{
+    try {
+        if (values)
+            for (std::size_t v = 0; v < h->cons.size(); ++v) {
+                if (auto* d = h->cons[v]->getConstraintAs<Gcs::DistanceConstraint>()) d->distance = values[v];
+                if (auto* a = h->cons[v]->getConstraintAs<Gcs::AngleConstraint>()) a->angle = values[v];
+            }
+        h->prog->solve();
+        for (std::size_t i = 0; i < h->elems.size(); ++i) readBack(*h->elems[i], el[i]);
+        return 0;
+    } catch (const std::exception& ex) {
+        return fail(ex);
+    }
+}
+
+GCS_API void gcs_host_program_destroy(gcs_host_program* h) { delete h; }
 
 }  // extern "C"

@@ -300,6 +300,62 @@ GCS_B200_API void gcs_b200_host_free(void* p);
 GCS_B200_API int gcs_b200_synth_pp(int device, void* cuda_stream, uint64_t seed, int64_t first,
     int64_t n, int perturb_of, double* const cols[6], uint8_t* code);
 
+/* ---- sketch programs (csrc/sketch_program.cu) ----
+ * The wave plan of a decomposed sketch as device-resident row recipes, run for K instances of the
+ * sketch's constraint values: topology and canvas are fixed, only the values vary per instance.  A
+ * run enqueues, per wave, one gather launch (writes the kind batches' input columns from the
+ * position and value tables, and the zero-fixed anchors into the position table), the kind batches
+ * through gcs_b200_solve_many (rows_k x K sub-systems each, 2 seeds), and one scatter launch (every
+ * row's output into its target slot), with no host synchronisation between waves. */
+typedef struct gcs_b200_program_row {
+    int32_t solver;   /* Gcs::B200::SolverId, 1..8 */
+    int32_t elem[3];  /* element slots of roles a, b, c (c receives the result) */
+    int32_t value[3]; /* value slots of v0, v1, v2; -1 where the solver reads none */
+    int32_t code;     /* orientation code of the row (GCS_MAKE_CODE) */
+    double sign[3];   /* signOf(canvas side) factor of v0..v2 (1 where the value is not signed) */
+    /* canvas constants: solvers 2, 5: gnx gny canvas_len; 6, 7: cfx cfy; 3, 8: gnx gny cfdx cfdy
+     * canvas_len, and for 3 also fdx fdy x1 x2 (direction and endpoints (x1,0), (x2,0) of the
+     * anchored line) */
+    double canvas[9];
+} gcs_b200_program_row;
+
+typedef struct gcs_b200_program_desc {
+    int32_t n_waves;
+    int32_t n_slots;
+    int32_t n_values;
+    int32_t reserved;
+    int64_t n_rows;
+    const gcs_b200_program_row* rows; /* [n_rows], wave-major, kind-minor */
+    const int64_t* offsets;           /* [n_waves * GCS_KIND_COUNT + 1]: rows of (wave w, kind k) are
+                                         offsets[w*5 + k-1] .. offsets[w*5 + k]; offsets[0] = 0,
+                                         non-decreasing, last = n_rows */
+    const uint8_t* slot_is_line;      /* [n_slots]: 0 point, 1 line */
+    const double* initial;            /* [n_slots][4]: positions before the first wave (point: x, y, -, -) */
+    const uint8_t* value_is_angle;    /* [n_values]: 1 = the slot holds cos(angle) (read as v0 of solvers 3, 8 only) */
+} gcs_b200_program_desc;
+
+typedef struct gcs_b200_program gcs_b200_program;
+
+/* Validates the descriptor (before any device call: slots, value slots, offsets, solver ids, the
+ * kind of every row's segment, role types) and uploads it to `device`.  Host pointers; nothing of
+ * them is kept.  GCS_E_INVALID with a message for a malformed descriptor, GCS_E_NO_DEVICE without
+ * a device. */
+GCS_B200_API int gcs_b200_program_create(const gcs_b200_program_desc* desc, int device, gcs_b200_program** out);
+/* Runs K = n_instances >= 1 instances, stream-ordered on `cuda_stream`; every pointer is a device
+ * pointer.  values [K][n_values] (angle slots hold cos(angle)); positions [K][n_slots][4] is
+ * written from the program's initial positions first, so no state carries over between runs;
+ * nonconverged [K] (may be NULL): per instance, the rows whose chosen Newton run did not converge.
+ * Runs of one program must not overlap (they share its batch buffers): order them on one stream.
+ * Launches per run: at most n_waves * (2 + kinds present), independent of K. */
+GCS_B200_API int gcs_b200_program_run(gcs_b200_program* prog, int64_t n_instances, const double* values, double* positions,
+    uint32_t* nonconverged, int variant, void* cuda_stream);
+/* The same with host buffers (pinned ones move asynchronously): values up, run, positions and
+ * counts down on the program's own stream, then synchronises.  ms (may be NULL) receives the
+ * device time of upload, run and download. */
+GCS_B200_API int gcs_b200_program_run_host(gcs_b200_program* prog, int64_t n_instances, const double* values, double* positions,
+    uint32_t* nonconverged, int variant, float ms[3]);
+GCS_B200_API void gcs_b200_program_destroy(gcs_b200_program* prog);
+
 /* Test hook: on-device self check of the hand-written division / square root / 2x2 QR fast paths
  * against the generic IEEE code (csrc/selftest.cu).  Fills counts[8]:
  *   [0] divisions on the fast path, [1] of those differing from a/b,
