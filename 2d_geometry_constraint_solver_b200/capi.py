@@ -113,6 +113,7 @@ EXPORTS = [
     "gcs_b200_solve_host_range_async", "gcs_b200_pcie_probe", "gcs_b200_solve_many",
     "gcs_b200_debug_path_buffer", "gcs_b200_resolve_variant",
     "gcs_b200_program_create", "gcs_b200_program_run", "gcs_b200_program_run_host", "gcs_b200_program_destroy",
+    "gcs_b200_program_run_tangents", "gcs_b200_program_run_tangents_host",
 ]
 
 
@@ -162,6 +163,10 @@ def load():
     lib.gcs_b200_program_run.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
     lib.gcs_b200_program_run_host.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
                                               C.POINTER(C.c_float)]
+    lib.gcs_b200_program_run_tangents.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
+                                                  C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
+    lib.gcs_b200_program_run_tangents_host.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
+                                                       C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_float)]
     lib.gcs_b200_program_destroy.argtypes = [C.c_void_p]
     _lib = lib
     return lib

@@ -8,6 +8,14 @@
 // the numeric half of the host packer (Gcs::B200 packNumeric, host/src/b200/leaf_batch.cpp): same
 // reads, same operations in the same order, built with --fmad=false like every kernel of the
 // library, so the columns it writes are the host's bit for bit.
+//
+// Tangent runs (gcs_b200_program_run_tangents) add one launch per wave after the scatter: the
+// tangent kernel, one thread per (row, instance, direction t) with t fastest, so that consecutive
+// threads read and write consecutive doubles of the instance-major tangent tables (dvalues
+// [K][n_values][T], dpositions [K][n_slots][4][T]).  It forms the row's input-column tangents the way
+// the gather forms the columns, linearises the row at its chosen root (csrc/newton_tangent.cuh) and
+// writes the target's tangents.  The K2 / K5 batches then also keep their candidate planes, whose
+// chosen normal is the row's unknown.
 #include <cuda_runtime.h>
 
 #include <cstdarg>
@@ -16,6 +24,7 @@
 #include <vector>
 
 #include "../../include/gcs_b200.h"
+#include "newton_tangent.cuh"
 
 namespace gcsk {
 int api_fail(int code, const char* msg);  // gcs_b200_api.cu: sets gcs_b200_last_error()
@@ -64,10 +73,14 @@ struct WaveArgs {
     uint8_t* code[kKinds];
     uint8_t* root[kKinds];
     uint8_t* conv[kKinds];     // [2][n] of the launch
+    double* cand[kKinds];      // [2][2][n] of the launch, K2 and K5 of tangent runs only
     double* pos;               // [K][n_slots][4]
     const double* val;         // [K][n_values]
     long long n_slots, n_values;
     uint32_t* nonconverged;    // [K] or null
+    long long T;               // directions of a tangent run (0: plain run)
+    double* dpos;              // [K][n_slots][4][T]
+    const double* dval;        // [K][n_values][T]
 };
 
 struct Where {
@@ -75,16 +88,22 @@ struct Where {
     int k;              // kind - 1
 };
 
-__device__ __forceinline__ bool locate(const WaveArgs& w, Where& at)
+// sub-system s = r * K + j of the wave
+__device__ __forceinline__ void place(const WaveArgs& w, long long s, Where& at)
 {
-    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= w.seg[kKinds] * w.K) return false;
-    at.r = t / w.K;
-    at.j = t - at.r * w.K;
+    at.r = s / w.K;
+    at.j = s - at.r * w.K;
     int k = 0;
     while (at.r >= w.seg[k + 1]) ++k;
     at.k = k;
     at.i = (at.r - w.seg[k]) * w.K + at.j;
+}
+
+__device__ __forceinline__ bool locate(const WaveArgs& w, Where& at)
+{
+    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= w.seg[kKinds] * w.K) return false;
+    place(w, t, at);
     return true;
 }
 
@@ -168,6 +187,102 @@ __global__ void __launch_bounds__(kThreads) program_scatter_kernel(const WaveArg
     }
 }
 
+// the row's unknown at the chosen root: the output point (K1, K3, K4) or the chosen seed's normal
+// (K2, K5; candidate planes [2][2][n])
+template <int KIND>
+__device__ __forceinline__ void row_tangent(const WaveArgs& w, const Where& at, unsigned root, long long n, const double* kd, double dout[4])
+{
+    constexpr int nin = gcsk::Sys<KIND>::kCols;
+    const double* const c = w.cols[at.k];
+    const long long cap = w.cap[at.k];
+    double k[nin];
+#pragma unroll
+    for (int q = 0; q < nin; ++q) k[q] = c[q * cap + at.i];
+    double ux, uy;
+    if constexpr (KIND == GCS_KIND_SDD || KIND == GCS_KIND_ANG) {
+        ux = w.cand[at.k][(root * 2 + 0) * n + at.i], uy = w.cand[at.k][(root * 2 + 1) * n + at.i];
+    } else {
+        ux = c[nin * cap + at.i], uy = c[(nin + 1) * cap + at.i];
+    }
+    gcsk::RowTangent<KIND> lin;
+    lin.init(k, ux, uy);
+    lin.apply(kd, dout);
+}
+
+__global__ void __launch_bounds__(kThreads) program_tangent_kernel(const WaveArgs w)
+{
+    const long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (g >= w.seg[kKinds] * w.K * w.T) return;
+    const long long T = w.T, s = g / T;
+    Where at;
+    place(w, s, at);
+    const gcs_b200_program_row& row = w.rows[at.r];
+    double* const dpos = w.dpos + at.j * w.n_slots * 4 * T + (g - s * T);
+    const double* const dval = w.dval + at.j * w.n_values * T + (g - s * T);
+    auto dp = [&](int slot, int q) -> double& { return dpos[(4 * (long long)slot + q) * T]; };
+    const int a = row.elem[0], b = row.elem[1];
+    const double v0 = row.value[0] >= 0 ? dval[row.value[0] * T] : 0.0;
+    const double v1 = row.value[1] >= 0 ? dval[row.value[1] * T] : 0.0;
+    const double v2 = row.value[2] >= 0 ? dval[row.value[2] * T] : 0.0;
+    // the gather's tangent: input-column tangents, and the zero-fixed anchors' tangents
+    double kd[13] = {};
+    switch (row.solver) {
+    case 1:
+        dp(a, 0) = 0.0, dp(a, 1) = 0.0, dp(b, 0) = v0, dp(b, 1) = 0.0;
+        kd[2] = v1, kd[3] = v0, kd[5] = v2;
+        break;
+    case 4:
+        kd[0] = dp(a, 0), kd[1] = dp(a, 1), kd[2] = v1, kd[3] = dp(b, 0), kd[4] = dp(b, 1), kd[5] = v2;
+        break;
+    case 2:
+        dp(a, 0) = 0.0, dp(a, 1) = 0.0, dp(b, 0) = v0, dp(b, 1) = 0.0;
+        kd[2] = v0, kd[4] = row.sign[1] * v1, kd[5] = row.sign[2] * v2;
+        break;
+    case 5:
+        kd[0] = dp(a, 0), kd[1] = dp(a, 1), kd[2] = dp(b, 0), kd[3] = dp(b, 1);
+        kd[4] = row.sign[1] * v1, kd[5] = row.sign[2] * v2;
+        break;
+    case 6:
+        kd[0] = dp(a, 0), kd[1] = dp(a, 1), kd[2] = v1, kd[3] = dp(b, 0), kd[4] = dp(b, 1), kd[5] = dp(b, 2), kd[6] = dp(b, 3);
+        kd[7] = row.sign[2] * v2;
+        break;
+    case 7:
+        kd[0] = dp(a, 0), kd[1] = dp(a, 1), kd[2] = dp(a, 2), kd[3] = dp(a, 3), kd[4] = row.sign[1] * v1;
+        kd[5] = dp(b, 0), kd[6] = dp(b, 1), kd[7] = dp(b, 2), kd[8] = dp(b, 3), kd[9] = row.sign[2] * v2;
+        break;
+    case 3: {
+        const double sd1 = row.sign[1] * v1;
+        dp(a, 0) = 0.0, dp(a, 1) = 0.0, dp(a, 2) = 0.0, dp(a, 3) = 0.0, dp(b, 0) = 0.0, dp(b, 1) = sd1;
+        kd[2] = v0, kd[8] = sd1, kd[9] = row.sign[2] * v2;
+        break;
+    }
+    case 8: {
+        const double p1x = dp(a, 0), p1y = dp(a, 1), p2x = dp(a, 2), p2y = dp(a, 3);
+        kd[0] = p2x - p1x, kd[1] = p2y - p1y, kd[2] = v0, kd[7] = dp(b, 0), kd[8] = dp(b, 1), kd[9] = row.sign[2] * v2;
+        kd[10] = (p1x + p2x) / 2.0, kd[11] = (p1y + p2y) / 2.0;
+        break;
+    }
+    }
+    const int kind = at.k + 1;
+    const int nout = (kind == GCS_KIND_SDD || kind == GCS_KIND_ANG) ? 4 : 2;
+    const long long n = (w.seg[at.k + 1] - w.seg[at.k]) * w.K;
+    const unsigned root = w.root[at.k][at.i];
+    double out[4];
+    if (root >= 2 || !w.conv[at.k][root * n + at.i]) {
+        // the scatter's test: not a root, so the implicit function theorem does not apply
+        out[0] = out[1] = out[2] = out[3] = __longlong_as_double(0x7ff8000000000000LL);
+    } else {
+        switch (kind) {
+        case GCS_KIND_PP: row_tangent<GCS_KIND_PP>(w, at, root, n, kd, out); break;
+        case GCS_KIND_SDD: row_tangent<GCS_KIND_SDD>(w, at, root, n, kd, out); break;
+        case GCS_KIND_PPL: row_tangent<GCS_KIND_PPL>(w, at, root, n, kd, out); break;
+        case GCS_KIND_PLL: row_tangent<GCS_KIND_PLL>(w, at, root, n, kd, out); break;
+        default: row_tangent<GCS_KIND_ANG>(w, at, root, n, kd, out); break;
+        }
+    }
+    for (int q = 0; q < nout; ++q) dp(row.elem[2], q) = out[q];
+}
+
 int validate_desc(const gcs_b200_program_desc* d)
 {
     if (!d) return failf(GCS_E_INVALID, "null program descriptor");
@@ -227,15 +342,18 @@ struct gcs_b200_program {
     gcs_b200_program_row* rows = nullptr;
     double* initial = nullptr;
     cudaStream_t stream = nullptr;  // uploads and gcs_b200_program_run_host
-    // kind batches, sized for `scratch_k` instances
+    // kind batches
     unsigned char* scratch = nullptr;
-    long long scratch_k = 0;
     size_t scratch_bytes = 0;
     // tables of gcs_b200_program_run_host, sized for `tables_k` instances
     double* values = nullptr;
     double* positions = nullptr;
     uint32_t* counts = nullptr;
     long long tables_k = 0;
+    // tangent tables of gcs_b200_program_run_tangents_host, sized for `tangents_kt` instances x directions
+    double* dvalues = nullptr;
+    double* dpositions = nullptr;
+    long long tangents_kt = 0;
     cudaEvent_t ev[4] = {};
 };
 
@@ -247,27 +365,32 @@ size_t align256(size_t v) { return (v + 255) / 256 * 256; }
 // of 32 so that every column starts 256-byte aligned like the library's other device batches
 long long kind_cap(const gcs_b200_program* p, int kind, long long K) { return (p->max_rows[kind - 1] * K + 31) / 32 * 32; }
 
-size_t kind_bytes(int kind, long long cap)
+bool has_cand(int kind, bool tangents) { return tangents && (kind == GCS_KIND_SDD || kind == GCS_KIND_ANG); }
+
+// input and output columns, then code, root and the two convergence planes, then (tangent runs, K2
+// and K5) the candidate planes
+size_t kind_bytes(int kind, long long cap, bool tangents)
 {
-    return align256((size_t)(kInCols[kind] + kOutCols[kind]) * cap * sizeof(double)) + 4 * align256((size_t)cap);
+    return align256((size_t)(kInCols[kind] + kOutCols[kind]) * cap * sizeof(double)) + 4 * align256((size_t)cap)
+        + (has_cand(kind, tangents) ? align256((size_t)4 * cap * sizeof(double)) : 0);
 }
 
 // device current; makes the kind batches hold K instances of the largest wave
-int ensure_scratch(gcs_b200_program* p, long long K, cudaStream_t st)
+int ensure_scratch(gcs_b200_program* p, long long K, bool tangents, cudaStream_t st)
 {
-    if (K <= p->scratch_k) return GCS_OK;
     size_t bytes = 0;
-    for (int k = 1; k <= kKinds; ++k) bytes += kind_bytes(k, kind_cap(p, k, K));
+    for (int k = 1; k <= kKinds; ++k) bytes += kind_bytes(k, kind_cap(p, k, K), tangents);
+    if (bytes <= p->scratch_bytes) return GCS_OK;
     if (p->scratch) {
         PROG_TRY(cudaStreamSynchronize(st));  // a run still in flight may use them
         PROG_TRY(cudaFree(p->scratch));
-        p->scratch = nullptr, p->scratch_k = 0, p->scratch_bytes = 0;
+        p->scratch = nullptr, p->scratch_bytes = 0;
     }
-    if (bytes && cudaMalloc(&p->scratch, bytes) != cudaSuccess) {
+    if (cudaMalloc(&p->scratch, bytes) != cudaSuccess) {
         cudaGetLastError();
         return failf(GCS_E_NOMEM, "cudaMalloc(%zu) for the kind batches of %lld instances failed", bytes, K);
     }
-    p->scratch_k = K, p->scratch_bytes = bytes;
+    p->scratch_bytes = bytes;
     return GCS_OK;
 }
 
@@ -284,10 +407,11 @@ struct CurrentDevice {
     }
 };
 
+// T = 0: a plain run.  T > 0: also the tangents along T directions (dvalues / dpositions).
 int run_on(gcs_b200_program* p, long long K, const double* values, double* positions, uint32_t* nonconverged, int variant,
-    cudaStream_t st)
+    cudaStream_t st, long long T = 0, const double* dvalues = nullptr, double* dpositions = nullptr)
 {
-    int rc = ensure_scratch(p, K, st);
+    int rc = ensure_scratch(p, K, T > 0, st);
     if (rc != GCS_OK) return rc;
     // every instance starts from the initial positions: one copy, then doubling copies
     const size_t table = (size_t)p->n_slots * 4 * sizeof(double);
@@ -301,11 +425,14 @@ int run_on(gcs_b200_program* p, long long K, const double* values, double* posit
         }
     }
     if (nonconverged) PROG_TRY(cudaMemsetAsync(nonconverged, 0, (size_t)K * sizeof(uint32_t), st));
+    // every slot's tangent is 0 before the first wave: the initial positions are constants
+    if (T > 0 && table) PROG_TRY(cudaMemsetAsync(dpositions, 0, (size_t)K * T * table, st));
     WaveArgs w;
     memset(&w, 0, sizeof(w));
     w.K = K;
     w.pos = positions, w.val = values, w.n_slots = p->n_slots, w.n_values = p->n_values;
     w.nonconverged = nonconverged;
+    w.T = T, w.dpos = dpositions, w.dval = dvalues;
     {
         unsigned char* at = p->scratch;
         for (int k = 1; k <= kKinds; ++k) {
@@ -314,7 +441,8 @@ int run_on(gcs_b200_program* p, long long K, const double* values, double* posit
             w.cap[k - 1] = cap;
             unsigned char* flags = at + align256((size_t)(kInCols[k] + kOutCols[k]) * cap * sizeof(double));
             w.code[k - 1] = flags, w.root[k - 1] = flags + align256((size_t)cap), w.conv[k - 1] = flags + 2 * align256((size_t)cap);
-            at += kind_bytes(k, cap);
+            if (has_cand(k, T > 0)) w.cand[k - 1] = reinterpret_cast<double*>(flags + 4 * align256((size_t)cap));
+            at += kind_bytes(k, cap, T > 0);
         }
     }
     for (int wave = 0; wave < p->n_waves; ++wave) {
@@ -325,6 +453,9 @@ int run_on(gcs_b200_program* p, long long K, const double* values, double* posit
         if (threads == 0) continue;
         const long long grid = (threads + kThreads - 1) / kThreads;
         if (grid > 0x7fffffffLL) return failf(GCS_E_INVALID, "wave %d: %lld sub-systems are too many for one launch", wave, threads);
+        const long long tgrid = (threads * T + kThreads - 1) / kThreads;
+        if (tgrid > 0x7fffffffLL)
+            return failf(GCS_E_INVALID, "wave %d: %lld sub-systems x %lld directions are too many for one launch", wave, threads, T);
         program_gather_kernel<<<(unsigned)grid, kThreads, 0, st>>>(w);
         gcsk::api_count_launch();
         PROG_TRY(cudaGetLastError());
@@ -340,7 +471,7 @@ int run_on(gcs_b200_program* p, long long K, const double* values, double* posit
             const long long cap = w.cap[k - 1];
             for (int c = 0; c < kInCols[k]; ++c) b.in[c] = w.cols[k - 1] + c * cap;
             for (int c = 0; c < kOutCols[k]; ++c) b.out[c] = w.cols[k - 1] + (kInCols[k] + c) * cap;
-            b.code = w.code[k - 1], b.root_index = w.root[k - 1], b.converged = w.conv[k - 1];
+            b.code = w.code[k - 1], b.root_index = w.root[k - 1], b.converged = w.conv[k - 1], b.cand = w.cand[k - 1];
             list[count++] = &b;
         }
         rc = gcs_b200_solve_many(list, count, p->device, st);
@@ -348,6 +479,11 @@ int run_on(gcs_b200_program* p, long long K, const double* values, double* posit
         program_scatter_kernel<<<(unsigned)grid, kThreads, 0, st>>>(w);
         gcsk::api_count_launch();
         PROG_TRY(cudaGetLastError());
+        if (T > 0) {
+            program_tangent_kernel<<<(unsigned)tgrid, kThreads, 0, st>>>(w);
+            gcsk::api_count_launch();
+            PROG_TRY(cudaGetLastError());
+        }
     }
     return GCS_OK;
 }
@@ -358,6 +494,66 @@ int check_run(const gcs_b200_program* p, long long K, const double* values, cons
     if (K < 1) return failf(GCS_E_INVALID, "n_instances must be >= 1 (got %lld)", K);
     if ((p->n_values > 0 && !values) || (p->n_slots > 0 && !positions)) return failf(GCS_E_INVALID, "null value or position table");
     if (variant < GCS_VARIANT_DEFAULT || variant > GCS_VARIANT_CONTRACTED_LINEAR) return failf(GCS_E_INVALID, "unknown variant %d", variant);
+    return GCS_OK;
+}
+
+// the checks that need no program come first; a null tangent table is refused unless the program
+// has nothing to put in it
+int check_tangent_run(const gcs_b200_program* p, long long K, const double* values, const double* positions, int T,
+    const double* dvalues, const double* dpositions, int variant)
+{
+    if (T < 1) return failf(GCS_E_INVALID, "n_tangents must be >= 1 (got %d)", T);
+    if (variant < GCS_VARIANT_DEFAULT || variant > GCS_VARIANT_CONTRACTED_LINEAR) return failf(GCS_E_INVALID, "unknown variant %d", variant);
+    if ((!dvalues && !(p && p->n_values == 0)) || (!dpositions && !(p && p->n_slots == 0)))
+        return failf(GCS_E_INVALID, "null tangent table (dvalues or dpositions)");
+    return check_run(p, K, values, positions, variant);
+}
+
+// device current, checks done
+int run_host(gcs_b200_program* p, long long K, const double* values, double* positions, uint32_t* nonconverged, int variant,
+    float ms[3], long long T, const double* dvalues, double* dpositions)
+{
+    const size_t vbytes = (size_t)K * p->n_values * sizeof(double), pbytes = (size_t)K * p->n_slots * 4 * sizeof(double);
+    if (K > p->tables_k) {
+        PROG_TRY(cudaStreamSynchronize(p->stream));
+        cudaFree(p->values), cudaFree(p->positions), cudaFree(p->counts);
+        p->values = p->positions = nullptr, p->counts = nullptr, p->tables_k = 0;
+        if ((vbytes && cudaMalloc(&p->values, vbytes) != cudaSuccess) || (pbytes && cudaMalloc(&p->positions, pbytes) != cudaSuccess)
+            || cudaMalloc(&p->counts, (size_t)K * sizeof(uint32_t)) != cudaSuccess) {
+            cudaGetLastError();
+            return failf(GCS_E_NOMEM, "cudaMalloc for the tables of %lld instances (%zu + %zu bytes) failed", (long long)K, vbytes, pbytes);
+        }
+        p->tables_k = K;
+    }
+    if (K * T > p->tangents_kt) {
+        PROG_TRY(cudaStreamSynchronize(p->stream));
+        cudaFree(p->dvalues), cudaFree(p->dpositions);
+        p->dvalues = p->dpositions = nullptr, p->tangents_kt = 0;
+        if ((vbytes && cudaMalloc(&p->dvalues, vbytes * T) != cudaSuccess) || (pbytes && cudaMalloc(&p->dpositions, pbytes * T) != cudaSuccess)) {
+            cudaGetLastError();
+            return failf(GCS_E_NOMEM, "cudaMalloc for the tangent tables of %lld instances x %lld directions (%zu + %zu bytes) failed",
+                (long long)K, T, vbytes * T, pbytes * T);
+        }
+        p->tangents_kt = K * T;
+    }
+    cudaStream_t st = p->stream;
+    PROG_TRY(cudaEventRecord(p->ev[0], st));
+    if (vbytes) PROG_TRY(cudaMemcpyAsync(p->values, values, vbytes, cudaMemcpyHostToDevice, st));
+    if (T > 0 && vbytes) PROG_TRY(cudaMemcpyAsync(p->dvalues, dvalues, vbytes * T, cudaMemcpyHostToDevice, st));
+    PROG_TRY(cudaEventRecord(p->ev[1], st));
+    int rc = run_on(p, K, p->values, p->positions, nonconverged ? p->counts : nullptr, variant, st, T, p->dvalues, p->dpositions);
+    if (rc != GCS_OK) {
+        cudaStreamSynchronize(st);
+        return rc;
+    }
+    PROG_TRY(cudaEventRecord(p->ev[2], st));
+    if (pbytes) PROG_TRY(cudaMemcpyAsync(positions, p->positions, pbytes, cudaMemcpyDeviceToHost, st));
+    if (T > 0 && pbytes) PROG_TRY(cudaMemcpyAsync(dpositions, p->dpositions, pbytes * T, cudaMemcpyDeviceToHost, st));
+    if (nonconverged) PROG_TRY(cudaMemcpyAsync(nonconverged, p->counts, (size_t)K * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    PROG_TRY(cudaEventRecord(p->ev[3], st));
+    PROG_TRY(cudaStreamSynchronize(st));
+    if (ms)
+        for (int q = 0; q < 3; ++q) PROG_TRY(cudaEventElapsedTime(&ms[q], p->ev[q], p->ev[q + 1]));
     return GCS_OK;
 }
 
@@ -418,35 +614,25 @@ int gcs_b200_program_run_host(gcs_b200_program* p, int64_t K, const double* valu
     int rc = check_run(p, K, values, positions, variant);
     if (rc != GCS_OK) return rc;
     CurrentDevice cur(p->device);
-    const size_t vbytes = (size_t)K * p->n_values * sizeof(double), pbytes = (size_t)K * p->n_slots * 4 * sizeof(double);
-    if (K > p->tables_k) {
-        PROG_TRY(cudaStreamSynchronize(p->stream));
-        cudaFree(p->values), cudaFree(p->positions), cudaFree(p->counts);
-        p->values = p->positions = nullptr, p->counts = nullptr, p->tables_k = 0;
-        if ((vbytes && cudaMalloc(&p->values, vbytes) != cudaSuccess) || (pbytes && cudaMalloc(&p->positions, pbytes) != cudaSuccess)
-            || cudaMalloc(&p->counts, (size_t)K * sizeof(uint32_t)) != cudaSuccess) {
-            cudaGetLastError();
-            return failf(GCS_E_NOMEM, "cudaMalloc for the tables of %lld instances (%zu + %zu bytes) failed", (long long)K, vbytes, pbytes);
-        }
-        p->tables_k = K;
-    }
-    cudaStream_t st = p->stream;
-    PROG_TRY(cudaEventRecord(p->ev[0], st));
-    if (vbytes) PROG_TRY(cudaMemcpyAsync(p->values, values, vbytes, cudaMemcpyHostToDevice, st));
-    PROG_TRY(cudaEventRecord(p->ev[1], st));
-    rc = run_on(p, K, p->values, p->positions, nonconverged ? p->counts : nullptr, variant, st);
-    if (rc != GCS_OK) {
-        cudaStreamSynchronize(st);
-        return rc;
-    }
-    PROG_TRY(cudaEventRecord(p->ev[2], st));
-    if (pbytes) PROG_TRY(cudaMemcpyAsync(positions, p->positions, pbytes, cudaMemcpyDeviceToHost, st));
-    if (nonconverged) PROG_TRY(cudaMemcpyAsync(nonconverged, p->counts, (size_t)K * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-    PROG_TRY(cudaEventRecord(p->ev[3], st));
-    PROG_TRY(cudaStreamSynchronize(st));
-    if (ms)
-        for (int q = 0; q < 3; ++q) PROG_TRY(cudaEventElapsedTime(&ms[q], p->ev[q], p->ev[q + 1]));
-    return GCS_OK;
+    return run_host(p, K, values, positions, nonconverged, variant, ms, 0, nullptr, nullptr);
+}
+
+int gcs_b200_program_run_tangents(gcs_b200_program* p, int64_t K, const double* values, double* positions, uint32_t* nonconverged,
+    int32_t T, const double* dvalues, double* dpositions, int variant, void* stream)
+{
+    int rc = check_tangent_run(p, K, values, positions, T, dvalues, dpositions, variant);
+    if (rc != GCS_OK) return rc;
+    CurrentDevice cur(p->device);
+    return run_on(p, K, values, positions, nonconverged, variant, static_cast<cudaStream_t>(stream), T, dvalues, dpositions);
+}
+
+int gcs_b200_program_run_tangents_host(gcs_b200_program* p, int64_t K, const double* values, double* positions,
+    uint32_t* nonconverged, int32_t T, const double* dvalues, double* dpositions, int variant, float ms[3])
+{
+    int rc = check_tangent_run(p, K, values, positions, T, dvalues, dpositions, variant);
+    if (rc != GCS_OK) return rc;
+    CurrentDevice cur(p->device);
+    return run_host(p, K, values, positions, nonconverged, variant, ms, T, dvalues, dpositions);
 }
 
 void gcs_b200_program_destroy(gcs_b200_program* p)
@@ -459,6 +645,7 @@ void gcs_b200_program_destroy(gcs_b200_program* p)
             if (e) cudaEventDestroy(e);
         cudaFree(p->rows), cudaFree(p->initial), cudaFree(p->scratch);
         cudaFree(p->values), cudaFree(p->positions), cudaFree(p->counts);
+        cudaFree(p->dvalues), cudaFree(p->dpositions);
         cudaGetLastError();
     }
     delete p;

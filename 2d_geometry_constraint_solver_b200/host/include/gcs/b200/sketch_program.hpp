@@ -55,6 +55,14 @@ public:
     // the CUDA library fails (no device: there is no CPU path).
     ProgramRunStats run(const double* values, std::int64_t K, double* positions, std::uint32_t* nonconverged = nullptr, int nDevices = 1);
 
+    // run(), plus the derivatives of the positions along T >= 1 directions in value space
+    // (gcs_b200_program_run_tangents): dvalues host [K][nValues()][T], in radians for angles like the
+    // values; dpositions host [K][nSlots()][4][T] receives sum_v dpositions/dvalues[v] * dvalues[v][t],
+    // NaN downstream of a row whose chosen run did not converge.  Positions and counts are run()'s.
+    // Throws std::invalid_argument for T < 1 before any device call.
+    ProgramRunStats runTangents(const double* values, std::int64_t K, const double* dvalues, int T, double* positions, double* dpositions,
+        std::uint32_t* nonconverged = nullptr, int nDevices = 1);
+
     // The edit loop: one instance with the constraints' current values, written into the elements -
     // the state solveLeaves leaves.
     ProgramRunStats solve();
@@ -68,11 +76,16 @@ public:
     const std::vector<std::int64_t>& rowLeaf() const { return m_rowLeaf; }  // leaf index of every row
     const std::vector<std::uint8_t>& solvedAfter() const { return m_solvedAfter; }  // per slot: solved after a run
     double compileSeconds() const { return m_compileSeconds; }
+    // the descriptor gcs_b200_program_create takes, pointing into this program's tables (valid while
+    // the program lives and is not moved from)
+    gcs_b200_program_desc desc() const;
 
 private:
     SketchProgram() = default;
     gcs_b200_program* onDevice(int device);
     void release();
+    ProgramRunStats runImpl(const double* values, std::int64_t K, const double* dvalues, int T, double* positions, double* dpositions,
+        std::uint32_t* nonconverged, int nDevices);
 
     BatchReport m_report;
     std::vector<gcs_b200_program_row> m_rows;
@@ -88,6 +101,9 @@ private:
     double* m_stagePositions = nullptr;
     std::uint32_t* m_stageCounts = nullptr;
     std::int64_t m_stageK = 0;
+    double* m_stageDValues = nullptr;
+    double* m_stageDPositions = nullptr;
+    std::int64_t m_stageKT = 0;  // instances x directions the tangent staging holds
 };
 
 }  // namespace Gcs::B200

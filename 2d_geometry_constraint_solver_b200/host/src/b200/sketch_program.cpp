@@ -128,6 +128,8 @@ SketchProgram& SketchProgram::operator=(SketchProgram&& o) noexcept
     o.m_device.clear();
     m_stageValues = o.m_stageValues, m_stagePositions = o.m_stagePositions, m_stageCounts = o.m_stageCounts, m_stageK = o.m_stageK;
     o.m_stageValues = o.m_stagePositions = nullptr, o.m_stageCounts = nullptr, o.m_stageK = 0;
+    m_stageDValues = o.m_stageDValues, m_stageDPositions = o.m_stageDPositions, m_stageKT = o.m_stageKT;
+    o.m_stageDValues = o.m_stageDPositions = nullptr, o.m_stageKT = 0;
     return *this;
 }
 
@@ -139,6 +141,20 @@ void SketchProgram::release()
     m_device.clear();
     gcs_b200_host_free(m_stageValues), gcs_b200_host_free(m_stagePositions), gcs_b200_host_free(m_stageCounts);
     m_stageValues = m_stagePositions = nullptr, m_stageCounts = nullptr, m_stageK = 0;
+    gcs_b200_host_free(m_stageDValues), gcs_b200_host_free(m_stageDPositions);
+    m_stageDValues = m_stageDPositions = nullptr, m_stageKT = 0;
+}
+
+gcs_b200_program_desc SketchProgram::desc() const
+{
+    gcs_b200_program_desc d {};
+    d.n_waves = static_cast<std::int32_t>(m_report.waves);
+    d.n_slots = static_cast<std::int32_t>(nSlots());
+    d.n_values = static_cast<std::int32_t>(nValues());
+    d.n_rows = static_cast<std::int64_t>(m_rows.size());
+    d.rows = m_rows.data(), d.offsets = m_offsets.data();
+    d.slot_is_line = m_slotIsLine.data(), d.initial = m_initial.data(), d.value_is_angle = m_valueIsAngle.data();
+    return d;
 }
 
 gcs_b200_program* SketchProgram::onDevice(int device)
@@ -146,13 +162,7 @@ gcs_b200_program* SketchProgram::onDevice(int device)
     if (static_cast<std::size_t>(device) >= m_device.size()) m_device.resize(static_cast<std::size_t>(device) + 1, nullptr);
     gcs_b200_program*& p = m_device[static_cast<std::size_t>(device)];
     if (!p) {
-        gcs_b200_program_desc d {};
-        d.n_waves = static_cast<std::int32_t>(m_report.waves);
-        d.n_slots = static_cast<std::int32_t>(nSlots());
-        d.n_values = static_cast<std::int32_t>(nValues());
-        d.n_rows = static_cast<std::int64_t>(m_rows.size());
-        d.rows = m_rows.data(), d.offsets = m_offsets.data();
-        d.slot_is_line = m_slotIsLine.data(), d.initial = m_initial.data(), d.value_is_angle = m_valueIsAngle.data();
+        const gcs_b200_program_desc d = desc();
         const int rc = gcs_b200_program_create(&d, device, &p);
         if (rc != GCS_OK) cudaFailure("gcs_b200_program_create", rc);
     }
@@ -160,6 +170,20 @@ gcs_b200_program* SketchProgram::onDevice(int device)
 }
 
 ProgramRunStats SketchProgram::run(const double* values, std::int64_t K, double* positions, std::uint32_t* nonconverged, int nDevices)
+{
+    return runImpl(values, K, nullptr, 0, positions, nullptr, nonconverged, nDevices);
+}
+
+ProgramRunStats SketchProgram::runTangents(const double* values, std::int64_t K, const double* dvalues, int T, double* positions,
+    double* dpositions, std::uint32_t* nonconverged, int nDevices)
+{
+    if (T < 1) throw std::invalid_argument("SketchProgram::runTangents: T must be >= 1 (got " + std::to_string(T) + ")");
+    return runImpl(values, K, dvalues, T, positions, dpositions, nonconverged, nDevices);
+}
+
+// T = 0: run(); T > 0: runTangents()
+ProgramRunStats SketchProgram::runImpl(const double* values, std::int64_t K, const double* dvalues, int T, double* positions,
+    double* dpositions, std::uint32_t* nonconverged, int nDevices)
 {
     const auto t0 = Clock::now();
     if (K < 1) throw std::invalid_argument("SketchProgram::run: K must be >= 1");
@@ -177,12 +201,29 @@ ProgramRunStats SketchProgram::run(const double* values, std::int64_t K, double*
         if (!m_stageValues || !m_stagePositions || !m_stageCounts) throw std::bad_alloc();
         m_stageK = K;
     }
+    const std::int64_t KT = K * T;
+    if (KT > m_stageKT) {
+        gcs_b200_host_free(m_stageDValues), gcs_b200_host_free(m_stageDPositions);
+        m_stageKT = 0;
+        m_stageDValues = static_cast<double*>(gcs_b200_host_alloc(std::max<std::size_t>(1, static_cast<std::size_t>(KT) * nv) * sizeof(double)));
+        m_stageDPositions = static_cast<double*>(gcs_b200_host_alloc(std::max<std::size_t>(1, static_cast<std::size_t>(KT) * table) * sizeof(double)));
+        if (!m_stageDValues || !m_stageDPositions) throw std::bad_alloc();
+        m_stageKT = KT;
+    }
     // angles go to the device as std::cos of the value: the host packer's rounding
     const long long nval = static_cast<long long>(K) * static_cast<long long>(nv);
     const std::uint8_t* angle = m_valueIsAngle.data();
     double* stage = m_stageValues;
 #pragma omp parallel for schedule(static) if (nval > 65536)
     for (long long q = 0; q < nval; ++q) stage[q] = angle[static_cast<std::size_t>(q) % nv] ? std::cos(values[q]) : values[q];
+    // and their directions as d(cos v) = -sin(v) dv
+    double* dstage = m_stageDValues;
+    const long long ndval = nval * T;
+#pragma omp parallel for schedule(static) if (ndval > 65536)
+    for (long long q = 0; q < ndval; ++q) {
+        const long long vq = q / T;
+        dstage[q] = angle[static_cast<std::size_t>(vq) % nv] ? -std::sin(values[vq]) * dvalues[q] : dvalues[q];
+    }
     for (int g = 0; g < nDevices; ++g) onDevice(g);
 
     const std::int64_t launches0 = gcs_b200_launch_count();
@@ -191,8 +232,14 @@ ProgramRunStats SketchProgram::run(const double* values, std::int64_t K, double*
     std::vector<std::array<float, 3>> ms(static_cast<std::size_t>(nDevices));
     auto part = [&](int g) {
         const std::int64_t lo = K * g / nDevices, hi = K * (g + 1) / nDevices;
-        rc[static_cast<std::size_t>(g)] = gcs_b200_program_run_host(m_device[static_cast<std::size_t>(g)], hi - lo, m_stageValues + lo * static_cast<std::int64_t>(nv),
-            m_stagePositions + lo * static_cast<std::int64_t>(table), nonconverged ? m_stageCounts + lo : nullptr, variant, ms[static_cast<std::size_t>(g)].data());
+        gcs_b200_program* p = m_device[static_cast<std::size_t>(g)];
+        const std::int64_t vo = lo * static_cast<std::int64_t>(nv), po = lo * static_cast<std::int64_t>(table);
+        std::uint32_t* counts = nonconverged ? m_stageCounts + lo : nullptr;
+        float* m = ms[static_cast<std::size_t>(g)].data();
+        rc[static_cast<std::size_t>(g)] = T == 0
+            ? gcs_b200_program_run_host(p, hi - lo, m_stageValues + vo, m_stagePositions + po, counts, variant, m)
+            : gcs_b200_program_run_tangents_host(p, hi - lo, m_stageValues + vo, m_stagePositions + po, counts, T, m_stageDValues + vo * T,
+                m_stageDPositions + po * T, variant, m);
     };
     if (nDevices == 1) {
         part(0);
@@ -202,11 +249,16 @@ ProgramRunStats SketchProgram::run(const double* values, std::int64_t K, double*
         for (auto& t : threads) t.join();
     }
     for (int g = 0; g < nDevices; ++g)
-        if (rc[static_cast<std::size_t>(g)] != GCS_OK) cudaFailure("gcs_b200_program_run_host", rc[static_cast<std::size_t>(g)]);
+        if (rc[static_cast<std::size_t>(g)] != GCS_OK)
+            cudaFailure(T == 0 ? "gcs_b200_program_run_host" : "gcs_b200_program_run_tangents_host", rc[static_cast<std::size_t>(g)]);
     const long long npos = static_cast<long long>(K) * static_cast<long long>(table);
     const double* from = m_stagePositions;
 #pragma omp parallel for schedule(static) if (npos > 65536)
     for (long long q = 0; q < npos; ++q) positions[q] = from[q];
+    const long long ndpos = npos * T;
+    const double* dfrom = m_stageDPositions;
+#pragma omp parallel for schedule(static) if (ndpos > 65536)
+    for (long long q = 0; q < ndpos; ++q) dpositions[q] = dfrom[q];
     if (nonconverged) std::memcpy(nonconverged, m_stageCounts, static_cast<std::size_t>(K) * sizeof(std::uint32_t));
     ProgramRunStats st;
     st.launches = gcs_b200_launch_count() - launches0;

@@ -876,6 +876,23 @@ GCS_API int gcs_host_program_describe(const gcs_host_program* h, int64_t* counts
     return 0;
 }
 
+// The descriptor of the compiled program (gcs_b200_program_desc), pointing into the program's own
+// tables: valid while the handle lives.  Returns 0.
+GCS_API int gcs_host_program_desc(const gcs_host_program* h, gcs_b200_program_desc* out)
+{
+    *out = h->prog->desc();
+    return 0;
+}
+
+static void programStats(const gcs_host_program* h, const Gcs::B200::ProgramRunStats& st, int n_devices, int64_t* stats)
+{
+    if (!stats) return;
+    stats[0] = st.launches, stats[1] = static_cast<int64_t>(h->prog->compileSeconds() * 1e6);
+    stats[2] = static_cast<int64_t>(st.uploadMs * 1e3), stats[3] = static_cast<int64_t>(st.deviceMs * 1e3);
+    stats[4] = static_cast<int64_t>(st.downloadMs * 1e3), stats[5] = static_cast<int64_t>(st.seconds * 1e6);
+    stats[6] = n_devices;
+}
+
 // K instances: values [K][n_values] (angles in radians), positions out [K][n_slots][4], nonconverged
 // [K] (may be NULL).  stats (may be NULL) holds 7 values: launches, compile us, upload us, device us,
 // download us (device time), run us (host clock), devices used.  Returns 0 or -1.
@@ -883,13 +900,20 @@ GCS_API int gcs_host_program_run(gcs_host_program* h, int64_t K, const double* v
     int n_devices, int64_t* stats)
 {
     try {
-        const auto st = h->prog->run(values, K, positions, nonconverged, n_devices);
-        if (stats) {
-            stats[0] = st.launches, stats[1] = static_cast<int64_t>(h->prog->compileSeconds() * 1e6);
-            stats[2] = static_cast<int64_t>(st.uploadMs * 1e3), stats[3] = static_cast<int64_t>(st.deviceMs * 1e3);
-            stats[4] = static_cast<int64_t>(st.downloadMs * 1e3), stats[5] = static_cast<int64_t>(st.seconds * 1e6);
-            stats[6] = n_devices;
-        }
+        programStats(h, h->prog->run(values, K, positions, nonconverged, n_devices), n_devices, stats);
+        return 0;
+    } catch (const std::exception& ex) {
+        return fail(ex);
+    }
+}
+
+// The same with the derivatives along T directions (SketchProgram::runTangents): dvalues [K][n_values][T]
+// (radians for angles), dpositions out [K][n_slots][4][T].  Returns 0 or -1.
+GCS_API int gcs_host_program_run_tangents(gcs_host_program* h, int64_t K, const double* values, int T, const double* dvalues,
+    double* positions, double* dpositions, uint32_t* nonconverged, int n_devices, int64_t* stats)
+{
+    try {
+        programStats(h, h->prog->runTangents(values, K, dvalues, T, positions, dpositions, nonconverged, n_devices), n_devices, stats);
         return 0;
     } catch (const std::exception& ex) {
         return fail(ex);

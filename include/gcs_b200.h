@@ -354,6 +354,31 @@ GCS_B200_API int gcs_b200_program_run(gcs_b200_program* prog, int64_t n_instance
  * device time of upload, run and download. */
 GCS_B200_API int gcs_b200_program_run_host(gcs_b200_program* prog, int64_t n_instances, const double* values, double* positions,
     uint32_t* nonconverged, int variant, float ms[3]);
+/* Tangent runs: gcs_b200_program_run, plus the directional derivatives of every position with
+ * respect to the values (forward mode).  For each instance k and T = n_tangents >= 1 directions
+ * dvalues[k][:][t]:
+ *     dpositions[k][s][c][t] = sum_v d positions[k][s][c] / d values[k][v] * dvalues[k][v][t]
+ * Layouts are instance-major with the direction innermost: dvalues [K][n_values][T], dpositions
+ * [K][n_slots][4][T].  With dvalues[k] the identity (T = n_values), dpositions[k] read as
+ * [n_slots * 4][T] is the full Jacobian of instance k.  An angle slot holds cos(angle), so its
+ * dvalues entry is d(cos(angle)).
+ * Every slot's tangent is 0 before the first wave (the initial positions are constants).  A row
+ * whose chosen Newton run did not converge (what `nonconverged` counts) is not a root, and the
+ * tangents of its target are NaN; they propagate to whatever depends on it.  A converged row's
+ * tangent is the implicit-function-theorem one, a 2x2 solve with the Jacobian at its root
+ * (csrc/newton_tangent.cuh states the operation order); a singular Jacobian gives what the IEEE
+ * division gives.  Root choice is piecewise constant and contributes nothing.
+ * Positions, nonconverged and the kernels that solve them are those of gcs_b200_program_run; the
+ * run adds one launch per wave.  Checked before any device call: n_tangents >= 1, dvalues non-null
+ * when n_values > 0, dpositions non-null when n_slots > 0, and what gcs_b200_program_run checks. */
+GCS_B200_API int gcs_b200_program_run_tangents(gcs_b200_program* prog, int64_t n_instances, const double* values,
+    double* positions, uint32_t* nonconverged, int32_t n_tangents, const double* dvalues, double* dpositions,
+    int variant, void* cuda_stream);
+/* The same with host buffers, as gcs_b200_program_run_host (dvalues go up with the values, dpositions
+ * come down with the positions). */
+GCS_B200_API int gcs_b200_program_run_tangents_host(gcs_b200_program* prog, int64_t n_instances, const double* values,
+    double* positions, uint32_t* nonconverged, int32_t n_tangents, const double* dvalues, double* dpositions,
+    int variant, float ms[3]);
 GCS_B200_API void gcs_b200_program_destroy(gcs_b200_program* prog);
 
 /* Test hook: on-device self check of the hand-written division / square root / 2x2 QR fast paths
