@@ -328,6 +328,29 @@ int validate_desc(const gcs_b200_program_desc* d)
                 return failf(GCS_E_INVALID, "row %lld: the three roles need three distinct slots", r);
         }
     }
+    // The footprint rule of the wave plan (makePlan, host/src/b200/leaf_batch.cpp): within one wave
+    // no slot is written by two rows, and no slot written by one row is read by another.  The rows
+    // of a wave run concurrently, so otherwise the scatter's writes race, or a zero-fixed row's
+    // anchors (written by the gather) race with another row's gather reading them.  Writes: a, b, c
+    // of solvers 1-3, c of 4-8; reads: a, b of 4-8.  Per slot, the last wave that touched it, the
+    // row that did and whether it wrote.
+    std::vector<int> wave_of((size_t)d->n_slots, -1);
+    std::vector<long long> row_of((size_t)d->n_slots);
+    std::vector<char> wrote((size_t)d->n_slots);
+    for (int wave = 0; wave < d->n_waves; ++wave) {
+        for (long long r = d->offsets[(long long)wave * kKinds]; r < d->offsets[(long long)(wave + 1) * kKinds]; ++r) {
+            const gcs_b200_program_row& row = d->rows[r];
+            const bool zero_fixed = row.solver <= 3;
+            for (int q = 0; q < 3; ++q) {
+                const size_t e = (size_t)row.elem[q];
+                const bool writes = zero_fixed || q == 2;
+                if (wave_of[e] == wave && (writes || wrote[e]))
+                    return failf(GCS_E_INVALID, "wave %d: slot %d is %s by row %lld and %s by row %lld; rows of one wave run concurrently", wave,
+                        (int)e, wrote[e] ? "written" : "read", row_of[e], writes ? "written" : "read", r);
+                if (wave_of[e] != wave || writes) wave_of[e] = wave, row_of[e] = r, wrote[e] = writes;
+            }
+        }
+    }
     return GCS_OK;
 }
 

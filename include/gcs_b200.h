@@ -337,9 +337,11 @@ typedef struct gcs_b200_program_desc {
 typedef struct gcs_b200_program gcs_b200_program;
 
 /* Validates the descriptor (before any device call: slots, value slots, offsets, solver ids, the
- * kind of every row's segment, role types) and uploads it to `device`.  Host pointers; nothing of
- * them is kept.  GCS_E_INVALID with a message for a malformed descriptor, GCS_E_NO_DEVICE without
- * a device. */
+ * kind of every row's segment, role types, and that the rows of one wave, which run concurrently,
+ * have disjoint footprints: no slot written by two rows of a wave, none written by one row and read
+ * by another; writes are roles a, b, c of solvers 1-3 and c of solvers 4-8, reads a, b of solvers
+ * 4-8; shared reads are fine) and uploads it to `device`.  Host pointers; nothing of them is kept.
+ * GCS_E_INVALID with a message for a malformed descriptor, GCS_E_NO_DEVICE without a device. */
 GCS_B200_API int gcs_b200_program_create(const gcs_b200_program_desc* desc, int device, gcs_b200_program** out);
 /* Runs K = n_instances >= 1 instances, stream-ordered on `cuda_stream`; every pointer is a device
  * pointer.  values [K][n_values] (angle slots hold cos(angle)); positions [K][n_slots][4] is

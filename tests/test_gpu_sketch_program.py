@@ -204,10 +204,11 @@ def test_a_program_is_reusable_and_solve_follows_edits(host):
 
 
 def test_the_contracted_class_agrees_to_the_tolerance(host):
-    """GCS_VARIANT_CONTRACTED on the chain of 400 dependent leaves of
+    """The contracted class on the chain of 400 dependent leaves of
     test_solve_gcs_with_the_contracted_kernels_agrees_to_the_tolerance: each leaf's coordinates are the
     next leaf's inputs, and the program agrees with the bit-identical class to 1e-9 relative, for the
-    drawn values and for value sets moved by up to 1e-7 relative."""
+    drawn values and for value sets moved by up to 1e-7 relative.  Every contracted variant:
+    GCS_VARIANT_CONTRACTED and the explicit mappings _STATIC, _SORTED, _SEQ and _LINEAR."""
     pts, el, lv = _triangle_strip(402)
     prog = P.Program(el, leaves=lv)
     assert prog.rc == 0, prog.error
@@ -216,16 +217,18 @@ def test_the_contracted_class_agrees_to_the_tolerance(host):
     vals = base_vals * (1.0 + 1e-7 * u)
     vals[0] = base_vals
     rc, base, nc_base, _ = prog.run(vals)
-    old = host.gcs_host_set_variant(5)
-    try:
-        rc2, fast, nc_fast, _ = prog.run(vals)
-    finally:
-        host.gcs_host_set_variant(old)
-    assert old == 0 and rc == rc2 == 0 and np.array_equal(nc_base, nc_fast) and not nc_base.any()
-    xy, fxy = base[:, :, :2], fast[:, :, :2]
+    assert rc == 0 and not nc_base.any()
+    xy = base[:, :, :2]
     scale = max(1.0, float(np.abs(xy).max()))
-    worst = float(np.abs(xy - fxy).max()) / scale
-    assert worst <= 1e-9, worst
+    for variant in (5, 6, 7, 8, 10):
+        old = host.gcs_host_set_variant(variant)
+        try:
+            rc2, fast, nc_fast, _ = prog.run(vals)
+        finally:
+            host.gcs_host_set_variant(old)
+        assert old == 0 and rc2 == 0 and np.array_equal(nc_base, nc_fast), variant
+        worst = float(np.abs(xy - fast[:, :, :2]).max()) / scale
+        assert worst <= 1e-9, (variant, worst)
 
 
 def test_results_do_not_depend_on_the_device_count(host, gcs):

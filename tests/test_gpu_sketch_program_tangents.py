@@ -13,13 +13,10 @@ import oracle_lib as O
 import program_tangents_lib as P
 import sketch_gen as S
 from test_gpu_host import WHOLE_SKETCHES, _ref_loops, _triangle_strip
-from tangent_oracle import tangent
+from program_restate import restate, rows
 from util import bits, digest
 
 pytestmark = pytest.mark.gpu
-
-IN_COLS = {1: 6, 2: 9, 3: 10, 4: 12, 5: 13}
-
 
 @pytest.fixture(scope="module")
 def host(gpu, built):
@@ -64,98 +61,6 @@ def test_a_tangent_run_leaves_the_positions_of_a_plain_run(host, case):
 
 # ---- 2. device equals the CPU restatement, bit for bit ----
 
-def _rows(desc):
-    n = desc.n_rows
-    rows = desc.rows
-    return {"solver": np.array([rows[r].solver for r in range(n)]), "elem": np.array([list(rows[r].elem) for r in range(n)]),
-            "value": np.array([list(rows[r].value) for r in range(n)]), "code": np.array([rows[r].code for r in range(n)], dtype=np.uint8),
-            "sign": np.array([list(rows[r].sign) for r in range(n)]), "canvas": np.array([list(rows[r].canvas) for r in range(n)])}
-
-
-def _gather(solver, sign, cst, pa, pb, v, dpa, dpb, dv):
-    """program_gather_kernel for one row over K instances and its tangent: (columns [nin][K], column
-    tangents [nin][K][T], anchors {role: (position [K][4] writes, tangent writes)})."""
-    K, T = v.shape[0], dv.shape[2]
-    z, dz = np.zeros(K), np.zeros((K, T))
-    v0, v1, v2 = v[:, 0], v[:, 1], v[:, 2]
-    d0, d1, d2 = dv[:, 0], dv[:, 1], dv[:, 2]
-    anchors = {}
-    if solver in (1, 2):
-        anchors = {0: ({0: z, 1: z}, {0: dz, 1: dz}), 1: ({0: v0, 1: z}, {0: d0, 1: dz})}
-    if solver == 1:
-        return [z, z, v1, v0, z, v2], [dz, dz, d1, d0, dz, d2], anchors
-    if solver == 4:
-        return [pa[:, 0], pa[:, 1], v1, pb[:, 0], pb[:, 1], v2], [dpa[:, 0], dpa[:, 1], d1, dpb[:, 0], dpb[:, 1], d2], anchors
-    c = [np.full(K, x) for x in cst]
-    if solver == 2:
-        return ([z, z, v0, z, sign[1] * v1, sign[2] * v2, c[0], c[1], c[2]],
-                [dz, dz, d0, dz, sign[1] * d1, sign[2] * d2, dz, dz, dz], anchors)
-    if solver == 5:
-        return ([pa[:, 0], pa[:, 1], pb[:, 0], pb[:, 1], sign[1] * v1, sign[2] * v2, c[0], c[1], c[2]],
-                [dpa[:, 0], dpa[:, 1], dpb[:, 0], dpb[:, 1], sign[1] * d1, sign[2] * d2, dz, dz, dz], anchors)
-    if solver == 6:
-        return ([pa[:, 0], pa[:, 1], v1, pb[:, 0], pb[:, 1], pb[:, 2], pb[:, 3], sign[2] * v2, c[0], c[1]],
-                [dpa[:, 0], dpa[:, 1], d1, dpb[:, 0], dpb[:, 1], dpb[:, 2], dpb[:, 3], sign[2] * d2, dz, dz], anchors)
-    if solver == 7:
-        return ([pa[:, 0], pa[:, 1], pa[:, 2], pa[:, 3], sign[1] * v1, pb[:, 0], pb[:, 1], pb[:, 2], pb[:, 3], sign[2] * v2, c[0], c[1]],
-                [dpa[:, 0], dpa[:, 1], dpa[:, 2], dpa[:, 3], sign[1] * d1, dpb[:, 0], dpb[:, 1], dpb[:, 2], dpb[:, 3], sign[2] * d2, dz, dz],
-                anchors)
-    if solver == 3:
-        sd1, dsd1 = sign[1] * v1, sign[1] * d1
-        anchors = {0: ({0: c[7], 1: z, 2: c[8], 3: z}, {0: dz, 1: dz, 2: dz, 3: dz}), 1: ({0: z, 1: sd1}, {0: dz, 1: dsd1})}
-        return ([c[5], c[6], v0, c[0], c[1], c[2], c[3], z, sd1, sign[2] * v2, z, z, c[4]],
-                [dz, dz, d0, dz, dz, dz, dz, dz, dsd1, sign[2] * d2, dz, dz, dz], anchors)
-    # solver 8
-    return ([pa[:, 2] - pa[:, 0], pa[:, 3] - pa[:, 1], v0, c[0], c[1], c[2], c[3], pb[:, 0], pb[:, 1], sign[2] * v2,
-             (pa[:, 0] + pa[:, 2]) / 2.0, (pa[:, 1] + pa[:, 3]) / 2.0, c[4]],
-            [dpa[:, 2] - dpa[:, 0], dpa[:, 3] - dpa[:, 1], d0, dz, dz, dz, dz, dpb[:, 0], dpb[:, 1], sign[2] * d2,
-             (dpa[:, 0] + dpa[:, 2]) / 2.0, (dpa[:, 1] + dpa[:, 3]) / 2.0, dz], anchors)
-
-
-def _restate(desc, vals, dvals):
-    """A tangent run restated wave by wave on the CPU: (positions [K][n_slots][4], tangents [K][n_slots][4][T])."""
-    K, T = dvals.shape[0], dvals.shape[2]
-    rows = _rows(desc)
-    init = np.array([desc.initial[i] for i in range(4 * desc.n_slots)]).reshape(desc.n_slots, 4)
-    pos = np.repeat(init[None], K, axis=0)
-    dpos = np.zeros((K, desc.n_slots, 4, T))
-    off = [desc.offsets[i] for i in range(5 * desc.n_waves + 1)]
-    for w in range(desc.n_waves):
-        anchors, solved = [], []
-        for k in range(1, 6):  # the gather reads the positions as the previous waves left them
-            lo, hi = off[5 * w + k - 1], off[5 * w + k]
-            if hi == lo:
-                continue
-            cols, dcols = [[] for _ in range(IN_COLS[k])], [[] for _ in range(IN_COLS[k])]
-            for r in range(lo, hi):
-                a, b = rows["elem"][r, 0], rows["elem"][r, 1]
-                vi = rows["value"][r]
-                v = np.stack([vals[:, i] if i >= 0 else np.zeros(K) for i in vi], axis=1)
-                dv = np.stack([dvals[:, i, :] if i >= 0 else np.zeros((K, T)) for i in vi], axis=1)
-                cs, dcs, anc = _gather(rows["solver"][r], rows["sign"][r], rows["canvas"][r], pos[:, a], pos[:, b], v,
-                                       dpos[:, a], dpos[:, b], dv)
-                for q in range(IN_COLS[k]):
-                    cols[q].append(cs[q])
-                    dcols[q].append(dcs[q])
-                anchors += [(a if role == 0 else b, p, dp) for role, (p, dp) in anc.items()]
-            code = np.repeat(rows["code"][lo:hi], K)  # sub-system (row i, instance j) at i * K + j
-            hb = O.capi.HostBatch(k, 2, [np.ascontiguousarray(np.concatenate(c)) for c in cols], np.ascontiguousarray(code))
-            O.solve(hb.alloc_outputs())
-            dout = tangent(hb, np.stack([np.concatenate(c) for c in dcols]))
-            solved.append((lo, hi, hb, dout))
-        for slot, p, dp in anchors:
-            for q in p:
-                pos[:, slot, q] = p[q]
-                dpos[:, slot, q] = dp[q]
-        for lo, hi, hb, dout in solved:  # the scatter and the tangent kernel
-            for r in range(lo, hi):
-                c, sl = rows["elem"][r, 2], slice((r - lo) * K, (r - lo + 1) * K)
-                for q in range(len(hb.out)):
-                    pos[:, c, q] = hb.out[q][sl]
-                    dpos[:, c, q, :] = dout[q, sl, :]
-    return pos, dpos
-
-
 def _desc_run(desc, vals, dvals, gcs):
     """gcs_b200_program_run_tangents_host on a C-ABI program built from `desc`."""
     lib = gcs.capi.load()
@@ -196,10 +101,11 @@ def test_device_tangents_equal_the_cpu_restatement(host, gcs, seed, first, n):
     cv = np.where(angle, np.cos(v), v)
     dcv = np.where(angle[None, :, None], -np.sin(v)[:, :, None] * dv, dv)
     pos, dpos, nc = _desc_run(desc, cv, dcv, gcs)
-    want, dwant = _restate(desc, cv, dcv)
+    want, dwant, wnc = restate(desc, cv, dcv)
     assert _same(pos, want)
     assert _same(dpos, dwant)
-    assert set(_rows(desc)["solver"]) <= set(range(1, 9))
+    assert np.array_equal(nc, wnc)
+    assert set(rows(desc)["solver"]) <= set(range(1, 9))
 
 
 def test_all_solvers_occur_in_the_restated_sketches(host):
@@ -435,9 +341,10 @@ def test_tangents_do_not_depend_on_the_device_count(host, gcs):
 
 
 def test_the_contracted_class_agrees_on_tangents(host):
-    """GCS_VARIANT_CONTRACTED on the 400-leaf strip: positions within 1e-9 and tangents within 1e-8
-    relative of the bit-identical class (the tangent of a chain amplifies the positions' differences
-    by the same factor it amplifies their derivatives)."""
+    """The contracted class on the 400-leaf strip: positions within 1e-9 and tangents within 1e-8
+    relative of the bit-identical class (the tangent of a chain amplifies the positions' differences by
+    the same factor it amplifies their derivatives).  Every contracted variant: GCS_VARIANT_CONTRACTED
+    and the explicit mappings _STATIC, _SORTED, _SEQ and _LINEAR."""
     pts, el, lv = _triangle_strip(402)
     prog = P.Program(el, leaves=lv)
     vals = np.array([e["value"] for lf in lv for e in lf["edges"] if e["type"] != S.VIRT])
@@ -445,13 +352,17 @@ def test_the_contracted_class_agrees_on_tangents(host):
     vals = vals * (1.0 + 1e-7 * u)
     dv = _directions(vals.shape[1], 4, 3, seed=4)
     rc, base, dbase, nc_base, _ = prog.run_tangents(vals, dv)
-    old = host.gcs_host_set_variant(5)
-    try:
-        rc2, fast, dfast, nc_fast, _ = prog.run_tangents(vals, dv)
-    finally:
-        host.gcs_host_set_variant(old)
-    assert rc == rc2 == 0 and np.array_equal(nc_base, nc_fast) and not nc_base.any()
+    assert rc == 0 and not nc_base.any()
     scale = max(1.0, float(np.abs(dbase).max()))
-    worst = float(np.abs(dbase - dfast).max()) / scale
-    print(f"contracted class: tangents within {worst:.3e} relative")
-    assert worst <= 1e-8, worst
+    pscale = max(1.0, float(np.abs(base[:, :, :2]).max()))
+    for variant in (5, 6, 7, 8, 10):
+        old = host.gcs_host_set_variant(variant)
+        try:
+            rc2, fast, dfast, nc_fast, _ = prog.run_tangents(vals, dv)
+        finally:
+            host.gcs_host_set_variant(old)
+        assert rc2 == 0 and np.array_equal(nc_base, nc_fast), variant
+        assert float(np.abs(base[:, :, :2] - fast[:, :, :2]).max()) / pscale <= 1e-9, variant
+        worst = float(np.abs(dbase - dfast).max()) / scale
+        print(f"contracted variant {variant}: tangents within {worst:.3e} relative")
+        assert worst <= 1e-8, (variant, worst)

@@ -8,6 +8,8 @@ import pytest
 
 import host_lib as H
 import program_lib as P
+import program_restate as R
+import program_tangents_lib as PT
 import sketch_gen as S
 
 GOLDEN_SKETCHES = [(31, 1, 3000), (32, 2, 3000), (33, 3, 3000)]
@@ -174,3 +176,68 @@ def test_a_valid_descriptor_needs_a_device(gcs, built):
         assert rc == capi.GCS_OK and h.value
         assert lib.gcs_b200_program_run_host(h, 0, None, None, None, 0, None) == capi.GCS_E_INVALID  # K < 1
         lib.gcs_b200_program_destroy(h)
+
+
+def _one_wave(rows):
+    """A one-wave program of K1 rows given as (solver, elem): solver 1 reads v0 v1 v2, solver 4 v1 v2."""
+    r = np.zeros(len(rows), dtype=R.ROW)
+    for i, (solver, elem) in enumerate(rows):
+        r[i]["solver"], r[i]["elem"], r[i]["sign"] = solver, elem, 1.0
+        r[i]["value"] = [3 * i, 3 * i + 1, 3 * i + 2] if solver == 1 else [-1, 3 * i + 1, 3 * i + 2]
+    n_slots = int(r["elem"].max()) + 1
+    return R.Arrays(r, [0] + [len(rows)] * 5, np.zeros(n_slots), np.zeros((n_slots, 4)), np.zeros(3 * len(rows)))
+
+
+def _create(gcs, arrays):
+    lib = gcs.capi.load()
+    h = C.c_void_p()
+    rc = lib.gcs_b200_program_create(C.byref(arrays.desc()), 0, C.byref(h))
+    if h.value:
+        lib.gcs_b200_program_destroy(h)
+    return rc, lib.gcs_b200_last_error().decode()
+
+
+def _valid(gcs):
+    """what gcs_b200_program_create returns for a valid descriptor on this machine"""
+    return gcs.capi.GCS_OK if gcs.capi.load().gcs_b200_device_count() > 0 else gcs.capi.GCS_E_NO_DEVICE
+
+
+@pytest.mark.parametrize("rows,written,read", [
+    ([(4, [0, 1, 4]), (4, [2, 3, 4])], "written by row 0", "written by row 1"),   # two rows target slot 4
+    ([(1, [0, 1, 2]), (4, [3, 0, 4])], "written by row 0", "read by row 1"),      # row 0 anchors slot 0 that row 1 reads
+    ([(4, [2, 3, 4]), (4, [0, 1, 2])], "read by row 0", "written by row 1"),      # row 1 targets slot 2 that row 0 reads
+])
+def test_rows_of_one_wave_with_overlapping_footprints_are_refused(gcs, built, rows, written, read):
+    """The rows of a wave run concurrently: a slot two of them write, or one writes and another reads,
+    would make the result depend on thread scheduling.  Refused before any device call, naming both rows."""
+    rc, msg = _create(gcs, _one_wave(rows))
+    assert rc == gcs.capi.GCS_E_INVALID
+    assert written in msg and read in msg, msg
+    # the same rows in two waves are a valid program
+    two = _one_wave(rows)
+    two = two.with_waves([[np.array([0]), *[np.zeros(0, dtype=np.int64)] * 4], [np.array([1]), *[np.zeros(0, dtype=np.int64)] * 4]])
+    assert _create(gcs, two)[0] == _valid(gcs), _create(gcs, two)[1]
+
+
+def test_rows_of_one_wave_may_share_what_they_read(gcs, built):
+    assert _create(gcs, _one_wave([(4, [0, 1, 2]), (4, [1, 0, 3]), (4, [0, 1, 4])]))[0] == _valid(gcs)
+
+
+@pytest.mark.parametrize("case", GOLDEN_SKETCHES + ["linkage20k"])
+def test_compiled_programs_and_their_wave_layouts_pass_validation(gcs, host, case):
+    """What SketchProgram::compile makes, and every layout of tests/program_restate.py (the layouts the
+    GPU tests require to leave every result unchanged), passes the footprint rule."""
+    if case == "linkage20k":
+        el, edges = S.make_linkage(20000, seed=6)
+        prog = PT.Program(el, edges)
+    else:
+        seed, first, n = case
+        el, lv = S.make_sketch(n, seed=seed, first_shape=first)
+        prog = PT.Program(el, leaves=lv)
+    assert prog.rc == 0, prog.error
+    p = R.Arrays.from_desc(prog.desc())
+    layouts = [("compiled", p)] + R.transforms(p) + [("relabelled", R.relabelled(p, seed=1)[0]),
+                                                     ("no_rows", R.without_rows(p, 0)), ("no_rows_3_waves", R.without_rows(p, 3))]
+    for name, q in layouts:
+        rc, msg = _create(gcs, q)
+        assert rc == _valid(gcs), (name, msg)
