@@ -114,6 +114,8 @@ EXPORTS = [
     "gcs_b200_debug_path_buffer", "gcs_b200_resolve_variant",
     "gcs_b200_program_create", "gcs_b200_program_run", "gcs_b200_program_run_host", "gcs_b200_program_destroy",
     "gcs_b200_program_run_tangents", "gcs_b200_program_run_tangents_host",
+    "gcs_b200_program_run_recorded", "gcs_b200_program_run_recorded_host", "gcs_b200_program_adjoints",
+    "gcs_b200_program_adjoints_host",
 ]
 
 
@@ -167,6 +169,11 @@ def load():
                                                   C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
     lib.gcs_b200_program_run_tangents_host.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
                                                        C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_float)]
+    lib.gcs_b200_program_run_recorded.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
+    lib.gcs_b200_program_run_recorded_host.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
+                                                       C.POINTER(C.c_float)]
+    lib.gcs_b200_program_adjoints.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.gcs_b200_program_adjoints_host.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.POINTER(C.c_float)]
     lib.gcs_b200_program_destroy.argtypes = [C.c_void_p]
     _lib = lib
     return lib

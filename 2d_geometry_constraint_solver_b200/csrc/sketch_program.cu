@@ -16,6 +16,17 @@
 // the gather forms the columns, linearises the row at its chosen root (csrc/newton_tangent.cuh) and
 // writes the target's tangents.  The K2 / K5 batches then also keep their candidate planes, whose
 // chosen normal is the row's unknown.
+//
+// Recorded runs (gcs_b200_program_run_recorded) place every (wave, kind) batch at its own offset of
+// one tape allocation instead of reusing one set of batches for every wave, so that the batches of
+// all waves (columns, flags, K2 / K5 candidate planes) survive the run.  The adjoint sweep
+// (gcs_b200_program_adjoints) reads them back, waves from last to first, with two launches per
+// wave: the adjoint kernel, one thread per (row, instance, cotangent t) with t fastest, takes the
+// adjoints of what the row wrote (its target, and the anchors of a zero-fixed row), zeroes them and
+// writes the row's contributions to the slots and values it read into a contribution buffer; the
+// reduce kernel adds those into the working slot-adjoint table and the value adjoints, each table
+// entry's contributions in ascending (row, role) order from reader lists built at create time.  No
+// atomics: the result does not depend on K, the stream or the schedule.
 #include <cuda_runtime.h>
 
 #include <cstdarg>
@@ -24,7 +35,7 @@
 #include <vector>
 
 #include "../../include/gcs_b200.h"
-#include "newton_tangent.cuh"
+#include "newton_adjoint.cuh"
 
 namespace gcsk {
 int api_fail(int code, const char* msg);  // gcs_b200_api.cu: sets gcs_b200_last_error()
@@ -78,9 +89,14 @@ struct WaveArgs {
     const double* val;         // [K][n_values]
     long long n_slots, n_values;
     uint32_t* nonconverged;    // [K] or null
-    long long T;               // directions of a tangent run (0: plain run)
+    long long T;               // directions of a tangent run, cotangents of a sweep (0: plain run)
     double* dpos;              // [K][n_slots][4][T]
     const double* dval;        // [K][n_values][T]
+    // adjoint sweep
+    double* apos;              // working slot adjoints [K][n_slots][4][T]
+    double* scon;              // slot contributions [rows][role a, b][4][K][T]
+    double* vcon;              // value contributions [rows][v0, v1, v2][K][T]
+    uint8_t* flag;             // [K][T]: a row without a root has a non-zero output adjoint
 };
 
 struct Where {
@@ -283,6 +299,165 @@ __global__ void __launch_bounds__(kThreads) program_tangent_kernel(const WaveArg
     for (int q = 0; q < nout; ++q) dp(row.elem[2], q) = out[q];
 }
 
+// input-column adjoints kb of a converged row for its output adjoints ob (csrc/newton_adjoint.cuh)
+template <int KIND>
+__device__ __forceinline__ void row_adjoint_at(const WaveArgs& w, const Where& at, unsigned root, long long n, const double ob[4], double* kb)
+{
+    constexpr int nin = gcsk::Sys<KIND>::kCols;
+    const double* const c = w.cols[at.k];
+    const long long cap = w.cap[at.k];
+    double k[nin];
+#pragma unroll
+    for (int q = 0; q < nin; ++q) k[q] = c[q * cap + at.i];
+    double ux, uy;
+    if constexpr (KIND == GCS_KIND_SDD || KIND == GCS_KIND_ANG) {
+        ux = w.cand[at.k][(root * 2 + 0) * n + at.i], uy = w.cand[at.k][(root * 2 + 1) * n + at.i];
+    } else {
+        ux = c[nin * cap + at.i], uy = c[(nin + 1) * cap + at.i];
+    }
+    gcsk::RowTangent<KIND> lin;
+    lin.init(k, ux, uy);
+    gcsk::row_adjoint<KIND>(lin, ob, kb);
+}
+
+// One wave of the adjoint sweep, over the batches a recorded run kept.  The transpose of the
+// scatter, the row's linearisation and the gather of program_tangent_kernel, in reverse:
+//   1. ob = the adjoints of the target's written coordinates, which are then zeroed; for solvers
+//      1-3 also the anchors the gather wrote (all zeroed; pb.x of solvers 1, 2 holds v0, pb.y of
+//      solver 3 holds sign1 * v1, the rest are constants);
+//   2. a row whose chosen run did not converge has no derivative: a non-zero (or NaN) ob sets the
+//      (instance, cotangent) flag and the row contributes kb = 0; otherwise kb = row_adjoint(ob);
+//   3. the gather's transpose, column adjoints first, then the anchor's:
+//      1: v0 = kb3 + pb.x, v1 = kb2, v2 = kb5          4: a = (kb0 kb1), v1 = kb2, b = (kb3 kb4), v2 = kb5
+//      2: v0 = kb2 + pb.x, v1 = s1*kb4, v2 = s2*kb5    5: a = (kb0 kb1), b = (kb2 kb3), v1 = s1*kb4, v2 = s2*kb5
+//      3: v0 = kb2, sd1 = kb8 + pb.y, v1 = s1*sd1, v2 = s2*kb9
+//      6: a = (kb0 kb1), v1 = kb2, b = (kb3 .. kb6), v2 = s2*kb7
+//      7: a = (kb0 .. kb3), v1 = s1*kb4, b = (kb5 .. kb8), v2 = s2*kb9
+//      8: a = (kb10/2.0 - kb0, kb11/2.0 - kb1, kb10/2.0 + kb0, kb11/2.0 + kb1), b = (kb7 kb8), v0 = kb2,
+//         v2 = s2*kb9
+//   written to the contribution buffer (program_adjoint_reduce_kernel adds them up).
+__global__ void __launch_bounds__(kThreads) program_adjoint_kernel(const WaveArgs w)
+{
+    const long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (g >= w.seg[kKinds] * w.K * w.T) return;
+    const long long T = w.T, KT = w.K * T, s = g / T, t = g - s * T;
+    Where at;
+    place(w, s, at);
+    const gcs_b200_program_row& row = w.rows[at.r];
+    double* const apos = w.apos + at.j * w.n_slots * 4 * T + t;
+    auto ap = [&](int slot, int q) -> double& { return apos[(4 * (long long)slot + q) * T]; };
+    const int a = row.elem[0], b = row.elem[1], tgt = row.elem[2];
+    const int kind = at.k + 1;
+    const int nout = (kind == GCS_KIND_SDD || kind == GCS_KIND_ANG) ? 4 : 2;
+    double ob[4] = {};
+    for (int q = 0; q < nout; ++q) ob[q] = ap(tgt, q), ap(tgt, q) = 0.0;
+    double anchor = 0.0;
+    if (row.solver <= 3) {
+        anchor = row.solver == 3 ? ap(b, 1) : ap(b, 0);
+        for (int q = 0; q < (row.solver == 3 ? 4 : 2); ++q) ap(a, q) = 0.0;
+        ap(b, 0) = 0.0, ap(b, 1) = 0.0;
+    }
+    const long long n = (w.seg[at.k + 1] - w.seg[at.k]) * w.K;
+    const unsigned root = w.root[at.k][at.i];
+    double kb[13] = {};
+    if (root >= 2 || !w.conv[at.k][root * n + at.i]) {
+        bool touched = false;
+        for (int q = 0; q < nout; ++q) touched |= !(ob[q] == 0.0);
+        if (touched) w.flag[at.j * T + t] = 1;
+    } else {
+        switch (kind) {
+        case GCS_KIND_PP: row_adjoint_at<GCS_KIND_PP>(w, at, root, n, ob, kb); break;
+        case GCS_KIND_SDD: row_adjoint_at<GCS_KIND_SDD>(w, at, root, n, ob, kb); break;
+        case GCS_KIND_PPL: row_adjoint_at<GCS_KIND_PPL>(w, at, root, n, ob, kb); break;
+        case GCS_KIND_PLL: row_adjoint_at<GCS_KIND_PLL>(w, at, root, n, ob, kb); break;
+        default: row_adjoint_at<GCS_KIND_ANG>(w, at, root, n, ob, kb); break;
+        }
+    }
+    const long long jt = at.j * T + t;
+    double* const sc = w.scon + at.r * 8 * KT + jt;  // [role][coordinate]
+    double* const vc = w.vcon + at.r * 3 * KT + jt;  // [q]
+    auto sa = [&](int role, int q, double v) { sc[(role * 4 + q) * KT] = v; };
+    auto va = [&](int q, double v) { vc[q * KT] = v; };
+    const double s1 = row.sign[1], s2 = row.sign[2];
+    switch (row.solver) {
+    case 1: va(0, kb[3] + anchor), va(1, kb[2]), va(2, kb[5]); break;
+    case 4:
+        sa(0, 0, kb[0]), sa(0, 1, kb[1]), va(1, kb[2]), sa(1, 0, kb[3]), sa(1, 1, kb[4]), va(2, kb[5]);
+        break;
+    case 2: va(0, kb[2] + anchor), va(1, s1 * kb[4]), va(2, s2 * kb[5]); break;
+    case 5:
+        sa(0, 0, kb[0]), sa(0, 1, kb[1]), sa(1, 0, kb[2]), sa(1, 1, kb[3]), va(1, s1 * kb[4]), va(2, s2 * kb[5]);
+        break;
+    case 6:
+        sa(0, 0, kb[0]), sa(0, 1, kb[1]), va(1, kb[2]);
+        sa(1, 0, kb[3]), sa(1, 1, kb[4]), sa(1, 2, kb[5]), sa(1, 3, kb[6]), va(2, s2 * kb[7]);
+        break;
+    case 7:
+        sa(0, 0, kb[0]), sa(0, 1, kb[1]), sa(0, 2, kb[2]), sa(0, 3, kb[3]), va(1, s1 * kb[4]);
+        sa(1, 0, kb[5]), sa(1, 1, kb[6]), sa(1, 2, kb[7]), sa(1, 3, kb[8]), va(2, s2 * kb[9]);
+        break;
+    case 3: va(0, kb[2]), va(1, s1 * (kb[8] + anchor)), va(2, s2 * kb[9]); break;
+    case 8: {
+        const double mx = kb[10] / 2.0, my = kb[11] / 2.0;
+        sa(0, 0, mx - kb[0]), sa(0, 1, my - kb[1]), sa(0, 2, mx + kb[0]), sa(0, 3, my + kb[1]);
+        sa(1, 0, kb[7]), sa(1, 1, kb[8]), va(0, kb[2]), va(2, s2 * kb[9]);
+        break;
+    }
+    }
+}
+
+// reader lists of one wave: slot entries first (target slot, coordinates read), then value entries
+struct AdjEntry {
+    int32_t target;
+    int32_t ncoord;  // 2 (point) or 4 (line) for a slot entry, 0 for a value entry
+};
+
+struct ReduceArgs {
+    const AdjEntry* ent;        // the wave's entries
+    const long long* begin;     // [n_ent + 1] into `readers`
+    const long long* readers;   // slot entry: row * 2 + role; value entry: row * 3 + q (rows relative to the wave)
+    long long n_ent, K, T;
+    double* apos;               // [K][n_slots][4][T]
+    double* aval;               // [K][n_values][T]
+    const double* scon;
+    const double* vcon;
+    long long n_slots, n_values;
+};
+
+// one thread per (entry, instance, cotangent): the entry's contributions added to its table entry
+// one at a time, in the reader list's ascending (row, role) order
+__global__ void __launch_bounds__(kThreads) program_adjoint_reduce_kernel(const ReduceArgs r)
+{
+    const long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const long long KT = r.K * r.T;
+    if (g >= r.n_ent * KT) return;
+    const long long e = g / KT, jt = g - e * KT, j = jt / r.T, t = jt - j * r.T;
+    const AdjEntry en = r.ent[e];
+    const long long lo = r.begin[e], hi = r.begin[e + 1];
+    if (en.ncoord > 0) {
+        double* const tab = r.apos + (j * r.n_slots + en.target) * 4 * r.T + t;
+        for (int c = 0; c < en.ncoord; ++c) {
+            double acc = tab[c * r.T];
+            for (long long i = lo; i < hi; ++i) acc = acc + r.scon[(r.readers[i] * 4 + c) * KT + jt];
+            tab[c * r.T] = acc;
+        }
+    } else {
+        double* const tab = r.aval + (j * r.n_values + en.target) * r.T + t;
+        double acc = *tab;
+        for (long long i = lo; i < hi; ++i) acc = acc + r.vcon[r.readers[i] * KT + jt];
+        *tab = acc;
+    }
+}
+
+// the NaN rule, after wave 0: adj_values[k][:][t] = NaN where the (k, t) flag is set
+__global__ void __launch_bounds__(kThreads) program_adjoint_flag_kernel(double* aval, const uint8_t* flag, long long K, long long n_values, long long T)
+{
+    const long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (g >= K * n_values * T) return;
+    const long long j = g / (n_values * T), t = g % T;
+    if (flag[j * T + t]) aval[g] = __longlong_as_double(0x7ff8000000000000LL);
+}
+
 int validate_desc(const gcs_b200_program_desc* d)
 {
     if (!d) return failf(GCS_E_INVALID, "null program descriptor");
@@ -377,6 +552,24 @@ struct gcs_b200_program {
     double* dvalues = nullptr;
     double* dpositions = nullptr;
     long long tangents_kt = 0;
+    // reader lists of the adjoint sweep, built at create time: the entries of wave w are
+    // [ent_off[w], ent_off[w+1]) of `ent` (slot entries, then value entries), the readers of entry e
+    // are readers[begin[e] .. begin[e+1])
+    std::vector<long long> ent_off;
+    AdjEntry* ent = nullptr;
+    long long* begin = nullptr;
+    long long* readers = nullptr;
+    long long max_wave_rows = 0;
+    // the tape of the last recorded run (every wave's kind batches) and its instance count (0: none)
+    unsigned char* tape = nullptr;
+    size_t tape_bytes = 0;
+    long long recorded_k = 0;
+    // working tables of the sweep, sized for `adj_kt` instances x cotangents
+    double* apos = nullptr;       // [K][n_slots][4][T]
+    double* contrib = nullptr;    // [max_wave_rows][11][K][T]: slot, then value contributions
+    uint8_t* flags = nullptr;     // [K][T]
+    double* avalues = nullptr;    // [K][n_values][T] of gcs_b200_program_adjoints_host
+    long long adj_kt = 0;
     cudaEvent_t ev[4] = {};
 };
 
@@ -430,12 +623,67 @@ struct CurrentDevice {
     }
 };
 
-// T = 0: a plain run.  T > 0: also the tangents along T directions (dvalues / dpositions).
-int run_on(gcs_b200_program* p, long long K, const double* values, double* positions, uint32_t* nonconverged, int variant,
-    cudaStream_t st, long long T = 0, const double* dvalues = nullptr, double* dpositions = nullptr)
+// the kind batches of one wave (or of the scratch) laid out from `at` with `cap[k]` sub-systems of
+// kind k + 1; returns the bytes they take
+size_t bind_batches(WaveArgs& w, unsigned char* at, const long long cap[kKinds], bool cand)
 {
-    int rc = ensure_scratch(p, K, T > 0, st);
+    size_t used = 0;
+    for (int k = 1; k <= kKinds; ++k) {
+        unsigned char* const base = at + used;
+        w.cols[k - 1] = reinterpret_cast<double*>(base);
+        w.cap[k - 1] = cap[k - 1];
+        unsigned char* flags = base + align256((size_t)(kInCols[k] + kOutCols[k]) * cap[k - 1] * sizeof(double));
+        w.code[k - 1] = flags, w.root[k - 1] = flags + align256((size_t)cap[k - 1]), w.conv[k - 1] = flags + 2 * align256((size_t)cap[k - 1]);
+        w.cand[k - 1] = has_cand(k, cand) ? reinterpret_cast<double*>(flags + 4 * align256((size_t)cap[k - 1])) : nullptr;
+        used += kind_bytes(k, cap[k - 1], cand);
+    }
+    return used;
+}
+
+// the tape's sub-system counts of wave `wave`: the wave's own rows x K, in multiples of 32
+void tape_caps(const gcs_b200_program* p, int wave, long long K, long long cap[kKinds])
+{
+    const long long* off = p->offsets.data() + (size_t)wave * kKinds;
+    for (int k = 0; k < kKinds; ++k) cap[k] = ((off[k + 1] - off[k]) * K + 31) / 32 * 32;
+}
+
+size_t tape_bytes(const gcs_b200_program* p, long long K)
+{
+    size_t bytes = 0;
+    for (int wave = 0; wave < p->n_waves; ++wave) {
+        long long cap[kKinds];
+        tape_caps(p, wave, K, cap);
+        for (int k = 1; k <= kKinds; ++k) bytes += kind_bytes(k, cap[k - 1], true);
+    }
+    return bytes;
+}
+
+// device current; makes the tape hold every wave's batches for K instances
+int ensure_tape(gcs_b200_program* p, long long K, cudaStream_t st)
+{
+    const size_t bytes = tape_bytes(p, K);
+    if (bytes <= p->tape_bytes) return GCS_OK;
+    if (p->tape) {
+        PROG_TRY(cudaStreamSynchronize(st));  // a sweep still in flight may read it
+        PROG_TRY(cudaFree(p->tape));
+        p->tape = nullptr, p->tape_bytes = 0;
+    }
+    if (cudaMalloc(&p->tape, bytes) != cudaSuccess) {
+        cudaGetLastError();
+        return failf(GCS_E_NOMEM, "cudaMalloc(%zu) for the tape of a recorded run of %lld instances failed", bytes, K);
+    }
+    p->tape_bytes = bytes;
+    return GCS_OK;
+}
+
+// T = 0: a plain run.  T > 0: also the tangents along T directions (dvalues / dpositions).
+// recorded: every wave's batches at their own place of the tape (T = 0 only)
+int run_on(gcs_b200_program* p, long long K, const double* values, double* positions, uint32_t* nonconverged, int variant,
+    cudaStream_t st, long long T = 0, const double* dvalues = nullptr, double* dpositions = nullptr, bool recorded = false)
+{
+    int rc = recorded ? ensure_tape(p, K, st) : ensure_scratch(p, K, T > 0, st);
     if (rc != GCS_OK) return rc;
+    if (recorded) p->recorded_k = 0;  // until this run is enqueued whole
     // every instance starts from the initial positions: one copy, then doubling copies
     const size_t table = (size_t)p->n_slots * 4 * sizeof(double);
     if (table) {
@@ -456,22 +704,21 @@ int run_on(gcs_b200_program* p, long long K, const double* values, double* posit
     w.pos = positions, w.val = values, w.n_slots = p->n_slots, w.n_values = p->n_values;
     w.nonconverged = nonconverged;
     w.T = T, w.dpos = dpositions, w.dval = dvalues;
-    {
-        unsigned char* at = p->scratch;
-        for (int k = 1; k <= kKinds; ++k) {
-            const long long cap = kind_cap(p, k, K);
-            w.cols[k - 1] = reinterpret_cast<double*>(at);
-            w.cap[k - 1] = cap;
-            unsigned char* flags = at + align256((size_t)(kInCols[k] + kOutCols[k]) * cap * sizeof(double));
-            w.code[k - 1] = flags, w.root[k - 1] = flags + align256((size_t)cap), w.conv[k - 1] = flags + 2 * align256((size_t)cap);
-            if (has_cand(k, T > 0)) w.cand[k - 1] = reinterpret_cast<double*>(flags + 4 * align256((size_t)cap));
-            at += kind_bytes(k, cap, T > 0);
-        }
+    if (!recorded) {
+        long long cap[kKinds];
+        for (int k = 1; k <= kKinds; ++k) cap[k - 1] = kind_cap(p, k, K);
+        bind_batches(w, p->scratch, cap, T > 0);
     }
+    unsigned char* tape = p->tape;
     for (int wave = 0; wave < p->n_waves; ++wave) {
         const long long* off = p->offsets.data() + (size_t)wave * kKinds;
         w.rows = p->rows + off[0];
         for (int k = 0; k <= kKinds; ++k) w.seg[k] = off[k] - off[0];
+        if (recorded) {
+            long long cap[kKinds];
+            tape_caps(p, wave, K, cap);
+            tape += bind_batches(w, tape, cap, true);
+        }
         const long long threads = w.seg[kKinds] * K;
         if (threads == 0) continue;
         const long long grid = (threads + kThreads - 1) / kThreads;
@@ -508,6 +755,99 @@ int run_on(gcs_b200_program* p, long long K, const double* values, double* posit
             PROG_TRY(cudaGetLastError());
         }
     }
+    if (recorded) p->recorded_k = K;
+    return GCS_OK;
+}
+
+// device current; the sweep's working tables for the recorded K x T cotangents
+int ensure_adjoint_tables(gcs_b200_program* p, long long T, cudaStream_t st)
+{
+    const long long KT = p->recorded_k * T;
+    if (KT <= p->adj_kt) return GCS_OK;
+    if (p->apos) PROG_TRY(cudaStreamSynchronize(st));
+    cudaFree(p->apos), cudaFree(p->contrib), cudaFree(p->flags), cudaFree(p->avalues);
+    p->apos = p->contrib = p->avalues = nullptr, p->flags = nullptr, p->adj_kt = 0;
+    const size_t pbytes = (size_t)KT * p->n_slots * 4 * sizeof(double), cbytes = (size_t)KT * p->max_wave_rows * 11 * sizeof(double);
+    const size_t vbytes = (size_t)KT * p->n_values * sizeof(double);
+    if ((pbytes && cudaMalloc(&p->apos, pbytes) != cudaSuccess) || (cbytes && cudaMalloc(&p->contrib, cbytes) != cudaSuccess)
+        || cudaMalloc(&p->flags, (size_t)KT) != cudaSuccess || (vbytes && cudaMalloc(&p->avalues, vbytes) != cudaSuccess)) {
+        cudaGetLastError();
+        return failf(GCS_E_NOMEM, "cudaMalloc for the adjoint tables of %lld instances x %lld cotangents (%zu + %zu + %zu bytes) failed",
+            p->recorded_k, T, pbytes, cbytes, vbytes);
+    }
+    p->adj_kt = KT;
+    return GCS_OK;
+}
+
+// device current, checks done, p->apos holds the cotangents of the recorded run's positions: the
+// sweep, waves from last to first, into adj_values [K][n_values][T]
+int sweep_on(gcs_b200_program* p, long long T, double* adj_values, cudaStream_t st)
+{
+    const long long K = p->recorded_k, KT = K * T;
+    if (p->n_values) PROG_TRY(cudaMemsetAsync(adj_values, 0, (size_t)KT * p->n_values * sizeof(double), st));
+    PROG_TRY(cudaMemsetAsync(p->flags, 0, (size_t)KT, st));
+    std::vector<unsigned char*> tape_at((size_t)p->n_waves + 1);
+    tape_at[0] = p->tape;
+    for (int wave = 0; wave < p->n_waves; ++wave) {
+        long long cap[kKinds];
+        tape_caps(p, wave, K, cap);
+        size_t bytes = 0;
+        for (int k = 1; k <= kKinds; ++k) bytes += kind_bytes(k, cap[k - 1], true);
+        tape_at[(size_t)wave + 1] = tape_at[(size_t)wave] + bytes;
+    }
+    WaveArgs w;
+    memset(&w, 0, sizeof(w));
+    w.K = K, w.T = T, w.n_slots = p->n_slots, w.n_values = p->n_values;
+    w.apos = p->apos, w.flag = p->flags;
+    w.scon = p->contrib, w.vcon = p->contrib + (size_t)p->max_wave_rows * 8 * KT;
+    ReduceArgs r;
+    memset(&r, 0, sizeof(r));
+    r.K = K, r.T = T, r.apos = p->apos, r.aval = adj_values, r.scon = w.scon, r.vcon = w.vcon;
+    r.n_slots = p->n_slots, r.n_values = p->n_values;
+    for (int wave = p->n_waves - 1; wave >= 0; --wave) {
+        const long long* off = p->offsets.data() + (size_t)wave * kKinds;
+        w.rows = p->rows + off[0];
+        for (int k = 0; k <= kKinds; ++k) w.seg[k] = off[k] - off[0];
+        const long long threads = w.seg[kKinds] * KT;
+        if (threads == 0) continue;
+        long long cap[kKinds];
+        tape_caps(p, wave, K, cap);
+        bind_batches(w, tape_at[(size_t)wave], cap, true);
+        r.ent = p->ent + p->ent_off[(size_t)wave];
+        r.begin = p->begin + p->ent_off[(size_t)wave];
+        r.readers = p->readers;
+        r.n_ent = p->ent_off[(size_t)wave + 1] - p->ent_off[(size_t)wave];
+        const long long grid = (threads + kThreads - 1) / kThreads, rgrid = (r.n_ent * KT + kThreads - 1) / kThreads;
+        if (grid > 0x7fffffffLL || rgrid > 0x7fffffffLL)
+            return failf(GCS_E_INVALID, "wave %d: %lld sub-systems x %lld cotangents are too many for one launch", wave, w.seg[kKinds] * K, T);
+        program_adjoint_kernel<<<(unsigned)grid, kThreads, 0, st>>>(w);
+        gcsk::api_count_launch();
+        PROG_TRY(cudaGetLastError());
+        if (rgrid == 0) continue;
+        program_adjoint_reduce_kernel<<<(unsigned)rgrid, kThreads, 0, st>>>(r);
+        gcsk::api_count_launch();
+        PROG_TRY(cudaGetLastError());
+    }
+    const long long nv = KT * p->n_values;
+    if (nv > 0) {
+        const long long grid = (nv + kThreads - 1) / kThreads;
+        if (grid > 0x7fffffffLL) return failf(GCS_E_INVALID, "%lld value adjoints are too many for one launch", nv);
+        program_adjoint_flag_kernel<<<(unsigned)grid, kThreads, 0, st>>>(adj_values, p->flags, K, p->n_values, T);
+        gcsk::api_count_launch();
+        PROG_TRY(cudaGetLastError());
+    }
+    return GCS_OK;
+}
+
+// the checks that need no program come first; a null table is refused unless the program has
+// nothing to put in it
+int check_adjoints(const gcs_b200_program* p, int T, const double* adj_positions, const double* adj_values)
+{
+    if (T < 1) return failf(GCS_E_INVALID, "n_cotangents must be >= 1 (got %d)", T);
+    if ((!adj_positions && !(p && p->n_slots == 0)) || (!adj_values && !(p && p->n_values == 0)))
+        return failf(GCS_E_INVALID, "null adjoint table (adj_positions or adj_values)");
+    if (!p) return failf(GCS_E_INVALID, "null program");
+    if (p->recorded_k < 1) return failf(GCS_E_INVALID, "no recorded run: call gcs_b200_program_run_recorded first");
     return GCS_OK;
 }
 
@@ -534,7 +874,7 @@ int check_tangent_run(const gcs_b200_program* p, long long K, const double* valu
 
 // device current, checks done
 int run_host(gcs_b200_program* p, long long K, const double* values, double* positions, uint32_t* nonconverged, int variant,
-    float ms[3], long long T, const double* dvalues, double* dpositions)
+    float ms[3], long long T, const double* dvalues, double* dpositions, bool recorded = false)
 {
     const size_t vbytes = (size_t)K * p->n_values * sizeof(double), pbytes = (size_t)K * p->n_slots * 4 * sizeof(double);
     if (K > p->tables_k) {
@@ -564,7 +904,7 @@ int run_host(gcs_b200_program* p, long long K, const double* values, double* pos
     if (vbytes) PROG_TRY(cudaMemcpyAsync(p->values, values, vbytes, cudaMemcpyHostToDevice, st));
     if (T > 0 && vbytes) PROG_TRY(cudaMemcpyAsync(p->dvalues, dvalues, vbytes * T, cudaMemcpyHostToDevice, st));
     PROG_TRY(cudaEventRecord(p->ev[1], st));
-    int rc = run_on(p, K, p->values, p->positions, nonconverged ? p->counts : nullptr, variant, st, T, p->dvalues, p->dpositions);
+    int rc = run_on(p, K, p->values, p->positions, nonconverged ? p->counts : nullptr, variant, st, T, p->dvalues, p->dpositions, recorded);
     if (rc != GCS_OK) {
         cudaStreamSynchronize(st);
         return rc;
@@ -614,8 +954,58 @@ int gcs_b200_program_create(const gcs_b200_program_desc* d, int device, gcs_b200
         cudaGetLastError();
         return bail(failf(GCS_E_NOMEM, "cudaMalloc for a program of %lld rows and %d slots failed", (long long)d->n_rows, d->n_slots));
     }
+    // The reader lists of the adjoint sweep.  Per wave, every slot read (roles a, b of solvers 4-8)
+    // and every value read gets one entry, slots first; its readers, (row, role) for a slot and (row,
+    // q) for a value with rows relative to the wave, are listed in ascending order.
+    std::vector<AdjEntry> ent;
+    std::vector<long long> begin(1, 0), readers;
+    {
+        std::vector<long long> slot_ent((size_t)d->n_slots, -1), value_ent((size_t)d->n_values, -1);
+        std::vector<std::vector<long long>> lists;
+        p->ent_off.assign(1, 0);
+        for (int wave = 0; wave < d->n_waves; ++wave) {
+            const long long lo = d->offsets[(long long)wave * kKinds], hi = d->offsets[(long long)(wave + 1) * kKinds];
+            if (hi - lo > p->max_wave_rows) p->max_wave_rows = hi - lo;
+            const size_t first = ent.size();
+            lists.clear();
+            for (int pass = 0; pass < 2; ++pass)  // slots, then values
+                for (long long r = lo; r < hi; ++r) {
+                    const gcs_b200_program_row& row = d->rows[r];
+                    for (int q = 0; q < 3; ++q) {
+                        const bool slot_read = pass == 0 && q < 2 && row.solver >= 4;
+                        const bool value_read = pass == 1 && row.value[q] >= 0;
+                        if (!slot_read && !value_read) continue;
+                        const int target = slot_read ? row.elem[q] : row.value[q];
+                        long long& e = (slot_read ? slot_ent : value_ent)[(size_t)target];
+                        if (e < 0) {
+                            e = (long long)lists.size();
+                            lists.emplace_back();
+                            ent.push_back({ target, slot_read ? (kRoleIsLine[row.solver][q] ? 4 : 2) : 0 });
+                        }
+                        lists[(size_t)e].push_back(slot_read ? (r - lo) * 2 + q : (r - lo) * 3 + q);
+                    }
+                }
+            for (size_t e = first; e < ent.size(); ++e) {
+                const std::vector<long long>& l = lists[e - first];
+                readers.insert(readers.end(), l.begin(), l.end());
+                begin.push_back((long long)readers.size());
+                (ent[e].ncoord ? slot_ent : value_ent)[(size_t)ent[e].target] = -1;
+            }
+            p->ent_off.push_back((long long)ent.size());
+        }
+    }
+    const size_t ent_bytes = ent.size() * sizeof(AdjEntry), begin_bytes = begin.size() * sizeof(long long);
+    const size_t reader_bytes = readers.size() * sizeof(long long);
+    if ((ent_bytes && cudaMalloc(&p->ent, ent_bytes) != cudaSuccess) || cudaMalloc(&p->begin, begin_bytes) != cudaSuccess
+        || (reader_bytes && cudaMalloc(&p->readers, reader_bytes) != cudaSuccess)) {
+        cudaGetLastError();
+        return bail(failf(GCS_E_NOMEM, "cudaMalloc for the reader lists of %zu entries failed", ent.size()));
+    }
     if ((row_bytes && cudaMemcpyAsync(p->rows, d->rows, row_bytes, cudaMemcpyHostToDevice, p->stream) != cudaSuccess)
         || (init_bytes && cudaMemcpyAsync(p->initial, d->initial, init_bytes, cudaMemcpyHostToDevice, p->stream) != cudaSuccess)
+        || (ent_bytes && cudaMemcpyAsync(p->ent, ent.data(), ent_bytes, cudaMemcpyHostToDevice, p->stream) != cudaSuccess)
+        || cudaMemcpyAsync(p->begin, begin.data(), begin_bytes, cudaMemcpyHostToDevice, p->stream) != cudaSuccess
+        || (reader_bytes && cudaMemcpyAsync(p->readers, readers.data(), reader_bytes, cudaMemcpyHostToDevice, p->stream) != cudaSuccess)
         || cudaStreamSynchronize(p->stream) != cudaSuccess)
         return bail(failf(GCS_E_CUDA, "program upload failed: %s", cudaGetErrorString(cudaGetLastError())));
     *out = p;
@@ -658,6 +1048,64 @@ int gcs_b200_program_run_tangents_host(gcs_b200_program* p, int64_t K, const dou
     return run_host(p, K, values, positions, nonconverged, variant, ms, T, dvalues, dpositions);
 }
 
+int gcs_b200_program_run_recorded(gcs_b200_program* p, int64_t K, const double* values, double* positions, uint32_t* nonconverged,
+    int variant, void* stream)
+{
+    int rc = check_run(p, K, values, positions, variant);
+    if (rc != GCS_OK) return rc;
+    CurrentDevice cur(p->device);
+    return run_on(p, K, values, positions, nonconverged, variant, static_cast<cudaStream_t>(stream), 0, nullptr, nullptr, true);
+}
+
+int gcs_b200_program_run_recorded_host(gcs_b200_program* p, int64_t K, const double* values, double* positions,
+    uint32_t* nonconverged, int variant, float ms[3])
+{
+    int rc = check_run(p, K, values, positions, variant);
+    if (rc != GCS_OK) return rc;
+    CurrentDevice cur(p->device);
+    return run_host(p, K, values, positions, nonconverged, variant, ms, 0, nullptr, nullptr, true);
+}
+
+int gcs_b200_program_adjoints(gcs_b200_program* p, int32_t T, const double* adj_positions, double* adj_values, void* stream)
+{
+    int rc = check_adjoints(p, T, adj_positions, adj_values);
+    if (rc != GCS_OK) return rc;
+    CurrentDevice cur(p->device);
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    rc = ensure_adjoint_tables(p, T, st);
+    if (rc != GCS_OK) return rc;
+    const size_t pbytes = (size_t)p->recorded_k * T * p->n_slots * 4 * sizeof(double);
+    if (pbytes) PROG_TRY(cudaMemcpyAsync(p->apos, adj_positions, pbytes, cudaMemcpyDeviceToDevice, st));
+    return sweep_on(p, T, adj_values, st);
+}
+
+int gcs_b200_program_adjoints_host(gcs_b200_program* p, int32_t T, const double* adj_positions, double* adj_values, float ms[3])
+{
+    int rc = check_adjoints(p, T, adj_positions, adj_values);
+    if (rc != GCS_OK) return rc;
+    CurrentDevice cur(p->device);
+    cudaStream_t st = p->stream;
+    rc = ensure_adjoint_tables(p, T, st);
+    if (rc != GCS_OK) return rc;
+    const size_t pbytes = (size_t)p->recorded_k * T * p->n_slots * 4 * sizeof(double);
+    const size_t vbytes = (size_t)p->recorded_k * T * p->n_values * sizeof(double);
+    PROG_TRY(cudaEventRecord(p->ev[0], st));
+    if (pbytes) PROG_TRY(cudaMemcpyAsync(p->apos, adj_positions, pbytes, cudaMemcpyHostToDevice, st));
+    PROG_TRY(cudaEventRecord(p->ev[1], st));
+    rc = sweep_on(p, T, p->avalues, st);
+    if (rc != GCS_OK) {
+        cudaStreamSynchronize(st);
+        return rc;
+    }
+    PROG_TRY(cudaEventRecord(p->ev[2], st));
+    if (vbytes) PROG_TRY(cudaMemcpyAsync(adj_values, p->avalues, vbytes, cudaMemcpyDeviceToHost, st));
+    PROG_TRY(cudaEventRecord(p->ev[3], st));
+    PROG_TRY(cudaStreamSynchronize(st));
+    if (ms)
+        for (int q = 0; q < 3; ++q) PROG_TRY(cudaEventElapsedTime(&ms[q], p->ev[q], p->ev[q + 1]));
+    return GCS_OK;
+}
+
 void gcs_b200_program_destroy(gcs_b200_program* p)
 {
     if (!p) return;
@@ -669,6 +1117,8 @@ void gcs_b200_program_destroy(gcs_b200_program* p)
         cudaFree(p->rows), cudaFree(p->initial), cudaFree(p->scratch);
         cudaFree(p->values), cudaFree(p->positions), cudaFree(p->counts);
         cudaFree(p->dvalues), cudaFree(p->dpositions);
+        cudaFree(p->ent), cudaFree(p->begin), cudaFree(p->readers), cudaFree(p->tape);
+        cudaFree(p->apos), cudaFree(p->contrib), cudaFree(p->flags), cudaFree(p->avalues);
         cudaGetLastError();
     }
     delete p;

@@ -63,6 +63,21 @@ public:
     ProgramRunStats runTangents(const double* values, std::int64_t K, const double* dvalues, int T, double* positions, double* dpositions,
         std::uint32_t* nonconverged = nullptr, int nDevices = 1);
 
+    // run(), also recording what adjoints() needs (gcs_b200_program_run_recorded): every wave's
+    // batches stay on the device, about n_rows x K x 100 bytes.  Positions and counts are run()'s.
+    ProgramRunStats record(const double* values, std::int64_t K, double* positions, std::uint32_t* nonconverged = nullptr,
+        int nDevices = 1);
+
+    // Reverse mode over the last record() (gcs_b200_program_adjoints), with its K and device split:
+    // adjPositions host [K][nSlots()][4][T] (T >= 1 cotangents, weights on the position coordinates),
+    // adjValues host [K][nValues()][T] receives sum_{s,c} adjPositions[k][s][c][t] * dpositions[k][s][c]
+    // / dvalues[k][v], with respect to radians for angles: the device gives the adjoint with respect
+    // to cos(v), and here adj = (-std::sin(v)) * adj_cos, v the recorded value.  NaN for every value
+    // of (k, t) when the cotangent reaches a row whose chosen run did not converge.  Throws
+    // std::logic_error before any device call when nothing was recorded, std::invalid_argument for
+    // T < 1.
+    ProgramRunStats adjoints(const double* adjPositions, int T, double* adjValues);
+
     // The edit loop: one instance with the constraints' current values, written into the elements -
     // the state solveLeaves leaves.
     ProgramRunStats solve();
@@ -76,6 +91,7 @@ public:
     const std::vector<std::int64_t>& rowLeaf() const { return m_rowLeaf; }  // leaf index of every row
     const std::vector<std::uint8_t>& solvedAfter() const { return m_solvedAfter; }  // per slot: solved after a run
     double compileSeconds() const { return m_compileSeconds; }
+    int recordedDevices() const { return m_recordedDevices; }  // devices of the last record() (0: none)
     // the descriptor gcs_b200_program_create takes, pointing into this program's tables (valid while
     // the program lives and is not moved from)
     gcs_b200_program_desc desc() const;
@@ -85,7 +101,7 @@ private:
     gcs_b200_program* onDevice(int device);
     void release();
     ProgramRunStats runImpl(const double* values, std::int64_t K, const double* dvalues, int T, double* positions, double* dpositions,
-        std::uint32_t* nonconverged, int nDevices);
+        std::uint32_t* nonconverged, int nDevices, bool recorded = false);
 
     BatchReport m_report;
     std::vector<gcs_b200_program_row> m_rows;
@@ -104,6 +120,10 @@ private:
     double* m_stageDValues = nullptr;
     double* m_stageDPositions = nullptr;
     std::int64_t m_stageKT = 0;  // instances x directions the tangent staging holds
+    // the last record(): its values (radians) and device split; m_recordedDevices = 0: none
+    std::vector<double> m_recordedValues;
+    std::int64_t m_recordedK = 0;
+    int m_recordedDevices = 0;
 };
 
 }  // namespace Gcs::B200

@@ -130,6 +130,8 @@ SketchProgram& SketchProgram::operator=(SketchProgram&& o) noexcept
     o.m_stageValues = o.m_stagePositions = nullptr, o.m_stageCounts = nullptr, o.m_stageK = 0;
     m_stageDValues = o.m_stageDValues, m_stageDPositions = o.m_stageDPositions, m_stageKT = o.m_stageKT;
     o.m_stageDValues = o.m_stageDPositions = nullptr, o.m_stageKT = 0;
+    m_recordedValues = std::move(o.m_recordedValues), m_recordedK = o.m_recordedK, m_recordedDevices = o.m_recordedDevices;
+    o.m_recordedK = 0, o.m_recordedDevices = 0;
     return *this;
 }
 
@@ -143,6 +145,7 @@ void SketchProgram::release()
     m_stageValues = m_stagePositions = nullptr, m_stageCounts = nullptr, m_stageK = 0;
     gcs_b200_host_free(m_stageDValues), gcs_b200_host_free(m_stageDPositions);
     m_stageDValues = m_stageDPositions = nullptr, m_stageKT = 0;
+    m_recordedValues.clear(), m_recordedK = 0, m_recordedDevices = 0;
 }
 
 gcs_b200_program_desc SketchProgram::desc() const
@@ -181,9 +184,62 @@ ProgramRunStats SketchProgram::runTangents(const double* values, std::int64_t K,
     return runImpl(values, K, dvalues, T, positions, dpositions, nonconverged, nDevices);
 }
 
-// T = 0: run(); T > 0: runTangents()
+ProgramRunStats SketchProgram::record(const double* values, std::int64_t K, double* positions, std::uint32_t* nonconverged, int nDevices)
+{
+    m_recordedDevices = 0;  // a failed record() leaves nothing to sweep
+    const ProgramRunStats st = runImpl(values, K, nullptr, 0, positions, nullptr, nonconverged, nDevices, true);
+    m_recordedValues.assign(values, values + static_cast<std::size_t>(K) * nValues());
+    m_recordedK = K;
+    // runImpl's split: instances in contiguous ranges over the first min(nDevices, devices, K) devices
+    m_recordedDevices = static_cast<int>(std::min<std::int64_t>(std::clamp(nDevices, 1, gcs_b200_device_count()), K));
+    return st;
+}
+
+ProgramRunStats SketchProgram::adjoints(const double* adjPositions, int T, double* adjValues)
+{
+    const auto t0 = Clock::now();
+    if (m_recordedDevices < 1) throw std::logic_error("SketchProgram::adjoints: no recorded run; call record() first");
+    if (T < 1) throw std::invalid_argument("SketchProgram::adjoints: T must be >= 1 (got " + std::to_string(T) + ")");
+    const std::int64_t K = m_recordedK;
+    const int nDevices = m_recordedDevices;
+    const std::size_t nv = nValues(), table = nSlots() * 4;
+    const std::int64_t launches0 = gcs_b200_launch_count();
+    std::vector<int> rc(static_cast<std::size_t>(nDevices), GCS_OK);
+    std::vector<std::array<float, 3>> ms(static_cast<std::size_t>(nDevices));
+    auto part = [&](int g) {
+        const std::int64_t lo = K * g / nDevices;
+        rc[static_cast<std::size_t>(g)] = gcs_b200_program_adjoints_host(m_device[static_cast<std::size_t>(g)], T,
+            adjPositions + lo * static_cast<std::int64_t>(table) * T, adjValues + lo * static_cast<std::int64_t>(nv) * T,
+            ms[static_cast<std::size_t>(g)].data());
+    };
+    if (nDevices == 1) {
+        part(0);
+    } else {
+        std::vector<std::thread> threads;
+        for (int g = 0; g < nDevices; ++g) threads.emplace_back(part, g);
+        for (auto& t : threads) t.join();
+    }
+    for (int g = 0; g < nDevices; ++g)
+        if (rc[static_cast<std::size_t>(g)] != GCS_OK) cudaFailure("gcs_b200_program_adjoints_host", rc[static_cast<std::size_t>(g)]);
+    // the device's adjoints of cos(v), to radians: adj = (-std::sin(v)) * adj_cos
+    const long long n = static_cast<long long>(K) * static_cast<long long>(nv) * T;
+    const std::uint8_t* angle = m_valueIsAngle.data();
+    const double* rec = m_recordedValues.data();
+#pragma omp parallel for schedule(static) if (n > 65536)
+    for (long long q = 0; q < n; ++q) {
+        const long long vq = q / T;
+        if (angle[static_cast<std::size_t>(vq) % nv]) adjValues[q] = -std::sin(rec[vq]) * adjValues[q];
+    }
+    ProgramRunStats st;
+    st.launches = gcs_b200_launch_count() - launches0;
+    for (const auto& m : ms) st.uploadMs += m[0], st.deviceMs += m[1], st.downloadMs += m[2];
+    st.seconds = std::chrono::duration<double>(Clock::now() - t0).count();
+    return st;
+}
+
+// T = 0: run() or record(); T > 0: runTangents()
 ProgramRunStats SketchProgram::runImpl(const double* values, std::int64_t K, const double* dvalues, int T, double* positions,
-    double* dpositions, std::uint32_t* nonconverged, int nDevices)
+    double* dpositions, std::uint32_t* nonconverged, int nDevices, bool recorded)
 {
     const auto t0 = Clock::now();
     if (K < 1) throw std::invalid_argument("SketchProgram::run: K must be >= 1");
@@ -236,8 +292,8 @@ ProgramRunStats SketchProgram::runImpl(const double* values, std::int64_t K, con
         const std::int64_t vo = lo * static_cast<std::int64_t>(nv), po = lo * static_cast<std::int64_t>(table);
         std::uint32_t* counts = nonconverged ? m_stageCounts + lo : nullptr;
         float* m = ms[static_cast<std::size_t>(g)].data();
-        rc[static_cast<std::size_t>(g)] = T == 0
-            ? gcs_b200_program_run_host(p, hi - lo, m_stageValues + vo, m_stagePositions + po, counts, variant, m)
+        rc[static_cast<std::size_t>(g)] = recorded ? gcs_b200_program_run_recorded_host(p, hi - lo, m_stageValues + vo, m_stagePositions + po, counts, variant, m)
+            : T == 0 ? gcs_b200_program_run_host(p, hi - lo, m_stageValues + vo, m_stagePositions + po, counts, variant, m)
             : gcs_b200_program_run_tangents_host(p, hi - lo, m_stageValues + vo, m_stagePositions + po, counts, T, m_stageDValues + vo * T,
                 m_stageDPositions + po * T, variant, m);
     };
@@ -250,7 +306,8 @@ ProgramRunStats SketchProgram::runImpl(const double* values, std::int64_t K, con
     }
     for (int g = 0; g < nDevices; ++g)
         if (rc[static_cast<std::size_t>(g)] != GCS_OK)
-            cudaFailure(T == 0 ? "gcs_b200_program_run_host" : "gcs_b200_program_run_tangents_host", rc[static_cast<std::size_t>(g)]);
+            cudaFailure(recorded ? "gcs_b200_program_run_recorded_host" : T == 0 ? "gcs_b200_program_run_host" : "gcs_b200_program_run_tangents_host",
+                rc[static_cast<std::size_t>(g)]);
     const long long npos = static_cast<long long>(K) * static_cast<long long>(table);
     const double* from = m_stagePositions;
 #pragma omp parallel for schedule(static) if (npos > 65536)

@@ -920,6 +920,32 @@ GCS_API int gcs_host_program_run_tangents(gcs_host_program* h, int64_t K, const 
     }
 }
 
+// run(), recording what gcs_host_program_adjoints needs (SketchProgram::record).  Returns 0 or -1.
+GCS_API int gcs_host_program_run_recorded(gcs_host_program* h, int64_t K, const double* values, double* positions, uint32_t* nonconverged,
+    int n_devices, int64_t* stats)
+{
+    try {
+        programStats(h, h->prog->record(values, K, positions, nonconverged, n_devices), n_devices, stats);
+        return 0;
+    } catch (const std::exception& ex) {
+        return fail(ex);
+    }
+}
+
+// Reverse mode over the last recorded run (SketchProgram::adjoints): adj_positions [K][n_slots][4][T],
+// adj_values out [K][n_values][T] (radians for angles); stats as gcs_host_program_run (devices: those of
+// the recorded run).  Returns 0 or -1.
+GCS_API int gcs_host_program_adjoints(gcs_host_program* h, int T, const double* adj_positions, double* adj_values, int64_t* stats)
+{
+    try {
+        const Gcs::B200::ProgramRunStats st = h->prog->adjoints(adj_positions, T, adj_values);
+        programStats(h, st, h->prog->recordedDevices(), stats);
+        return 0;
+    } catch (const std::exception& ex) {
+        return fail(ex);
+    }
+}
+
 // The edit loop: values (may be NULL: keep the current ones) become the constraints' values, then
 // SketchProgram::solve(); el receives every element's solved flag and position.  Returns 0 or -1.
 GCS_API int gcs_host_program_solve(gcs_host_program* h, const double* values, gcs_host_element* el)

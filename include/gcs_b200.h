@@ -381,6 +381,50 @@ GCS_B200_API int gcs_b200_program_run_tangents(gcs_b200_program* prog, int64_t n
 GCS_B200_API int gcs_b200_program_run_tangents_host(gcs_b200_program* prog, int64_t n_instances, const double* values,
     double* positions, uint32_t* nonconverged, int32_t n_tangents, const double* dvalues, double* dpositions,
     int variant, float ms[3]);
+/* Recorded runs: gcs_b200_program_run, plus a tape that the adjoint sweep below reads.  Every (wave,
+ * kind) batch gets its own place in one program-owned tape allocation (input and output columns,
+ * code, root and convergence planes, and the candidate planes of K2 / K5), each starting at a
+ * multiple of 32 sub-systems, instead of one set of batches reused by every wave.  Positions,
+ * nonconverged, the kernels that solve them and the launch count are those of gcs_b200_program_run.
+ * The tape takes about  sum over waves and kinds of rows x K x (8 x (in + out columns) + 4, + 32 for
+ * K2 / K5)  bytes: it grows with n_rows x K, not with the largest wave as a plain run's batches do.
+ * It is kept until the next recorded run replaces it; plain and tangent runs leave it alone. */
+GCS_B200_API int gcs_b200_program_run_recorded(gcs_b200_program* prog, int64_t n_instances, const double* values, double* positions,
+    uint32_t* nonconverged, int variant, void* cuda_stream);
+/* The same with host buffers, as gcs_b200_program_run_host. */
+GCS_B200_API int gcs_b200_program_run_recorded_host(gcs_b200_program* prog, int64_t n_instances, const double* values,
+    double* positions, uint32_t* nonconverged, int variant, float ms[3]);
+/* Adjoints (reverse mode) of the program's last recorded run, with that run's K: for each instance k
+ * and T = n_cotangents >= 1 cotangents adj_positions[k][:][:][t] (a weight on every position
+ * coordinate),
+ *     adj_values[k][v][t] = sum_{s,c} adj_positions[k][s][c][t] * d positions[k][s][c] / d values[k][v]
+ * the transpose of the Jacobian whose columns gcs_b200_program_run_tangents computes.  Layouts are
+ * instance-major with the cotangent innermost: adj_positions [K][n_slots][4][T] (device, read, not
+ * changed), adj_values [K][n_values][T] (device, fully written).  An angle slot holds cos(angle), so
+ * its adjoint is with respect to cos(angle).
+ * Order of summation (deterministic: independent of K, the stream and the schedule): a working copy
+ * of adj_positions is swept over the waves from last to first.  Per wave, each row takes the adjoints
+ * of the slot coordinates it wrote (its target, and for solvers 1-3 the anchors) and zeroes them,
+ * maps them through the transpose of its linearisation and of the gather (csrc/newton_adjoint.cuh,
+ * csrc/sketch_program.cu state the operation order), and every slot and value entry the wave read
+ * then receives its rows' contributions in ascending (row, role) order, each added to the running
+ * entry one at a time.  What is left in the working table after wave 0 belongs to the initial
+ * positions, which are constants, and is dropped.
+ * Rows without a root: a row whose chosen Newton run did not converge has no derivative.  If its
+ * output adjoint for (k, t) is not all zero (NaN counts as non-zero), adj_values[k][:][t] is NaN
+ * entirely (forward mode gives NaN for every value it depends on); if it is all zero, the row
+ * contributes nothing.
+ * Stream-ordered on `cuda_stream` and must come after its recorded run there (the tape is read on the
+ * device); does not synchronise.  Launches: at most 2 per non-empty wave + 1.  Memory: working tables
+ * of K x T x (n_slots x 32 + n_values x 8 + rows of the largest wave x 88 + 1) bytes.  Checked before
+ * any device call: a null program, n_cotangents >= 1, adj_positions non-null when n_slots > 0,
+ * adj_values non-null when n_values > 0, and that the program has a recorded run. */
+GCS_B200_API int gcs_b200_program_adjoints(gcs_b200_program* prog, int32_t n_cotangents, const double* adj_positions,
+    double* adj_values, void* cuda_stream);
+/* The same with host buffers: adj_positions up, the sweep, adj_values down on the program's own
+ * stream, then synchronises; ms (may be NULL) receives the device time of the three. */
+GCS_B200_API int gcs_b200_program_adjoints_host(gcs_b200_program* prog, int32_t n_cotangents, const double* adj_positions,
+    double* adj_values, float ms[3]);
 GCS_B200_API void gcs_b200_program_destroy(gcs_b200_program* prog);
 
 /* Test hook: on-device self check of the hand-written division / square root / 2x2 QR fast paths
