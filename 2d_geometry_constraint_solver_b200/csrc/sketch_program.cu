@@ -4,26 +4,27 @@
 // Device layout.  The caller's tables are instance-major (values [K][n_values], positions
 // [K][n_slots][4]).  The kind batches of a wave put the K instances of one row next to each other
 // (sub-system (row r, instance j) at index r*K + j of its kind's batch), so the threads of a warp
-// share a row recipe and write consecutive column entries.  The gather kernel is the device copy of
-// the numeric half of the host packer (Gcs::B200 packNumeric, host/src/b200/leaf_batch.cpp): same
-// reads, same operations in the same order, built with --fmad=false like every kernel of the
-// library, so the columns it writes are the host's bit for bit.
+// share a row recipe and write consecutive column entries.  The gather (gather_row, run by the
+// gather kernel) is the device copy of the numeric half of the host packer (Gcs::B200 packNumeric,
+// host/src/b200/leaf_batch.cpp): same reads, same operations in the same order, built with
+// --fmad=false like every kernel of the library, so the columns it writes are the host's bit for bit.
 //
 // Tangent runs (gcs_b200_program_run_tangents) add one launch per wave after the scatter: the
 // tangent kernel, one thread per (row, instance, direction t) with t fastest, so that consecutive
 // threads read and write consecutive doubles of the instance-major tangent tables (dvalues
-// [K][n_values][T], dpositions [K][n_slots][4][T]).  It forms the row's input-column tangents the way
-// the gather forms the columns, linearises the row at its chosen root (csrc/newton_tangent.cuh) and
+// [K][n_values][T], dpositions [K][n_slots][4][T]).  It runs gather_row on the tangents to form the
+// row's input-column tangents, linearises the row at its chosen root (csrc/newton_tangent.cuh) and
 // writes the target's tangents.  The K2 / K5 batches then also keep their candidate planes, whose
 // chosen normal is the row's unknown.
 //
 // Recorded runs (gcs_b200_program_run_recorded) place every (wave, kind) batch at its own offset of
-// one tape allocation instead of reusing one set of batches for every wave, so that the batches of
-// all waves (columns, flags, K2 / K5 candidate planes) survive the run.  The adjoint sweep
-// (gcs_b200_program_adjoints) reads them back, waves from last to first, with two launches per
+// one tape allocation (tape_layout) instead of reusing one set of batches for every wave, so that
+// the batches of all waves (columns, flags, K2 / K5 candidate planes) survive the run.  The adjoint
+// sweep (gcs_b200_program_adjoints) reads them back, waves from last to first, with two launches per
 // wave: the adjoint kernel, one thread per (row, instance, cotangent t) with t fastest, takes the
 // adjoints of what the row wrote (its target, and the anchors of a zero-fixed row), zeroes them and
-// writes the row's contributions to the slots and values it read into a contribution buffer; the
+// writes the row's contributions to the slots and values it read (gather_row_transpose) into a
+// contribution buffer; the
 // reduce kernel adds those into the working slot-adjoint table and the value adjoints, each table
 // entry's contributions in ascending (row, role) order from reader lists built at create time.  No
 // atomics: the result does not depend on K, the stream or the schedule.
@@ -32,6 +33,8 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <initializer_list>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/gcs_b200.h"
@@ -61,6 +64,12 @@ int failf(int code, const char* fmt, ...)
             __FILE__, __LINE__);                                                                          \
     } while (0)
 
+#define PROG_RC(expr)                  \
+    do {                               \
+        const int rc_ = (expr);        \
+        if (rc_ != GCS_OK) return rc_; \
+    } while (0)
+
 constexpr int kKinds = GCS_KIND_COUNT;
 constexpr int kThreads = 256;
 
@@ -71,8 +80,33 @@ constexpr bool kRoleIsLine[9][3] = { {}, { 0, 0, 0 }, { 0, 0, 1 }, { 1, 0, 1 }, 
     { 1, 1, 0 }, { 1, 0, 1 } };
 constexpr bool kReads[9][3] = { {}, { 1, 1, 1 }, { 1, 1, 1 }, { 1, 1, 1 }, { 0, 1, 1 }, { 0, 1, 1 }, { 0, 1, 1 },
     { 0, 1, 1 }, { 1, 0, 1 } };
-constexpr int kInCols[kKinds + 1] = { 0, 6, 9, 10, 12, 13 };
-constexpr int kOutCols[kKinds + 1] = { 0, 2, 4, 2, 2, 4 };
+
+// f(std::integral_constant<int, kind>()): f sees a kind known at run time as a compile-time
+// constant.  The host (in_cols, out_cols) and the kernels' device lambdas share it; the pragma lets
+// the one template call either.
+#pragma nv_exec_check_disable
+template <class F>
+__host__ __device__ __forceinline__ auto with_kind(int kind, F&& f)
+{
+    switch (kind) {
+    case GCS_KIND_PP: return f(std::integral_constant<int, GCS_KIND_PP>());
+    case GCS_KIND_SDD: return f(std::integral_constant<int, GCS_KIND_SDD>());
+    case GCS_KIND_PPL: return f(std::integral_constant<int, GCS_KIND_PPL>());
+    case GCS_KIND_PLL: return f(std::integral_constant<int, GCS_KIND_PLL>());
+    default: return f(std::integral_constant<int, GCS_KIND_ANG>());
+    }
+}
+
+// a kind's input and output columns
+__host__ __device__ __forceinline__ int in_cols(int kind)
+{
+    return with_kind(kind, [](auto K) { return gcsk::Sys<decltype(K)::value>::kCols; });
+}
+
+__host__ __device__ __forceinline__ int out_cols(int kind)
+{
+    return with_kind(kind, [](auto K) { return gcsk::Sys<decltype(K)::value>::kOut; });
+}
 
 // one wave: rows [seg[0], seg[5]) of the program relative to `rows`, kind k + 1 at [seg[k], seg[k+1])
 struct WaveArgs {
@@ -123,261 +157,84 @@ __device__ __forceinline__ bool locate(const WaveArgs& w, Where& at)
     return true;
 }
 
-__global__ void __launch_bounds__(kThreads) program_gather_kernel(const WaveArgs w)
+// The gather of one row, solver by solver: its input columns and, for the zero-fixed solvers 1-3,
+// the anchors it writes into the positions.  S provides
+//   slot(role, q)  coordinate q of role a (0) or b (1), as a double&;
+//   value(q)       v0 .. v2;
+//   cst(i)         canvas constant i;
+//   in(col, v)     writes input column col.
+// program_gather_kernel runs it on the positions and values (GatherColumns), program_tangent_kernel
+// on their tangents (GatherTangents, where every canvas constant is 0), so that each statement of the
+// latter is the exact derivative of the former's.
+template <class S>
+__device__ __forceinline__ void gather_row(const gcs_b200_program_row& row, S& s)
 {
-    Where at;
-    if (!locate(w, at)) return;
-    const gcs_b200_program_row& row = w.rows[at.r];
-    double* const pos = w.pos + at.j * w.n_slots * 4;
-    const double* const val = w.val + at.j * w.n_values;
-    double* const c = w.cols[at.k];
-    const long long cap = w.cap[at.k], i = at.i;
-    auto in = [&](int col, double v) { c[col * cap + i] = v; };
-    double* const pa = pos + 4 * (long long)row.elem[0];
-    double* const pb = pos + 4 * (long long)row.elem[1];
-    const double v0 = row.value[0] >= 0 ? val[row.value[0]] : 0.0;
-    const double v1 = row.value[1] >= 0 ? val[row.value[1]] : 0.0;
-    const double v2 = row.value[2] >= 0 ? val[row.value[2]] : 0.0;
-    const double* const cst = row.canvas;
-    w.code[at.k][i] = (uint8_t)row.code;
+    auto pa = [&](int q) -> double& { return s.slot(0, q); };
+    auto pb = [&](int q) -> double& { return s.slot(1, q); };
+    auto cst = [&](int i) { return s.cst(i); };
+    auto in = [&](int col, double v) { s.in(col, v); };
+    const double v0 = s.value(0), v1 = s.value(1), v2 = s.value(2);
     switch (row.solver) {
     case 1:  // ZeroFixedPointsTriangle: P1 -> (0, 0), P2 -> (d12, 0)
-        pa[0] = 0.0, pa[1] = 0.0, pb[0] = v0, pb[1] = 0.0;
+        pa(0) = 0.0, pa(1) = 0.0, pb(0) = v0, pb(1) = 0.0;
         in(0, 0.0), in(1, 0.0), in(2, v1), in(3, v0), in(4, 0.0), in(5, v2);
         break;
     case 4:  // TwoFixedPointsDistance
-        in(0, pa[0]), in(1, pa[1]), in(2, v1), in(3, pb[0]), in(4, pb[1]), in(5, v2);
+        in(0, pa(0)), in(1, pa(1)), in(2, v1), in(3, pb(0)), in(4, pb(1)), in(5, v2);
         break;
     case 2:  // ZeroFixedPPLTriangle
-        pa[0] = 0.0, pa[1] = 0.0, pb[0] = v0, pb[1] = 0.0;
+        pa(0) = 0.0, pa(1) = 0.0, pb(0) = v0, pb(1) = 0.0;
         in(0, 0.0), in(1, 0.0), in(2, v0), in(3, 0.0);
-        in(4, row.sign[1] * v1), in(5, row.sign[2] * v2), in(6, cst[0]), in(7, cst[1]), in(8, cst[2]);
+        in(4, row.sign[1] * v1), in(5, row.sign[2] * v2), in(6, cst(0)), in(7, cst(1)), in(8, cst(2));
         break;
     case 5:  // TwoFixedPointsLine
-        in(0, pa[0]), in(1, pa[1]), in(2, pb[0]), in(3, pb[1]);
-        in(4, row.sign[1] * v1), in(5, row.sign[2] * v2), in(6, cst[0]), in(7, cst[1]), in(8, cst[2]);
+        in(0, pa(0)), in(1, pa(1)), in(2, pb(0)), in(3, pb(1));
+        in(4, row.sign[1] * v1), in(5, row.sign[2] * v2), in(6, cst(0)), in(7, cst(1)), in(8, cst(2));
         break;
     case 6:  // FixedPointAndLineFreePoint: a point, b line
-        in(0, pa[0]), in(1, pa[1]), in(2, v1), in(3, pb[0]), in(4, pb[1]), in(5, pb[2]), in(6, pb[3]);
-        in(7, row.sign[2] * v2), in(8, cst[0]), in(9, cst[1]);
+        in(0, pa(0)), in(1, pa(1)), in(2, v1), in(3, pb(0)), in(4, pb(1)), in(5, pb(2)), in(6, pb(3));
+        in(7, row.sign[2] * v2), in(8, cst(0)), in(9, cst(1));
         break;
     case 7:  // TwoFixedLinesFreePoint
-        in(0, pa[0]), in(1, pa[1]), in(2, pa[2]), in(3, pa[3]), in(4, row.sign[1] * v1);
-        in(5, pb[0]), in(6, pb[1]), in(7, pb[2]), in(8, pb[3]), in(9, row.sign[2] * v2);
-        in(10, cst[0]), in(11, cst[1]);
+        in(0, pa(0)), in(1, pa(1)), in(2, pa(2)), in(3, pa(3)), in(4, row.sign[1] * v1);
+        in(5, pb(0)), in(6, pb(1)), in(7, pb(2)), in(8, pb(3)), in(9, row.sign[2] * v2);
+        in(10, cst(0)), in(11, cst(1));
         break;
     case 3: {  // ZeroFixedLLPAngleTriangle: line1 -> (x1, 0)-(x2, 0), point -> (0, sign * d(P, line1)); v0 holds cos(angle)
         const double sd1 = row.sign[1] * v1;
-        pa[0] = cst[7], pa[1] = 0.0, pa[2] = cst[8], pa[3] = 0.0;
-        pb[0] = 0.0, pb[1] = sd1;
-        in(0, cst[5]), in(1, cst[6]), in(2, v0), in(3, cst[0]), in(4, cst[1]), in(5, cst[2]), in(6, cst[3]);
-        in(7, 0.0), in(8, sd1), in(9, row.sign[2] * v2), in(10, 0.0), in(11, 0.0), in(12, cst[4]);
+        pa(0) = cst(7), pa(1) = 0.0, pa(2) = cst(8), pa(3) = 0.0;
+        pb(0) = 0.0, pb(1) = sd1;
+        in(0, cst(5)), in(1, cst(6)), in(2, v0), in(3, cst(0)), in(4, cst(1)), in(5, cst(2)), in(6, cst(3));
+        in(7, 0.0), in(8, sd1), in(9, row.sign[2] * v2), in(10, 0.0), in(11, 0.0), in(12, cst(4));
         break;
     }
     case 8: {  // FixedLineAndPointFreeLine: a fixed line, b point; v0 holds cos(angle)
-        const double p1x = pa[0], p1y = pa[1], p2x = pa[2], p2y = pa[3];
-        in(0, p2x - p1x), in(1, p2y - p1y), in(2, v0), in(3, cst[0]), in(4, cst[1]), in(5, cst[2]), in(6, cst[3]);
-        in(7, pb[0]), in(8, pb[1]), in(9, row.sign[2] * v2), in(10, (p1x + p2x) / 2.0), in(11, (p1y + p2y) / 2.0);
-        in(12, cst[4]);
+        const double p1x = pa(0), p1y = pa(1), p2x = pa(2), p2y = pa(3);
+        in(0, p2x - p1x), in(1, p2y - p1y), in(2, v0), in(3, cst(0)), in(4, cst(1)), in(5, cst(2)), in(6, cst(3));
+        in(7, pb(0)), in(8, pb(1)), in(9, row.sign[2] * v2), in(10, (p1x + p2x) / 2.0), in(11, (p1y + p2y) / 2.0);
+        in(12, cst(4));
         break;
     }
     }
 }
 
-__global__ void __launch_bounds__(kThreads) program_scatter_kernel(const WaveArgs w)
+// The transpose of gather_row, for program_adjoint_kernel: from the input-column adjoints kb and the
+// adjoint `anchor` of the anchor coordinate that holds a value (pb.x of solvers 1, 2 holds v0, pb.y
+// of solver 3 holds sign1 * v1; the other anchor coordinates are constants), column adjoints first:
+//   1: v0 = kb3 + pb.x, v1 = kb2, v2 = kb5          4: a = (kb0 kb1), v1 = kb2, b = (kb3 kb4), v2 = kb5
+//   2: v0 = kb2 + pb.x, v1 = s1*kb4, v2 = s2*kb5    5: a = (kb0 kb1), b = (kb2 kb3), v1 = s1*kb4, v2 = s2*kb5
+//   3: v0 = kb2, sd1 = kb8 + pb.y, v1 = s1*sd1, v2 = s2*kb9
+//   6: a = (kb0 kb1), v1 = kb2, b = (kb3 .. kb6), v2 = s2*kb7
+//   7: a = (kb0 .. kb3), v1 = s1*kb4, b = (kb5 .. kb8), v2 = s2*kb9
+//   8: a = (kb10/2.0 - kb0, kb11/2.0 - kb1, kb10/2.0 + kb0, kb11/2.0 + kb1), b = (kb7 kb8), v0 = kb2,
+//      v2 = s2*kb9
+// sa(role, q, x) receives the adjoint of coordinate q of role a (0) or b (1), va(q, x) that of vq.
+// Written out rather than derived from gather_row: the restatement in the test suite pins these
+// addition orders and signed zeros, which a mechanical transpose of the recipe would change in
+// cases 1, 2, 3 and 8.
+template <class SA, class VA>
+__device__ __forceinline__ void gather_row_transpose(const gcs_b200_program_row& row, const double* kb, double anchor, SA&& sa, VA&& va)
 {
-    Where at;
-    if (!locate(w, at)) return;
-    const gcs_b200_program_row& row = w.rows[at.r];
-    const int kind = at.k + 1;
-    const int nin = kind == 1 ? 6 : kind == 2 ? 9 : kind == 3 ? 10 : kind == 4 ? 12 : 13;
-    const int nout = (kind == GCS_KIND_SDD || kind == GCS_KIND_ANG) ? 4 : 2;
-    const double* const c = w.cols[at.k];
-    const long long cap = w.cap[at.k], i = at.i;
-    double* const dst = w.pos + at.j * w.n_slots * 4 + 4 * (long long)row.elem[2];
-    for (int q = 0; q < nout; ++q) dst[q] = c[(nin + q) * cap + i];
-    if (w.nonconverged) {
-        const long long n = (w.seg[at.k + 1] - w.seg[at.k]) * w.K;
-        const unsigned root = w.root[at.k][i];
-        if (root >= 2 || !w.conv[at.k][root * n + i]) atomicAdd(w.nonconverged + at.j, 1u);
-    }
-}
-
-// the row's unknown at the chosen root: the output point (K1, K3, K4) or the chosen seed's normal
-// (K2, K5; candidate planes [2][2][n])
-template <int KIND>
-__device__ __forceinline__ void row_tangent(const WaveArgs& w, const Where& at, unsigned root, long long n, const double* kd, double dout[4])
-{
-    constexpr int nin = gcsk::Sys<KIND>::kCols;
-    const double* const c = w.cols[at.k];
-    const long long cap = w.cap[at.k];
-    double k[nin];
-#pragma unroll
-    for (int q = 0; q < nin; ++q) k[q] = c[q * cap + at.i];
-    double ux, uy;
-    if constexpr (KIND == GCS_KIND_SDD || KIND == GCS_KIND_ANG) {
-        ux = w.cand[at.k][(root * 2 + 0) * n + at.i], uy = w.cand[at.k][(root * 2 + 1) * n + at.i];
-    } else {
-        ux = c[nin * cap + at.i], uy = c[(nin + 1) * cap + at.i];
-    }
-    gcsk::RowTangent<KIND> lin;
-    lin.init(k, ux, uy);
-    lin.apply(kd, dout);
-}
-
-__global__ void __launch_bounds__(kThreads) program_tangent_kernel(const WaveArgs w)
-{
-    const long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (g >= w.seg[kKinds] * w.K * w.T) return;
-    const long long T = w.T, s = g / T;
-    Where at;
-    place(w, s, at);
-    const gcs_b200_program_row& row = w.rows[at.r];
-    double* const dpos = w.dpos + at.j * w.n_slots * 4 * T + (g - s * T);
-    const double* const dval = w.dval + at.j * w.n_values * T + (g - s * T);
-    auto dp = [&](int slot, int q) -> double& { return dpos[(4 * (long long)slot + q) * T]; };
-    const int a = row.elem[0], b = row.elem[1];
-    const double v0 = row.value[0] >= 0 ? dval[row.value[0] * T] : 0.0;
-    const double v1 = row.value[1] >= 0 ? dval[row.value[1] * T] : 0.0;
-    const double v2 = row.value[2] >= 0 ? dval[row.value[2] * T] : 0.0;
-    // the gather's tangent: input-column tangents, and the zero-fixed anchors' tangents
-    double kd[13] = {};
-    switch (row.solver) {
-    case 1:
-        dp(a, 0) = 0.0, dp(a, 1) = 0.0, dp(b, 0) = v0, dp(b, 1) = 0.0;
-        kd[2] = v1, kd[3] = v0, kd[5] = v2;
-        break;
-    case 4:
-        kd[0] = dp(a, 0), kd[1] = dp(a, 1), kd[2] = v1, kd[3] = dp(b, 0), kd[4] = dp(b, 1), kd[5] = v2;
-        break;
-    case 2:
-        dp(a, 0) = 0.0, dp(a, 1) = 0.0, dp(b, 0) = v0, dp(b, 1) = 0.0;
-        kd[2] = v0, kd[4] = row.sign[1] * v1, kd[5] = row.sign[2] * v2;
-        break;
-    case 5:
-        kd[0] = dp(a, 0), kd[1] = dp(a, 1), kd[2] = dp(b, 0), kd[3] = dp(b, 1);
-        kd[4] = row.sign[1] * v1, kd[5] = row.sign[2] * v2;
-        break;
-    case 6:
-        kd[0] = dp(a, 0), kd[1] = dp(a, 1), kd[2] = v1, kd[3] = dp(b, 0), kd[4] = dp(b, 1), kd[5] = dp(b, 2), kd[6] = dp(b, 3);
-        kd[7] = row.sign[2] * v2;
-        break;
-    case 7:
-        kd[0] = dp(a, 0), kd[1] = dp(a, 1), kd[2] = dp(a, 2), kd[3] = dp(a, 3), kd[4] = row.sign[1] * v1;
-        kd[5] = dp(b, 0), kd[6] = dp(b, 1), kd[7] = dp(b, 2), kd[8] = dp(b, 3), kd[9] = row.sign[2] * v2;
-        break;
-    case 3: {
-        const double sd1 = row.sign[1] * v1;
-        dp(a, 0) = 0.0, dp(a, 1) = 0.0, dp(a, 2) = 0.0, dp(a, 3) = 0.0, dp(b, 0) = 0.0, dp(b, 1) = sd1;
-        kd[2] = v0, kd[8] = sd1, kd[9] = row.sign[2] * v2;
-        break;
-    }
-    case 8: {
-        const double p1x = dp(a, 0), p1y = dp(a, 1), p2x = dp(a, 2), p2y = dp(a, 3);
-        kd[0] = p2x - p1x, kd[1] = p2y - p1y, kd[2] = v0, kd[7] = dp(b, 0), kd[8] = dp(b, 1), kd[9] = row.sign[2] * v2;
-        kd[10] = (p1x + p2x) / 2.0, kd[11] = (p1y + p2y) / 2.0;
-        break;
-    }
-    }
-    const int kind = at.k + 1;
-    const int nout = (kind == GCS_KIND_SDD || kind == GCS_KIND_ANG) ? 4 : 2;
-    const long long n = (w.seg[at.k + 1] - w.seg[at.k]) * w.K;
-    const unsigned root = w.root[at.k][at.i];
-    double out[4];
-    if (root >= 2 || !w.conv[at.k][root * n + at.i]) {
-        // the scatter's test: not a root, so the implicit function theorem does not apply
-        out[0] = out[1] = out[2] = out[3] = __longlong_as_double(0x7ff8000000000000LL);
-    } else {
-        switch (kind) {
-        case GCS_KIND_PP: row_tangent<GCS_KIND_PP>(w, at, root, n, kd, out); break;
-        case GCS_KIND_SDD: row_tangent<GCS_KIND_SDD>(w, at, root, n, kd, out); break;
-        case GCS_KIND_PPL: row_tangent<GCS_KIND_PPL>(w, at, root, n, kd, out); break;
-        case GCS_KIND_PLL: row_tangent<GCS_KIND_PLL>(w, at, root, n, kd, out); break;
-        default: row_tangent<GCS_KIND_ANG>(w, at, root, n, kd, out); break;
-        }
-    }
-    for (int q = 0; q < nout; ++q) dp(row.elem[2], q) = out[q];
-}
-
-// input-column adjoints kb of a converged row for its output adjoints ob (csrc/newton_adjoint.cuh)
-template <int KIND>
-__device__ __forceinline__ void row_adjoint_at(const WaveArgs& w, const Where& at, unsigned root, long long n, const double ob[4], double* kb)
-{
-    constexpr int nin = gcsk::Sys<KIND>::kCols;
-    const double* const c = w.cols[at.k];
-    const long long cap = w.cap[at.k];
-    double k[nin];
-#pragma unroll
-    for (int q = 0; q < nin; ++q) k[q] = c[q * cap + at.i];
-    double ux, uy;
-    if constexpr (KIND == GCS_KIND_SDD || KIND == GCS_KIND_ANG) {
-        ux = w.cand[at.k][(root * 2 + 0) * n + at.i], uy = w.cand[at.k][(root * 2 + 1) * n + at.i];
-    } else {
-        ux = c[nin * cap + at.i], uy = c[(nin + 1) * cap + at.i];
-    }
-    gcsk::RowTangent<KIND> lin;
-    lin.init(k, ux, uy);
-    gcsk::row_adjoint<KIND>(lin, ob, kb);
-}
-
-// One wave of the adjoint sweep, over the batches a recorded run kept.  The transpose of the
-// scatter, the row's linearisation and the gather of program_tangent_kernel, in reverse:
-//   1. ob = the adjoints of the target's written coordinates, which are then zeroed; for solvers
-//      1-3 also the anchors the gather wrote (all zeroed; pb.x of solvers 1, 2 holds v0, pb.y of
-//      solver 3 holds sign1 * v1, the rest are constants);
-//   2. a row whose chosen run did not converge has no derivative: a non-zero (or NaN) ob sets the
-//      (instance, cotangent) flag and the row contributes kb = 0; otherwise kb = row_adjoint(ob);
-//   3. the gather's transpose, column adjoints first, then the anchor's:
-//      1: v0 = kb3 + pb.x, v1 = kb2, v2 = kb5          4: a = (kb0 kb1), v1 = kb2, b = (kb3 kb4), v2 = kb5
-//      2: v0 = kb2 + pb.x, v1 = s1*kb4, v2 = s2*kb5    5: a = (kb0 kb1), b = (kb2 kb3), v1 = s1*kb4, v2 = s2*kb5
-//      3: v0 = kb2, sd1 = kb8 + pb.y, v1 = s1*sd1, v2 = s2*kb9
-//      6: a = (kb0 kb1), v1 = kb2, b = (kb3 .. kb6), v2 = s2*kb7
-//      7: a = (kb0 .. kb3), v1 = s1*kb4, b = (kb5 .. kb8), v2 = s2*kb9
-//      8: a = (kb10/2.0 - kb0, kb11/2.0 - kb1, kb10/2.0 + kb0, kb11/2.0 + kb1), b = (kb7 kb8), v0 = kb2,
-//         v2 = s2*kb9
-//   written to the contribution buffer (program_adjoint_reduce_kernel adds them up).
-__global__ void __launch_bounds__(kThreads) program_adjoint_kernel(const WaveArgs w)
-{
-    const long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (g >= w.seg[kKinds] * w.K * w.T) return;
-    const long long T = w.T, KT = w.K * T, s = g / T, t = g - s * T;
-    Where at;
-    place(w, s, at);
-    const gcs_b200_program_row& row = w.rows[at.r];
-    double* const apos = w.apos + at.j * w.n_slots * 4 * T + t;
-    auto ap = [&](int slot, int q) -> double& { return apos[(4 * (long long)slot + q) * T]; };
-    const int a = row.elem[0], b = row.elem[1], tgt = row.elem[2];
-    const int kind = at.k + 1;
-    const int nout = (kind == GCS_KIND_SDD || kind == GCS_KIND_ANG) ? 4 : 2;
-    double ob[4] = {};
-    for (int q = 0; q < nout; ++q) ob[q] = ap(tgt, q), ap(tgt, q) = 0.0;
-    double anchor = 0.0;
-    if (row.solver <= 3) {
-        anchor = row.solver == 3 ? ap(b, 1) : ap(b, 0);
-        for (int q = 0; q < (row.solver == 3 ? 4 : 2); ++q) ap(a, q) = 0.0;
-        ap(b, 0) = 0.0, ap(b, 1) = 0.0;
-    }
-    const long long n = (w.seg[at.k + 1] - w.seg[at.k]) * w.K;
-    const unsigned root = w.root[at.k][at.i];
-    double kb[13] = {};
-    if (root >= 2 || !w.conv[at.k][root * n + at.i]) {
-        bool touched = false;
-        for (int q = 0; q < nout; ++q) touched |= !(ob[q] == 0.0);
-        if (touched) w.flag[at.j * T + t] = 1;
-    } else {
-        switch (kind) {
-        case GCS_KIND_PP: row_adjoint_at<GCS_KIND_PP>(w, at, root, n, ob, kb); break;
-        case GCS_KIND_SDD: row_adjoint_at<GCS_KIND_SDD>(w, at, root, n, ob, kb); break;
-        case GCS_KIND_PPL: row_adjoint_at<GCS_KIND_PPL>(w, at, root, n, ob, kb); break;
-        case GCS_KIND_PLL: row_adjoint_at<GCS_KIND_PLL>(w, at, root, n, ob, kb); break;
-        default: row_adjoint_at<GCS_KIND_ANG>(w, at, root, n, ob, kb); break;
-        }
-    }
-    const long long jt = at.j * T + t;
-    double* const sc = w.scon + at.r * 8 * KT + jt;  // [role][coordinate]
-    double* const vc = w.vcon + at.r * 3 * KT + jt;  // [q]
-    auto sa = [&](int role, int q, double v) { sc[(role * 4 + q) * KT] = v; };
-    auto va = [&](int q, double v) { vc[q * KT] = v; };
     const double s1 = row.sign[1], s2 = row.sign[2];
     switch (row.solver) {
     case 1: va(0, kb[3] + anchor), va(1, kb[2]), va(2, kb[5]); break;
@@ -406,6 +263,175 @@ __global__ void __launch_bounds__(kThreads) program_adjoint_kernel(const WaveArg
     }
 }
 
+// value vq of a row, from a table whose entries are `stride` doubles apart (0 where it reads none)
+__device__ __forceinline__ double row_value(const gcs_b200_program_row& row, int q, const double* val, long long stride)
+{
+    return row.value[q] >= 0 ? val[row.value[q] * stride] : 0.0;
+}
+
+// gather_row's two sides.  Both take what the row reads (its slots a, b and v0 .. v2) once, before
+// the switch: with the accessors reading row.elem / row.value at every use, the compiler reloads
+// them, and the gather kernel takes a quarter more instructions.
+struct GatherColumns {  // instance j: anchors into its positions, columns into the kind batch
+    double* pa;
+    double* pb;
+    double v[3];
+    const double* canvas;
+    double* cols;
+    long long cap, i;
+    __device__ __forceinline__ double& slot(int role, int q) { return (role ? pb : pa)[q]; }
+    __device__ __forceinline__ double value(int q) const { return v[q]; }
+    __device__ __forceinline__ double cst(int c) const { return canvas[c]; }
+    __device__ __forceinline__ void in(int col, double x) { cols[col * cap + i] = x; }
+};
+
+struct GatherTangents {  // their tangents along one direction, coordinates T apart; columns into kd
+    double* pa;
+    double* pb;
+    double v[3];
+    long long T;
+    double kd[13];
+    __device__ __forceinline__ double& slot(int role, int q) { return (role ? pb : pa)[q * T]; }
+    __device__ __forceinline__ double value(int q) const { return v[q]; }
+    __device__ __forceinline__ double cst(int) const { return 0.0; }
+    __device__ __forceinline__ void in(int col, double x) { kd[col] = x; }
+};
+
+__global__ void __launch_bounds__(kThreads) program_gather_kernel(const WaveArgs w)
+{
+    Where at;
+    if (!locate(w, at)) return;
+    const gcs_b200_program_row& row = w.rows[at.r];
+    double* const pos = w.pos + at.j * w.n_slots * 4;
+    const double* const val = w.val + at.j * w.n_values;
+    GatherColumns s { pos + 4 * (long long)row.elem[0], pos + 4 * (long long)row.elem[1],
+        { row_value(row, 0, val, 1), row_value(row, 1, val, 1), row_value(row, 2, val, 1) }, row.canvas, w.cols[at.k],
+        w.cap[at.k], at.i };
+    w.code[at.k][at.i] = (uint8_t)row.code;
+    gather_row(row, s);
+}
+
+// The scatter's test: the row's chosen run converged, so its output is a root.  Also gives the
+// chosen seed and n, the kind's sub-systems in the launch.
+__device__ __forceinline__ bool chosen_root(const WaveArgs& w, const Where& at, unsigned& root, long long& n)
+{
+    n = (w.seg[at.k + 1] - w.seg[at.k]) * w.K;
+    root = w.root[at.k][at.i];
+    if (root >= 2) return false;
+    return w.conv[at.k][root * n + at.i] != 0;
+}
+
+__global__ void __launch_bounds__(kThreads) program_scatter_kernel(const WaveArgs w)
+{
+    Where at;
+    if (!locate(w, at)) return;
+    const gcs_b200_program_row& row = w.rows[at.r];
+    const int nin = in_cols(at.k + 1), nout = out_cols(at.k + 1);
+    const double* const c = w.cols[at.k];
+    const long long cap = w.cap[at.k], i = at.i;
+    double* const dst = w.pos + at.j * w.n_slots * 4 + 4 * (long long)row.elem[2];
+    for (int q = 0; q < nout; ++q) dst[q] = c[(nin + q) * cap + i];
+    unsigned root;
+    long long n;
+    if (w.nonconverged && !chosen_root(w, at, root, n)) atomicAdd(w.nonconverged + at.j, 1u);
+}
+
+// The linearisation of a converged row at its chosen root (chosen_root): its input columns, and the
+// unknown there, the output point (K1, K3, K4) or the chosen seed's normal (K2, K5; candidate planes
+// [2][2][n]).
+template <int KIND>
+__device__ __forceinline__ gcsk::RowTangent<KIND> linearisation(std::integral_constant<int, KIND>, const WaveArgs& w, const Where& at,
+    unsigned root, long long n)
+{
+    constexpr int nin = gcsk::Sys<KIND>::kCols;
+    const double* const c = w.cols[at.k];
+    const long long cap = w.cap[at.k];
+    double k[nin];
+#pragma unroll
+    for (int q = 0; q < nin; ++q) k[q] = c[q * cap + at.i];
+    double ux, uy;
+    if constexpr (KIND == GCS_KIND_SDD || KIND == GCS_KIND_ANG) {
+        ux = w.cand[at.k][(root * 2 + 0) * n + at.i], uy = w.cand[at.k][(root * 2 + 1) * n + at.i];
+    } else {
+        ux = c[nin * cap + at.i], uy = c[(nin + 1) * cap + at.i];
+    }
+    gcsk::RowTangent<KIND> lin;
+    lin.init(k, ux, uy);
+    return lin;
+}
+
+__global__ void __launch_bounds__(kThreads) program_tangent_kernel(const WaveArgs w)
+{
+    const long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (g >= w.seg[kKinds] * w.K * w.T) return;
+    const long long T = w.T, s = g / T;
+    Where at;
+    place(w, s, at);
+    const gcs_b200_program_row& row = w.rows[at.r];
+    double* const dpos = w.dpos + at.j * w.n_slots * 4 * T + (g - s * T);
+    const double* const dval = w.dval + at.j * w.n_values * T + (g - s * T);
+    GatherTangents d { dpos + 4 * (long long)row.elem[0] * T, dpos + 4 * (long long)row.elem[1] * T,
+        { row_value(row, 0, dval, T), row_value(row, 1, dval, T), row_value(row, 2, dval, T) }, T, {} };
+    gather_row(row, d);
+    const int kind = at.k + 1;
+    unsigned root;
+    long long n;
+    double out[4];
+    if (!chosen_root(w, at, root, n)) {
+        // not a root, so the implicit function theorem does not apply
+        out[0] = out[1] = out[2] = out[3] = __longlong_as_double(0x7ff8000000000000LL);
+    } else {
+        with_kind(kind, [&](auto K) { linearisation(K, w, at, root, n).apply(d.kd, out); });
+    }
+    double* const dst = dpos + 4 * (long long)row.elem[2] * T;
+    for (int q = 0; q < out_cols(kind); ++q) dst[q * T] = out[q];
+}
+
+// One wave of the adjoint sweep, over the batches a recorded run kept.  The transpose of the
+// scatter, the row's linearisation and the gather of program_tangent_kernel, in reverse:
+//   1. ob = the adjoints of the target's written coordinates, which are then zeroed; for solvers
+//      1-3 also the anchors the gather wrote (all zeroed, the one that holds a value kept);
+//   2. a row whose chosen run did not converge has no derivative: a non-zero (or NaN) ob sets the
+//      (instance, cotangent) flag and the row contributes kb = 0; otherwise kb = row_adjoint(ob);
+//   3. gather_row_transpose, written to the contribution buffer (program_adjoint_reduce_kernel
+//      adds them up).
+__global__ void __launch_bounds__(kThreads) program_adjoint_kernel(const WaveArgs w)
+{
+    const long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (g >= w.seg[kKinds] * w.K * w.T) return;
+    const long long T = w.T, KT = w.K * T, s = g / T, t = g - s * T;
+    Where at;
+    place(w, s, at);
+    const gcs_b200_program_row& row = w.rows[at.r];
+    double* const apos = w.apos + at.j * w.n_slots * 4 * T + t;
+    auto ap = [&](int slot, int q) -> double& { return apos[(4 * (long long)slot + q) * T]; };
+    const int a = row.elem[0], b = row.elem[1], tgt = row.elem[2];
+    const int kind = at.k + 1, nout = out_cols(kind);
+    double ob[4] = {};
+    for (int q = 0; q < nout; ++q) ob[q] = ap(tgt, q), ap(tgt, q) = 0.0;
+    double anchor = 0.0;
+    if (row.solver <= 3) {
+        anchor = row.solver == 3 ? ap(b, 1) : ap(b, 0);
+        for (int q = 0; q < (row.solver == 3 ? 4 : 2); ++q) ap(a, q) = 0.0;
+        ap(b, 0) = 0.0, ap(b, 1) = 0.0;
+    }
+    unsigned root;
+    long long n;
+    double kb[13] = {};
+    if (!chosen_root(w, at, root, n)) {
+        bool touched = false;
+        for (int q = 0; q < nout; ++q) touched |= !(ob[q] == 0.0);
+        if (touched) w.flag[at.j * T + t] = 1;
+    } else {
+        with_kind(kind, [&](auto K) { gcsk::row_adjoint(linearisation(K, w, at, root, n), ob, kb); });
+    }
+    const long long jt = at.j * T + t;
+    double* const sc = w.scon + at.r * 8 * KT + jt;  // [role][coordinate]
+    double* const vc = w.vcon + at.r * 3 * KT + jt;  // [q]
+    gather_row_transpose(row, kb, anchor, [&](int role, int q, double v) { sc[(role * 4 + q) * KT] = v; },
+        [&](int q, double v) { vc[q * KT] = v; });
+}
+
 // reader lists of one wave: slot entries first (target slot, coordinates read), then value entries
 struct AdjEntry {
     int32_t target;
@@ -422,6 +448,7 @@ struct ReduceArgs {
     const double* scon;
     const double* vcon;
     long long n_slots, n_values;
+    const uint8_t* flag;        // [K][T] of the sweep (program_adjoint_flag_kernel)
 };
 
 // one thread per (entry, instance, cotangent): the entry's contributions added to its table entry
@@ -450,12 +477,12 @@ __global__ void __launch_bounds__(kThreads) program_adjoint_reduce_kernel(const 
 }
 
 // the NaN rule, after wave 0: adj_values[k][:][t] = NaN where the (k, t) flag is set
-__global__ void __launch_bounds__(kThreads) program_adjoint_flag_kernel(double* aval, const uint8_t* flag, long long K, long long n_values, long long T)
+__global__ void __launch_bounds__(kThreads) program_adjoint_flag_kernel(const ReduceArgs r)
 {
     const long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (g >= K * n_values * T) return;
-    const long long j = g / (n_values * T), t = g % T;
-    if (flag[j * T + t]) aval[g] = __longlong_as_double(0x7ff8000000000000LL);
+    if (g >= r.K * r.n_values * r.T) return;
+    const long long j = g / (r.n_values * r.T), t = g % r.T;
+    if (r.flag[j * r.T + t]) r.aval[g] = __longlong_as_double(0x7ff8000000000000LL);
 }
 
 int validate_desc(const gcs_b200_program_desc* d)
@@ -529,6 +556,38 @@ int validate_desc(const gcs_b200_program_desc* d)
     return GCS_OK;
 }
 
+// A device buffer that only grows.
+template <class T>
+struct DeviceBuffer {
+    T* ptr = nullptr;
+    size_t bytes = 0;  // allocated
+
+    // device current; makes the buffer at least `need` bytes long.  The old buffer is freed once
+    // `st`, whose work in flight may still use it, is done.  A failed allocation leaves the buffer
+    // empty and fails with GCS_E_NOMEM, naming what the buffer is for (`what`, printf-style).
+    int grow(size_t need, cudaStream_t st, const char* what, ...)
+    {
+        if (need <= bytes) return GCS_OK;
+        if (ptr) {
+            PROG_TRY(cudaStreamSynchronize(st));
+            PROG_TRY(cudaFree(ptr));
+            ptr = nullptr, bytes = 0;
+        }
+        if (cudaMalloc(&ptr, need) != cudaSuccess) {
+            cudaGetLastError();
+            ptr = nullptr;
+            char buf[300];
+            va_list ap;
+            va_start(ap, what);
+            vsnprintf(buf, sizeof(buf), what, ap);
+            va_end(ap);
+            return failf(GCS_E_NOMEM, "cudaMalloc(%zu) for %s failed", need, buf);
+        }
+        bytes = need;
+        return GCS_OK;
+    }
+};
+
 }  // namespace
 
 struct gcs_b200_program {
@@ -539,19 +598,14 @@ struct gcs_b200_program {
     long long max_rows[kKinds] = {};  // most rows of a kind in one wave
     gcs_b200_program_row* rows = nullptr;
     double* initial = nullptr;
-    cudaStream_t stream = nullptr;  // uploads and gcs_b200_program_run_host
-    // kind batches
-    unsigned char* scratch = nullptr;
-    size_t scratch_bytes = 0;
-    // tables of gcs_b200_program_run_host, sized for `tables_k` instances
-    double* values = nullptr;
-    double* positions = nullptr;
-    uint32_t* counts = nullptr;
-    long long tables_k = 0;
-    // tangent tables of gcs_b200_program_run_tangents_host, sized for `tangents_kt` instances x directions
-    double* dvalues = nullptr;
-    double* dpositions = nullptr;
-    long long tangents_kt = 0;
+    cudaStream_t stream = nullptr;  // uploads and the _host entry points
+    // the kind batches of plain and tangent runs, reused by every wave
+    DeviceBuffer<unsigned char> scratch;
+    // tables of the _host entry points: gcs_b200_program_run_host, and the tangent tables of
+    // gcs_b200_program_run_tangents_host
+    DeviceBuffer<double> values, positions;
+    DeviceBuffer<uint32_t> counts;
+    DeviceBuffer<double> dvalues, dpositions;
     // reader lists of the adjoint sweep, built at create time: the entries of wave w are
     // [ent_off[w], ent_off[w+1]) of `ent` (slot entries, then value entries), the readers of entry e
     // are readers[begin[e] .. begin[e+1])
@@ -561,15 +615,13 @@ struct gcs_b200_program {
     long long* readers = nullptr;
     long long max_wave_rows = 0;
     // the tape of the last recorded run (every wave's kind batches) and its instance count (0: none)
-    unsigned char* tape = nullptr;
-    size_t tape_bytes = 0;
+    DeviceBuffer<unsigned char> tape;
     long long recorded_k = 0;
-    // working tables of the sweep, sized for `adj_kt` instances x cotangents
-    double* apos = nullptr;       // [K][n_slots][4][T]
-    double* contrib = nullptr;    // [max_wave_rows][11][K][T]: slot, then value contributions
-    uint8_t* flags = nullptr;     // [K][T]
-    double* avalues = nullptr;    // [K][n_values][T] of gcs_b200_program_adjoints_host
-    long long adj_kt = 0;
+    // working tables of the sweep
+    DeviceBuffer<double> apos;     // [K][n_slots][4][T]
+    DeviceBuffer<double> contrib;  // [max_wave_rows][11][K][T]: slot, then value contributions
+    DeviceBuffer<uint8_t> flags;   // [K][T]
+    DeviceBuffer<double> avalues;  // [K][n_values][T] of gcs_b200_program_adjoints_host
     cudaEvent_t ev[4] = {};
 };
 
@@ -587,27 +639,16 @@ bool has_cand(int kind, bool tangents) { return tangents && (kind == GCS_KIND_SD
 // and K5) the candidate planes
 size_t kind_bytes(int kind, long long cap, bool tangents)
 {
-    return align256((size_t)(kInCols[kind] + kOutCols[kind]) * cap * sizeof(double)) + 4 * align256((size_t)cap)
+    return align256((size_t)(in_cols(kind) + out_cols(kind)) * cap * sizeof(double)) + 4 * align256((size_t)cap)
         + (has_cand(kind, tangents) ? align256((size_t)4 * cap * sizeof(double)) : 0);
 }
 
-// device current; makes the kind batches hold K instances of the largest wave
-int ensure_scratch(gcs_b200_program* p, long long K, bool tangents, cudaStream_t st)
+// the kind batches with `cap[k]` sub-systems of kind k + 1
+size_t batches_bytes(const long long cap[kKinds], bool cand)
 {
     size_t bytes = 0;
-    for (int k = 1; k <= kKinds; ++k) bytes += kind_bytes(k, kind_cap(p, k, K), tangents);
-    if (bytes <= p->scratch_bytes) return GCS_OK;
-    if (p->scratch) {
-        PROG_TRY(cudaStreamSynchronize(st));  // a run still in flight may use them
-        PROG_TRY(cudaFree(p->scratch));
-        p->scratch = nullptr, p->scratch_bytes = 0;
-    }
-    if (cudaMalloc(&p->scratch, bytes) != cudaSuccess) {
-        cudaGetLastError();
-        return failf(GCS_E_NOMEM, "cudaMalloc(%zu) for the kind batches of %lld instances failed", bytes, K);
-    }
-    p->scratch_bytes = bytes;
-    return GCS_OK;
+    for (int k = 1; k <= kKinds; ++k) bytes += kind_bytes(k, cap[k - 1], cand);
+    return bytes;
 }
 
 struct CurrentDevice {
@@ -624,20 +665,17 @@ struct CurrentDevice {
 };
 
 // the kind batches of one wave (or of the scratch) laid out from `at` with `cap[k]` sub-systems of
-// kind k + 1; returns the bytes they take
-size_t bind_batches(WaveArgs& w, unsigned char* at, const long long cap[kKinds], bool cand)
+// kind k + 1
+void bind_batches(WaveArgs& w, unsigned char* at, const long long cap[kKinds], bool cand)
 {
-    size_t used = 0;
     for (int k = 1; k <= kKinds; ++k) {
-        unsigned char* const base = at + used;
-        w.cols[k - 1] = reinterpret_cast<double*>(base);
+        w.cols[k - 1] = reinterpret_cast<double*>(at);
         w.cap[k - 1] = cap[k - 1];
-        unsigned char* flags = base + align256((size_t)(kInCols[k] + kOutCols[k]) * cap[k - 1] * sizeof(double));
+        unsigned char* flags = at + align256((size_t)(in_cols(k) + out_cols(k)) * cap[k - 1] * sizeof(double));
         w.code[k - 1] = flags, w.root[k - 1] = flags + align256((size_t)cap[k - 1]), w.conv[k - 1] = flags + 2 * align256((size_t)cap[k - 1]);
         w.cand[k - 1] = has_cand(k, cand) ? reinterpret_cast<double*>(flags + 4 * align256((size_t)cap[k - 1])) : nullptr;
-        used += kind_bytes(k, cap[k - 1], cand);
+        at += kind_bytes(k, cap[k - 1], cand);
     }
-    return used;
 }
 
 // the tape's sub-system counts of wave `wave`: the wave's own rows x K, in multiples of 32
@@ -647,32 +685,51 @@ void tape_caps(const gcs_b200_program* p, int wave, long long K, long long cap[k
     for (int k = 0; k < kKinds; ++k) cap[k] = ((off[k + 1] - off[k]) * K + 31) / 32 * 32;
 }
 
-size_t tape_bytes(const gcs_b200_program* p, long long K)
+// The tape of a recorded run of K instances: the byte offset of every wave's kind batches (candidate
+// planes included), then the tape's size.
+std::vector<size_t> tape_layout(const gcs_b200_program* p, long long K)
 {
-    size_t bytes = 0;
+    std::vector<size_t> at(1, 0);
     for (int wave = 0; wave < p->n_waves; ++wave) {
         long long cap[kKinds];
         tape_caps(p, wave, K, cap);
-        for (int k = 1; k <= kKinds; ++k) bytes += kind_bytes(k, cap[k - 1], true);
+        at.push_back(at.back() + batches_bytes(cap, true));
     }
-    return bytes;
+    return at;
 }
 
-// device current; makes the tape hold every wave's batches for K instances
-int ensure_tape(gcs_b200_program* p, long long K, cudaStream_t st)
+// w's rows and segments for wave `wave`; with a tape layout (tape_layout of w.K), also its batches
+// on the tape
+void bind_wave(const gcs_b200_program* p, WaveArgs& w, int wave, const std::vector<size_t>* tape_at = nullptr)
 {
-    const size_t bytes = tape_bytes(p, K);
-    if (bytes <= p->tape_bytes) return GCS_OK;
-    if (p->tape) {
-        PROG_TRY(cudaStreamSynchronize(st));  // a sweep still in flight may read it
-        PROG_TRY(cudaFree(p->tape));
-        p->tape = nullptr, p->tape_bytes = 0;
+    const long long* off = p->offsets.data() + (size_t)wave * kKinds;
+    w.rows = p->rows + off[0];
+    for (int k = 0; k <= kKinds; ++k) w.seg[k] = off[k] - off[0];
+    if (tape_at) {
+        long long cap[kKinds];
+        tape_caps(p, wave, w.K, cap);
+        bind_batches(w, p->tape.ptr + (*tape_at)[(size_t)wave], cap, true);
     }
-    if (cudaMalloc(&p->tape, bytes) != cudaSuccess) {
-        cudaGetLastError();
-        return failf(GCS_E_NOMEM, "cudaMalloc(%zu) for the tape of a recorded run of %lld instances failed", bytes, K);
+}
+
+// Launches `kernel` on `st` over `threads` threads (nothing when there are none) and counts the
+// launch.  A grid beyond 31 bits fails, naming the work (`what`, printf-style).
+template <class A>
+int launch(void (*kernel)(A), long long threads, cudaStream_t st, const A& args, const char* what, ...)
+{
+    if (threads == 0) return GCS_OK;
+    const long long grid = (threads + kThreads - 1) / kThreads;
+    if (grid > 0x7fffffffLL) {
+        char buf[300];
+        va_list ap;
+        va_start(ap, what);
+        vsnprintf(buf, sizeof(buf), what, ap);
+        va_end(ap);
+        return failf(GCS_E_INVALID, "%s are too many for one launch", buf);
     }
-    p->tape_bytes = bytes;
+    kernel<<<(unsigned)grid, kThreads, 0, st>>>(args);
+    gcsk::api_count_launch();
+    PROG_TRY(cudaGetLastError());
     return GCS_OK;
 }
 
@@ -681,9 +738,24 @@ int ensure_tape(gcs_b200_program* p, long long K, cudaStream_t st)
 int run_on(gcs_b200_program* p, long long K, const double* values, double* positions, uint32_t* nonconverged, int variant,
     cudaStream_t st, long long T = 0, const double* dvalues = nullptr, double* dpositions = nullptr, bool recorded = false)
 {
-    int rc = recorded ? ensure_tape(p, K, st) : ensure_scratch(p, K, T > 0, st);
-    if (rc != GCS_OK) return rc;
-    if (recorded) p->recorded_k = 0;  // until this run is enqueued whole
+    WaveArgs w;
+    memset(&w, 0, sizeof(w));
+    w.K = K;
+    w.pos = positions, w.val = values, w.n_slots = p->n_slots, w.n_values = p->n_values;
+    w.nonconverged = nonconverged;
+    w.T = T, w.dpos = dpositions, w.dval = dvalues;
+    std::vector<size_t> tape_at;
+    if (recorded) {
+        p->recorded_k = 0;  // until this run is enqueued whole
+        tape_at = tape_layout(p, K);
+        PROG_RC(p->tape.grow(tape_at.back(), st, "the tape of a recorded run of %lld instances", K));
+    } else {
+        // K instances of every kind's largest wave
+        long long cap[kKinds];
+        for (int k = 1; k <= kKinds; ++k) cap[k - 1] = kind_cap(p, k, K);
+        PROG_RC(p->scratch.grow(batches_bytes(cap, T > 0), st, "the kind batches of %lld instances", K));
+        bind_batches(w, p->scratch.ptr, cap, T > 0);
+    }
     // every instance starts from the initial positions: one copy, then doubling copies
     const size_t table = (size_t)p->n_slots * 4 * sizeof(double);
     if (table) {
@@ -698,37 +770,11 @@ int run_on(gcs_b200_program* p, long long K, const double* values, double* posit
     if (nonconverged) PROG_TRY(cudaMemsetAsync(nonconverged, 0, (size_t)K * sizeof(uint32_t), st));
     // every slot's tangent is 0 before the first wave: the initial positions are constants
     if (T > 0 && table) PROG_TRY(cudaMemsetAsync(dpositions, 0, (size_t)K * T * table, st));
-    WaveArgs w;
-    memset(&w, 0, sizeof(w));
-    w.K = K;
-    w.pos = positions, w.val = values, w.n_slots = p->n_slots, w.n_values = p->n_values;
-    w.nonconverged = nonconverged;
-    w.T = T, w.dpos = dpositions, w.dval = dvalues;
-    if (!recorded) {
-        long long cap[kKinds];
-        for (int k = 1; k <= kKinds; ++k) cap[k - 1] = kind_cap(p, k, K);
-        bind_batches(w, p->scratch, cap, T > 0);
-    }
-    unsigned char* tape = p->tape;
     for (int wave = 0; wave < p->n_waves; ++wave) {
-        const long long* off = p->offsets.data() + (size_t)wave * kKinds;
-        w.rows = p->rows + off[0];
-        for (int k = 0; k <= kKinds; ++k) w.seg[k] = off[k] - off[0];
-        if (recorded) {
-            long long cap[kKinds];
-            tape_caps(p, wave, K, cap);
-            tape += bind_batches(w, tape, cap, true);
-        }
-        const long long threads = w.seg[kKinds] * K;
-        if (threads == 0) continue;
-        const long long grid = (threads + kThreads - 1) / kThreads;
-        if (grid > 0x7fffffffLL) return failf(GCS_E_INVALID, "wave %d: %lld sub-systems are too many for one launch", wave, threads);
-        const long long tgrid = (threads * T + kThreads - 1) / kThreads;
-        if (tgrid > 0x7fffffffLL)
-            return failf(GCS_E_INVALID, "wave %d: %lld sub-systems x %lld directions are too many for one launch", wave, threads, T);
-        program_gather_kernel<<<(unsigned)grid, kThreads, 0, st>>>(w);
-        gcsk::api_count_launch();
-        PROG_TRY(cudaGetLastError());
+        bind_wave(p, w, wave, recorded ? &tape_at : nullptr);
+        const long long subs = w.seg[kKinds] * K;
+        if (subs == 0) continue;
+        PROG_RC(launch(program_gather_kernel, subs, st, w, "wave %d: %lld sub-systems", wave, subs));
         gcs_b200_batch batch[kKinds];
         const gcs_b200_batch* list[kKinds];
         int count = 0;
@@ -739,21 +785,15 @@ int run_on(gcs_b200_program* p, long long K, const double* values, double* posit
             memset(&b, 0, sizeof(b));
             b.kind = k, b.n_seeds = 2, b.n = n, b.mem = GCS_MEM_DEVICE, b.variant = variant;
             const long long cap = w.cap[k - 1];
-            for (int c = 0; c < kInCols[k]; ++c) b.in[c] = w.cols[k - 1] + c * cap;
-            for (int c = 0; c < kOutCols[k]; ++c) b.out[c] = w.cols[k - 1] + (kInCols[k] + c) * cap;
+            for (int c = 0; c < in_cols(k); ++c) b.in[c] = w.cols[k - 1] + c * cap;
+            for (int c = 0; c < out_cols(k); ++c) b.out[c] = w.cols[k - 1] + (in_cols(k) + c) * cap;
             b.code = w.code[k - 1], b.root_index = w.root[k - 1], b.converged = w.conv[k - 1], b.cand = w.cand[k - 1];
             list[count++] = &b;
         }
-        rc = gcs_b200_solve_many(list, count, p->device, st);
-        if (rc != GCS_OK) return rc;
-        program_scatter_kernel<<<(unsigned)grid, kThreads, 0, st>>>(w);
-        gcsk::api_count_launch();
-        PROG_TRY(cudaGetLastError());
-        if (T > 0) {
-            program_tangent_kernel<<<(unsigned)tgrid, kThreads, 0, st>>>(w);
-            gcsk::api_count_launch();
-            PROG_TRY(cudaGetLastError());
-        }
+        PROG_RC(gcs_b200_solve_many(list, count, p->device, st));
+        PROG_RC(launch(program_scatter_kernel, subs, st, w, "wave %d: %lld sub-systems", wave, subs));
+        if (T > 0)
+            PROG_RC(launch(program_tangent_kernel, subs * T, st, w, "wave %d: %lld sub-systems x %lld directions", wave, subs, T));
     }
     if (recorded) p->recorded_k = K;
     return GCS_OK;
@@ -762,21 +802,14 @@ int run_on(gcs_b200_program* p, long long K, const double* values, double* posit
 // device current; the sweep's working tables for the recorded K x T cotangents
 int ensure_adjoint_tables(gcs_b200_program* p, long long T, cudaStream_t st)
 {
-    const long long KT = p->recorded_k * T;
-    if (KT <= p->adj_kt) return GCS_OK;
-    if (p->apos) PROG_TRY(cudaStreamSynchronize(st));
-    cudaFree(p->apos), cudaFree(p->contrib), cudaFree(p->flags), cudaFree(p->avalues);
-    p->apos = p->contrib = p->avalues = nullptr, p->flags = nullptr, p->adj_kt = 0;
+    const long long K = p->recorded_k, KT = K * T;
     const size_t pbytes = (size_t)KT * p->n_slots * 4 * sizeof(double), cbytes = (size_t)KT * p->max_wave_rows * 11 * sizeof(double);
     const size_t vbytes = (size_t)KT * p->n_values * sizeof(double);
-    if ((pbytes && cudaMalloc(&p->apos, pbytes) != cudaSuccess) || (cbytes && cudaMalloc(&p->contrib, cbytes) != cudaSuccess)
-        || cudaMalloc(&p->flags, (size_t)KT) != cudaSuccess || (vbytes && cudaMalloc(&p->avalues, vbytes) != cudaSuccess)) {
-        cudaGetLastError();
-        return failf(GCS_E_NOMEM, "cudaMalloc for the adjoint tables of %lld instances x %lld cotangents (%zu + %zu + %zu bytes) failed",
-            p->recorded_k, T, pbytes, cbytes, vbytes);
-    }
-    p->adj_kt = KT;
-    return GCS_OK;
+    const char* what = "the %s of %lld instances x %lld cotangents";
+    PROG_RC(p->apos.grow(pbytes, st, what, "slot adjoints", K, T));
+    PROG_RC(p->contrib.grow(cbytes, st, what, "adjoint contributions", K, T));
+    PROG_RC(p->flags.grow((size_t)KT, st, what, "NaN flags", K, T));
+    return p->avalues.grow(vbytes, st, what, "value adjoints", K, T);
 }
 
 // device current, checks done, p->apos holds the cotangents of the recorded run's positions: the
@@ -785,58 +818,30 @@ int sweep_on(gcs_b200_program* p, long long T, double* adj_values, cudaStream_t 
 {
     const long long K = p->recorded_k, KT = K * T;
     if (p->n_values) PROG_TRY(cudaMemsetAsync(adj_values, 0, (size_t)KT * p->n_values * sizeof(double), st));
-    PROG_TRY(cudaMemsetAsync(p->flags, 0, (size_t)KT, st));
-    std::vector<unsigned char*> tape_at((size_t)p->n_waves + 1);
-    tape_at[0] = p->tape;
-    for (int wave = 0; wave < p->n_waves; ++wave) {
-        long long cap[kKinds];
-        tape_caps(p, wave, K, cap);
-        size_t bytes = 0;
-        for (int k = 1; k <= kKinds; ++k) bytes += kind_bytes(k, cap[k - 1], true);
-        tape_at[(size_t)wave + 1] = tape_at[(size_t)wave] + bytes;
-    }
+    PROG_TRY(cudaMemsetAsync(p->flags.ptr, 0, (size_t)KT, st));
+    const std::vector<size_t> tape_at = tape_layout(p, K);
     WaveArgs w;
     memset(&w, 0, sizeof(w));
     w.K = K, w.T = T, w.n_slots = p->n_slots, w.n_values = p->n_values;
-    w.apos = p->apos, w.flag = p->flags;
-    w.scon = p->contrib, w.vcon = p->contrib + (size_t)p->max_wave_rows * 8 * KT;
+    w.apos = p->apos.ptr, w.flag = p->flags.ptr;
+    w.scon = p->contrib.ptr, w.vcon = p->contrib.ptr + (size_t)p->max_wave_rows * 8 * KT;
     ReduceArgs r;
     memset(&r, 0, sizeof(r));
-    r.K = K, r.T = T, r.apos = p->apos, r.aval = adj_values, r.scon = w.scon, r.vcon = w.vcon;
-    r.n_slots = p->n_slots, r.n_values = p->n_values;
+    r.K = K, r.T = T, r.apos = p->apos.ptr, r.aval = adj_values, r.scon = w.scon, r.vcon = w.vcon;
+    r.n_slots = p->n_slots, r.n_values = p->n_values, r.flag = p->flags.ptr;
     for (int wave = p->n_waves - 1; wave >= 0; --wave) {
-        const long long* off = p->offsets.data() + (size_t)wave * kKinds;
-        w.rows = p->rows + off[0];
-        for (int k = 0; k <= kKinds; ++k) w.seg[k] = off[k] - off[0];
-        const long long threads = w.seg[kKinds] * KT;
-        if (threads == 0) continue;
-        long long cap[kKinds];
-        tape_caps(p, wave, K, cap);
-        bind_batches(w, tape_at[(size_t)wave], cap, true);
+        bind_wave(p, w, wave, &tape_at);
+        const long long subs = w.seg[kKinds] * K;
+        if (subs == 0) continue;
         r.ent = p->ent + p->ent_off[(size_t)wave];
         r.begin = p->begin + p->ent_off[(size_t)wave];
         r.readers = p->readers;
         r.n_ent = p->ent_off[(size_t)wave + 1] - p->ent_off[(size_t)wave];
-        const long long grid = (threads + kThreads - 1) / kThreads, rgrid = (r.n_ent * KT + kThreads - 1) / kThreads;
-        if (grid > 0x7fffffffLL || rgrid > 0x7fffffffLL)
-            return failf(GCS_E_INVALID, "wave %d: %lld sub-systems x %lld cotangents are too many for one launch", wave, w.seg[kKinds] * K, T);
-        program_adjoint_kernel<<<(unsigned)grid, kThreads, 0, st>>>(w);
-        gcsk::api_count_launch();
-        PROG_TRY(cudaGetLastError());
-        if (rgrid == 0) continue;
-        program_adjoint_reduce_kernel<<<(unsigned)rgrid, kThreads, 0, st>>>(r);
-        gcsk::api_count_launch();
-        PROG_TRY(cudaGetLastError());
+        const char* what = "wave %d: %lld sub-systems x %lld cotangents";
+        PROG_RC(launch(program_adjoint_kernel, subs * T, st, w, what, wave, subs, T));
+        PROG_RC(launch(program_adjoint_reduce_kernel, r.n_ent * KT, st, r, what, wave, subs, T));
     }
-    const long long nv = KT * p->n_values;
-    if (nv > 0) {
-        const long long grid = (nv + kThreads - 1) / kThreads;
-        if (grid > 0x7fffffffLL) return failf(GCS_E_INVALID, "%lld value adjoints are too many for one launch", nv);
-        program_adjoint_flag_kernel<<<(unsigned)grid, kThreads, 0, st>>>(adj_values, p->flags, K, p->n_values, T);
-        gcsk::api_count_launch();
-        PROG_TRY(cudaGetLastError());
-    }
-    return GCS_OK;
+    return launch(program_adjoint_flag_kernel, KT * p->n_values, st, r, "%lld value adjoints", KT * p->n_values);
 }
 
 // the checks that need no program come first; a null table is refused unless the program has
@@ -872,52 +877,58 @@ int check_tangent_run(const gcs_b200_program* p, long long K, const double* valu
     return check_run(p, K, values, positions, variant);
 }
 
-// device current, checks done
-int run_host(gcs_b200_program* p, long long K, const double* values, double* positions, uint32_t* nonconverged, int variant,
-    float ms[3], long long T, const double* dvalues, double* dpositions, bool recorded = false)
+// one copy of the _host entry points; none when `bytes` is 0
+struct Copy {
+    void* dst;
+    const void* src;
+    size_t bytes;
+};
+
+// Device current, checks done: a _host entry point on the program's stream.  The uploads, work(st),
+// the downloads, then a synchronise; ms[0 .. 2] (unless null) the upload, device and download times.
+template <class Work>
+int on_host(gcs_b200_program* p, std::initializer_list<Copy> up, Work&& work, std::initializer_list<Copy> down, float ms[3])
 {
-    const size_t vbytes = (size_t)K * p->n_values * sizeof(double), pbytes = (size_t)K * p->n_slots * 4 * sizeof(double);
-    if (K > p->tables_k) {
-        PROG_TRY(cudaStreamSynchronize(p->stream));
-        cudaFree(p->values), cudaFree(p->positions), cudaFree(p->counts);
-        p->values = p->positions = nullptr, p->counts = nullptr, p->tables_k = 0;
-        if ((vbytes && cudaMalloc(&p->values, vbytes) != cudaSuccess) || (pbytes && cudaMalloc(&p->positions, pbytes) != cudaSuccess)
-            || cudaMalloc(&p->counts, (size_t)K * sizeof(uint32_t)) != cudaSuccess) {
-            cudaGetLastError();
-            return failf(GCS_E_NOMEM, "cudaMalloc for the tables of %lld instances (%zu + %zu bytes) failed", (long long)K, vbytes, pbytes);
-        }
-        p->tables_k = K;
-    }
-    if (K * T > p->tangents_kt) {
-        PROG_TRY(cudaStreamSynchronize(p->stream));
-        cudaFree(p->dvalues), cudaFree(p->dpositions);
-        p->dvalues = p->dpositions = nullptr, p->tangents_kt = 0;
-        if ((vbytes && cudaMalloc(&p->dvalues, vbytes * T) != cudaSuccess) || (pbytes && cudaMalloc(&p->dpositions, pbytes * T) != cudaSuccess)) {
-            cudaGetLastError();
-            return failf(GCS_E_NOMEM, "cudaMalloc for the tangent tables of %lld instances x %lld directions (%zu + %zu bytes) failed",
-                (long long)K, T, vbytes * T, pbytes * T);
-        }
-        p->tangents_kt = K * T;
-    }
-    cudaStream_t st = p->stream;
+    const cudaStream_t st = p->stream;
     PROG_TRY(cudaEventRecord(p->ev[0], st));
-    if (vbytes) PROG_TRY(cudaMemcpyAsync(p->values, values, vbytes, cudaMemcpyHostToDevice, st));
-    if (T > 0 && vbytes) PROG_TRY(cudaMemcpyAsync(p->dvalues, dvalues, vbytes * T, cudaMemcpyHostToDevice, st));
+    for (const Copy& c : up)
+        if (c.bytes) PROG_TRY(cudaMemcpyAsync(c.dst, c.src, c.bytes, cudaMemcpyHostToDevice, st));
     PROG_TRY(cudaEventRecord(p->ev[1], st));
-    int rc = run_on(p, K, p->values, p->positions, nonconverged ? p->counts : nullptr, variant, st, T, p->dvalues, p->dpositions, recorded);
+    const int rc = work(st);
     if (rc != GCS_OK) {
         cudaStreamSynchronize(st);
         return rc;
     }
     PROG_TRY(cudaEventRecord(p->ev[2], st));
-    if (pbytes) PROG_TRY(cudaMemcpyAsync(positions, p->positions, pbytes, cudaMemcpyDeviceToHost, st));
-    if (T > 0 && pbytes) PROG_TRY(cudaMemcpyAsync(dpositions, p->dpositions, pbytes * T, cudaMemcpyDeviceToHost, st));
-    if (nonconverged) PROG_TRY(cudaMemcpyAsync(nonconverged, p->counts, (size_t)K * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    for (const Copy& c : down)
+        if (c.bytes) PROG_TRY(cudaMemcpyAsync(c.dst, c.src, c.bytes, cudaMemcpyDeviceToHost, st));
     PROG_TRY(cudaEventRecord(p->ev[3], st));
     PROG_TRY(cudaStreamSynchronize(st));
     if (ms)
         for (int q = 0; q < 3; ++q) PROG_TRY(cudaEventElapsedTime(&ms[q], p->ev[q], p->ev[q + 1]));
     return GCS_OK;
+}
+
+// device current, checks done
+int run_host(gcs_b200_program* p, long long K, const double* values, double* positions, uint32_t* nonconverged, int variant,
+    float ms[3], long long T = 0, const double* dvalues = nullptr, double* dpositions = nullptr, bool recorded = false)
+{
+    const size_t vbytes = (size_t)K * p->n_values * sizeof(double), pbytes = (size_t)K * p->n_slots * 4 * sizeof(double);
+    const size_t cbytes = (size_t)K * sizeof(uint32_t);
+    const cudaStream_t st = p->stream;
+    PROG_RC(p->values.grow(vbytes, st, "the values of %lld instances", K));
+    PROG_RC(p->positions.grow(pbytes, st, "the positions of %lld instances", K));
+    PROG_RC(p->counts.grow(cbytes, st, "the nonconverged counts of %lld instances", K));
+    PROG_RC(p->dvalues.grow(vbytes * T, st, "the value tangents of %lld instances x %lld directions", K, T));
+    PROG_RC(p->dpositions.grow(pbytes * T, st, "the position tangents of %lld instances x %lld directions", K, T));
+    return on_host(p, { { p->values.ptr, values, vbytes }, { p->dvalues.ptr, dvalues, vbytes * T } },
+        [&](cudaStream_t s) {
+            return run_on(p, K, p->values.ptr, p->positions.ptr, nonconverged ? p->counts.ptr : nullptr, variant, s, T, p->dvalues.ptr,
+                p->dpositions.ptr, recorded);
+        },
+        { { positions, p->positions.ptr, pbytes }, { dpositions, p->dpositions.ptr, pbytes * T },
+            { nonconverged, p->counts.ptr, nonconverged ? cbytes : 0 } },
+        ms);
 }
 
 }  // namespace
@@ -1015,8 +1026,7 @@ int gcs_b200_program_create(const gcs_b200_program_desc* d, int device, gcs_b200
 int gcs_b200_program_run(gcs_b200_program* p, int64_t K, const double* values, double* positions, uint32_t* nonconverged, int variant,
     void* stream)
 {
-    int rc = check_run(p, K, values, positions, variant);
-    if (rc != GCS_OK) return rc;
+    PROG_RC(check_run(p, K, values, positions, variant));
     CurrentDevice cur(p->device);
     return run_on(p, K, values, positions, nonconverged, variant, static_cast<cudaStream_t>(stream));
 }
@@ -1024,17 +1034,15 @@ int gcs_b200_program_run(gcs_b200_program* p, int64_t K, const double* values, d
 int gcs_b200_program_run_host(gcs_b200_program* p, int64_t K, const double* values, double* positions, uint32_t* nonconverged,
     int variant, float ms[3])
 {
-    int rc = check_run(p, K, values, positions, variant);
-    if (rc != GCS_OK) return rc;
+    PROG_RC(check_run(p, K, values, positions, variant));
     CurrentDevice cur(p->device);
-    return run_host(p, K, values, positions, nonconverged, variant, ms, 0, nullptr, nullptr);
+    return run_host(p, K, values, positions, nonconverged, variant, ms);
 }
 
 int gcs_b200_program_run_tangents(gcs_b200_program* p, int64_t K, const double* values, double* positions, uint32_t* nonconverged,
     int32_t T, const double* dvalues, double* dpositions, int variant, void* stream)
 {
-    int rc = check_tangent_run(p, K, values, positions, T, dvalues, dpositions, variant);
-    if (rc != GCS_OK) return rc;
+    PROG_RC(check_tangent_run(p, K, values, positions, T, dvalues, dpositions, variant));
     CurrentDevice cur(p->device);
     return run_on(p, K, values, positions, nonconverged, variant, static_cast<cudaStream_t>(stream), T, dvalues, dpositions);
 }
@@ -1042,8 +1050,7 @@ int gcs_b200_program_run_tangents(gcs_b200_program* p, int64_t K, const double* 
 int gcs_b200_program_run_tangents_host(gcs_b200_program* p, int64_t K, const double* values, double* positions,
     uint32_t* nonconverged, int32_t T, const double* dvalues, double* dpositions, int variant, float ms[3])
 {
-    int rc = check_tangent_run(p, K, values, positions, T, dvalues, dpositions, variant);
-    if (rc != GCS_OK) return rc;
+    PROG_RC(check_tangent_run(p, K, values, positions, T, dvalues, dpositions, variant));
     CurrentDevice cur(p->device);
     return run_host(p, K, values, positions, nonconverged, variant, ms, T, dvalues, dpositions);
 }
@@ -1051,8 +1058,7 @@ int gcs_b200_program_run_tangents_host(gcs_b200_program* p, int64_t K, const dou
 int gcs_b200_program_run_recorded(gcs_b200_program* p, int64_t K, const double* values, double* positions, uint32_t* nonconverged,
     int variant, void* stream)
 {
-    int rc = check_run(p, K, values, positions, variant);
-    if (rc != GCS_OK) return rc;
+    PROG_RC(check_run(p, K, values, positions, variant));
     CurrentDevice cur(p->device);
     return run_on(p, K, values, positions, nonconverged, variant, static_cast<cudaStream_t>(stream), 0, nullptr, nullptr, true);
 }
@@ -1060,50 +1066,31 @@ int gcs_b200_program_run_recorded(gcs_b200_program* p, int64_t K, const double* 
 int gcs_b200_program_run_recorded_host(gcs_b200_program* p, int64_t K, const double* values, double* positions,
     uint32_t* nonconverged, int variant, float ms[3])
 {
-    int rc = check_run(p, K, values, positions, variant);
-    if (rc != GCS_OK) return rc;
+    PROG_RC(check_run(p, K, values, positions, variant));
     CurrentDevice cur(p->device);
     return run_host(p, K, values, positions, nonconverged, variant, ms, 0, nullptr, nullptr, true);
 }
 
 int gcs_b200_program_adjoints(gcs_b200_program* p, int32_t T, const double* adj_positions, double* adj_values, void* stream)
 {
-    int rc = check_adjoints(p, T, adj_positions, adj_values);
-    if (rc != GCS_OK) return rc;
+    PROG_RC(check_adjoints(p, T, adj_positions, adj_values));
     CurrentDevice cur(p->device);
     const cudaStream_t st = static_cast<cudaStream_t>(stream);
-    rc = ensure_adjoint_tables(p, T, st);
-    if (rc != GCS_OK) return rc;
+    PROG_RC(ensure_adjoint_tables(p, T, st));
     const size_t pbytes = (size_t)p->recorded_k * T * p->n_slots * 4 * sizeof(double);
-    if (pbytes) PROG_TRY(cudaMemcpyAsync(p->apos, adj_positions, pbytes, cudaMemcpyDeviceToDevice, st));
+    if (pbytes) PROG_TRY(cudaMemcpyAsync(p->apos.ptr, adj_positions, pbytes, cudaMemcpyDeviceToDevice, st));
     return sweep_on(p, T, adj_values, st);
 }
 
 int gcs_b200_program_adjoints_host(gcs_b200_program* p, int32_t T, const double* adj_positions, double* adj_values, float ms[3])
 {
-    int rc = check_adjoints(p, T, adj_positions, adj_values);
-    if (rc != GCS_OK) return rc;
+    PROG_RC(check_adjoints(p, T, adj_positions, adj_values));
     CurrentDevice cur(p->device);
-    cudaStream_t st = p->stream;
-    rc = ensure_adjoint_tables(p, T, st);
-    if (rc != GCS_OK) return rc;
+    PROG_RC(ensure_adjoint_tables(p, T, p->stream));
     const size_t pbytes = (size_t)p->recorded_k * T * p->n_slots * 4 * sizeof(double);
     const size_t vbytes = (size_t)p->recorded_k * T * p->n_values * sizeof(double);
-    PROG_TRY(cudaEventRecord(p->ev[0], st));
-    if (pbytes) PROG_TRY(cudaMemcpyAsync(p->apos, adj_positions, pbytes, cudaMemcpyHostToDevice, st));
-    PROG_TRY(cudaEventRecord(p->ev[1], st));
-    rc = sweep_on(p, T, p->avalues, st);
-    if (rc != GCS_OK) {
-        cudaStreamSynchronize(st);
-        return rc;
-    }
-    PROG_TRY(cudaEventRecord(p->ev[2], st));
-    if (vbytes) PROG_TRY(cudaMemcpyAsync(adj_values, p->avalues, vbytes, cudaMemcpyDeviceToHost, st));
-    PROG_TRY(cudaEventRecord(p->ev[3], st));
-    PROG_TRY(cudaStreamSynchronize(st));
-    if (ms)
-        for (int q = 0; q < 3; ++q) PROG_TRY(cudaEventElapsedTime(&ms[q], p->ev[q], p->ev[q + 1]));
-    return GCS_OK;
+    return on_host(p, { { p->apos.ptr, adj_positions, pbytes } }, [&](cudaStream_t st) { return sweep_on(p, T, p->avalues.ptr, st); },
+        { { adj_values, p->avalues.ptr, vbytes } }, ms);
 }
 
 void gcs_b200_program_destroy(gcs_b200_program* p)
@@ -1114,11 +1101,11 @@ void gcs_b200_program_destroy(gcs_b200_program* p)
         if (p->stream) cudaStreamSynchronize(p->stream), cudaStreamDestroy(p->stream);
         for (auto e : p->ev)
             if (e) cudaEventDestroy(e);
-        cudaFree(p->rows), cudaFree(p->initial), cudaFree(p->scratch);
-        cudaFree(p->values), cudaFree(p->positions), cudaFree(p->counts);
-        cudaFree(p->dvalues), cudaFree(p->dpositions);
-        cudaFree(p->ent), cudaFree(p->begin), cudaFree(p->readers), cudaFree(p->tape);
-        cudaFree(p->apos), cudaFree(p->contrib), cudaFree(p->flags), cudaFree(p->avalues);
+        cudaFree(p->rows), cudaFree(p->initial), cudaFree(p->scratch.ptr);
+        cudaFree(p->values.ptr), cudaFree(p->positions.ptr), cudaFree(p->counts.ptr);
+        cudaFree(p->dvalues.ptr), cudaFree(p->dpositions.ptr);
+        cudaFree(p->ent), cudaFree(p->begin), cudaFree(p->readers), cudaFree(p->tape.ptr);
+        cudaFree(p->apos.ptr), cudaFree(p->contrib.ptr), cudaFree(p->flags.ptr), cudaFree(p->avalues.ptr);
         cudaGetLastError();
     }
     delete p;

@@ -356,7 +356,7 @@ CanvasRow detail::packCanvas(const Roles& r)
 namespace {
 
 // Numeric half of pack(): reads solved positions, places anchors, fills the batch row.  The
-// sketch program's gather kernel (csrc/sketch_program.cu) is the device's copy of this function.
+// sketch program's gather_row (csrc/sketch_program.cu) is the device's copy of this function.
 PackedLeaf packNumeric(const Roles& r)
 {
     const CanvasRow cv = detail::packCanvas(r);

@@ -31,6 +31,35 @@ using Clock = std::chrono::steady_clock;
 
 bool isZeroFixed(int solver) { return solver >= 1 && solver <= 3; }
 
+// K instances over devices 0 .. nDevices-1, one host thread per device: part(g, lo, hi, ms) runs
+// instances [lo, hi) = [K*g/n, K*(g+1)/n) on device g through the C entry point `entry`, returns its
+// code and fills ms[3].  A failed part throws, naming `entry`.  Returns the launches and the summed
+// times; seconds are the caller's.
+template <class Part>
+ProgramRunStats fanOut(std::int64_t K, int nDevices, const char* entry, Part&& part)
+{
+    const std::int64_t launches0 = gcs_b200_launch_count();
+    std::vector<int> rc(static_cast<std::size_t>(nDevices), GCS_OK);
+    std::vector<std::array<float, 3>> ms(static_cast<std::size_t>(nDevices));
+    auto one = [&](int g) {
+        const std::size_t i = static_cast<std::size_t>(g);
+        rc[i] = part(g, K * g / nDevices, K * (g + 1) / nDevices, ms[i].data());
+    };
+    if (nDevices == 1) {
+        one(0);
+    } else {
+        std::vector<std::thread> threads;
+        for (int g = 0; g < nDevices; ++g) threads.emplace_back(one, g);
+        for (auto& t : threads) t.join();
+    }
+    for (int r : rc)
+        if (r != GCS_OK) cudaFailure(entry, r);
+    ProgramRunStats st;
+    st.launches = gcs_b200_launch_count() - launches0;
+    for (const auto& m : ms) st.uploadMs += m[0], st.deviceMs += m[1], st.downloadMs += m[2];
+    return st;
+}
+
 }  // namespace
 
 SketchProgram SketchProgram::compile(const std::vector<ConstraintGraph>& leaves, const std::vector<std::shared_ptr<Element>>& elements,
@@ -201,26 +230,11 @@ ProgramRunStats SketchProgram::adjoints(const double* adjPositions, int T, doubl
     if (m_recordedDevices < 1) throw std::logic_error("SketchProgram::adjoints: no recorded run; call record() first");
     if (T < 1) throw std::invalid_argument("SketchProgram::adjoints: T must be >= 1 (got " + std::to_string(T) + ")");
     const std::int64_t K = m_recordedK;
-    const int nDevices = m_recordedDevices;
     const std::size_t nv = nValues(), table = nSlots() * 4;
-    const std::int64_t launches0 = gcs_b200_launch_count();
-    std::vector<int> rc(static_cast<std::size_t>(nDevices), GCS_OK);
-    std::vector<std::array<float, 3>> ms(static_cast<std::size_t>(nDevices));
-    auto part = [&](int g) {
-        const std::int64_t lo = K * g / nDevices;
-        rc[static_cast<std::size_t>(g)] = gcs_b200_program_adjoints_host(m_device[static_cast<std::size_t>(g)], T,
-            adjPositions + lo * static_cast<std::int64_t>(table) * T, adjValues + lo * static_cast<std::int64_t>(nv) * T,
-            ms[static_cast<std::size_t>(g)].data());
-    };
-    if (nDevices == 1) {
-        part(0);
-    } else {
-        std::vector<std::thread> threads;
-        for (int g = 0; g < nDevices; ++g) threads.emplace_back(part, g);
-        for (auto& t : threads) t.join();
-    }
-    for (int g = 0; g < nDevices; ++g)
-        if (rc[static_cast<std::size_t>(g)] != GCS_OK) cudaFailure("gcs_b200_program_adjoints_host", rc[static_cast<std::size_t>(g)]);
+    ProgramRunStats st = fanOut(K, m_recordedDevices, "gcs_b200_program_adjoints_host", [&](int g, std::int64_t lo, std::int64_t, float* ms) {
+        return gcs_b200_program_adjoints_host(m_device[static_cast<std::size_t>(g)], T, adjPositions + lo * static_cast<std::int64_t>(table) * T,
+            adjValues + lo * static_cast<std::int64_t>(nv) * T, ms);
+    });
     // the device's adjoints of cos(v), to radians: adj = (-std::sin(v)) * adj_cos
     const long long n = static_cast<long long>(K) * static_cast<long long>(nv) * T;
     const std::uint8_t* angle = m_valueIsAngle.data();
@@ -230,9 +244,6 @@ ProgramRunStats SketchProgram::adjoints(const double* adjPositions, int T, doubl
         const long long vq = q / T;
         if (angle[static_cast<std::size_t>(vq) % nv]) adjValues[q] = -std::sin(rec[vq]) * adjValues[q];
     }
-    ProgramRunStats st;
-    st.launches = gcs_b200_launch_count() - launches0;
-    for (const auto& m : ms) st.uploadMs += m[0], st.deviceMs += m[1], st.downloadMs += m[2];
     st.seconds = std::chrono::duration<double>(Clock::now() - t0).count();
     return st;
 }
@@ -282,32 +293,17 @@ ProgramRunStats SketchProgram::runImpl(const double* values, std::int64_t K, con
     }
     for (int g = 0; g < nDevices; ++g) onDevice(g);
 
-    const std::int64_t launches0 = gcs_b200_launch_count();
     const int variant = kernelVariant();
-    std::vector<int> rc(static_cast<std::size_t>(nDevices), GCS_OK);
-    std::vector<std::array<float, 3>> ms(static_cast<std::size_t>(nDevices));
-    auto part = [&](int g) {
-        const std::int64_t lo = K * g / nDevices, hi = K * (g + 1) / nDevices;
+    const char* entry = recorded ? "gcs_b200_program_run_recorded_host" : T == 0 ? "gcs_b200_program_run_host" : "gcs_b200_program_run_tangents_host";
+    ProgramRunStats st = fanOut(K, nDevices, entry, [&](int g, std::int64_t lo, std::int64_t hi, float* ms) {
         gcs_b200_program* p = m_device[static_cast<std::size_t>(g)];
         const std::int64_t vo = lo * static_cast<std::int64_t>(nv), po = lo * static_cast<std::int64_t>(table);
         std::uint32_t* counts = nonconverged ? m_stageCounts + lo : nullptr;
-        float* m = ms[static_cast<std::size_t>(g)].data();
-        rc[static_cast<std::size_t>(g)] = recorded ? gcs_b200_program_run_recorded_host(p, hi - lo, m_stageValues + vo, m_stagePositions + po, counts, variant, m)
-            : T == 0 ? gcs_b200_program_run_host(p, hi - lo, m_stageValues + vo, m_stagePositions + po, counts, variant, m)
+        return recorded ? gcs_b200_program_run_recorded_host(p, hi - lo, m_stageValues + vo, m_stagePositions + po, counts, variant, ms)
+            : T == 0 ? gcs_b200_program_run_host(p, hi - lo, m_stageValues + vo, m_stagePositions + po, counts, variant, ms)
             : gcs_b200_program_run_tangents_host(p, hi - lo, m_stageValues + vo, m_stagePositions + po, counts, T, m_stageDValues + vo * T,
-                m_stageDPositions + po * T, variant, m);
-    };
-    if (nDevices == 1) {
-        part(0);
-    } else {
-        std::vector<std::thread> threads;
-        for (int g = 0; g < nDevices; ++g) threads.emplace_back(part, g);
-        for (auto& t : threads) t.join();
-    }
-    for (int g = 0; g < nDevices; ++g)
-        if (rc[static_cast<std::size_t>(g)] != GCS_OK)
-            cudaFailure(recorded ? "gcs_b200_program_run_recorded_host" : T == 0 ? "gcs_b200_program_run_host" : "gcs_b200_program_run_tangents_host",
-                rc[static_cast<std::size_t>(g)]);
+                m_stageDPositions + po * T, variant, ms);
+    });
     const long long npos = static_cast<long long>(K) * static_cast<long long>(table);
     const double* from = m_stagePositions;
 #pragma omp parallel for schedule(static) if (npos > 65536)
@@ -317,9 +313,6 @@ ProgramRunStats SketchProgram::runImpl(const double* values, std::int64_t K, con
 #pragma omp parallel for schedule(static) if (ndpos > 65536)
     for (long long q = 0; q < ndpos; ++q) dpositions[q] = dfrom[q];
     if (nonconverged) std::memcpy(nonconverged, m_stageCounts, static_cast<std::size_t>(K) * sizeof(std::uint32_t));
-    ProgramRunStats st;
-    st.launches = gcs_b200_launch_count() - launches0;
-    for (const auto& m : ms) st.uploadMs += m[0], st.deviceMs += m[1], st.downloadMs += m[2];
     st.seconds = std::chrono::duration<double>(Clock::now() - t0).count();
     return st;
 }

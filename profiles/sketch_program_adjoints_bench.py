@@ -42,7 +42,7 @@ def median(xs):
 
 
 def tape_bytes(offsets, K):
-    """the tape of a recorded run (csrc/sketch_program.cu: tape_bytes), from the program's offsets"""
+    """the tape of a recorded run (csrc/sketch_program.cu: tape_layout), from the program's offsets"""
     a256 = lambda v: (v + 255) // 256 * 256  # noqa: E731
     total = 0
     for s in range(len(offsets) - 1):

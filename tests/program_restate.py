@@ -149,8 +149,8 @@ def transforms(p):
 # ---- the CPU restatement ----
 
 def gather(solver, sign, cst, pa, pb, v, dpa, dpb, dv):
-    """program_gather_kernel for one row over K instances and its tangent: (columns [nin][K], column
-    tangents [nin][K][T], anchors {role: (position [K][4] writes, tangent writes)})."""
+    """gather_row (csrc/sketch_program.cu) for one row over K instances and its tangent: (columns
+    [nin][K], column tangents [nin][K][T], anchors {role: (position [K][4] writes, tangent writes)})."""
     K, T = v.shape[0], dv.shape[2]
     z, dz = np.zeros(K), np.zeros((K, T))
     v0, v1, v2 = v[:, 0], v[:, 1], v[:, 2]

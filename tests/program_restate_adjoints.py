@@ -1,7 +1,7 @@
 """The adjoint sweep of a sketch program (gcs_b200_program_adjoints) restated wave by wave on the CPU:
 the forward run of tests/program_restate.py keeping every wave's solved batches, then the waves from
-last to first with the row adjoint of tests/adjoint_oracle.py, the gather's transpose and the reader
-lists' summation order of csrc/sketch_program.cu.  Also the forward/reverse contractions the duality
+last to first with the row adjoint of tests/adjoint_oracle.py, the gather's transpose
+(gather_row_transpose) and the reader lists' summation order of csrc/sketch_program.cu.  Also the forward/reverse contractions the duality
 tests compare."""
 import numpy as np
 
