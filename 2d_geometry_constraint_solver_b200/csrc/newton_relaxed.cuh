@@ -105,6 +105,21 @@ __device__ __forceinline__ int abs_hi(double v) { return __double2hiint(v) & 0x7
 // high word of a non-negative double, rounded outwards (thresholds of integer comparisons)
 __device__ __forceinline__ int hi_floor(double v) { return v > 0.0 ? __double2hiint(v) : 0; }
 
+// K2 / K5 pair a linear row of size L with the unit-normal row (size 2).  The literal solve's column-
+// pivoted QR rounds relative to the columns' norms, which the larger row dominates: its error in the
+// smaller row's equation is eps times the ratio of the rows, which the guards' eps S cond budget does not
+// contain.  Where the ratio leaves 2^-16 .. 2^16 the run goes to the literal code (det_root < 0 below:
+// G1 on the first update).  Found by tests/test_gpu_ranges.py at 2^-45 .. 2^-43 and on K2 fixed points
+// 2^-20 apart.
+__device__ __forceinline__ bool rows_comparable(double len) { return len >= 0x1p-16 && len <= 0x1p16; }
+
+// K4 lands with its first update; from a seed at |G| (20000 for the default seeds) the landing carries an
+// absolute rounding error ~eps cond |G|, and a system whose coordinates are smaller than that is solved
+// to noise in both arithmetics: the two seeds' candidates differ by that noise and the nearest-to-canvas
+// selection decides on it, beyond what (G5) budgets (2^-36 S).  Under 2^-20 the run goes literal.
+// Found by tests/test_gpu_ranges.py at 2^-513 .. 2^-100.
+constexpr double kMinLinearScale = 0x1p-20;
+
 // Per-run constants of the guards, derived once per run from the system's scale.
 struct RelaxGuard {
     int lo_h, hi_h;  // hi(|s|) < lo_h: converged for certain; >= hi_h: not converged for certain
@@ -208,8 +223,11 @@ struct Rsys<GCS_KIND_SDD> {
         dX = k[2] - k[0], dY = k[3] - k[1];
         c0 = k[4] - k[5];
         const double l1 = fabs(dX) + fabs(dY);
-        // iterates are unit normals; the linear residual carries the offsets in units of |delta|
-        if constexpr (kGuard) g.init(1.0 + (fabs(k[4]) + fabs(k[5])) * rcp_relaxed(l1), 2.0 * l1 * 0.70710678118654746, kStepScale);
+        // iterates are unit normals; the linear residual carries the offsets in units of |delta|.
+        // Rows far apart in size (|delta| outside 2^-16 .. 2^16 of the unit-normal row): run literally.
+        if constexpr (kGuard)
+            g.init(1.0 + (fabs(k[4]) + fabs(k[5])) * rcp_relaxed(l1), rows_comparable(l1) ? 2.0 * l1 * 0.70710678118654746 : -1.0,
+                kStepScale);
     }
     __device__ __forceinline__ void eval(
         double x, double y, double& a, double& b, double& c, double& d, double& r0, double& r1) const
@@ -276,7 +294,9 @@ struct Rsys<GCS_KIND_PLL> {
     {
         l1.set(k[0], k[1], k[2], k[3], k[4]);
         l2.set(k[5], k[6], k[7], k[8], k[9]);
-        if constexpr (kGuard) g.init(fabs(k[0]) + fabs(k[1]) + fabs(k[5]) + fabs(k[6]) + fabs(k[4]) + fabs(k[9]), l1.len * l2.len, kStepScale);
+        // Systems under 2^-20 in their coordinates: run literally (see kMinLinearScale).
+        const double sc = fabs(k[0]) + fabs(k[1]) + fabs(k[5]) + fabs(k[6]) + fabs(k[4]) + fabs(k[9]);
+        if constexpr (kGuard) g.init(sc, sc >= kMinLinearScale ? l1.len * l2.len : -1.0, kStepScale);
     }
     __device__ __forceinline__ void eval(
         double x, double y, double& a, double& b, double& c, double& d, double& r0, double& r1) const
@@ -301,8 +321,9 @@ struct Rsys<GCS_KIND_ANG> {
         rl = rsqrt_relaxed(l2);  // see RP2L::set
         len = l2 * rl;
         cl = k[2] * len;
-        // unit normals; the linear residual is L (cos(phi) - cosA): scale 2; det J = 2 L sin(.)
-        if constexpr (kGuard) g.init(2.0, 2.0 * len, kStepScale);
+        // unit normals; the linear residual is L (cos(phi) - cosA): scale 2; det J = 2 L sin(.).
+        // Rows far apart in size (L outside 2^-16 .. 2^16): run literally, as K2.
+        if constexpr (kGuard) g.init(2.0, rows_comparable(len) ? 2.0 * len : -1.0, kStepScale);
     }
     __device__ __forceinline__ void eval(
         double x, double y, double& a, double& b, double& c, double& d, double& r0, double& r1) const
