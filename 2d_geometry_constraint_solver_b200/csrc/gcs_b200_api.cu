@@ -17,6 +17,7 @@
 #include <vector>
 
 #include "../../include/gcs_b200.h"
+#include "api_common.cuh"
 #include "newton_kernels.cuh"
 
 using namespace gcsk;
@@ -24,23 +25,6 @@ using namespace gcsk;
 namespace {
 
 thread_local char g_err[512] = "";
-
-int fail(int code, const char* fmt, ...)
-{
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(g_err, sizeof(g_err), fmt, ap);
-    va_end(ap);
-    return code;
-}
-
-#define CUDA_TRY(expr)                                                                         \
-    do {                                                                                       \
-        cudaError_t e_ = (expr);                                                               \
-        if (e_ != cudaSuccess)                                                                 \
-            return fail(GCS_E_CUDA, "%s -> %s (%s:%d)", #expr, cudaGetErrorString(e_), __FILE__, \
-                __LINE__);                                                                     \
-    } while (0)
 
 // GCS_VARIANT_DEFAULT: the sorted kernel from kSortedMinRuns Newton runs per launch (measured faster
 // on every kind and seed count there, profiles/), the static kernel below (a sorted CTA lives
@@ -133,11 +117,13 @@ int ensure_init()
     return GCS_OK;
 }
 
+// the tickets, streams and events of device `d`, made on first use
 int prepare_device(DeviceState* d)
 {
     std::lock_guard<std::mutex> lk(g_mu);  // two first-time callers on one device must not both allocate
     if (d->tickets) return GCS_OK;
-    CUDA_TRY(cudaSetDevice(d->device));
+    DeviceScope on(d->device);
+    RC_TRY(on.rc);
     cudaDeviceProp prop;
     CUDA_TRY(cudaGetDeviceProperties(&prop, d->device));
     d->sm_count = prop.multiProcessorCount;
@@ -154,13 +140,33 @@ int prepare_device(DeviceState* d)
     return GCS_OK;
 }
 
+// The prologue of an entry point on `device`: ensure_init, find_dev and, when `prepare`,
+// prepare_device.  Null, with the failure's code in rc, when one of them fails.
+DeviceState* device_state(int device, int& rc, bool prepare = true)
+{
+    rc = ensure_init();
+    if (rc != GCS_OK) return nullptr;
+    DeviceState* d = find_dev(device);
+    if (!d) {
+        rc = fail(GCS_E_NO_DEVICE, "device %d not present", device);
+        return nullptr;
+    }
+    if (prepare) rc = prepare_device(d);
+    return rc == GCS_OK ? d : nullptr;
+}
+
 }  // namespace
 
-// for the other translation units of the library (sketch_program.cu)
-namespace gcsk {
-int api_fail(int code, const char* msg) { return fail(code, "%s", msg); }
-void api_count_launch() { g_launches.fetch_add(1); }
-}  // namespace gcsk
+int gcsk::fail(int code, const char* fmt, ...)
+{
+    va_list ap;
+    va_start(ap, fmt);
+    vsnprintf(g_err, sizeof(g_err), fmt, ap);
+    va_end(ap);
+    return code;
+}
+
+void gcsk::count_launch() { g_launches.fetch_add(1); }
 
 extern "C" int gcs_b200_column_may_be_null(int kind, int c)
 {
@@ -281,74 +287,34 @@ long long wave_subs(DeviceState* d, Kern kern, int block, int subs_per_block)
     return (long long)d->sm_count * bps * subs_per_block;
 }
 
+int batch_too_large() { return fail(GCS_E_INVALID, "batch too large for one launch"); }
+
 template <int KIND, int NS, bool RLX = false>
-int launch_static(DeviceState*, const BatchDev& p, cudaStream_t st)
+int launch_static(const BatchDev& p, cudaStream_t st)
 {
-    const long long threads = p.n * NS;
     static const int block = static_block_size();
-    const long long grid = (threads + block - 1) / block;
-    if (grid > 0x7fffffffLL) return fail(GCS_E_INVALID, "batch too large for one launch");
-    newton_static_kernel<KIND, NS, RLX><<<(unsigned)grid, block, 0, st>>>(p);
-    g_launches.fetch_add(1);
-    CUDA_TRY(cudaGetLastError());
-    return GCS_OK;
+    return launch_kernel(newton_static_kernel<KIND, NS, RLX>, (p.n * NS + block - 1) / block, block, 0, st, batch_too_large, p);
 }
 
-template <int KIND, int NS, bool RLX>
-int launch_seq(DeviceState* d, BatchDev p, cudaStream_t st)
+// one lane per sub-system (the seq and linear kernels), with the L2 prefetch looking ahead
+// prefetch_waves() waves of the kernel's resident CTAs
+template <auto kernel>
+int launch_lanes(DeviceState* d, BatchDev p, cudaStream_t st)
 {
-    const long long grid = (p.n + 127) / 128;
-    if (grid > 0x7fffffffLL) return fail(GCS_E_INVALID, "batch too large for one launch");
     static thread_local long long wave[64] = {};
     if (prefetch_waves() > 0) {
         long long& w = wave[d->device & 63];
-        if (w == 0) w = wave_subs(d, newton_seq_kernel<KIND, NS, RLX>, 128, 128);
+        if (w == 0) w = wave_subs(d, kernel, 128, 128);
         p.pf = w * prefetch_waves();
     }
-    newton_seq_kernel<KIND, NS, RLX><<<(unsigned)grid, 128, 0, st>>>(p);
-    g_launches.fetch_add(1);
-    CUDA_TRY(cudaGetLastError());
-    return GCS_OK;
-}
-
-template <int NS>
-int launch_linear(DeviceState* d, BatchDev p, cudaStream_t st)
-{
-    const long long grid = (p.n + 127) / 128;
-    if (grid > 0x7fffffffLL) return fail(GCS_E_INVALID, "batch too large for one launch");
-    static thread_local long long wave[64] = {};
-    if (prefetch_waves() > 0) {
-        long long& w = wave[d->device & 63];
-        if (w == 0) w = wave_subs(d, newton_linear_kernel<NS>, 128, 128);
-        p.pf = w * prefetch_waves();
-    }
-    newton_linear_kernel<NS><<<(unsigned)grid, 128, 0, st>>>(p);
-    g_launches.fetch_add(1);
-    CUDA_TRY(cudaGetLastError());
-    return GCS_OK;
-}
-
-template <int KIND>
-int launch_pair(const BatchDev& p, cudaStream_t st)
-{
-    const long long grid = (p.n + 127) / 128;
-    if (grid > 0x7fffffffLL) return fail(GCS_E_INVALID, "batch too large for one launch");
-    newton_pair_kernel<KIND><<<(unsigned)grid, 128, 0, st>>>(p);
-    g_launches.fetch_add(1);
-    CUDA_TRY(cudaGetLastError());
-    return GCS_OK;
+    return launch_kernel(kernel, (p.n + 127) / 128, 128, 0, st, batch_too_large, p);
 }
 
 template <int KIND, int NS, bool RLX = false>
 int launch_sorted(const BatchDev& p, cudaStream_t st)
 {
     constexpr int T = GCS_SORTED_THREADS, TILE = 2 * T / NS;  // two runs per lane
-    const long long grid = (p.n + TILE - 1) / TILE;
-    if (grid > 0x7fffffffLL) return fail(GCS_E_INVALID, "batch too large for one launch");
-    newton_sorted_kernel<KIND, NS, TILE, T, RLX><<<(unsigned)grid, T, 0, st>>>(p);
-    g_launches.fetch_add(1);
-    CUDA_TRY(cudaGetLastError());
-    return GCS_OK;
+    return launch_kernel(newton_sorted_kernel<KIND, NS, TILE, T, RLX>, (p.n + TILE - 1) / TILE, T, 0, st, batch_too_large, p);
 }
 
 template <int KIND, int NS>
@@ -376,51 +342,39 @@ int launch_refill(DeviceState* d, const BatchDev& p, cudaStream_t st)
     for (int c = 0; c < Sys<KIND>::kCols; ++c)
         aligned = aligned && ((reinterpret_cast<uintptr_t>(p.in[c]) & 15) == 0);
     unsigned* tk = d->tickets + 2 * (d->ticket_rr.fetch_add(1) % kTicketSlots);
-    kern<<<(unsigned)grid, W * 32, smem, st>>>(p, tk, aligned ? 1 : 0);
-    g_launches.fetch_add(1);
-    CUDA_TRY(cudaGetLastError());
-    return GCS_OK;
+    return launch_kernel(kern, grid, W * 32, smem, st, batch_too_large, p, tk, aligned ? 1 : 0);
 }
 
-template <int KIND>
-int launch_kind(DeviceState* d, const gcs_b200_batch* b, const BatchDev& p, cudaStream_t st)
+// The kernel of a resolved variant.  PAIR exists for 2 seeds only (8 seeds run the static kernel),
+// CONTRACTED_LINEAR for K4 only (resolve_variant maps it to another contracted variant elsewhere).
+template <int KIND, int NS>
+int launch_kind(DeviceState* d, int variant, const BatchDev& p, cudaStream_t st)
 {
-    const int variant = resolve_variant(b->variant, KIND, p.n, b->n_seeds);
-    constexpr bool column_guess = (KIND == GCS_KIND_SDD || KIND == GCS_KIND_ANG);
-    if constexpr (KIND == GCS_KIND_PLL) {
-        if (variant == GCS_VARIANT_CONTRACTED_LINEAR) return b->n_seeds == 2 ? launch_linear<2>(d, p, st) : launch_linear<8>(d, p, st);
-    }
-    if (b->n_seeds == 2) {
-        if (variant == GCS_VARIANT_CONTRACTED_SEQ) return launch_seq<KIND, 2, true>(d, p, st);
-        if (variant == GCS_VARIANT_SEQ) return launch_seq<KIND, 2, false>(d, p, st);
-        if (variant == GCS_VARIANT_CONTRACTED_SORTED) return launch_sorted<KIND, 2, true>(p, st);
-        if (variant == GCS_VARIANT_CONTRACTED_STATIC) return launch_static<KIND, 2, true>(d, p, st);
-        if (variant == GCS_VARIANT_SORTED) return launch_sorted<KIND, 2>(p, st);
-        if (variant == GCS_VARIANT_PAIR) return launch_pair<KIND>(p, st);
-        return variant == GCS_VARIANT_REFILL ? launch_refill<KIND, 2>(d, p, st) : launch_static<KIND, 2>(d, p, st);
-    }
-    if constexpr (!column_guess) {
-        if (variant == GCS_VARIANT_CONTRACTED_SEQ) return launch_seq<KIND, 8, true>(d, p, st);
-        if (variant == GCS_VARIANT_SEQ) return launch_seq<KIND, 8, false>(d, p, st);
-        if (variant == GCS_VARIANT_CONTRACTED_SORTED) return launch_sorted<KIND, 8, true>(p, st);
-        if (variant == GCS_VARIANT_CONTRACTED_STATIC) return launch_static<KIND, 8, true>(d, p, st);
-        if (variant == GCS_VARIANT_SORTED) return launch_sorted<KIND, 8>(p, st);
-        return variant == GCS_VARIANT_REFILL ? launch_refill<KIND, 8>(d, p, st) : launch_static<KIND, 8>(d, p, st);
-    }
-    return fail(GCS_E_INVALID, "unsupported seed count");
+    if constexpr (KIND == GCS_KIND_PLL)
+        if (variant == GCS_VARIANT_CONTRACTED_LINEAR) return launch_lanes<newton_linear_kernel<NS>>(d, p, st);
+    if (variant == GCS_VARIANT_CONTRACTED_SEQ) return launch_lanes<newton_seq_kernel<KIND, NS, true>>(d, p, st);
+    if (variant == GCS_VARIANT_SEQ) return launch_lanes<newton_seq_kernel<KIND, NS, false>>(d, p, st);
+    if (variant == GCS_VARIANT_CONTRACTED_SORTED) return launch_sorted<KIND, NS, true>(p, st);
+    if (variant == GCS_VARIANT_CONTRACTED_STATIC) return launch_static<KIND, NS, true>(p, st);
+    if (variant == GCS_VARIANT_SORTED) return launch_sorted<KIND, NS>(p, st);
+    if constexpr (NS == 2)
+        if (variant == GCS_VARIANT_PAIR) return launch_kernel(newton_pair_kernel<KIND>, (p.n + 127) / 128, 128, 0, st, batch_too_large, p);
+    return variant == GCS_VARIANT_REFILL ? launch_refill<KIND, NS>(d, p, st) : launch_static<KIND, NS>(p, st);
 }
 
+// the column-guess kinds K2 / K5 take 2 seeds only
 int solve_dev(DeviceState* d, const gcs_b200_batch* b, const BatchDev& p, cudaStream_t st)
 {
     if (p.n == 0) return GCS_OK;
-    switch (b->kind) {
-    case GCS_KIND_PP: return launch_kind<GCS_KIND_PP>(d, b, p, st);
-    case GCS_KIND_SDD: return launch_kind<GCS_KIND_SDD>(d, b, p, st);
-    case GCS_KIND_PPL: return launch_kind<GCS_KIND_PPL>(d, b, p, st);
-    case GCS_KIND_PLL: return launch_kind<GCS_KIND_PLL>(d, b, p, st);
-    case GCS_KIND_ANG: return launch_kind<GCS_KIND_ANG>(d, b, p, st);
-    }
-    return fail(GCS_E_INVALID, "unknown kind");
+    const int variant = resolve_variant(b->variant, b->kind, p.n, b->n_seeds);
+    return with_kind(b->kind, [&](auto K) {
+        constexpr int KIND = decltype(K)::value;
+        if (b->n_seeds == 2) return launch_kind<KIND, 2>(d, variant, p, st);
+        if constexpr (KIND == GCS_KIND_SDD || KIND == GCS_KIND_ANG)
+            return fail(GCS_E_INVALID, "unsupported seed count");
+        else
+            return launch_kind<KIND, 8>(d, variant, p, st);
+    });
 }
 
 int solve_on(DeviceState* d, const gcs_b200_batch* b, cudaStream_t st)
@@ -503,17 +457,9 @@ __global__ void fp64_curve_kernel(double* out, long long* cycles, int iters, dou
 
 extern "C" {
 
-int gcs_b200_kind_in_cols(int kind)
-{
-    static const int t[GCS_KIND_COUNT + 1] = { 0, 6, 9, 10, 12, 13 };
-    return (kind >= 1 && kind <= GCS_KIND_COUNT) ? t[kind] : 0;
-}
+int gcs_b200_kind_in_cols(int kind) { return (kind >= 1 && kind <= GCS_KIND_COUNT) ? in_cols(kind) : 0; }
 
-int gcs_b200_kind_out_cols(int kind)
-{
-    static const int t[GCS_KIND_COUNT + 1] = { 0, 2, 4, 2, 2, 4 };
-    return (kind >= 1 && kind <= GCS_KIND_COUNT) ? t[kind] : 0;
-}
+int gcs_b200_kind_out_cols(int kind) { return (kind >= 1 && kind <= GCS_KIND_COUNT) ? out_cols(kind) : 0; }
 
 void* gcs_b200_host_alloc(size_t bytes) { return gcs_b200_host_alloc_ex(bytes, 0); }
 
@@ -570,7 +516,7 @@ void gcs_b200_shutdown(void)
     std::lock_guard<std::mutex> lk(g_mu);
     for (auto* d : g_devs) {
         if (d->tickets || d->arena || d->stream) {
-            cudaSetDevice(d->device);
+            DeviceScope on(d->device);  // released whether or not the switch succeeded
             if (d->stream) cudaStreamSynchronize(d->stream), cudaStreamDestroy(d->stream);
             if (d->h2d) cudaStreamSynchronize(d->h2d), cudaStreamDestroy(d->h2d);
             if (d->d2h) cudaStreamSynchronize(d->d2h), cudaStreamDestroy(d->d2h);
@@ -627,18 +573,11 @@ int gcs_b200_solve(const gcs_b200_batch* b, int device, void* cuda_stream)
     int rc = validate(b);
     if (rc != GCS_OK) return rc;
     if (b->mem != GCS_MEM_DEVICE) return fail(GCS_E_INVALID, "gcs_b200_solve needs device pointers (mem=GCS_MEM_DEVICE)");
-    rc = ensure_init();
-    if (rc != GCS_OK) return rc;
-    DeviceState* d = find_dev(device);
-    if (!d) return fail(GCS_E_NO_DEVICE, "device %d not present", device);
-    rc = prepare_device(d);
-    if (rc != GCS_OK) return rc;
-    int cur = -1;
-    CUDA_TRY(cudaGetDevice(&cur));
-    if (cur != device) CUDA_TRY(cudaSetDevice(device));
-    rc = solve_on(d, b, static_cast<cudaStream_t>(cuda_stream));
-    if (cur != device && cur >= 0) cudaSetDevice(cur);
-    return rc;
+    DeviceState* d = device_state(device, rc);
+    if (!d) return rc;
+    DeviceScope on(device);
+    RC_TRY(on.rc);
+    return solve_on(d, b, static_cast<cudaStream_t>(cuda_stream));
 }
 
 int gcs_b200_solve_many(const gcs_b200_batch* const* batches, int count, int device, void* cuda_stream)
@@ -651,15 +590,11 @@ int gcs_b200_solve_many(const gcs_b200_batch* const* batches, int count, int dev
     }
     if (count == 0) return GCS_OK;
     if (count == 1) return gcs_b200_solve(batches[0], device, cuda_stream);
-    int rc = ensure_init();
-    if (rc != GCS_OK) return rc;
-    DeviceState* d = find_dev(device);
-    if (!d) return fail(GCS_E_NO_DEVICE, "device %d not present", device);
-    rc = prepare_device(d);
-    if (rc != GCS_OK) return rc;
-    int cur = -1;
-    CUDA_TRY(cudaGetDevice(&cur));
-    if (cur != device) CUDA_TRY(cudaSetDevice(device));
+    int rc;
+    DeviceState* d = device_state(device, rc);
+    if (!d) return rc;
+    DeviceScope on(device);
+    RC_TRY(on.rc);
     cudaStream_t user = static_cast<cudaStream_t>(cuda_stream);
     {
         // The batches are independent jobs: the first stays on the caller's stream, the others go
@@ -687,7 +622,6 @@ int gcs_b200_solve_many(const gcs_b200_batch* const* batches, int count, int dev
                 if (rc == GCS_OK) rc = fail(GCS_E_CUDA, "joining the side streams failed");
         }
     }
-    if (cur != device && cur >= 0) cudaSetDevice(cur);
     return rc;
 }
 
@@ -1005,23 +939,18 @@ int enqueue_host(DeviceState* d, const gcs_b200_batch* b, int64_t first, int64_t
 // index range [first, first + count) of a validated host batch on `device`
 int host_range_entry(const gcs_b200_batch* b, int device, int64_t first, int64_t count, bool wait)
 {
-    int rc = ensure_init();
-    if (rc != GCS_OK) return rc;
-    DeviceState* d = find_dev(device);
-    if (!d) return fail(GCS_E_NO_DEVICE, "device %d not present", device);
-    rc = prepare_device(d);
-    if (rc != GCS_OK) return rc;
+    int rc;
+    DeviceState* d = device_state(device, rc);
+    if (!d) return rc;
     std::lock_guard<std::mutex> lk(d->arena_mu);
-    int cur = -1;
-    CUDA_TRY(cudaGetDevice(&cur));
-    if (cur != device) CUDA_TRY(cudaSetDevice(device));
+    DeviceScope on(device);
+    RC_TRY(on.rc);
     if (count > 0) rc = enqueue_host(d, b, first, count);
     if (rc != GCS_OK) {
         drain(d);  // leave nothing behind a failed call
     } else if (wait && d->in_flight) {
         rc = drain(d);
     }
-    if (cur != device && cur >= 0) cudaSetDevice(cur);
     return rc;
 }
 
@@ -1052,18 +981,14 @@ int gcs_b200_solve_host_range_async(const gcs_b200_batch* b, int device, int64_t
 
 int gcs_b200_wait(int device)
 {
-    int rc = ensure_init();
-    if (rc != GCS_OK) return rc;
-    DeviceState* d = find_dev(device);
-    if (!d) return fail(GCS_E_NO_DEVICE, "device %d not present", device);
+    int rc;
+    DeviceState* d = device_state(device, rc, false);
+    if (!d) return rc;
     if (!d->tickets) return GCS_OK;  // never used
     std::lock_guard<std::mutex> lk(d->arena_mu);
-    int cur = -1;
-    CUDA_TRY(cudaGetDevice(&cur));
-    if (cur != device) CUDA_TRY(cudaSetDevice(device));
-    rc = drain(d);
-    if (cur != device && cur >= 0) cudaSetDevice(cur);
-    return rc;
+    DeviceScope on(device);
+    RC_TRY(on.rc);
+    return drain(d);
 }
 
 int gcs_b200_solve_sharded(const gcs_b200_batch* b, int n_dev)
@@ -1109,10 +1034,9 @@ int gcs_b200_contracted_stats_ex(int device, uint64_t out[8], int reset);
 
 int gcs_b200_debug_path_buffer(int device, uint8_t* dev_buf, int64_t capacity)
 {
-    int rc = ensure_init();
-    if (rc != GCS_OK) return rc;
-    DeviceState* d = find_dev(device);
-    if (!d) return fail(GCS_E_NO_DEVICE, "device %d not present", device);
+    int rc;
+    DeviceState* d = device_state(device, rc, false);
+    if (!d) return rc;
     if (capacity < 0) return fail(GCS_E_INVALID, "negative capacity");
     d->dbg_path = capacity > 0 ? dev_buf : nullptr;
     d->dbg_path_cap = d->dbg_path ? capacity : 0;
@@ -1135,13 +1059,10 @@ int gcs_b200_contracted_stats(int device, uint64_t out[2], int reset)
 
 int gcs_b200_contracted_stats_ex(int device, uint64_t out[8], int reset)
 {
-    int rc = ensure_init();
-    if (rc != GCS_OK) return rc;
-    DeviceState* d = find_dev(device);
-    if (!d) return fail(GCS_E_NO_DEVICE, "device %d not present", device);
-    int cur = -1;
-    CUDA_TRY(cudaGetDevice(&cur));
-    if (cur != device) CUDA_TRY(cudaSetDevice(device));
+    int rc;
+    if (!device_state(device, rc, false)) return rc;
+    DeviceScope on(device);
+    RC_TRY(on.rc);
     CUDA_TRY(cudaDeviceSynchronize());
     unsigned long long v[gcsk::kWhyCount] = {};
     CUDA_TRY(cudaMemcpyFromSymbol(v, gcsk::g_relax_reruns, sizeof(v)));
@@ -1151,19 +1072,16 @@ int gcs_b200_contracted_stats_ex(int device, uint64_t out[8], int reset)
     }
     if (out)
         for (int k = 0; k < gcsk::kWhyCount; ++k) out[k] = v[k];
-    if (cur != device && cur >= 0) cudaSetDevice(cur);
     return GCS_OK;
 }
 
 double gcs_b200_fp64_probe(int device, int what)
 {
-    int rc = ensure_init();
-    if (rc != GCS_OK) return (double)rc;
-    DeviceState* d = find_dev(device);
-    if (!d) return (double)fail(GCS_E_NO_DEVICE, "device %d not present", device);
-    rc = prepare_device(d);
-    if (rc != GCS_OK) return (double)rc;
-    if (cudaSetDevice(device) != cudaSuccess) return (double)GCS_E_CUDA;
+    int rc;
+    DeviceState* d = device_state(device, rc);
+    if (!d) return (double)rc;
+    DeviceScope on(device);
+    if (on.rc != GCS_OK) return (double)on.rc;
     double* out = nullptr;
     const int blocks = d->sm_count * 8, threads = 256, iters = 20000;
     if (cudaMalloc(&out, sizeof(double) * blocks * threads + 64) != cudaSuccess) return (double)GCS_E_NOMEM;
@@ -1235,15 +1153,11 @@ double gcs_b200_fp64_probe(int device, int what)
 int gcs_b200_pcie_probe(int device, size_t bytes_up, size_t bytes_down, int pieces, int write_combined, int reps, double out[4])
 {
     if (!out || pieces < 1 || reps < 1 || bytes_up == 0 || bytes_down == 0) return fail(GCS_E_INVALID, "bad probe arguments");
-    int rc = ensure_init();
-    if (rc != GCS_OK) return rc;
-    DeviceState* d = find_dev(device);
-    if (!d) return fail(GCS_E_NO_DEVICE, "device %d not present", device);
-    rc = prepare_device(d);
-    if (rc != GCS_OK) return rc;
-    int cur = -1;
-    CUDA_TRY(cudaGetDevice(&cur));
-    if (cur != device) CUDA_TRY(cudaSetDevice(device));
+    int rc;
+    DeviceState* d = device_state(device, rc);
+    if (!d) return rc;
+    DeviceScope on(device);
+    RC_TRY(on.rc);
     void *hu = nullptr, *hd = nullptr, *du = nullptr, *dd = nullptr;
     cudaEvent_t e[4] = {};
     auto cleanup = [&]() {
@@ -1253,7 +1167,6 @@ int gcs_b200_pcie_probe(int device, size_t bytes_up, size_t bytes_down, int piec
         if (dd) cudaFree(dd);
         for (auto ev : e)
             if (ev) cudaEventDestroy(ev);
-        if (cur != device && cur >= 0) cudaSetDevice(cur);
     };
     cudaError_t ce = cudaHostAlloc(&hu, bytes_up, cudaHostAllocPortable | (write_combined ? cudaHostAllocWriteCombined : 0u));
     if (ce == cudaSuccess) ce = cudaHostAlloc(&hd, bytes_down, cudaHostAllocPortable);
@@ -1313,18 +1226,16 @@ int gcs_b200_selftest_launch(uint64_t seed, long long n, unsigned long long* dev
 int gcs_b200_selftest(int device, uint64_t seed, int64_t n, uint64_t counts[8])
 {
     if (!counts || n < 0) return fail(GCS_E_INVALID, "bad selftest arguments");
-    int rc = ensure_init();
-    if (rc != GCS_OK) return rc;
-    DeviceState* d = find_dev(device);
-    if (!d) return fail(GCS_E_NO_DEVICE, "device %d not present", device);
-    rc = prepare_device(d);
-    if (rc != GCS_OK) return rc;
-    CUDA_TRY(cudaSetDevice(device));
+    int rc;
+    DeviceState* d = device_state(device, rc);
+    if (!d) return rc;
+    DeviceScope on(device);
+    RC_TRY(on.rc);
     unsigned long long* dc = nullptr;
     CUDA_TRY(cudaMalloc(&dc, 8 * sizeof(unsigned long long)));
     CUDA_TRY(cudaMemset(dc, 0, 8 * sizeof(unsigned long long)));
     rc = gcs_b200_selftest_launch(seed, (long long)n, dc, d->sm_count);
-    g_launches.fetch_add(1);
+    count_launch();
     cudaError_t e = cudaDeviceSynchronize();
     unsigned long long h[8] = {};
     if (e == cudaSuccess) e = cudaMemcpy(h, dc, sizeof(h), cudaMemcpyDeviceToHost);
@@ -1343,15 +1254,12 @@ int gcs_b200_synth_pp(int device, void* cuda_stream, uint64_t seed, int64_t firs
     if (n < 0 || !cols || !code) return fail(GCS_E_INVALID, "bad synth arguments");
     for (int c = 0; c < 6; ++c)
         if (!cols[c]) return fail(GCS_E_INVALID, "synth column %d is null", c);
-    int rc = ensure_init();
-    if (rc != GCS_OK) return rc;
-    if (!find_dev(device)) return fail(GCS_E_NO_DEVICE, "device %d not present", device);
-    int cur = -1;
-    CUDA_TRY(cudaGetDevice(&cur));
-    if (cur != device) CUDA_TRY(cudaSetDevice(device));
+    int rc;
+    if (!device_state(device, rc, false)) return rc;
+    DeviceScope on(device);
+    RC_TRY(on.rc);
     rc = gcs_b200_synth_pp_launch(cuda_stream, seed, first, n, perturb_of, cols, code);
-    g_launches.fetch_add(1);
-    if (cur != device && cur >= 0) cudaSetDevice(cur);
+    count_launch();
     if (rc != 0) return fail(GCS_E_CUDA, "synth launch failed: %s", cudaGetErrorString(cudaGetLastError()));
     return GCS_OK;
 }

@@ -38,37 +38,16 @@
 #include <vector>
 
 #include "../../include/gcs_b200.h"
+#include "api_common.cuh"
 #include "newton_adjoint.cuh"
 
-namespace gcsk {
-int api_fail(int code, const char* msg);  // gcs_b200_api.cu: sets gcs_b200_last_error()
-void api_count_launch();
-}  // namespace gcsk
+using gcsk::DeviceScope;
+using gcsk::fail;
+using gcsk::in_cols;
+using gcsk::out_cols;
+using gcsk::with_kind;
 
 namespace {
-
-int failf(int code, const char* fmt, ...)
-{
-    char buf[400];
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(buf, sizeof(buf), fmt, ap);
-    va_end(ap);
-    return gcsk::api_fail(code, buf);
-}
-
-#define PROG_TRY(expr)                                                                                    \
-    do {                                                                                                  \
-        cudaError_t e_ = (expr);                                                                          \
-        if (e_ != cudaSuccess) return failf(GCS_E_CUDA, "%s -> %s (%s:%d)", #expr, cudaGetErrorString(e_), \
-            __FILE__, __LINE__);                                                                          \
-    } while (0)
-
-#define PROG_RC(expr)                  \
-    do {                               \
-        const int rc_ = (expr);        \
-        if (rc_ != GCS_OK) return rc_; \
-    } while (0)
 
 constexpr int kKinds = GCS_KIND_COUNT;
 constexpr int kThreads = 256;
@@ -80,33 +59,6 @@ constexpr bool kRoleIsLine[9][3] = { {}, { 0, 0, 0 }, { 0, 0, 1 }, { 1, 0, 1 }, 
     { 1, 1, 0 }, { 1, 0, 1 } };
 constexpr bool kReads[9][3] = { {}, { 1, 1, 1 }, { 1, 1, 1 }, { 1, 1, 1 }, { 0, 1, 1 }, { 0, 1, 1 }, { 0, 1, 1 },
     { 0, 1, 1 }, { 1, 0, 1 } };
-
-// f(std::integral_constant<int, kind>()): f sees a kind known at run time as a compile-time
-// constant.  The host (in_cols, out_cols) and the kernels' device lambdas share it; the pragma lets
-// the one template call either.
-#pragma nv_exec_check_disable
-template <class F>
-__host__ __device__ __forceinline__ auto with_kind(int kind, F&& f)
-{
-    switch (kind) {
-    case GCS_KIND_PP: return f(std::integral_constant<int, GCS_KIND_PP>());
-    case GCS_KIND_SDD: return f(std::integral_constant<int, GCS_KIND_SDD>());
-    case GCS_KIND_PPL: return f(std::integral_constant<int, GCS_KIND_PPL>());
-    case GCS_KIND_PLL: return f(std::integral_constant<int, GCS_KIND_PLL>());
-    default: return f(std::integral_constant<int, GCS_KIND_ANG>());
-    }
-}
-
-// a kind's input and output columns
-__host__ __device__ __forceinline__ int in_cols(int kind)
-{
-    return with_kind(kind, [](auto K) { return gcsk::Sys<decltype(K)::value>::kCols; });
-}
-
-__host__ __device__ __forceinline__ int out_cols(int kind)
-{
-    return with_kind(kind, [](auto K) { return gcsk::Sys<decltype(K)::value>::kOut; });
-}
 
 // one wave: rows [seg[0], seg[5]) of the program relative to `rows`, kind k + 1 at [seg[k], seg[k+1])
 struct WaveArgs {
@@ -487,47 +439,47 @@ __global__ void __launch_bounds__(kThreads) program_adjoint_flag_kernel(const Re
 
 int validate_desc(const gcs_b200_program_desc* d)
 {
-    if (!d) return failf(GCS_E_INVALID, "null program descriptor");
+    if (!d) return fail(GCS_E_INVALID, "null program descriptor");
     if (d->n_waves < 0 || d->n_slots < 0 || d->n_values < 0 || d->n_rows < 0)
-        return failf(GCS_E_INVALID, "negative count in the program descriptor");
-    if (!d->offsets) return failf(GCS_E_INVALID, "null offsets");
+        return fail(GCS_E_INVALID, "negative count in the program descriptor");
+    if (!d->offsets) return fail(GCS_E_INVALID, "null offsets");
     if ((d->n_rows > 0 && !d->rows) || (d->n_slots > 0 && (!d->slot_is_line || !d->initial)) || (d->n_values > 0 && !d->value_is_angle))
-        return failf(GCS_E_INVALID, "null table in the program descriptor");
+        return fail(GCS_E_INVALID, "null table in the program descriptor");
     const long long nseg = (long long)d->n_waves * kKinds;
-    if (d->offsets[0] != 0) return failf(GCS_E_INVALID, "offsets[0] is %lld, not 0", (long long)d->offsets[0]);
+    if (d->offsets[0] != 0) return fail(GCS_E_INVALID, "offsets[0] is %lld, not 0", (long long)d->offsets[0]);
     for (long long s = 0; s < nseg; ++s)
         if (d->offsets[s + 1] < d->offsets[s])
-            return failf(GCS_E_INVALID, "offsets decrease at segment %lld (%lld after %lld)", s, (long long)d->offsets[s + 1], (long long)d->offsets[s]);
+            return fail(GCS_E_INVALID, "offsets decrease at segment %lld (%lld after %lld)", s, (long long)d->offsets[s + 1], (long long)d->offsets[s]);
     if (d->offsets[nseg] != d->n_rows)
-        return failf(GCS_E_INVALID, "offsets end at %lld, not at n_rows = %lld", (long long)d->offsets[nseg], (long long)d->n_rows);
+        return fail(GCS_E_INVALID, "offsets end at %lld, not at n_rows = %lld", (long long)d->offsets[nseg], (long long)d->n_rows);
     for (int s = 0; s < d->n_slots; ++s)
-        if (d->slot_is_line[s] > 1) return failf(GCS_E_INVALID, "slot %d: type %d is neither point (0) nor line (1)", s, d->slot_is_line[s]);
+        if (d->slot_is_line[s] > 1) return fail(GCS_E_INVALID, "slot %d: type %d is neither point (0) nor line (1)", s, d->slot_is_line[s]);
     for (long long s = 0; s < nseg; ++s) {
         const int kind = (int)(s % kKinds) + 1;
         for (long long r = d->offsets[s]; r < d->offsets[s + 1]; ++r) {
             const gcs_b200_program_row& row = d->rows[r];
-            if (row.solver < 1 || row.solver > 8) return failf(GCS_E_INVALID, "row %lld: unknown solver id %d", r, row.solver);
+            if (row.solver < 1 || row.solver > 8) return fail(GCS_E_INVALID, "row %lld: unknown solver id %d", r, row.solver);
             if (kKindOfSolver[row.solver] != kind)
-                return failf(GCS_E_INVALID, "row %lld: solver %d (kind %d) in a kind-%d segment", r, row.solver, kKindOfSolver[row.solver], kind);
-            if (row.code < 0 || row.code > 255) return failf(GCS_E_INVALID, "row %lld: code %d out of range", r, row.code);
+                return fail(GCS_E_INVALID, "row %lld: solver %d (kind %d) in a kind-%d segment", r, row.solver, kKindOfSolver[row.solver], kind);
+            if (row.code < 0 || row.code > 255) return fail(GCS_E_INVALID, "row %lld: code %d out of range", r, row.code);
             for (int q = 0; q < 3; ++q) {
                 const int e = row.elem[q];
-                if (e < 0 || e >= d->n_slots) return failf(GCS_E_INVALID, "row %lld: element slot %d out of range (%d slots)", r, e, d->n_slots);
+                if (e < 0 || e >= d->n_slots) return fail(GCS_E_INVALID, "row %lld: element slot %d out of range (%d slots)", r, e, d->n_slots);
                 if ((d->slot_is_line[e] != 0) != kRoleIsLine[row.solver][q])
-                    return failf(GCS_E_INVALID, "row %lld: slot %d of role %c has the wrong element type for solver %d", r, e, 'a' + q, row.solver);
+                    return fail(GCS_E_INVALID, "row %lld: slot %d of role %c has the wrong element type for solver %d", r, e, 'a' + q, row.solver);
                 const int v = row.value[q];
                 if (!kReads[row.solver][q]) {
-                    if (v != -1) return failf(GCS_E_INVALID, "row %lld: solver %d reads no v%d, value slot must be -1 (got %d)", r, row.solver, q, v);
+                    if (v != -1) return fail(GCS_E_INVALID, "row %lld: solver %d reads no v%d, value slot must be -1 (got %d)", r, row.solver, q, v);
                     continue;
                 }
-                if (v < 0 || v >= d->n_values) return failf(GCS_E_INVALID, "row %lld: value slot %d out of range (%d values)", r, v, d->n_values);
+                if (v < 0 || v >= d->n_values) return fail(GCS_E_INVALID, "row %lld: value slot %d out of range (%d values)", r, v, d->n_values);
                 const bool cosine = q == 0 && (row.solver == 3 || row.solver == 8);
                 if ((d->value_is_angle[v] != 0) != cosine)
-                    return failf(GCS_E_INVALID, "row %lld: value slot %d is %s an angle slot, v%d of solver %d needs %s", r, v,
+                    return fail(GCS_E_INVALID, "row %lld: value slot %d is %s an angle slot, v%d of solver %d needs %s", r, v,
                         d->value_is_angle[v] ? "" : "not", q, row.solver, cosine ? "one" : "a distance");
             }
             if (row.elem[0] == row.elem[1] || row.elem[0] == row.elem[2] || row.elem[1] == row.elem[2])
-                return failf(GCS_E_INVALID, "row %lld: the three roles need three distinct slots", r);
+                return fail(GCS_E_INVALID, "row %lld: the three roles need three distinct slots", r);
         }
     }
     // The footprint rule of the wave plan (makePlan, host/src/b200/leaf_batch.cpp): within one wave
@@ -547,7 +499,7 @@ int validate_desc(const gcs_b200_program_desc* d)
                 const size_t e = (size_t)row.elem[q];
                 const bool writes = zero_fixed || q == 2;
                 if (wave_of[e] == wave && (writes || wrote[e]))
-                    return failf(GCS_E_INVALID, "wave %d: slot %d is %s by row %lld and %s by row %lld; rows of one wave run concurrently", wave,
+                    return fail(GCS_E_INVALID, "wave %d: slot %d is %s by row %lld and %s by row %lld; rows of one wave run concurrently", wave,
                         (int)e, wrote[e] ? "written" : "read", row_of[e], writes ? "written" : "read", r);
                 if (wave_of[e] != wave || writes) wave_of[e] = wave, row_of[e] = r, wrote[e] = writes;
             }
@@ -569,8 +521,8 @@ struct DeviceBuffer {
     {
         if (need <= bytes) return GCS_OK;
         if (ptr) {
-            PROG_TRY(cudaStreamSynchronize(st));
-            PROG_TRY(cudaFree(ptr));
+            CUDA_TRY(cudaStreamSynchronize(st));
+            CUDA_TRY(cudaFree(ptr));
             ptr = nullptr, bytes = 0;
         }
         if (cudaMalloc(&ptr, need) != cudaSuccess) {
@@ -581,7 +533,7 @@ struct DeviceBuffer {
             va_start(ap, what);
             vsnprintf(buf, sizeof(buf), what, ap);
             va_end(ap);
-            return failf(GCS_E_NOMEM, "cudaMalloc(%zu) for %s failed", need, buf);
+            return fail(GCS_E_NOMEM, "cudaMalloc(%zu) for %s failed", need, buf);
         }
         bytes = need;
         return GCS_OK;
@@ -651,19 +603,6 @@ size_t batches_bytes(const long long cap[kKinds], bool cand)
     return bytes;
 }
 
-struct CurrentDevice {
-    int prev = -1;
-    explicit CurrentDevice(int dev)
-    {
-        if (cudaGetDevice(&prev) != cudaSuccess) cudaGetLastError(), prev = -1;
-        if (prev != dev) cudaSetDevice(dev);
-    }
-    ~CurrentDevice()
-    {
-        if (prev >= 0) cudaSetDevice(prev);
-    }
-};
-
 // the kind batches of one wave (or of the scratch) laid out from `at` with `cap[k]` sub-systems of
 // kind k + 1
 void bind_batches(WaveArgs& w, unsigned char* at, const long long cap[kKinds], bool cand)
@@ -712,25 +651,13 @@ void bind_wave(const gcs_b200_program* p, WaveArgs& w, int wave, const std::vect
     }
 }
 
-// Launches `kernel` on `st` over `threads` threads (nothing when there are none) and counts the
-// launch.  A grid beyond 31 bits fails, naming the work (`what`, printf-style).
-template <class A>
-int launch(void (*kernel)(A), long long threads, cudaStream_t st, const A& args, const char* what, ...)
+// Launches `kernel` on `st` over `threads` threads, nothing when there are none.  too_many(): the
+// failure when they need a grid beyond 31 bits.
+template <class A, class TooMany>
+int launch(void (*kernel)(A), long long threads, cudaStream_t st, const A& args, TooMany&& too_many)
 {
     if (threads == 0) return GCS_OK;
-    const long long grid = (threads + kThreads - 1) / kThreads;
-    if (grid > 0x7fffffffLL) {
-        char buf[300];
-        va_list ap;
-        va_start(ap, what);
-        vsnprintf(buf, sizeof(buf), what, ap);
-        va_end(ap);
-        return failf(GCS_E_INVALID, "%s are too many for one launch", buf);
-    }
-    kernel<<<(unsigned)grid, kThreads, 0, st>>>(args);
-    gcsk::api_count_launch();
-    PROG_TRY(cudaGetLastError());
-    return GCS_OK;
+    return gcsk::launch_kernel(kernel, (threads + kThreads - 1) / kThreads, kThreads, 0, st, too_many, args);
 }
 
 // T = 0: a plain run.  T > 0: also the tangents along T directions (dvalues / dpositions).
@@ -748,33 +675,34 @@ int run_on(gcs_b200_program* p, long long K, const double* values, double* posit
     if (recorded) {
         p->recorded_k = 0;  // until this run is enqueued whole
         tape_at = tape_layout(p, K);
-        PROG_RC(p->tape.grow(tape_at.back(), st, "the tape of a recorded run of %lld instances", K));
+        RC_TRY(p->tape.grow(tape_at.back(), st, "the tape of a recorded run of %lld instances", K));
     } else {
         // K instances of every kind's largest wave
         long long cap[kKinds];
         for (int k = 1; k <= kKinds; ++k) cap[k - 1] = kind_cap(p, k, K);
-        PROG_RC(p->scratch.grow(batches_bytes(cap, T > 0), st, "the kind batches of %lld instances", K));
+        RC_TRY(p->scratch.grow(batches_bytes(cap, T > 0), st, "the kind batches of %lld instances", K));
         bind_batches(w, p->scratch.ptr, cap, T > 0);
     }
     // every instance starts from the initial positions: one copy, then doubling copies
     const size_t table = (size_t)p->n_slots * 4 * sizeof(double);
     if (table) {
-        PROG_TRY(cudaMemcpyAsync(positions, p->initial, table, cudaMemcpyDeviceToDevice, st));
+        CUDA_TRY(cudaMemcpyAsync(positions, p->initial, table, cudaMemcpyDeviceToDevice, st));
         for (long long have = 1; have < K;) {
             const long long n = have < K - have ? have : K - have;
-            PROG_TRY(cudaMemcpyAsync(reinterpret_cast<unsigned char*>(positions) + (size_t)have * table, positions, (size_t)n * table,
+            CUDA_TRY(cudaMemcpyAsync(reinterpret_cast<unsigned char*>(positions) + (size_t)have * table, positions, (size_t)n * table,
                 cudaMemcpyDeviceToDevice, st));
             have += n;
         }
     }
-    if (nonconverged) PROG_TRY(cudaMemsetAsync(nonconverged, 0, (size_t)K * sizeof(uint32_t), st));
+    if (nonconverged) CUDA_TRY(cudaMemsetAsync(nonconverged, 0, (size_t)K * sizeof(uint32_t), st));
     // every slot's tangent is 0 before the first wave: the initial positions are constants
-    if (T > 0 && table) PROG_TRY(cudaMemsetAsync(dpositions, 0, (size_t)K * T * table, st));
+    if (T > 0 && table) CUDA_TRY(cudaMemsetAsync(dpositions, 0, (size_t)K * T * table, st));
     for (int wave = 0; wave < p->n_waves; ++wave) {
         bind_wave(p, w, wave, recorded ? &tape_at : nullptr);
         const long long subs = w.seg[kKinds] * K;
         if (subs == 0) continue;
-        PROG_RC(launch(program_gather_kernel, subs, st, w, "wave %d: %lld sub-systems", wave, subs));
+        const auto too_many = [&] { return fail(GCS_E_INVALID, "wave %d: %lld sub-systems are too many for one launch", wave, subs); };
+        RC_TRY(launch(program_gather_kernel, subs, st, w, too_many));
         gcs_b200_batch batch[kKinds];
         const gcs_b200_batch* list[kKinds];
         int count = 0;
@@ -790,10 +718,12 @@ int run_on(gcs_b200_program* p, long long K, const double* values, double* posit
             b.code = w.code[k - 1], b.root_index = w.root[k - 1], b.converged = w.conv[k - 1], b.cand = w.cand[k - 1];
             list[count++] = &b;
         }
-        PROG_RC(gcs_b200_solve_many(list, count, p->device, st));
-        PROG_RC(launch(program_scatter_kernel, subs, st, w, "wave %d: %lld sub-systems", wave, subs));
+        RC_TRY(gcs_b200_solve_many(list, count, p->device, st));
+        RC_TRY(launch(program_scatter_kernel, subs, st, w, too_many));
         if (T > 0)
-            PROG_RC(launch(program_tangent_kernel, subs * T, st, w, "wave %d: %lld sub-systems x %lld directions", wave, subs, T));
+            RC_TRY(launch(program_tangent_kernel, subs * T, st, w, [&] {
+                return fail(GCS_E_INVALID, "wave %d: %lld sub-systems x %lld directions are too many for one launch", wave, subs, T);
+            }));
     }
     if (recorded) p->recorded_k = K;
     return GCS_OK;
@@ -806,9 +736,9 @@ int ensure_adjoint_tables(gcs_b200_program* p, long long T, cudaStream_t st)
     const size_t pbytes = (size_t)KT * p->n_slots * 4 * sizeof(double), cbytes = (size_t)KT * p->max_wave_rows * 11 * sizeof(double);
     const size_t vbytes = (size_t)KT * p->n_values * sizeof(double);
     const char* what = "the %s of %lld instances x %lld cotangents";
-    PROG_RC(p->apos.grow(pbytes, st, what, "slot adjoints", K, T));
-    PROG_RC(p->contrib.grow(cbytes, st, what, "adjoint contributions", K, T));
-    PROG_RC(p->flags.grow((size_t)KT, st, what, "NaN flags", K, T));
+    RC_TRY(p->apos.grow(pbytes, st, what, "slot adjoints", K, T));
+    RC_TRY(p->contrib.grow(cbytes, st, what, "adjoint contributions", K, T));
+    RC_TRY(p->flags.grow((size_t)KT, st, what, "NaN flags", K, T));
     return p->avalues.grow(vbytes, st, what, "value adjoints", K, T);
 }
 
@@ -817,8 +747,8 @@ int ensure_adjoint_tables(gcs_b200_program* p, long long T, cudaStream_t st)
 int sweep_on(gcs_b200_program* p, long long T, double* adj_values, cudaStream_t st)
 {
     const long long K = p->recorded_k, KT = K * T;
-    if (p->n_values) PROG_TRY(cudaMemsetAsync(adj_values, 0, (size_t)KT * p->n_values * sizeof(double), st));
-    PROG_TRY(cudaMemsetAsync(p->flags.ptr, 0, (size_t)KT, st));
+    if (p->n_values) CUDA_TRY(cudaMemsetAsync(adj_values, 0, (size_t)KT * p->n_values * sizeof(double), st));
+    CUDA_TRY(cudaMemsetAsync(p->flags.ptr, 0, (size_t)KT, st));
     const std::vector<size_t> tape_at = tape_layout(p, K);
     WaveArgs w;
     memset(&w, 0, sizeof(w));
@@ -837,31 +767,34 @@ int sweep_on(gcs_b200_program* p, long long T, double* adj_values, cudaStream_t 
         r.begin = p->begin + p->ent_off[(size_t)wave];
         r.readers = p->readers;
         r.n_ent = p->ent_off[(size_t)wave + 1] - p->ent_off[(size_t)wave];
-        const char* what = "wave %d: %lld sub-systems x %lld cotangents";
-        PROG_RC(launch(program_adjoint_kernel, subs * T, st, w, what, wave, subs, T));
-        PROG_RC(launch(program_adjoint_reduce_kernel, r.n_ent * KT, st, r, what, wave, subs, T));
+        const auto too_many = [&] {
+            return fail(GCS_E_INVALID, "wave %d: %lld sub-systems x %lld cotangents are too many for one launch", wave, subs, T);
+        };
+        RC_TRY(launch(program_adjoint_kernel, subs * T, st, w, too_many));
+        RC_TRY(launch(program_adjoint_reduce_kernel, r.n_ent * KT, st, r, too_many));
     }
-    return launch(program_adjoint_flag_kernel, KT * p->n_values, st, r, "%lld value adjoints", KT * p->n_values);
+    return launch(program_adjoint_flag_kernel, KT * p->n_values, st, r,
+        [&] { return fail(GCS_E_INVALID, "%lld value adjoints are too many for one launch", KT * p->n_values); });
 }
 
 // the checks that need no program come first; a null table is refused unless the program has
 // nothing to put in it
 int check_adjoints(const gcs_b200_program* p, int T, const double* adj_positions, const double* adj_values)
 {
-    if (T < 1) return failf(GCS_E_INVALID, "n_cotangents must be >= 1 (got %d)", T);
+    if (T < 1) return fail(GCS_E_INVALID, "n_cotangents must be >= 1 (got %d)", T);
     if ((!adj_positions && !(p && p->n_slots == 0)) || (!adj_values && !(p && p->n_values == 0)))
-        return failf(GCS_E_INVALID, "null adjoint table (adj_positions or adj_values)");
-    if (!p) return failf(GCS_E_INVALID, "null program");
-    if (p->recorded_k < 1) return failf(GCS_E_INVALID, "no recorded run: call gcs_b200_program_run_recorded first");
+        return fail(GCS_E_INVALID, "null adjoint table (adj_positions or adj_values)");
+    if (!p) return fail(GCS_E_INVALID, "null program");
+    if (p->recorded_k < 1) return fail(GCS_E_INVALID, "no recorded run: call gcs_b200_program_run_recorded first");
     return GCS_OK;
 }
 
 int check_run(const gcs_b200_program* p, long long K, const double* values, const double* positions, int variant)
 {
-    if (!p) return failf(GCS_E_INVALID, "null program");
-    if (K < 1) return failf(GCS_E_INVALID, "n_instances must be >= 1 (got %lld)", K);
-    if ((p->n_values > 0 && !values) || (p->n_slots > 0 && !positions)) return failf(GCS_E_INVALID, "null value or position table");
-    if (variant < GCS_VARIANT_DEFAULT || variant > GCS_VARIANT_CONTRACTED_LINEAR) return failf(GCS_E_INVALID, "unknown variant %d", variant);
+    if (!p) return fail(GCS_E_INVALID, "null program");
+    if (K < 1) return fail(GCS_E_INVALID, "n_instances must be >= 1 (got %lld)", K);
+    if ((p->n_values > 0 && !values) || (p->n_slots > 0 && !positions)) return fail(GCS_E_INVALID, "null value or position table");
+    if (variant < GCS_VARIANT_DEFAULT || variant > GCS_VARIANT_CONTRACTED_LINEAR) return fail(GCS_E_INVALID, "unknown variant %d", variant);
     return GCS_OK;
 }
 
@@ -870,10 +803,10 @@ int check_run(const gcs_b200_program* p, long long K, const double* values, cons
 int check_tangent_run(const gcs_b200_program* p, long long K, const double* values, const double* positions, int T,
     const double* dvalues, const double* dpositions, int variant)
 {
-    if (T < 1) return failf(GCS_E_INVALID, "n_tangents must be >= 1 (got %d)", T);
-    if (variant < GCS_VARIANT_DEFAULT || variant > GCS_VARIANT_CONTRACTED_LINEAR) return failf(GCS_E_INVALID, "unknown variant %d", variant);
+    if (T < 1) return fail(GCS_E_INVALID, "n_tangents must be >= 1 (got %d)", T);
+    if (variant < GCS_VARIANT_DEFAULT || variant > GCS_VARIANT_CONTRACTED_LINEAR) return fail(GCS_E_INVALID, "unknown variant %d", variant);
     if ((!dvalues && !(p && p->n_values == 0)) || (!dpositions && !(p && p->n_slots == 0)))
-        return failf(GCS_E_INVALID, "null tangent table (dvalues or dpositions)");
+        return fail(GCS_E_INVALID, "null tangent table (dvalues or dpositions)");
     return check_run(p, K, values, positions, variant);
 }
 
@@ -890,22 +823,22 @@ template <class Work>
 int on_host(gcs_b200_program* p, std::initializer_list<Copy> up, Work&& work, std::initializer_list<Copy> down, float ms[3])
 {
     const cudaStream_t st = p->stream;
-    PROG_TRY(cudaEventRecord(p->ev[0], st));
+    CUDA_TRY(cudaEventRecord(p->ev[0], st));
     for (const Copy& c : up)
-        if (c.bytes) PROG_TRY(cudaMemcpyAsync(c.dst, c.src, c.bytes, cudaMemcpyHostToDevice, st));
-    PROG_TRY(cudaEventRecord(p->ev[1], st));
+        if (c.bytes) CUDA_TRY(cudaMemcpyAsync(c.dst, c.src, c.bytes, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaEventRecord(p->ev[1], st));
     const int rc = work(st);
     if (rc != GCS_OK) {
         cudaStreamSynchronize(st);
         return rc;
     }
-    PROG_TRY(cudaEventRecord(p->ev[2], st));
+    CUDA_TRY(cudaEventRecord(p->ev[2], st));
     for (const Copy& c : down)
-        if (c.bytes) PROG_TRY(cudaMemcpyAsync(c.dst, c.src, c.bytes, cudaMemcpyDeviceToHost, st));
-    PROG_TRY(cudaEventRecord(p->ev[3], st));
-    PROG_TRY(cudaStreamSynchronize(st));
+        if (c.bytes) CUDA_TRY(cudaMemcpyAsync(c.dst, c.src, c.bytes, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaEventRecord(p->ev[3], st));
+    CUDA_TRY(cudaStreamSynchronize(st));
     if (ms)
-        for (int q = 0; q < 3; ++q) PROG_TRY(cudaEventElapsedTime(&ms[q], p->ev[q], p->ev[q + 1]));
+        for (int q = 0; q < 3; ++q) CUDA_TRY(cudaEventElapsedTime(&ms[q], p->ev[q], p->ev[q + 1]));
     return GCS_OK;
 }
 
@@ -916,11 +849,11 @@ int run_host(gcs_b200_program* p, long long K, const double* values, double* pos
     const size_t vbytes = (size_t)K * p->n_values * sizeof(double), pbytes = (size_t)K * p->n_slots * 4 * sizeof(double);
     const size_t cbytes = (size_t)K * sizeof(uint32_t);
     const cudaStream_t st = p->stream;
-    PROG_RC(p->values.grow(vbytes, st, "the values of %lld instances", K));
-    PROG_RC(p->positions.grow(pbytes, st, "the positions of %lld instances", K));
-    PROG_RC(p->counts.grow(cbytes, st, "the nonconverged counts of %lld instances", K));
-    PROG_RC(p->dvalues.grow(vbytes * T, st, "the value tangents of %lld instances x %lld directions", K, T));
-    PROG_RC(p->dpositions.grow(pbytes * T, st, "the position tangents of %lld instances x %lld directions", K, T));
+    RC_TRY(p->values.grow(vbytes, st, "the values of %lld instances", K));
+    RC_TRY(p->positions.grow(pbytes, st, "the positions of %lld instances", K));
+    RC_TRY(p->counts.grow(cbytes, st, "the nonconverged counts of %lld instances", K));
+    RC_TRY(p->dvalues.grow(vbytes * T, st, "the value tangents of %lld instances x %lld directions", K, T));
+    RC_TRY(p->dpositions.grow(pbytes * T, st, "the position tangents of %lld instances x %lld directions", K, T));
     return on_host(p, { { p->values.ptr, values, vbytes }, { p->dvalues.ptr, dvalues, vbytes * T } },
         [&](cudaStream_t s) {
             return run_on(p, K, p->values.ptr, p->positions.ptr, nonconverged ? p->counts.ptr : nullptr, variant, s, T, p->dvalues.ptr,
@@ -937,14 +870,15 @@ extern "C" {
 
 int gcs_b200_program_create(const gcs_b200_program_desc* d, int device, gcs_b200_program** out)
 {
-    if (!out) return failf(GCS_E_INVALID, "null output handle");
+    if (!out) return fail(GCS_E_INVALID, "null output handle");
     *out = nullptr;
     int rc = validate_desc(d);
     if (rc != GCS_OK) return rc;
     const int ndev = gcs_b200_device_count();
-    if (ndev <= 0) return failf(GCS_E_NO_DEVICE, "no CUDA device; this library has no CPU fallback");
-    if (device < 0 || device >= ndev) return failf(GCS_E_NO_DEVICE, "device %d out of range (%d present)", device, ndev);
-    CurrentDevice cur(device);
+    if (ndev <= 0) return fail(GCS_E_NO_DEVICE, "no CUDA device; this library has no CPU fallback");
+    if (device < 0 || device >= ndev) return fail(GCS_E_NO_DEVICE, "device %d out of range (%d present)", device, ndev);
+    DeviceScope on(device);
+    RC_TRY(on.rc);
     auto* p = new gcs_b200_program();
     p->device = device, p->n_waves = d->n_waves, p->n_slots = d->n_slots, p->n_values = d->n_values, p->n_rows = d->n_rows;
     p->offsets.assign(d->offsets, d->offsets + (size_t)d->n_waves * kKinds + 1);
@@ -957,13 +891,13 @@ int gcs_b200_program_create(const gcs_b200_program_desc* d, int device, gcs_b200
         gcs_b200_program_destroy(p);
         return code;
     };
-    if (cudaStreamCreateWithFlags(&p->stream, cudaStreamNonBlocking) != cudaSuccess) return bail(failf(GCS_E_CUDA, "stream creation failed"));
+    if (cudaStreamCreateWithFlags(&p->stream, cudaStreamNonBlocking) != cudaSuccess) return bail(fail(GCS_E_CUDA, "stream creation failed"));
     for (auto& e : p->ev)
-        if (cudaEventCreate(&e) != cudaSuccess) return bail(failf(GCS_E_CUDA, "event creation failed"));
+        if (cudaEventCreate(&e) != cudaSuccess) return bail(fail(GCS_E_CUDA, "event creation failed"));
     const size_t row_bytes = (size_t)d->n_rows * sizeof(gcs_b200_program_row), init_bytes = (size_t)d->n_slots * 4 * sizeof(double);
     if ((row_bytes && cudaMalloc(&p->rows, row_bytes) != cudaSuccess) || (init_bytes && cudaMalloc(&p->initial, init_bytes) != cudaSuccess)) {
         cudaGetLastError();
-        return bail(failf(GCS_E_NOMEM, "cudaMalloc for a program of %lld rows and %d slots failed", (long long)d->n_rows, d->n_slots));
+        return bail(fail(GCS_E_NOMEM, "cudaMalloc for a program of %lld rows and %d slots failed", (long long)d->n_rows, d->n_slots));
     }
     // The reader lists of the adjoint sweep.  Per wave, every slot read (roles a, b of solvers 4-8)
     // and every value read gets one entry, slots first; its readers, (row, role) for a slot and (row,
@@ -1010,7 +944,7 @@ int gcs_b200_program_create(const gcs_b200_program_desc* d, int device, gcs_b200
     if ((ent_bytes && cudaMalloc(&p->ent, ent_bytes) != cudaSuccess) || cudaMalloc(&p->begin, begin_bytes) != cudaSuccess
         || (reader_bytes && cudaMalloc(&p->readers, reader_bytes) != cudaSuccess)) {
         cudaGetLastError();
-        return bail(failf(GCS_E_NOMEM, "cudaMalloc for the reader lists of %zu entries failed", ent.size()));
+        return bail(fail(GCS_E_NOMEM, "cudaMalloc for the reader lists of %zu entries failed", ent.size()));
     }
     if ((row_bytes && cudaMemcpyAsync(p->rows, d->rows, row_bytes, cudaMemcpyHostToDevice, p->stream) != cudaSuccess)
         || (init_bytes && cudaMemcpyAsync(p->initial, d->initial, init_bytes, cudaMemcpyHostToDevice, p->stream) != cudaSuccess)
@@ -1018,7 +952,7 @@ int gcs_b200_program_create(const gcs_b200_program_desc* d, int device, gcs_b200
         || cudaMemcpyAsync(p->begin, begin.data(), begin_bytes, cudaMemcpyHostToDevice, p->stream) != cudaSuccess
         || (reader_bytes && cudaMemcpyAsync(p->readers, readers.data(), reader_bytes, cudaMemcpyHostToDevice, p->stream) != cudaSuccess)
         || cudaStreamSynchronize(p->stream) != cudaSuccess)
-        return bail(failf(GCS_E_CUDA, "program upload failed: %s", cudaGetErrorString(cudaGetLastError())));
+        return bail(fail(GCS_E_CUDA, "program upload failed: %s", cudaGetErrorString(cudaGetLastError())));
     *out = p;
     return GCS_OK;
 }
@@ -1026,67 +960,75 @@ int gcs_b200_program_create(const gcs_b200_program_desc* d, int device, gcs_b200
 int gcs_b200_program_run(gcs_b200_program* p, int64_t K, const double* values, double* positions, uint32_t* nonconverged, int variant,
     void* stream)
 {
-    PROG_RC(check_run(p, K, values, positions, variant));
-    CurrentDevice cur(p->device);
+    RC_TRY(check_run(p, K, values, positions, variant));
+    DeviceScope on(p->device);
+    RC_TRY(on.rc);
     return run_on(p, K, values, positions, nonconverged, variant, static_cast<cudaStream_t>(stream));
 }
 
 int gcs_b200_program_run_host(gcs_b200_program* p, int64_t K, const double* values, double* positions, uint32_t* nonconverged,
     int variant, float ms[3])
 {
-    PROG_RC(check_run(p, K, values, positions, variant));
-    CurrentDevice cur(p->device);
+    RC_TRY(check_run(p, K, values, positions, variant));
+    DeviceScope on(p->device);
+    RC_TRY(on.rc);
     return run_host(p, K, values, positions, nonconverged, variant, ms);
 }
 
 int gcs_b200_program_run_tangents(gcs_b200_program* p, int64_t K, const double* values, double* positions, uint32_t* nonconverged,
     int32_t T, const double* dvalues, double* dpositions, int variant, void* stream)
 {
-    PROG_RC(check_tangent_run(p, K, values, positions, T, dvalues, dpositions, variant));
-    CurrentDevice cur(p->device);
+    RC_TRY(check_tangent_run(p, K, values, positions, T, dvalues, dpositions, variant));
+    DeviceScope on(p->device);
+    RC_TRY(on.rc);
     return run_on(p, K, values, positions, nonconverged, variant, static_cast<cudaStream_t>(stream), T, dvalues, dpositions);
 }
 
 int gcs_b200_program_run_tangents_host(gcs_b200_program* p, int64_t K, const double* values, double* positions,
     uint32_t* nonconverged, int32_t T, const double* dvalues, double* dpositions, int variant, float ms[3])
 {
-    PROG_RC(check_tangent_run(p, K, values, positions, T, dvalues, dpositions, variant));
-    CurrentDevice cur(p->device);
+    RC_TRY(check_tangent_run(p, K, values, positions, T, dvalues, dpositions, variant));
+    DeviceScope on(p->device);
+    RC_TRY(on.rc);
     return run_host(p, K, values, positions, nonconverged, variant, ms, T, dvalues, dpositions);
 }
 
 int gcs_b200_program_run_recorded(gcs_b200_program* p, int64_t K, const double* values, double* positions, uint32_t* nonconverged,
     int variant, void* stream)
 {
-    PROG_RC(check_run(p, K, values, positions, variant));
-    CurrentDevice cur(p->device);
+    RC_TRY(check_run(p, K, values, positions, variant));
+    DeviceScope on(p->device);
+    RC_TRY(on.rc);
     return run_on(p, K, values, positions, nonconverged, variant, static_cast<cudaStream_t>(stream), 0, nullptr, nullptr, true);
 }
 
 int gcs_b200_program_run_recorded_host(gcs_b200_program* p, int64_t K, const double* values, double* positions,
     uint32_t* nonconverged, int variant, float ms[3])
 {
-    PROG_RC(check_run(p, K, values, positions, variant));
-    CurrentDevice cur(p->device);
+    RC_TRY(check_run(p, K, values, positions, variant));
+    DeviceScope on(p->device);
+    RC_TRY(on.rc);
     return run_host(p, K, values, positions, nonconverged, variant, ms, 0, nullptr, nullptr, true);
 }
 
 int gcs_b200_program_adjoints(gcs_b200_program* p, int32_t T, const double* adj_positions, double* adj_values, void* stream)
 {
-    PROG_RC(check_adjoints(p, T, adj_positions, adj_values));
-    CurrentDevice cur(p->device);
+    RC_TRY(check_adjoints(p, T, adj_positions, adj_values));
+    DeviceScope on(p->device);
+    RC_TRY(on.rc);
     const cudaStream_t st = static_cast<cudaStream_t>(stream);
-    PROG_RC(ensure_adjoint_tables(p, T, st));
+    RC_TRY(ensure_adjoint_tables(p, T, st));
     const size_t pbytes = (size_t)p->recorded_k * T * p->n_slots * 4 * sizeof(double);
-    if (pbytes) PROG_TRY(cudaMemcpyAsync(p->apos.ptr, adj_positions, pbytes, cudaMemcpyDeviceToDevice, st));
+    if (pbytes) CUDA_TRY(cudaMemcpyAsync(p->apos.ptr, adj_positions, pbytes, cudaMemcpyDeviceToDevice, st));
     return sweep_on(p, T, adj_values, st);
 }
 
 int gcs_b200_program_adjoints_host(gcs_b200_program* p, int32_t T, const double* adj_positions, double* adj_values, float ms[3])
 {
-    PROG_RC(check_adjoints(p, T, adj_positions, adj_values));
-    CurrentDevice cur(p->device);
-    PROG_RC(ensure_adjoint_tables(p, T, p->stream));
+    RC_TRY(check_adjoints(p, T, adj_positions, adj_values));
+    DeviceScope on(p->device);
+    RC_TRY(on.rc);
+    RC_TRY(ensure_adjoint_tables(p, T, p->stream));
     const size_t pbytes = (size_t)p->recorded_k * T * p->n_slots * 4 * sizeof(double);
     const size_t vbytes = (size_t)p->recorded_k * T * p->n_values * sizeof(double);
     return on_host(p, { { p->apos.ptr, adj_positions, pbytes } }, [&](cudaStream_t st) { return sweep_on(p, T, p->avalues.ptr, st); },
@@ -1097,7 +1039,7 @@ void gcs_b200_program_destroy(gcs_b200_program* p)
 {
     if (!p) return;
     {
-        CurrentDevice cur(p->device);
+        DeviceScope on(p->device);  // released whether or not the switch succeeded
         if (p->stream) cudaStreamSynchronize(p->stream), cudaStreamDestroy(p->stream);
         for (auto e : p->ev)
             if (e) cudaEventDestroy(e);
