@@ -99,6 +99,42 @@ class CProgramDesc(C.Structure):
     ]
 
 
+class CFitDesc(C.Structure):
+    """gcs_b200_fit_desc."""
+    _fields_ = [
+        ("n_free", C.c_int32),
+        ("n_obs", C.c_int32),
+        ("free_values", C.POINTER(C.c_int32)),
+        ("lower", C.POINTER(C.c_double)),
+        ("upper", C.POINTER(C.c_double)),
+        ("obs_slots", C.POINTER(C.c_int32)),
+        ("obs_coords", C.POINTER(C.c_int32)),
+        ("weights", C.POINTER(C.c_double)),
+        ("max_iterations", C.c_int32),
+        ("reserved", C.c_int32),
+        ("lambda0", C.c_double),
+        ("cost_tol", C.c_double),
+        ("ftol", C.c_double),
+        ("xtol", C.c_double),
+        ("gtol", C.c_double),
+    ]
+
+
+class CFitResult(C.Structure):
+    """gcs_b200_fit_result."""
+    _fields_ = [
+        ("status", C.c_int32),
+        ("iterations", C.c_int32),
+        ("cost", C.c_double),
+        ("grad_inf", C.c_double),
+        ("lambda_", C.c_double),
+    ]
+
+
+# gcs_b200_fit_result.status
+FIT_RUNNING, FIT_COST, FIT_GTOL, FIT_FTOL, FIT_XTOL, FIT_STALLED, FIT_START_FAILED = range(7)
+
+
 _PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 # GCS_B200_LIB: developer override to A/B an experimental build of the same library
 LIB_PATH = os.environ.get("GCS_B200_LIB") or os.path.join(_PKG_DIR, "libgcs_b200.so")
@@ -115,7 +151,7 @@ EXPORTS = [
     "gcs_b200_program_create", "gcs_b200_program_run", "gcs_b200_program_run_host", "gcs_b200_program_destroy",
     "gcs_b200_program_run_tangents", "gcs_b200_program_run_tangents_host",
     "gcs_b200_program_run_recorded", "gcs_b200_program_run_recorded_host", "gcs_b200_program_adjoints",
-    "gcs_b200_program_adjoints_host",
+    "gcs_b200_program_adjoints_host", "gcs_b200_program_fit", "gcs_b200_program_fit_host", "gcs_b200_fit_check",
 ]
 
 
@@ -174,6 +210,11 @@ def load():
                                                        C.POINTER(C.c_float)]
     lib.gcs_b200_program_adjoints.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.gcs_b200_program_adjoints_host.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.POINTER(C.c_float)]
+    lib.gcs_b200_program_fit.argtypes = [C.c_void_p, C.POINTER(CFitDesc), C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                         C.c_void_p, C.c_int, C.c_void_p]
+    lib.gcs_b200_program_fit_host.argtypes = [C.c_void_p, C.POINTER(CFitDesc), C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
+                                              C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_float)]
+    lib.gcs_b200_fit_check.argtypes = [C.POINTER(CProgramDesc), C.POINTER(CFitDesc)]
     lib.gcs_b200_program_destroy.argtypes = [C.c_void_p]
     _lib = lib
     return lib

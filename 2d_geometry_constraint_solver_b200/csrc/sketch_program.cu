@@ -30,6 +30,7 @@
 // atomics: the result does not depend on K, the stream or the schedule.
 #include <cuda_runtime.h>
 
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
@@ -437,6 +438,220 @@ __global__ void __launch_bounds__(kThreads) program_adjoint_flag_kernel(const Re
     if (r.flag[j * r.T + t]) r.aval[g] = __longlong_as_double(0x7ff8000000000000LL);
 }
 
+// ---- fitting values to targets (gcs_b200_program_fit) ----
+// Per instance the working state is one row of `work`, `stride` = 3 n^2 + 5 n + 3 doubles (n = n_free):
+// x, xt (trial), x0 (the caller's start), g, gt [n], A, At [n][n] (upper triangle used), L [n][n]
+// (Cholesky factor, lower), c, ct, failed.  The trial's (xt, At, gt, ct, failed) come from the
+// tangent run at xt and program_fit_normal_kernel.
+constexpr int kFitPoll = 4;  // gcs_b200_program_fit_host reads the running count every kFitPoll iterations
+
+struct FitArgs {
+    long long K, n, n_obs, n_values, n_slots, stride;
+    const double* lo;          // [n] box, intersected with [-1, 1] for an angle slot
+    const double* hi;
+    const double* w;           // [n_obs]
+    const int32_t* free;       // [n] value slots
+    const int32_t* obs;        // [n_obs] slot * 4 + coordinate
+    double* val;               // [K][n_values], the runs' value table
+    double* dval;              // [K][n_values][n]: the selector
+    const double* pos;         // [K][n_slots][4] of the last tangent run
+    const double* dpos;        // [K][n_slots][4][n]
+    const uint32_t* nc;        // [K]
+    const double* target;      // [K][n_obs]
+    double* work;              // [K][stride]
+    gcs_b200_fit_result* res;  // [K]
+    uint32_t* running;         // [max_iterations + 1]: instances still running after iteration it
+    int it, last, max_it;
+    double lambda0, cost_tol, ftol, xtol, gtol;
+};
+
+struct FitState {
+    double *x, *xt, *x0, *g, *gt, *A, *At, *L, *c;  // c[0] = c, c[1] = ct, c[2] = failed
+    __device__ FitState(const FitArgs& f, long long k)
+    {
+        const long long n = f.n;
+        x = f.work + k * f.stride, xt = x + n, x0 = xt + n, g = x0 + n, gt = g + n, A = gt + n, At = A + n * n, L = At + n * n;
+        c = L + n * n;
+    }
+};
+
+// x clamped into [lo, hi]; NaN stays NaN
+__device__ __forceinline__ double clamp_box(double x, double lo, double hi) { return x < lo ? lo : (x > hi ? hi : x); }
+
+// One thread per max(K x n_values x n, max_iterations + 1): the selector dvalues[k][v][t] = (v ==
+// free[t]); for the first K x n threads, x0 = the caller's value, x = xt = clamp_box(x0) written back
+// into the value table; for the first K, a RUNNING result with lambda0; the running counts zeroed.
+__global__ void __launch_bounds__(kThreads) program_fit_start_kernel(const FitArgs f)
+{
+    const long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const long long n = f.n;
+    if (g < f.K * f.n_values * n) f.dval[g] = (g / n) % f.n_values == f.free[g % n] ? 1.0 : 0.0;
+    if (g < f.K * n) {
+        const long long k = g / n, i = g % n;
+        FitState s(f, k);
+        double& v = f.val[k * f.n_values + f.free[i]];
+        s.x0[i] = v;
+        s.x[i] = s.xt[i] = v = clamp_box(v, f.lo[i], f.hi[i]);
+    }
+    if (g < f.K) {
+        const double nan = __longlong_as_double(0x7ff8000000000000LL);
+        f.res[g] = gcs_b200_fit_result { GCS_FIT_RUNNING, 0, nan, nan, f.lambda0 };
+    }
+    if (g <= f.max_it) f.running[g] = 0;
+}
+
+// One thread per (instance k, entry e), e in [0, P + n] with P = n (n + 1) / 2: e < P is A_ij (i <= j,
+// row-major over the upper triangle), P <= e < P + n is g_{e-P}, e = P + n is c and the failure flag.
+// With r_o = p_o - target_o and J_oi = dpos[k][obs_o][i], every sum runs over o = 0 .. n_obs-1, one
+// term at a time from 0.0:
+//   A_ij = A_ij + (w_o * J_oi) * J_oj,   g_i = g_i + (w_o * J_oi) * r_o,   c = c + (w_o * r_o) * r_o
+// failed: nonconverged[k] > 0, or some observed p_o or J_oi is not finite.
+__global__ void __launch_bounds__(kThreads) program_fit_normal_kernel(const FitArgs f)
+{
+    const long long n = f.n, P = n * (n + 1) / 2, E = P + n + 1;
+    const long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (g >= f.K * E) return;
+    const long long k = g / E, e = g - k * E;
+    FitState s(f, k);
+    const double* const pos = f.pos + k * f.n_slots * 4;
+    const double* const dpos = f.dpos + k * f.n_slots * 4 * n;
+    const double* const tgt = f.target + k * f.n_obs;
+    if (e < P) {
+        long long i = 0, r = e;
+        while (r >= n - i) r -= n - i, ++i;
+        const long long j = i + r;
+        double a = 0.0;
+        for (long long o = 0; o < f.n_obs; ++o) {
+            const double* const J = dpos + f.obs[o] * n;
+            a = a + (f.w[o] * J[i]) * J[j];
+        }
+        s.At[i * n + j] = a;
+    } else if (e < P + n) {
+        const long long i = e - P;
+        double a = 0.0;
+        for (long long o = 0; o < f.n_obs; ++o) a = a + (f.w[o] * dpos[f.obs[o] * n + i]) * (pos[f.obs[o]] - tgt[o]);
+        s.gt[i] = a;
+    } else {
+        double c = 0.0;
+        bool failed = f.nc[k] > 0;
+        for (long long o = 0; o < f.n_obs; ++o) {
+            const double p = pos[f.obs[o]], r = p - tgt[o];
+            c = c + (f.w[o] * r) * r;
+            failed |= !isfinite(p);
+            for (long long i = 0; i < n; ++i) failed |= !isfinite(dpos[f.obs[o] * n + i]);
+        }
+        s.c[1] = c, s.c[2] = failed ? 1.0 : 0.0;
+    }
+}
+
+// L L^T = A + lambda D (A upper, row-major), D_jj = max(A_jj, floor), column by column:
+//   s = A_jj + lambda * D_jj, then s = s - L_jk * L_jk for k = 0 .. j-1; a pivot s that is not > 0
+//   fails; L_jj = sqrt(s); for i > j: s = A_ji, s = s - L_ik * L_jk for k = 0 .. j-1, L_ij = s / L_jj
+__device__ __forceinline__ bool fit_cholesky(const double* A, double lambda, double floor, double* L, long long n)
+{
+    for (long long j = 0; j < n; ++j) {
+        const double ajj = A[j * n + j];
+        double s = ajj + lambda * (ajj > floor ? ajj : floor);
+        for (long long q = 0; q < j; ++q) s = s - L[j * n + q] * L[j * n + q];
+        if (!(s > 0.0)) return false;
+        const double d = sqrt(s);
+        L[j * n + j] = d;
+        for (long long i = j + 1; i < n; ++i) {
+            double t = A[j * n + i];
+            for (long long q = 0; q < j; ++q) t = t - L[i * n + q] * L[j * n + q];
+            L[i * n + j] = t / d;
+        }
+    }
+    return true;
+}
+
+// One thread per instance; a finished instance returns at once (frozen).  In order:
+//   1. iterations += 1.  Iteration 0: a failed trial is START_FAILED (x0 back into the values, done);
+//      otherwise accept.  Later: accept when !failed and ct < c.  Accept: x, g, A, c <- xt, gt, At, ct
+//      and, after iteration 0, lambda = max(lambda / 10, 1e-12); then gi = max_i |g_i| (ascending i,
+//      `a > gi ? a : gi` from 0.0), COST if c <= cost_tol, else GTOL if gi <= gtol, else (after
+//      iteration 0) FTOL if c_old - c <= ftol * c_old.  Reject: lambda = 10 * max(lambda, 1e-12),
+//      STALLED if lambda > 1e16.
+//   2. Still running: floor = 1e-12 * max_j A_jj (as gi, from 0.0); fit_cholesky, and while it fails
+//      lambda = 10 * max(lambda, 1e-12), STALLED once lambda > 1e16.
+//   3. Still running: y_i = (-g_i - sum_{q < i} L_iq y_q) / L_ii (ascending i; the sum as s = s -
+//      L_iq * y_q from s = -g_i), then d_i = (y_i - sum_{q > i} L_qi d_q) / L_ii (descending i, q
+//      ascending); xt_i = clamp_box(x_i + d_i); XTOL if max_i |xt_i - x_i| <= xtol * (max_i |x_i| +
+//      xtol) (both maxima as gi).
+//   4. The values get xt while running, x once finished or after the last iteration.
+__global__ void __launch_bounds__(kThreads) program_fit_update_kernel(const FitArgs f)
+{
+    const long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= f.K) return;
+    gcs_b200_fit_result& res = f.res[k];
+    if (res.status != GCS_FIT_RUNNING) return;
+    const long long n = f.n;
+    FitState s(f, k);
+    double* const val = f.val + k * f.n_values;
+    res.iterations += 1;
+    const bool failed = s.c[2] != 0.0;
+    if (f.it == 0 && failed) {
+        for (long long i = 0; i < n; ++i) val[f.free[i]] = s.x0[i];
+        res.status = GCS_FIT_START_FAILED;
+        return;
+    }
+    int status = GCS_FIT_RUNNING;
+    double lambda = res.lambda;
+    const auto reject = [&] {
+        lambda = 10.0 * (lambda > 1e-12 ? lambda : 1e-12);
+        if (lambda > 1e16) status = GCS_FIT_STALLED;
+    };
+    if (!failed && (f.it == 0 || s.c[1] < s.c[0])) {
+        const double c_old = s.c[0], c = s.c[1];
+        for (long long i = 0; i < n; ++i) s.x[i] = s.xt[i], s.g[i] = s.gt[i];
+        for (long long q = 0; q < n * n; ++q) s.A[q] = s.At[q];
+        s.c[0] = c;
+        if (f.it > 0) lambda = lambda / 10.0 > 1e-12 ? lambda / 10.0 : 1e-12;
+        double gi = 0.0;
+        for (long long i = 0; i < n; ++i) {
+            const double a = fabs(s.g[i]);
+            gi = a > gi ? a : gi;
+        }
+        if (c <= f.cost_tol) status = GCS_FIT_COST;
+        else if (gi <= f.gtol) status = GCS_FIT_GTOL;
+        else if (f.it > 0 && c_old - c <= f.ftol * c_old) status = GCS_FIT_FTOL;
+        res.cost = c, res.grad_inf = gi;
+    } else {
+        reject();
+    }
+    if (status == GCS_FIT_RUNNING) {
+        double amax = 0.0;
+        for (long long j = 0; j < n; ++j) amax = s.A[j * n + j] > amax ? s.A[j * n + j] : amax;
+        const double floor = 1e-12 * amax;
+        while (status == GCS_FIT_RUNNING && !fit_cholesky(s.A, lambda, floor, s.L, n)) reject();
+    }
+    if (status == GCS_FIT_RUNNING) {
+        double* const d = s.xt;  // y, then d, then the trial
+        for (long long i = 0; i < n; ++i) {
+            double t = -s.g[i];
+            for (long long q = 0; q < i; ++q) t = t - s.L[i * n + q] * d[q];
+            d[i] = t / s.L[i * n + i];
+        }
+        for (long long i = n - 1; i >= 0; --i) {
+            double t = d[i];
+            for (long long q = i + 1; q < n; ++q) t = t - s.L[q * n + i] * d[q];
+            d[i] = t / s.L[i * n + i];
+        }
+        double step = 0.0, xmax = 0.0;
+        for (long long i = 0; i < n; ++i) {
+            d[i] = clamp_box(s.x[i] + d[i], f.lo[i], f.hi[i]);
+            const double a = fabs(d[i] - s.x[i]), b = fabs(s.x[i]);
+            step = a > step ? a : step;
+            xmax = b > xmax ? b : xmax;
+        }
+        if (step <= f.xtol * (xmax + f.xtol)) status = GCS_FIT_XTOL;
+    }
+    res.status = status, res.lambda = lambda;
+    const double* const next = status == GCS_FIT_RUNNING && !f.last ? s.xt : s.x;
+    for (long long i = 0; i < n; ++i) val[f.free[i]] = next[i];
+    if (status == GCS_FIT_RUNNING) atomicAdd(f.running + f.it, 1u);
+}
+
 int validate_desc(const gcs_b200_program_desc* d)
 {
     if (!d) return fail(GCS_E_INVALID, "null program descriptor");
@@ -508,6 +723,43 @@ int validate_desc(const gcs_b200_program_desc* d)
     return GCS_OK;
 }
 
+// gcs_b200_fit_check's checks, against a program's counts and slot and value types
+int validate_fit(const gcs_b200_fit_desc* f, int n_slots, int n_values, const uint8_t* slot_is_line, const uint8_t* value_is_angle)
+{
+    if (!f) return fail(GCS_E_INVALID, "null fit descriptor");
+    if (f->n_free < 1 || f->n_free > 32) return fail(GCS_E_INVALID, "n_free must be in 1..32 (got %d)", f->n_free);
+    if (f->n_obs < 1) return fail(GCS_E_INVALID, "n_obs must be >= 1 (got %d)", f->n_obs);
+    if (!f->free_values || !f->obs_slots || !f->obs_coords) return fail(GCS_E_INVALID, "null table in the fit descriptor");
+    for (int i = 0; i < f->n_free; ++i) {
+        const int v = f->free_values[i];
+        if (v < 0 || v >= n_values) return fail(GCS_E_INVALID, "free value %d: value slot %d out of range (%d values)", i, v, n_values);
+        for (int j = 0; j < i; ++j)
+            if (f->free_values[j] == v) return fail(GCS_E_INVALID, "free value %d: value slot %d is already free value %d", i, v, j);
+        const double lo = f->lower ? f->lower[i] : -INFINITY, hi = f->upper ? f->upper[i] : INFINITY;
+        if (std::isnan(lo) || std::isnan(hi)) return fail(GCS_E_INVALID, "free value %d: NaN bound", i);
+        if (lo > hi) return fail(GCS_E_INVALID, "free value %d: lower bound %g above upper bound %g", i, lo, hi);
+        if (value_is_angle[v] && (lo > 1.0 || hi < -1.0))
+            return fail(GCS_E_INVALID, "free value %d: the box [%g, %g] of an angle slot (a cosine) does not meet [-1, 1]", i, lo, hi);
+    }
+    for (int o = 0; o < f->n_obs; ++o) {
+        const int s = f->obs_slots[o], c = f->obs_coords[o];
+        if (s < 0 || s >= n_slots) return fail(GCS_E_INVALID, "observation %d: slot %d out of range (%d slots)", o, s, n_slots);
+        const int ncoord = slot_is_line[s] ? 4 : 2;
+        if (c < 0 || c >= ncoord)
+            return fail(GCS_E_INVALID, "observation %d: coordinate %d of a %s slot (0..%d)", o, c, slot_is_line[s] ? "line" : "point", ncoord - 1);
+        if (f->weights && !(std::isfinite(f->weights[o]) && f->weights[o] > 0.0))
+            return fail(GCS_E_INVALID, "observation %d: weight %g is not finite and positive", o, f->weights[o]);
+    }
+    if (f->max_iterations < 0) return fail(GCS_E_INVALID, "max_iterations must be >= 0 (got %d)", f->max_iterations);
+    const struct {
+        const char* name;
+        double v;
+    } tol[] = { { "lambda0", f->lambda0 }, { "cost_tol", f->cost_tol }, { "ftol", f->ftol }, { "xtol", f->xtol }, { "gtol", f->gtol } };
+    for (const auto& t : tol)
+        if (!(std::isfinite(t.v) && t.v >= 0.0)) return fail(GCS_E_INVALID, "%s must be finite and >= 0 (got %g)", t.name, t.v);
+    return GCS_OK;
+}
+
 // A device buffer that only grows.
 template <class T>
 struct DeviceBuffer {
@@ -574,6 +826,14 @@ struct gcs_b200_program {
     DeviceBuffer<double> contrib;  // [max_wave_rows][11][K][T]: slot, then value contributions
     DeviceBuffer<uint8_t> flags;   // [K][T]
     DeviceBuffer<double> avalues;  // [K][n_values][T] of gcs_b200_program_adjoints_host
+    // fits: host copies of the element and value types (for the descriptor checks); the descriptor's
+    // tables, the selector and tangent tables, the counts of the tangent runs, the working state and
+    // the running counts; targets and results of gcs_b200_program_fit_host
+    std::vector<uint8_t> slot_is_line, value_is_angle;
+    DeviceBuffer<unsigned char> fit_desc;
+    DeviceBuffer<double> fit_dvalues, fit_dpositions, fit_work, fit_targets;
+    DeviceBuffer<uint32_t> fit_counts, fit_running;
+    DeviceBuffer<gcs_b200_fit_result> fit_results;
     cudaEvent_t ev[4] = {};
 };
 
@@ -864,6 +1124,73 @@ int run_host(gcs_b200_program* p, long long K, const double* values, double* pos
         ms);
 }
 
+int check_fit(const gcs_b200_program* p, const gcs_b200_fit_desc* fit, long long K, const double* values, const double* targets,
+    const double* positions, const gcs_b200_fit_result* results, int variant)
+{
+    RC_TRY(check_run(p, K, values, positions, variant));
+    if (!targets || !results) return fail(GCS_E_INVALID, "null target or result table");
+    return validate_fit(fit, p->n_slots, p->n_values, p->slot_is_line.data(), p->value_is_angle.data());
+}
+
+// Device current, checks done: the fit on `st` (gcs_b200_program_fit).  poll: read the running count
+// back every kFitPoll iterations and stop when it is 0 (gcs_b200_program_fit_host).
+int fit_on(gcs_b200_program* p, const gcs_b200_fit_desc* fit, long long K, double* values, const double* targets, double* positions,
+    uint32_t* nonconverged, gcs_b200_fit_result* results, int variant, cudaStream_t st, bool poll)
+{
+    const long long n = fit->n_free, n_obs = fit->n_obs, nv = p->n_values, ns = p->n_slots;
+    // the descriptor's tables: lo, hi [n], w [n_obs] (doubles), then free [n], obs [n_obs] (int32)
+    std::vector<double> dbl((size_t)(2 * n + n_obs));
+    std::vector<int32_t> idx((size_t)(n + n_obs));
+    for (long long i = 0; i < n; ++i) {
+        const bool angle = p->value_is_angle[(size_t)fit->free_values[i]] != 0;
+        double lo = fit->lower ? fit->lower[i] : -INFINITY, hi = fit->upper ? fit->upper[i] : INFINITY;
+        if (angle) lo = lo > -1.0 ? lo : -1.0, hi = hi < 1.0 ? hi : 1.0;
+        dbl[(size_t)i] = lo, dbl[(size_t)(n + i)] = hi;
+        idx[(size_t)i] = fit->free_values[i];
+    }
+    for (long long o = 0; o < n_obs; ++o) {
+        dbl[(size_t)(2 * n + o)] = fit->weights ? fit->weights[o] : 1.0;
+        idx[(size_t)(n + o)] = fit->obs_slots[o] * 4 + fit->obs_coords[o];
+    }
+    const size_t dbytes = dbl.size() * sizeof(double), ibytes = idx.size() * sizeof(int32_t);
+    const long long stride = 3 * n * n + 5 * n + 3;
+    const char* what = "the %s of a fit of %lld instances";
+    RC_TRY(p->fit_desc.grow(dbytes + ibytes, st, what, "descriptor", K));
+    RC_TRY(p->fit_dvalues.grow((size_t)(K * nv * n) * sizeof(double), st, what, "selector", K));
+    RC_TRY(p->fit_dpositions.grow((size_t)(K * ns * 4 * n) * sizeof(double), st, what, "position tangents", K));
+    RC_TRY(p->fit_work.grow((size_t)(K * stride) * sizeof(double), st, what, "working state", K));
+    RC_TRY(p->fit_counts.grow((size_t)K * sizeof(uint32_t), st, what, "nonconverged counts", K));
+    RC_TRY(p->fit_running.grow((size_t)(fit->max_iterations + 1) * sizeof(uint32_t), st, what, "running counts", K));
+    CUDA_TRY(cudaMemcpyAsync(p->fit_desc.ptr, dbl.data(), dbytes, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(p->fit_desc.ptr + dbytes, idx.data(), ibytes, cudaMemcpyHostToDevice, st));
+    FitArgs f;
+    memset(&f, 0, sizeof(f));
+    f.K = K, f.n = n, f.n_obs = n_obs, f.n_values = nv, f.n_slots = ns, f.stride = stride;
+    const double* d = reinterpret_cast<const double*>(p->fit_desc.ptr);
+    f.lo = d, f.hi = d + n, f.w = d + 2 * n;
+    f.free = reinterpret_cast<const int32_t*>(p->fit_desc.ptr + dbytes), f.obs = f.free + n;
+    f.val = values, f.dval = p->fit_dvalues.ptr, f.pos = positions, f.dpos = p->fit_dpositions.ptr, f.nc = p->fit_counts.ptr;
+    f.target = targets, f.work = p->fit_work.ptr, f.res = results, f.running = p->fit_running.ptr;
+    f.max_it = fit->max_iterations;
+    f.lambda0 = fit->lambda0, f.cost_tol = fit->cost_tol, f.ftol = fit->ftol, f.xtol = fit->xtol, f.gtol = fit->gtol;
+    const auto too_many = [&] { return fail(GCS_E_INVALID, "a fit of %lld instances x %lld free values is too large for one launch", K, n); };
+    const long long start = K * nv * n > f.max_it + 1 ? K * nv * n : f.max_it + 1;
+    RC_TRY(launch(program_fit_start_kernel, start, st, f, too_many));
+    for (int it = 0; it <= f.max_it; ++it) {
+        RC_TRY(run_on(p, K, values, positions, p->fit_counts.ptr, variant, st, n, p->fit_dvalues.ptr, p->fit_dpositions.ptr));
+        f.it = it, f.last = it == f.max_it;
+        RC_TRY(launch(program_fit_normal_kernel, K * (n * (n + 1) / 2 + n + 1), st, f, too_many));
+        RC_TRY(launch(program_fit_update_kernel, K, st, f, too_many));
+        if (poll && !f.last && it % kFitPoll == kFitPoll - 1) {
+            uint32_t running = 0;
+            CUDA_TRY(cudaMemcpyAsync(&running, p->fit_running.ptr + it, sizeof(running), cudaMemcpyDeviceToHost, st));
+            CUDA_TRY(cudaStreamSynchronize(st));
+            if (running == 0) break;  // every instance frozen: the values hold the results
+        }
+    }
+    return run_on(p, K, values, positions, nonconverged, variant, st);
+}
+
 }  // namespace
 
 extern "C" {
@@ -882,6 +1209,8 @@ int gcs_b200_program_create(const gcs_b200_program_desc* d, int device, gcs_b200
     auto* p = new gcs_b200_program();
     p->device = device, p->n_waves = d->n_waves, p->n_slots = d->n_slots, p->n_values = d->n_values, p->n_rows = d->n_rows;
     p->offsets.assign(d->offsets, d->offsets + (size_t)d->n_waves * kKinds + 1);
+    p->slot_is_line.assign(d->slot_is_line, d->slot_is_line + d->n_slots);
+    p->value_is_angle.assign(d->value_is_angle, d->value_is_angle + d->n_values);
     for (int w = 0; w < d->n_waves; ++w)
         for (int k = 0; k < kKinds; ++k) {
             const long long rows = p->offsets[(size_t)w * kKinds + k + 1] - p->offsets[(size_t)w * kKinds + k];
@@ -1035,6 +1364,46 @@ int gcs_b200_program_adjoints_host(gcs_b200_program* p, int32_t T, const double*
         { { adj_values, p->avalues.ptr, vbytes } }, ms);
 }
 
+int gcs_b200_program_fit(gcs_b200_program* p, const gcs_b200_fit_desc* fit, int64_t K, double* values, const double* targets,
+    double* positions, uint32_t* nonconverged, gcs_b200_fit_result* results, int variant, void* stream)
+{
+    RC_TRY(check_fit(p, fit, K, values, targets, positions, results, variant));
+    DeviceScope on(p->device);
+    RC_TRY(on.rc);
+    return fit_on(p, fit, K, values, targets, positions, nonconverged, results, variant, static_cast<cudaStream_t>(stream), false);
+}
+
+int gcs_b200_program_fit_host(gcs_b200_program* p, const gcs_b200_fit_desc* fit, int64_t K, double* values, const double* targets,
+    double* positions, uint32_t* nonconverged, gcs_b200_fit_result* results, int variant, float ms[3])
+{
+    RC_TRY(check_fit(p, fit, K, values, targets, positions, results, variant));
+    DeviceScope on(p->device);
+    RC_TRY(on.rc);
+    const size_t vbytes = (size_t)K * p->n_values * sizeof(double), pbytes = (size_t)K * p->n_slots * 4 * sizeof(double);
+    const size_t cbytes = (size_t)K * sizeof(uint32_t), tbytes = (size_t)K * fit->n_obs * sizeof(double);
+    const size_t rbytes = (size_t)K * sizeof(gcs_b200_fit_result);
+    const cudaStream_t st = p->stream;
+    RC_TRY(p->values.grow(vbytes, st, "the values of %lld instances", (long long)K));
+    RC_TRY(p->positions.grow(pbytes, st, "the positions of %lld instances", (long long)K));
+    RC_TRY(p->counts.grow(cbytes, st, "the nonconverged counts of %lld instances", (long long)K));
+    RC_TRY(p->fit_targets.grow(tbytes, st, "the targets of %lld instances", (long long)K));
+    RC_TRY(p->fit_results.grow(rbytes, st, "the fit results of %lld instances", (long long)K));
+    return on_host(p, { { p->values.ptr, values, vbytes }, { p->fit_targets.ptr, targets, tbytes } },
+        [&](cudaStream_t s) {
+            return fit_on(p, fit, K, p->values.ptr, p->fit_targets.ptr, p->positions.ptr, nonconverged ? p->counts.ptr : nullptr,
+                p->fit_results.ptr, variant, s, true);
+        },
+        { { values, p->values.ptr, vbytes }, { positions, p->positions.ptr, pbytes }, { nonconverged, p->counts.ptr, nonconverged ? cbytes : 0 },
+            { results, p->fit_results.ptr, rbytes } },
+        ms);
+}
+
+int gcs_b200_fit_check(const gcs_b200_program_desc* d, const gcs_b200_fit_desc* fit)
+{
+    RC_TRY(validate_desc(d));
+    return validate_fit(fit, d->n_slots, d->n_values, d->slot_is_line, d->value_is_angle);
+}
+
 void gcs_b200_program_destroy(gcs_b200_program* p)
 {
     if (!p) return;
@@ -1048,6 +1417,8 @@ void gcs_b200_program_destroy(gcs_b200_program* p)
         cudaFree(p->dvalues.ptr), cudaFree(p->dpositions.ptr);
         cudaFree(p->ent), cudaFree(p->begin), cudaFree(p->readers), cudaFree(p->tape.ptr);
         cudaFree(p->apos.ptr), cudaFree(p->contrib.ptr), cudaFree(p->flags.ptr), cudaFree(p->avalues.ptr);
+        cudaFree(p->fit_desc.ptr), cudaFree(p->fit_dvalues.ptr), cudaFree(p->fit_dpositions.ptr), cudaFree(p->fit_work.ptr);
+        cudaFree(p->fit_targets.ptr), cudaFree(p->fit_counts.ptr), cudaFree(p->fit_running.ptr), cudaFree(p->fit_results.ptr);
         cudaGetLastError();
     }
     delete p;

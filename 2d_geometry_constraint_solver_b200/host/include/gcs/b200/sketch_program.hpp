@@ -30,6 +30,18 @@ struct ProgramRunStats {
     double seconds = 0;                     // host clock, call to return
 };
 
+// What fit() fits (gcs_b200_fit_desc of include/gcs_b200.h): free value indices, their box (empty:
+// none; in the C ABI's units, so an angle's bounds are on cos(angle)), observations (slot, coordinate,
+// weight; empty weights: all 1) and the Levenberg-Marquardt controls.
+struct FitSpec {
+    std::vector<std::int32_t> freeValues;
+    std::vector<double> lower, upper;
+    std::vector<std::int32_t> obsSlots, obsCoords;
+    std::vector<double> weights;
+    int maxIterations = 50;
+    double lambda0 = 1e-3, costTol = 0.0, ftol = 1e-15, xtol = 1e-15, gtol = 0.0;
+};
+
 class GCS_API SketchProgram {
 public:
     // leaves: as decomposeConstraintGraph returns them.  elements / constraints: the slot order of
@@ -77,6 +89,16 @@ public:
     // std::logic_error before any device call when nothing was recorded, std::invalid_argument for
     // T < 1.
     ProgramRunStats adjoints(const double* adjPositions, int T, double* adjValues);
+
+    // Fits the free values of K instances to targets on the device (gcs_b200_program_fit_host).
+    // values host [K][nValues()] in-out, radians for angles: a free angle starts at std::cos(v) and
+    // returns std::acos(c) with the sign of its start (the program reads only cos), every other entry
+    // and every START_FAILED instance is left as it was.  targets host [K][n_obs]; positions host
+    // [K][nSlots()][4] and nonconverged (may be null) receive run() at the returned values; results
+    // host [K].  Instances split over devices as run() splits them.  Throws std::invalid_argument for
+    // a malformed spec (gcs_b200_fit_check's message) before any device call.
+    ProgramRunStats fit(double* values, std::int64_t K, const FitSpec& spec, const double* targets, double* positions,
+        gcs_b200_fit_result* results, std::uint32_t* nonconverged = nullptr, int nDevices = 1);
 
     // The edit loop: one instance with the constraints' current values, written into the elements -
     // the state solveLeaves leaves.

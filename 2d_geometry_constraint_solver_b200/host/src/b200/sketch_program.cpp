@@ -248,6 +248,54 @@ ProgramRunStats SketchProgram::adjoints(const double* adjPositions, int T, doubl
     return st;
 }
 
+ProgramRunStats SketchProgram::fit(double* values, std::int64_t K, const FitSpec& spec, const double* targets, double* positions,
+    gcs_b200_fit_result* results, std::uint32_t* nonconverged, int nDevices)
+{
+    const auto t0 = Clock::now();
+    const auto bad = [](const std::string& what) { throw std::invalid_argument("SketchProgram::fit: " + what); };
+    if (K < 1) bad("K must be >= 1");
+    const std::size_t nf = spec.freeValues.size(), nobs = spec.obsSlots.size();
+    if ((!spec.lower.empty() && spec.lower.size() != nf) || (!spec.upper.empty() && spec.upper.size() != nf))
+        bad("lower and upper hold one bound per free value, or none");
+    if (spec.obsCoords.size() != nobs || (!spec.weights.empty() && spec.weights.size() != nobs))
+        bad("obsCoords (and weights, if any) hold one entry per observation");
+    gcs_b200_fit_desc f {};
+    f.n_free = static_cast<std::int32_t>(std::min<std::size_t>(nf, 1u << 30));
+    f.n_obs = static_cast<std::int32_t>(std::min<std::size_t>(nobs, 1u << 30));
+    f.free_values = spec.freeValues.data(), f.obs_slots = spec.obsSlots.data(), f.obs_coords = spec.obsCoords.data();
+    f.lower = spec.lower.empty() ? nullptr : spec.lower.data();
+    f.upper = spec.upper.empty() ? nullptr : spec.upper.data();
+    f.weights = spec.weights.empty() ? nullptr : spec.weights.data();
+    f.max_iterations = spec.maxIterations, f.lambda0 = spec.lambda0;
+    f.cost_tol = spec.costTol, f.ftol = spec.ftol, f.xtol = spec.xtol, f.gtol = spec.gtol;
+    const gcs_b200_program_desc d = desc();
+    if (gcs_b200_fit_check(&d, &f) != GCS_OK) bad(gcs_b200_last_error());
+    const int avail = gcs_b200_device_count();
+    if (avail < 1) cudaFailure("gcs_b200_device_count", GCS_E_NO_DEVICE);
+    nDevices = static_cast<int>(std::min<std::int64_t>(std::clamp(nDevices, 1, avail), K));
+    const std::size_t nv = nValues(), table = nSlots() * 4;
+    // angles go to the device as std::cos of the value, as in run()
+    std::vector<double> cv(values, values + static_cast<std::size_t>(K) * nv);
+    for (std::size_t q = 0; q < cv.size(); ++q)
+        if (m_valueIsAngle[q % nv]) cv[q] = std::cos(cv[q]);
+    for (int g = 0; g < nDevices; ++g) onDevice(g);
+    const int variant = kernelVariant();
+    ProgramRunStats st = fanOut(K, nDevices, "gcs_b200_program_fit_host", [&](int g, std::int64_t lo, std::int64_t hi, float* ms) {
+        return gcs_b200_program_fit_host(m_device[static_cast<std::size_t>(g)], &f, hi - lo, cv.data() + lo * static_cast<std::int64_t>(nv),
+            targets + lo * static_cast<std::int64_t>(nobs), positions + lo * static_cast<std::int64_t>(table),
+            nonconverged ? nonconverged + lo : nullptr, results + lo, variant, ms);
+    });
+    for (std::int64_t k = 0; k < K; ++k) {
+        if (results[k].status == GCS_FIT_START_FAILED) continue;
+        for (std::size_t i = 0; i < nf; ++i) {
+            const std::size_t q = static_cast<std::size_t>(k) * nv + static_cast<std::size_t>(spec.freeValues[i]);
+            values[q] = m_valueIsAngle[static_cast<std::size_t>(spec.freeValues[i])] ? std::copysign(std::acos(cv[q]), values[q]) : cv[q];
+        }
+    }
+    st.seconds = std::chrono::duration<double>(Clock::now() - t0).count();
+    return st;
+}
+
 // T = 0: run() or record(); T > 0: runTangents()
 ProgramRunStats SketchProgram::runImpl(const double* values, std::int64_t K, const double* dvalues, int T, double* positions,
     double* dpositions, std::uint32_t* nonconverged, int nDevices, bool recorded)

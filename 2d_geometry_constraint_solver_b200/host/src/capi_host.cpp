@@ -144,6 +144,13 @@ Gcs::ConstraintGraph makeSketch(std::vector<std::shared_ptr<Gcs::Element>>& elem
     return g;
 }
 
+// a table of n entries, or none for NULL
+template <class T>
+std::vector<T> take(const T* p, int n)
+{
+    return p ? std::vector<T>(p, p + std::max(n, 0)) : std::vector<T>();
+}
+
 int fail(const std::exception& ex)
 {
     std::snprintf(g_msg, sizeof(g_msg), "%s", ex.what());
@@ -940,6 +947,29 @@ GCS_API int gcs_host_program_adjoints(gcs_host_program* h, int T, const double* 
     try {
         const Gcs::B200::ProgramRunStats st = h->prog->adjoints(adj_positions, T, adj_values);
         programStats(h, st, h->prog->recordedDevices(), stats);
+        return 0;
+    } catch (const std::exception& ex) {
+        return fail(ex);
+    }
+}
+
+// Fit values to targets (SketchProgram::fit) for the descriptor `fit` (gcs_b200_fit_desc; host
+// tables): values in-out [K][n_values] (radians for angles), targets [K][n_obs], positions out
+// [K][n_slots][4], results out [K], nonconverged [K] (may be NULL); stats as gcs_host_program_run.
+// Returns 0 or -1.
+GCS_API int gcs_host_program_fit(gcs_host_program* h, const gcs_b200_fit_desc* fit, int64_t K, double* values, const double* targets,
+    double* positions, gcs_b200_fit_result* results, uint32_t* nonconverged, int n_devices, int64_t* stats)
+{
+    try {
+        if (!fit) throw std::invalid_argument("gcs_host_program_fit: null fit descriptor");
+        Gcs::B200::FitSpec spec;
+        spec.freeValues = take(fit->free_values, fit->n_free);
+        spec.lower = take(fit->lower, fit->n_free), spec.upper = take(fit->upper, fit->n_free);
+        spec.obsSlots = take(fit->obs_slots, fit->n_obs), spec.obsCoords = take(fit->obs_coords, fit->n_obs);
+        spec.weights = take(fit->weights, fit->n_obs);
+        spec.maxIterations = fit->max_iterations, spec.lambda0 = fit->lambda0;
+        spec.costTol = fit->cost_tol, spec.ftol = fit->ftol, spec.xtol = fit->xtol, spec.gtol = fit->gtol;
+        programStats(h, h->prog->fit(values, K, spec, targets, positions, results, nonconverged, n_devices), n_devices, stats);
         return 0;
     } catch (const std::exception& ex) {
         return fail(ex);

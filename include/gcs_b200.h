@@ -427,6 +427,89 @@ GCS_B200_API int gcs_b200_program_adjoints_host(gcs_b200_program* prog, int32_t 
     double* adj_values, float ms[3]);
 GCS_B200_API void gcs_b200_program_destroy(gcs_b200_program* prog);
 
+/* Fitting values to targets: for each instance k, Levenberg-Marquardt over n_free of its values
+ *     minimise  c(x) = sum_o w_o (positions[k][slot_o][coord_o](x) - target[k][o])^2
+ * with every other value held at the instance's own.  Units are the C ABI's: an angle slot's free
+ * value is cos(angle), and its box is intersected with [-1, 1]. */
+typedef struct gcs_b200_fit_desc {
+    int32_t n_free;                /* 1 .. 32 */
+    int32_t n_obs;                 /* >= 1 */
+    const int32_t* free_values;    /* [n_free] distinct value slots */
+    const double* lower;           /* [n_free] box, or NULL (no lower bounds) */
+    const double* upper;           /* [n_free] box, or NULL (no upper bounds) */
+    const int32_t* obs_slots;      /* [n_obs] element slots */
+    const int32_t* obs_coords;     /* [n_obs] 0..1 of a point slot, 0..3 (p1.x p1.y p2.x p2.y) of a line slot */
+    const double* weights;         /* [n_obs] finite, > 0, or NULL (all 1) */
+    int32_t max_iterations;        /* >= 0 */
+    int32_t reserved;
+    double lambda0;                /* initial damping, finite, >= 0 */
+    double cost_tol, ftol, xtol, gtol;  /* finite, >= 0 */
+} gcs_b200_fit_desc;
+
+#define GCS_FIT_RUNNING 0      /* max_iterations reached */
+#define GCS_FIT_COST 1         /* c <= cost_tol */
+#define GCS_FIT_GTOL 2         /* max_i |g_i| <= gtol */
+#define GCS_FIT_FTOL 3         /* an accepted step gained c_old - c <= ftol c_old */
+#define GCS_FIT_XTOL 4         /* the next (clamped) step has max_i |d_i| <= xtol (max_i |x_i| + xtol) */
+#define GCS_FIT_STALLED 5      /* lambda went above 1e16 */
+#define GCS_FIT_START_FAILED 6 /* the clamped start fails (see below); values unchanged */
+
+typedef struct gcs_b200_fit_result {
+    int32_t status;      /* GCS_FIT_* */
+    int32_t iterations;  /* tangent runs the instance used, iteration 0 included */
+    double cost;         /* c at the accepted values (NaN for START_FAILED) */
+    double grad_inf;     /* max_i |g_i| there (NaN for START_FAILED) */
+    double lambda;       /* damping at the end */
+} gcs_b200_fit_result;
+
+/* The fit of K = n_instances instances in lockstep, stream-ordered on `cuda_stream`; every table is a
+ * device pointer.  values [K][n_values] in-out: only the free entries change, to the fitted values;
+ * the table is the working table of the call.  targets [K][n_obs]; positions [K][n_slots][4] and
+ * nonconverged [K] (may be NULL) receive a plain run at the returned values, bit for bit what
+ * gcs_b200_program_run gives there; results [K].
+ * Iterations.  Iteration 0 is one tangent run (T = n_free, dvalues the selector: 1 at
+ * (free_values[t], t), 0 elsewhere) at the start clamped into the box, then iterations 1 ..
+ * max_iterations one tangent run each at every instance's trial values.  After each run two kernels:
+ *   program_fit_normal_kernel: per instance r_o = p_o - target_o, J_oi = dp_o / dx_i, and in ascending
+ *     o, one term at a time,  c += (w_o r_o) r_o,  g_i += (w_o J_oi) r_o,  A_ij += (w_o J_oi) J_oj
+ *     (i <= j).  The trial fails when nonconverged[k] > 0 (even if the observed coordinates are
+ *     finite: a fitted instance is always a fully solved sketch) or an observed position or
+ *     tangent is not finite.
+ *   program_fit_update_kernel, per running instance:
+ *     1. accept the trial if it did not fail and c' < c: x, A, g, c <- the trial's, lambda <-
+ *        max(lambda / 10, 1e-12); else reject: lambda <- 10 max(lambda, 1e-12), STALLED once lambda
+ *        > 1e16.  Iteration 0 accepts the start unless it failed (then START_FAILED) and keeps
+ *        lambda0.
+ *     2. on accept, in this order: COST, GTOL, FTOL (not at iteration 0).
+ *     3. the step: Cholesky of A + lambda D, D_ii = max(A_ii, 1e-12 max_j A_jj); a non-positive
+ *        pivot is a reject (step 1's rule, then retry); d solves (A + lambda D) d = -g; the trial is
+ *        x + d clamped into the box.
+ *     4. XTOL on the clamped step (before any trial: an exact fit would otherwise stall at the
+ *        rounding floor).
+ *     5. the trial's free values into `values`.  A finished instance is frozen and its trial is its
+ *        result, so later runs leave it bit-unchanged; after the last iteration a running instance
+ *        writes its accepted values.
+ * Then one plain run at the returned values.  csrc/sketch_program.cu states the operation order.
+ * Launches: 1 + (max_iterations + 1) x (a tangent run's + 2) + a plain run's; exactly
+ * max_iterations iterations are enqueued and nothing synchronises.  Memory: selector and tangent
+ * tables of K x n_free x (8 n_values + 32 n_slots) bytes, and K x (24 n_free^2 + 40 n_free + 24)
+ * bytes of working state.
+ * Checked before any device call (GCS_E_INVALID with a message): what gcs_b200_program_run checks,
+ * a null target or result table, and gcs_b200_fit_check's checks. */
+GCS_B200_API int gcs_b200_program_fit(gcs_b200_program* prog, const gcs_b200_fit_desc* fit, int64_t n_instances, double* values,
+    const double* targets, double* positions, uint32_t* nonconverged, gcs_b200_fit_result* results, int variant, void* cuda_stream);
+/* The same with host buffers on the program's own stream.  It may stop early: every 4 iterations it
+ * reads back the count of running instances and stops at 0.  Finished instances are frozen, so the
+ * results equal gcs_b200_program_fit's bit for bit.  ms (may be NULL) receives the device time of
+ * upload, fit and download. */
+GCS_B200_API int gcs_b200_program_fit_host(gcs_b200_program* prog, const gcs_b200_fit_desc* fit, int64_t n_instances, double* values,
+    const double* targets, double* positions, uint32_t* nonconverged, gcs_b200_fit_result* results, int variant, float ms[3]);
+/* The fit descriptor's checks against a program descriptor, without a device: n_free in 1..32,
+ * distinct free value slots in range, observation slots in range with a coordinate their element
+ * has, finite positive weights, bounds that are not NaN with lower <= upper (and, for an angle slot,
+ * a box that meets [-1, 1]), max_iterations >= 0, lambda0 and tolerances finite and >= 0. */
+GCS_B200_API int gcs_b200_fit_check(const gcs_b200_program_desc* prog, const gcs_b200_fit_desc* fit);
+
 /* Test hook: on-device self check of the hand-written division / square root / 2x2 QR fast paths
  * against the generic IEEE code (csrc/selftest.cu).  Fills counts[8]:
  *   [0] divisions on the fast path, [1] of those differing from a/b,
