@@ -805,8 +805,8 @@ struct gcs_b200_program {
     cudaStream_t stream = nullptr;  // uploads and the _host entry points
     // the kind batches of plain and tangent runs, reused by every wave
     DeviceBuffer<unsigned char> scratch;
-    // tables of the _host entry points: gcs_b200_program_run_host, and the tangent tables of
-    // gcs_b200_program_run_tangents_host
+    // tables of the _host entry points, and the counts and tangent tables of _host runs and of fits
+    // (grow_tables)
     DeviceBuffer<double> values, positions;
     DeviceBuffer<uint32_t> counts;
     DeviceBuffer<double> dvalues, dpositions;
@@ -826,13 +826,12 @@ struct gcs_b200_program {
     DeviceBuffer<double> contrib;  // [max_wave_rows][11][K][T]: slot, then value contributions
     DeviceBuffer<uint8_t> flags;   // [K][T]
     DeviceBuffer<double> avalues;  // [K][n_values][T] of gcs_b200_program_adjoints_host
-    // fits: host copies of the element and value types (for the descriptor checks); the descriptor's
-    // tables, the selector and tangent tables, the counts of the tangent runs, the working state and
-    // the running counts; targets and results of gcs_b200_program_fit_host
+    // fits: host copies of the element and value types (for the descriptor checks); the working
+    // state, descriptor tables and running counts (fit_on); targets and results of
+    // gcs_b200_program_fit_host
     std::vector<uint8_t> slot_is_line, value_is_angle;
-    DeviceBuffer<unsigned char> fit_desc;
-    DeviceBuffer<double> fit_dvalues, fit_dpositions, fit_work, fit_targets;
-    DeviceBuffer<uint32_t> fit_counts, fit_running;
+    DeviceBuffer<unsigned char> fit_state;
+    DeviceBuffer<double> fit_targets;
     DeviceBuffer<gcs_b200_fit_result> fit_results;
     cudaEvent_t ev[4] = {};
 };
@@ -1102,18 +1101,27 @@ int on_host(gcs_b200_program* p, std::initializer_list<Copy> up, Work&& work, st
     return GCS_OK;
 }
 
+// device current: the counts and tangent tables for K instances and T directions of the runs the
+// program drives itself (_host runs, fits); host: also the _host entry points' values and positions
+int grow_tables(gcs_b200_program* p, long long K, long long T, bool host, cudaStream_t st)
+{
+    const size_t vbytes = (size_t)K * p->n_values * sizeof(double), pbytes = (size_t)K * p->n_slots * 4 * sizeof(double);
+    if (host) {
+        RC_TRY(p->values.grow(vbytes, st, "the values of %lld instances", K));
+        RC_TRY(p->positions.grow(pbytes, st, "the positions of %lld instances", K));
+    }
+    RC_TRY(p->counts.grow((size_t)K * sizeof(uint32_t), st, "the nonconverged counts of %lld instances", K));
+    RC_TRY(p->dvalues.grow(vbytes * T, st, "the value tangents of %lld instances x %lld directions", K, T));
+    return p->dpositions.grow(pbytes * T, st, "the position tangents of %lld instances x %lld directions", K, T);
+}
+
 // device current, checks done
 int run_host(gcs_b200_program* p, long long K, const double* values, double* positions, uint32_t* nonconverged, int variant,
     float ms[3], long long T = 0, const double* dvalues = nullptr, double* dpositions = nullptr, bool recorded = false)
 {
     const size_t vbytes = (size_t)K * p->n_values * sizeof(double), pbytes = (size_t)K * p->n_slots * 4 * sizeof(double);
     const size_t cbytes = (size_t)K * sizeof(uint32_t);
-    const cudaStream_t st = p->stream;
-    RC_TRY(p->values.grow(vbytes, st, "the values of %lld instances", K));
-    RC_TRY(p->positions.grow(pbytes, st, "the positions of %lld instances", K));
-    RC_TRY(p->counts.grow(cbytes, st, "the nonconverged counts of %lld instances", K));
-    RC_TRY(p->dvalues.grow(vbytes * T, st, "the value tangents of %lld instances x %lld directions", K, T));
-    RC_TRY(p->dpositions.grow(pbytes * T, st, "the position tangents of %lld instances x %lld directions", K, T));
+    RC_TRY(grow_tables(p, K, T, true, p->stream));
     return on_host(p, { { p->values.ptr, values, vbytes }, { p->dvalues.ptr, dvalues, vbytes * T } },
         [&](cudaStream_t s) {
             return run_on(p, K, p->values.ptr, p->positions.ptr, nonconverged ? p->counts.ptr : nullptr, variant, s, T, p->dvalues.ptr,
@@ -1132,8 +1140,8 @@ int check_fit(const gcs_b200_program* p, const gcs_b200_fit_desc* fit, long long
     return validate_fit(fit, p->n_slots, p->n_values, p->slot_is_line.data(), p->value_is_angle.data());
 }
 
-// Device current, checks done: the fit on `st` (gcs_b200_program_fit).  poll: read the running count
-// back every kFitPoll iterations and stop when it is 0 (gcs_b200_program_fit_host).
+// Device current, checks done, grow_tables(K, n_free): the fit on `st` (gcs_b200_program_fit).  poll:
+// read the running count back every kFitPoll iterations and stop when it is 0 (gcs_b200_program_fit_host).
 int fit_on(gcs_b200_program* p, const gcs_b200_fit_desc* fit, long long K, double* values, const double* targets, double* positions,
     uint32_t* nonconverged, gcs_b200_fit_result* results, int variant, cudaStream_t st, bool poll)
 {
@@ -1152,38 +1160,35 @@ int fit_on(gcs_b200_program* p, const gcs_b200_fit_desc* fit, long long K, doubl
         dbl[(size_t)(2 * n + o)] = fit->weights ? fit->weights[o] : 1.0;
         idx[(size_t)(n + o)] = fit->obs_slots[o] * 4 + fit->obs_coords[o];
     }
-    const size_t dbytes = dbl.size() * sizeof(double), ibytes = idx.size() * sizeof(int32_t);
+    // one allocation: the working state, the descriptor's tables, the running counts
     const long long stride = 3 * n * n + 5 * n + 3;
-    const char* what = "the %s of a fit of %lld instances";
-    RC_TRY(p->fit_desc.grow(dbytes + ibytes, st, what, "descriptor", K));
-    RC_TRY(p->fit_dvalues.grow((size_t)(K * nv * n) * sizeof(double), st, what, "selector", K));
-    RC_TRY(p->fit_dpositions.grow((size_t)(K * ns * 4 * n) * sizeof(double), st, what, "position tangents", K));
-    RC_TRY(p->fit_work.grow((size_t)(K * stride) * sizeof(double), st, what, "working state", K));
-    RC_TRY(p->fit_counts.grow((size_t)K * sizeof(uint32_t), st, what, "nonconverged counts", K));
-    RC_TRY(p->fit_running.grow((size_t)(fit->max_iterations + 1) * sizeof(uint32_t), st, what, "running counts", K));
-    CUDA_TRY(cudaMemcpyAsync(p->fit_desc.ptr, dbl.data(), dbytes, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(cudaMemcpyAsync(p->fit_desc.ptr + dbytes, idx.data(), ibytes, cudaMemcpyHostToDevice, st));
+    const size_t wbytes = (size_t)(K * stride) * sizeof(double), dbytes = dbl.size() * sizeof(double), ibytes = idx.size() * sizeof(int32_t);
+    RC_TRY(p->fit_state.grow(wbytes + dbytes + ibytes + (size_t)(fit->max_iterations + 1) * sizeof(uint32_t), st,
+        "the working state of a fit of %lld instances", K));
+    unsigned char* const at = p->fit_state.ptr;
+    CUDA_TRY(cudaMemcpyAsync(at + wbytes, dbl.data(), dbytes, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(at + wbytes + dbytes, idx.data(), ibytes, cudaMemcpyHostToDevice, st));
     FitArgs f;
     memset(&f, 0, sizeof(f));
     f.K = K, f.n = n, f.n_obs = n_obs, f.n_values = nv, f.n_slots = ns, f.stride = stride;
-    const double* d = reinterpret_cast<const double*>(p->fit_desc.ptr);
-    f.lo = d, f.hi = d + n, f.w = d + 2 * n;
-    f.free = reinterpret_cast<const int32_t*>(p->fit_desc.ptr + dbytes), f.obs = f.free + n;
-    f.val = values, f.dval = p->fit_dvalues.ptr, f.pos = positions, f.dpos = p->fit_dpositions.ptr, f.nc = p->fit_counts.ptr;
-    f.target = targets, f.work = p->fit_work.ptr, f.res = results, f.running = p->fit_running.ptr;
+    f.work = reinterpret_cast<double*>(at), f.lo = f.work + K * stride, f.hi = f.lo + n, f.w = f.lo + 2 * n;
+    f.free = reinterpret_cast<const int32_t*>(at + wbytes + dbytes), f.obs = f.free + n;
+    f.running = reinterpret_cast<uint32_t*>(at + wbytes + dbytes + ibytes);
+    f.val = values, f.dval = p->dvalues.ptr, f.pos = positions, f.dpos = p->dpositions.ptr, f.nc = p->counts.ptr;
+    f.target = targets, f.res = results;
     f.max_it = fit->max_iterations;
     f.lambda0 = fit->lambda0, f.cost_tol = fit->cost_tol, f.ftol = fit->ftol, f.xtol = fit->xtol, f.gtol = fit->gtol;
     const auto too_many = [&] { return fail(GCS_E_INVALID, "a fit of %lld instances x %lld free values is too large for one launch", K, n); };
     const long long start = K * nv * n > f.max_it + 1 ? K * nv * n : f.max_it + 1;
     RC_TRY(launch(program_fit_start_kernel, start, st, f, too_many));
     for (int it = 0; it <= f.max_it; ++it) {
-        RC_TRY(run_on(p, K, values, positions, p->fit_counts.ptr, variant, st, n, p->fit_dvalues.ptr, p->fit_dpositions.ptr));
+        RC_TRY(run_on(p, K, values, positions, p->counts.ptr, variant, st, n, p->dvalues.ptr, p->dpositions.ptr));
         f.it = it, f.last = it == f.max_it;
         RC_TRY(launch(program_fit_normal_kernel, K * (n * (n + 1) / 2 + n + 1), st, f, too_many));
         RC_TRY(launch(program_fit_update_kernel, K, st, f, too_many));
         if (poll && !f.last && it % kFitPoll == kFitPoll - 1) {
             uint32_t running = 0;
-            CUDA_TRY(cudaMemcpyAsync(&running, p->fit_running.ptr + it, sizeof(running), cudaMemcpyDeviceToHost, st));
+            CUDA_TRY(cudaMemcpyAsync(&running, f.running + it, sizeof(running), cudaMemcpyDeviceToHost, st));
             CUDA_TRY(cudaStreamSynchronize(st));
             if (running == 0) break;  // every instance frozen: the values hold the results
         }
@@ -1370,7 +1375,9 @@ int gcs_b200_program_fit(gcs_b200_program* p, const gcs_b200_fit_desc* fit, int6
     RC_TRY(check_fit(p, fit, K, values, targets, positions, results, variant));
     DeviceScope on(p->device);
     RC_TRY(on.rc);
-    return fit_on(p, fit, K, values, targets, positions, nonconverged, results, variant, static_cast<cudaStream_t>(stream), false);
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    RC_TRY(grow_tables(p, K, fit->n_free, false, st));
+    return fit_on(p, fit, K, values, targets, positions, nonconverged, results, variant, st, false);
 }
 
 int gcs_b200_program_fit_host(gcs_b200_program* p, const gcs_b200_fit_desc* fit, int64_t K, double* values, const double* targets,
@@ -1383,9 +1390,7 @@ int gcs_b200_program_fit_host(gcs_b200_program* p, const gcs_b200_fit_desc* fit,
     const size_t cbytes = (size_t)K * sizeof(uint32_t), tbytes = (size_t)K * fit->n_obs * sizeof(double);
     const size_t rbytes = (size_t)K * sizeof(gcs_b200_fit_result);
     const cudaStream_t st = p->stream;
-    RC_TRY(p->values.grow(vbytes, st, "the values of %lld instances", (long long)K));
-    RC_TRY(p->positions.grow(pbytes, st, "the positions of %lld instances", (long long)K));
-    RC_TRY(p->counts.grow(cbytes, st, "the nonconverged counts of %lld instances", (long long)K));
+    RC_TRY(grow_tables(p, K, fit->n_free, true, st));
     RC_TRY(p->fit_targets.grow(tbytes, st, "the targets of %lld instances", (long long)K));
     RC_TRY(p->fit_results.grow(rbytes, st, "the fit results of %lld instances", (long long)K));
     return on_host(p, { { p->values.ptr, values, vbytes }, { p->fit_targets.ptr, targets, tbytes } },
@@ -1417,8 +1422,7 @@ void gcs_b200_program_destroy(gcs_b200_program* p)
         cudaFree(p->dvalues.ptr), cudaFree(p->dpositions.ptr);
         cudaFree(p->ent), cudaFree(p->begin), cudaFree(p->readers), cudaFree(p->tape.ptr);
         cudaFree(p->apos.ptr), cudaFree(p->contrib.ptr), cudaFree(p->flags.ptr), cudaFree(p->avalues.ptr);
-        cudaFree(p->fit_desc.ptr), cudaFree(p->fit_dvalues.ptr), cudaFree(p->fit_dpositions.ptr), cudaFree(p->fit_work.ptr);
-        cudaFree(p->fit_targets.ptr), cudaFree(p->fit_counts.ptr), cudaFree(p->fit_running.ptr), cudaFree(p->fit_results.ptr);
+        cudaFree(p->fit_state.ptr), cudaFree(p->fit_targets.ptr), cudaFree(p->fit_results.ptr);
         cudaGetLastError();
     }
     delete p;

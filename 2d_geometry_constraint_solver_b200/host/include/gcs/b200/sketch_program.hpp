@@ -122,6 +122,7 @@ private:
     SketchProgram() = default;
     gcs_b200_program* onDevice(int device);
     void release();
+    void stage(const double* values, std::int64_t K, const double* dvalues, int T);
     ProgramRunStats runImpl(const double* values, std::int64_t K, const double* dvalues, int T, double* positions, double* dpositions,
         std::uint32_t* nonconverged, int nDevices, bool recorded = false);
 
@@ -134,7 +135,7 @@ private:
     std::vector<std::shared_ptr<Constraint>> m_constraints;
     double m_compileSeconds = 0;
     std::vector<gcs_b200_program*> m_device;  // uploaded lazily, by device ordinal
-    // page-locked staging of run()
+    // page-locked staging of run() and fit() (stage)
     double* m_stageValues = nullptr;
     double* m_stagePositions = nullptr;
     std::uint32_t* m_stageCounts = nullptr;

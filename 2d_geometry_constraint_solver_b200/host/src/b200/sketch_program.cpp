@@ -31,6 +31,14 @@ using Clock = std::chrono::steady_clock;
 
 bool isZeroFixed(int solver) { return solver >= 1 && solver <= 3; }
 
+// the devices K >= 1 instances split over: nDevices clamped to [1, devices present], at most K
+int devicesFor(int nDevices, std::int64_t K)
+{
+    const int avail = gcs_b200_device_count();
+    if (avail < 1) cudaFailure("gcs_b200_device_count", GCS_E_NO_DEVICE);
+    return static_cast<int>(std::min<std::int64_t>(std::clamp(nDevices, 1, avail), K));
+}
+
 // K instances over devices 0 .. nDevices-1, one host thread per device: part(g, lo, hi, ms) runs
 // instances [lo, hi) = [K*g/n, K*(g+1)/n) on device g through the C entry point `entry`, returns its
 // code and fills ms[3].  A failed part throws, naming `entry`.  Returns the launches and the summed
@@ -219,8 +227,8 @@ ProgramRunStats SketchProgram::record(const double* values, std::int64_t K, doub
     const ProgramRunStats st = runImpl(values, K, nullptr, 0, positions, nullptr, nonconverged, nDevices, true);
     m_recordedValues.assign(values, values + static_cast<std::size_t>(K) * nValues());
     m_recordedK = K;
-    // runImpl's split: instances in contiguous ranges over the first min(nDevices, devices, K) devices
-    m_recordedDevices = static_cast<int>(std::min<std::int64_t>(std::clamp(nDevices, 1, gcs_b200_device_count()), K));
+    // runImpl's split: instances in contiguous ranges over the first devicesFor(nDevices, K) devices
+    m_recordedDevices = devicesFor(nDevices, K);
     return st;
 }
 
@@ -270,18 +278,14 @@ ProgramRunStats SketchProgram::fit(double* values, std::int64_t K, const FitSpec
     f.cost_tol = spec.costTol, f.ftol = spec.ftol, f.xtol = spec.xtol, f.gtol = spec.gtol;
     const gcs_b200_program_desc d = desc();
     if (gcs_b200_fit_check(&d, &f) != GCS_OK) bad(gcs_b200_last_error());
-    const int avail = gcs_b200_device_count();
-    if (avail < 1) cudaFailure("gcs_b200_device_count", GCS_E_NO_DEVICE);
-    nDevices = static_cast<int>(std::min<std::int64_t>(std::clamp(nDevices, 1, avail), K));
+    nDevices = devicesFor(nDevices, K);
     const std::size_t nv = nValues(), table = nSlots() * 4;
-    // angles go to the device as std::cos of the value, as in run()
-    std::vector<double> cv(values, values + static_cast<std::size_t>(K) * nv);
-    for (std::size_t q = 0; q < cv.size(); ++q)
-        if (m_valueIsAngle[q % nv]) cv[q] = std::cos(cv[q]);
+    stage(values, K, nullptr, 0);
+    double* const cv = m_stageValues;
     for (int g = 0; g < nDevices; ++g) onDevice(g);
     const int variant = kernelVariant();
     ProgramRunStats st = fanOut(K, nDevices, "gcs_b200_program_fit_host", [&](int g, std::int64_t lo, std::int64_t hi, float* ms) {
-        return gcs_b200_program_fit_host(m_device[static_cast<std::size_t>(g)], &f, hi - lo, cv.data() + lo * static_cast<std::int64_t>(nv),
+        return gcs_b200_program_fit_host(m_device[static_cast<std::size_t>(g)], &f, hi - lo, cv + lo * static_cast<std::int64_t>(nv),
             targets + lo * static_cast<std::int64_t>(nobs), positions + lo * static_cast<std::int64_t>(table),
             nonconverged ? nonconverged + lo : nullptr, results + lo, variant, ms);
     });
@@ -296,16 +300,9 @@ ProgramRunStats SketchProgram::fit(double* values, std::int64_t K, const FitSpec
     return st;
 }
 
-// T = 0: run() or record(); T > 0: runTangents()
-ProgramRunStats SketchProgram::runImpl(const double* values, std::int64_t K, const double* dvalues, int T, double* positions,
-    double* dpositions, std::uint32_t* nonconverged, int nDevices, bool recorded)
+// values [K][nValues()] and dvalues [K][nValues()][T] (radians) into the page-locked staging, in the C ABI's units
+void SketchProgram::stage(const double* values, std::int64_t K, const double* dvalues, int T)
 {
-    const auto t0 = Clock::now();
-    if (K < 1) throw std::invalid_argument("SketchProgram::run: K must be >= 1");
-    const int avail = gcs_b200_device_count();
-    if (avail < 1) cudaFailure("gcs_b200_device_count", GCS_E_NO_DEVICE);
-    nDevices = std::clamp(nDevices, 1, avail);
-    if (nDevices > K) nDevices = static_cast<int>(K);
     const std::size_t nv = nValues(), table = nSlots() * 4;
     if (K > m_stageK) {
         gcs_b200_host_free(m_stageValues), gcs_b200_host_free(m_stagePositions), gcs_b200_host_free(m_stageCounts);
@@ -339,6 +336,17 @@ ProgramRunStats SketchProgram::runImpl(const double* values, std::int64_t K, con
         const long long vq = q / T;
         dstage[q] = angle[static_cast<std::size_t>(vq) % nv] ? -std::sin(values[vq]) * dvalues[q] : dvalues[q];
     }
+}
+
+// T = 0: run() or record(); T > 0: runTangents()
+ProgramRunStats SketchProgram::runImpl(const double* values, std::int64_t K, const double* dvalues, int T, double* positions,
+    double* dpositions, std::uint32_t* nonconverged, int nDevices, bool recorded)
+{
+    const auto t0 = Clock::now();
+    if (K < 1) throw std::invalid_argument("SketchProgram::run: K must be >= 1");
+    nDevices = devicesFor(nDevices, K);
+    const std::size_t nv = nValues(), table = nSlots() * 4;
+    stage(values, K, dvalues, T);
     for (int g = 0; g < nDevices; ++g) onDevice(g);
 
     const int variant = kernelVariant();

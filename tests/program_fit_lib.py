@@ -12,8 +12,6 @@ from program_restate import Arrays, restate
 from program_restate_fit import Fit
 from program_tangents_lib import capi
 
-_KEYS = ("launches", "compile_us", "upload_us", "device_us", "download_us", "run_us", "devices")
-
 
 def cfit(fit):
     """capi.CFitDesc over a program_restate_fit.Fit (its tables live as long as the descriptor)."""
@@ -128,7 +126,7 @@ class Program(program_adjoints_lib.Program):
         stats = np.zeros(7, dtype=np.int64)
         rc = lib.gcs_host_program_fit(self.handle, C.byref(cfit(fit)), K, _dp(vals), _dp(targets), _dp(pos), res,
                                       nc.ctypes.data_as(C.POINTER(C.c_uint32)), n_devices, stats.ctypes.data_as(C.POINTER(C.c_int64)))
-        return rc, vals, pos, nc, results(res), dict(zip(_KEYS, (int(v) for v in stats)))
+        return rc, vals, pos, nc, results(res), dict(zip(program_adjoints_lib._KEYS, (int(v) for v in stats)))
 
 
 def problem(p, cv, n_free, seed, max_obs=48):
