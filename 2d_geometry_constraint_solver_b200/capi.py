@@ -152,6 +152,7 @@ EXPORTS = [
     "gcs_b200_program_run_tangents", "gcs_b200_program_run_tangents_host",
     "gcs_b200_program_run_recorded", "gcs_b200_program_run_recorded_host", "gcs_b200_program_adjoints",
     "gcs_b200_program_adjoints_host", "gcs_b200_program_fit", "gcs_b200_program_fit_host", "gcs_b200_fit_check",
+    "gcs_b200_program_run_fused", "gcs_b200_program_run_fused_host",
 ]
 
 
@@ -208,6 +209,10 @@ def load():
     lib.gcs_b200_program_run_recorded.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
     lib.gcs_b200_program_run_recorded_host.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
                                                        C.POINTER(C.c_float)]
+    lib.gcs_b200_program_run_fused.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p,
+                                               C.c_void_p, C.c_void_p]
+    lib.gcs_b200_program_run_fused_host.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
+                                                    C.c_void_p, C.c_void_p, C.POINTER(C.c_float)]
     lib.gcs_b200_program_adjoints.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.gcs_b200_program_adjoints_host.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.POINTER(C.c_float)]
     lib.gcs_b200_program_fit.argtypes = [C.c_void_p, C.POINTER(CFitDesc), C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,

@@ -75,6 +75,21 @@ int launch_kernel(void (*kernel)(P...), long long grid, int block, size_t smem, 
     return GCS_OK;
 }
 
+// The cooperative sibling of launch_kernel: cudaLaunchCooperativeKernel, counted.  Every block of
+// the grid must be co-resident; a grid that is not fails here as a launch error (GCS_E_CUDA)
+// instead of waiting at a grid barrier for blocks that never run.
+template <class... P, class... A>
+int launch_cooperative(void (*kernel)(P...), unsigned grid, int block, size_t smem, cudaStream_t st, const A&... args)
+{
+    void* params[] = { const_cast<A*>(&args)... };
+    const cudaError_t e = cudaLaunchCooperativeKernel(reinterpret_cast<const void*>(kernel), dim3(grid), dim3(block), params, smem, st);
+    count_launch();
+    cudaGetLastError();  // the launch's error is e
+    if (e != cudaSuccess)
+        return fail(GCS_E_CUDA, "cudaLaunchCooperativeKernel(%u blocks of %d threads) -> %s", grid, block, cudaGetErrorString(e));
+    return GCS_OK;
+}
+
 // f(std::integral_constant<int, kind>()): f sees a kind known at run time as a compile-time
 // constant; a kind outside 1..4 is K5.  The host and the kernels' device lambdas share it; the
 // pragma lets the one template call either.

@@ -28,6 +28,7 @@
 // reduce kernel adds those into the working slot-adjoint table and the value adjoints, each table
 // entry's contributions in ascending (row, role) order from reader lists built at create time.  No
 // atomics: the result does not depend on K, the stream or the schedule.
+#include <cooperative_groups.h>
 #include <cuda_runtime.h>
 
 #include <cmath>
@@ -338,6 +339,148 @@ __global__ void __launch_bounds__(kThreads) program_tangent_kernel(const WaveArg
     }
     double* const dst = dpos + 4 * (long long)row.elem[2] * T;
     for (int q = 0; q < out_cols(kind); ++q) dst[q * T] = out[q];
+}
+
+// ---- fused runs (gcs_b200_program_run_fused): every wave in one cooperative launch ----
+// One thread per (row, instance) of a wave does what the wave path spreads over the gather, the kind
+// batch's solve, the scatter and the tangent kernel, with the columns in registers instead of a kind
+// batch: gather_row, then newton_pair_kernel's body (same device functions, same operations in the
+// same order, so the same bits as every bit-identical mapping), then the scatter's writes and count,
+// then the tangents along every direction.  A grid barrier separates the waves.
+constexpr int kFusedThreads = 128;
+
+struct FusedArgs {
+    const gcs_b200_program_row* rows;
+    const long long* offsets;  // device copy of the descriptor's offsets
+    int n_waves;
+    long long K, n_slots, n_values, T;
+    const double* initial;     // [n_slots][4]
+    // Other blocks write positions and dpositions during the launch (earlier waves' targets, which
+    // later waves read): they are read with plain loads, never __ldg, and are not `const __restrict__`.
+    // The grid barrier between waves orders those writes before the reads.
+    double* pos;               // [K][n_slots][4]
+    double* dpos;              // [K][n_slots][4][T]
+    const double* val;         // [K][n_values]
+    const double* dval;        // [K][n_values][T]
+    uint32_t* nonconverged;    // [K] or null
+};
+
+// kKindOfSolver on the device
+__device__ __forceinline__ int kind_of_solver(int solver)
+{
+    switch (solver) {
+    case 1: case 4: return GCS_KIND_PP;
+    case 2: case 5: return GCS_KIND_SDD;
+    case 6: return GCS_KIND_PPL;
+    case 7: return GCS_KIND_PLL;
+    default: return GCS_KIND_ANG;
+    }
+}
+
+// gather_row's side for a fused run: anchors into the positions, columns into registers
+struct GatherRegisters {
+    double* pa;
+    double* pb;
+    double v[3];
+    const double* canvas;
+    double k[13];
+    __device__ __forceinline__ double& slot(int role, int q) { return (role ? pb : pa)[q]; }
+    __device__ __forceinline__ double value(int q) const { return v[q]; }
+    __device__ __forceinline__ double cst(int c) const { return canvas[c]; }
+    __device__ __forceinline__ void in(int col, double x) { k[col] = x; }
+};
+
+// Row `row` (of kind KIND) for instance j.  Out of line per kind, so that the kernel holds one
+// kind's registers at a time rather than the union of all five.
+template <int KIND>
+__device__ __noinline__ void fused_row(const FusedArgs& f, const gcs_b200_program_row& row, long long j)
+{
+    using S = gcsk::Sys<KIND>;
+    double* const pos = f.pos + j * f.n_slots * 4;
+    const double* const val = f.val + j * f.n_values;
+    GatherRegisters g { pos + 4 * (long long)row.elem[0], pos + 4 * (long long)row.elem[1],
+        { row_value(row, 0, val, 1), row_value(row, 1, val, 1), row_value(row, 2, val, 1) }, row.canvas, {} };
+    gather_row(row, g);
+    // newton_pair_kernel
+    S sys;
+    sys.load(g.k);
+    double cx[2], cy[2];
+    if constexpr (S::kGuessFromCols) {
+        gcsk::column_seed<KIND>(g.k, 0, cx[0], cy[0]);
+        gcsk::column_seed<KIND>(g.k, 1, cx[1], cy[1]);
+    } else {
+        gcsk::default_seed(0, cx[0], cy[0]);
+        gcsk::default_seed(1, cx[1], cy[1]);
+    }
+    gcsk::FastConsts fc;
+    fc.init((double)(f.K >> 62));  // 0.0, opaque to the compiler
+    bool cva = fabs(0.0 - cx[0]) < fc.tol && fabs(0.0 - cy[0]) < fc.tol;
+    bool cvb = fabs(0.0 - cx[1]) < fc.tol && fabs(0.0 - cy[1]) < fc.tol;
+    int ita = 0, itb = 0;
+    gcsk::newton_run2<KIND>(sys, sys, fc, cx[0], cy[0], ita, cva, !cva, cx[1], cy[1], itb, cvb, !cvb);
+    double out[4];
+    const int root = gcsk::select_and_finish<KIND, 2>(g.k, (uint8_t)row.code, cx, cy, out);
+    // program_scatter_kernel, with chosen_root's test
+    double* const dst = pos + 4 * (long long)row.elem[2];
+#pragma unroll
+    for (int q = 0; q < S::kOut; ++q) dst[q] = out[q];
+    const bool converged = root ? cvb : cva;
+    if (f.nonconverged && !converged) atomicAdd(f.nonconverged + j, 1u);
+    if (f.T == 0) return;
+    // program_tangent_kernel, one direction after the other; the unknown at the root is the output
+    // point (K1, K3, K4) or the chosen seed's normal (K2, K5), which is the chosen candidate either way
+    const long long T = f.T;
+    double* const dpos = f.dpos + j * f.n_slots * 4 * T;
+    const double* const dval = f.dval + j * f.n_values * T;
+    gcsk::RowTangent<KIND> lin;
+    if (converged) lin.init(g.k, root ? cx[1] : cx[0], root ? cy[1] : cy[0]);
+#pragma unroll 1
+    for (long long t = 0; t < T; ++t) {
+        GatherTangents d { dpos + 4 * (long long)row.elem[0] * T + t, dpos + 4 * (long long)row.elem[1] * T + t,
+            { row_value(row, 0, dval + t, T), row_value(row, 1, dval + t, T), row_value(row, 2, dval + t, T) }, T, {} };
+        gather_row(row, d);
+        double dout[4];
+        if (!converged) {
+            // not a root, so the implicit function theorem does not apply
+            dout[0] = dout[1] = dout[2] = dout[3] = __longlong_as_double(0x7ff8000000000000LL);
+        } else {
+            lin.apply(d.kd, dout);
+        }
+        double* const ddst = dpos + 4 * (long long)row.elem[2] * T + t;
+#pragma unroll
+        for (int q = 0; q < S::kOut; ++q) ddst[q * T] = dout[q];
+    }
+}
+
+// A persistent grid, launched cooperatively (launch_cooperative) with at most as many blocks as
+// can be co-resident.  Every thread reaches every grid.sync(): there is no early return, the loops
+// are grid-stride, and the wave bounds come from the device copy of the offsets, the same for every
+// thread.
+__global__ void __launch_bounds__(kFusedThreads) program_fused_kernel(const __grid_constant__ FusedArgs f)
+{
+    cooperative_groups::grid_group grid = cooperative_groups::this_grid();
+    const long long first = (long long)blockIdx.x * blockDim.x + threadIdx.x, step = (long long)gridDim.x * blockDim.x;
+    // what run_on's copies and memsets do: every instance starts from the initial positions (copied
+    // as bits), the counts and every slot's tangent from 0
+    const long long table = f.n_slots * 4;
+    const long long* const init = reinterpret_cast<const long long*>(f.initial);
+    long long* const pos = reinterpret_cast<long long*>(f.pos);
+    for (long long q = first; q < f.K * table; q += step) pos[q] = init[q % table];
+    if (f.nonconverged)
+        for (long long q = first; q < f.K; q += step) f.nonconverged[q] = 0;
+    for (long long q = first; q < f.K * table * f.T; q += step) f.dpos[q] = 0.0;
+    grid.sync();
+    for (int wave = 0; wave < f.n_waves; ++wave) {
+        const long long lo = f.offsets[wave * kKinds], hi = f.offsets[(wave + 1) * kKinds];
+        if (hi == lo) continue;  // the same for every thread: no barrier for an empty wave
+        // sub-system s = r * K + j as place() orders them
+        for (long long s = first; s < (hi - lo) * f.K; s += step) {
+            const long long r = s / f.K, j = s - r * f.K;
+            const gcs_b200_program_row& row = f.rows[lo + r];
+            with_kind(kind_of_solver(row.solver), [&](auto K) { fused_row<decltype(K)::value>(f, row, j); });
+        }
+        grid.sync();
+    }
 }
 
 // One wave of the adjoint sweep, over the batches a recorded run kept.  The transpose of the
@@ -803,6 +946,10 @@ struct gcs_b200_program {
     gcs_b200_program_row* rows = nullptr;
     double* initial = nullptr;
     cudaStream_t stream = nullptr;  // uploads and the _host entry points
+    // fused runs: the device copy of `offsets`, and the co-resident blocks of program_fused_kernel on
+    // the program's device (0 until the first fused run asks)
+    long long* offsets_dev = nullptr;
+    long long fused_capacity = 0;
     // the kind batches of plain and tangent runs, reused by every wave
     DeviceBuffer<unsigned char> scratch;
     // tables of the _host entry points, and the counts and tangent tables of _host runs and of fits
@@ -919,6 +1066,11 @@ int launch(void (*kernel)(A), long long threads, cudaStream_t st, const A& args,
     return gcsk::launch_kernel(kernel, (threads + kThreads - 1) / kThreads, kThreads, 0, st, too_many, args);
 }
 
+// how a run goes: wave by wave through the kind batches (gcs_b200_program_run[_tangents]), the same
+// keeping every wave's batches on the tape (gcs_b200_program_run_recorded), or in one cooperative
+// launch (gcs_b200_program_run_fused)
+enum class RunKind { waves, recorded, fused };
+
 // T = 0: a plain run.  T > 0: also the tangents along T directions (dvalues / dpositions).
 // recorded: every wave's batches at their own place of the tape (T = 0 only)
 int run_on(gcs_b200_program* p, long long K, const double* values, double* positions, uint32_t* nonconverged, int variant,
@@ -986,6 +1138,29 @@ int run_on(gcs_b200_program* p, long long K, const double* values, double* posit
     }
     if (recorded) p->recorded_k = K;
     return GCS_OK;
+}
+
+// Device current, checks done: a fused run (T = 0: plain) on `st`, one cooperative launch.  The grid:
+// as many blocks as the largest wave's rows x K sub-systems fill, at most as many as can be
+// co-resident on the device, at least one.
+int fused_on(gcs_b200_program* p, long long K, const double* values, double* positions, uint32_t* nonconverged, cudaStream_t st,
+    long long T, const double* dvalues, double* dpositions)
+{
+    if (p->fused_capacity == 0) {
+        int per_sm = 0, sms = 0;
+        CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, program_fused_kernel, kFusedThreads, 0));
+        CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, p->device));
+        p->fused_capacity = (long long)per_sm * sms;
+    }
+    const long long need = (p->max_wave_rows * K + kFusedThreads - 1) / kFusedThreads;
+    long long grid = need < p->fused_capacity ? need : p->fused_capacity;
+    if (grid < 1) grid = 1;
+    FusedArgs f;
+    memset(&f, 0, sizeof(f));
+    f.rows = p->rows, f.offsets = p->offsets_dev, f.n_waves = p->n_waves;
+    f.K = K, f.n_slots = p->n_slots, f.n_values = p->n_values, f.T = T;
+    f.initial = p->initial, f.pos = positions, f.dpos = dpositions, f.val = values, f.dval = dvalues, f.nonconverged = nonconverged;
+    return gcsk::launch_cooperative(program_fused_kernel, (unsigned)grid, kFusedThreads, 0, st, f);
 }
 
 // device current; the sweep's working tables for the recorded K x T cotangents
@@ -1069,6 +1244,15 @@ int check_tangent_run(const gcs_b200_program* p, long long K, const double* valu
     return check_run(p, K, values, positions, variant);
 }
 
+// a fused run's checks: n_tangents >= 0, then a plain run's (T = 0) or a tangent run's
+int check_fused_run(const gcs_b200_program* p, long long K, const double* values, const double* positions, int T, const double* dvalues,
+    const double* dpositions)
+{
+    if (T < 0) return fail(GCS_E_INVALID, "n_tangents must be >= 0 (got %d)", T);
+    if (T == 0) return check_run(p, K, values, positions, GCS_VARIANT_DEFAULT);
+    return check_tangent_run(p, K, values, positions, T, dvalues, dpositions, GCS_VARIANT_DEFAULT);
+}
+
 // one copy of the _host entry points; none when `bytes` is 0
 struct Copy {
     void* dst;
@@ -1117,15 +1301,17 @@ int grow_tables(gcs_b200_program* p, long long K, long long T, bool host, cudaSt
 
 // device current, checks done
 int run_host(gcs_b200_program* p, long long K, const double* values, double* positions, uint32_t* nonconverged, int variant,
-    float ms[3], long long T = 0, const double* dvalues = nullptr, double* dpositions = nullptr, bool recorded = false)
+    float ms[3], long long T = 0, const double* dvalues = nullptr, double* dpositions = nullptr, RunKind how = RunKind::waves)
 {
     const size_t vbytes = (size_t)K * p->n_values * sizeof(double), pbytes = (size_t)K * p->n_slots * 4 * sizeof(double);
     const size_t cbytes = (size_t)K * sizeof(uint32_t);
     RC_TRY(grow_tables(p, K, T, true, p->stream));
     return on_host(p, { { p->values.ptr, values, vbytes }, { p->dvalues.ptr, dvalues, vbytes * T } },
         [&](cudaStream_t s) {
-            return run_on(p, K, p->values.ptr, p->positions.ptr, nonconverged ? p->counts.ptr : nullptr, variant, s, T, p->dvalues.ptr,
-                p->dpositions.ptr, recorded);
+            uint32_t* const counts = nonconverged ? p->counts.ptr : nullptr;
+            if (how == RunKind::fused) return fused_on(p, K, p->values.ptr, p->positions.ptr, counts, s, T, p->dvalues.ptr, p->dpositions.ptr);
+            return run_on(p, K, p->values.ptr, p->positions.ptr, counts, variant, s, T, p->dvalues.ptr, p->dpositions.ptr,
+                how == RunKind::recorded);
         },
         { { positions, p->positions.ptr, pbytes }, { dpositions, p->dpositions.ptr, pbytes * T },
             { nonconverged, p->counts.ptr, nonconverged ? cbytes : 0 } },
@@ -1229,7 +1415,9 @@ int gcs_b200_program_create(const gcs_b200_program_desc* d, int device, gcs_b200
     for (auto& e : p->ev)
         if (cudaEventCreate(&e) != cudaSuccess) return bail(fail(GCS_E_CUDA, "event creation failed"));
     const size_t row_bytes = (size_t)d->n_rows * sizeof(gcs_b200_program_row), init_bytes = (size_t)d->n_slots * 4 * sizeof(double);
-    if ((row_bytes && cudaMalloc(&p->rows, row_bytes) != cudaSuccess) || (init_bytes && cudaMalloc(&p->initial, init_bytes) != cudaSuccess)) {
+    const size_t off_bytes = p->offsets.size() * sizeof(long long);
+    if ((row_bytes && cudaMalloc(&p->rows, row_bytes) != cudaSuccess) || (init_bytes && cudaMalloc(&p->initial, init_bytes) != cudaSuccess)
+        || cudaMalloc(&p->offsets_dev, off_bytes) != cudaSuccess) {
         cudaGetLastError();
         return bail(fail(GCS_E_NOMEM, "cudaMalloc for a program of %lld rows and %d slots failed", (long long)d->n_rows, d->n_slots));
     }
@@ -1282,6 +1470,7 @@ int gcs_b200_program_create(const gcs_b200_program_desc* d, int device, gcs_b200
     }
     if ((row_bytes && cudaMemcpyAsync(p->rows, d->rows, row_bytes, cudaMemcpyHostToDevice, p->stream) != cudaSuccess)
         || (init_bytes && cudaMemcpyAsync(p->initial, d->initial, init_bytes, cudaMemcpyHostToDevice, p->stream) != cudaSuccess)
+        || cudaMemcpyAsync(p->offsets_dev, p->offsets.data(), off_bytes, cudaMemcpyHostToDevice, p->stream) != cudaSuccess
         || (ent_bytes && cudaMemcpyAsync(p->ent, ent.data(), ent_bytes, cudaMemcpyHostToDevice, p->stream) != cudaSuccess)
         || cudaMemcpyAsync(p->begin, begin.data(), begin_bytes, cudaMemcpyHostToDevice, p->stream) != cudaSuccess
         || (reader_bytes && cudaMemcpyAsync(p->readers, readers.data(), reader_bytes, cudaMemcpyHostToDevice, p->stream) != cudaSuccess)
@@ -1342,7 +1531,25 @@ int gcs_b200_program_run_recorded_host(gcs_b200_program* p, int64_t K, const dou
     RC_TRY(check_run(p, K, values, positions, variant));
     DeviceScope on(p->device);
     RC_TRY(on.rc);
-    return run_host(p, K, values, positions, nonconverged, variant, ms, 0, nullptr, nullptr, true);
+    return run_host(p, K, values, positions, nonconverged, variant, ms, 0, nullptr, nullptr, RunKind::recorded);
+}
+
+int gcs_b200_program_run_fused(gcs_b200_program* p, int64_t K, const double* values, double* positions, uint32_t* nonconverged,
+    int32_t T, const double* dvalues, double* dpositions, void* stream)
+{
+    RC_TRY(check_fused_run(p, K, values, positions, T, dvalues, dpositions));
+    DeviceScope on(p->device);
+    RC_TRY(on.rc);
+    return fused_on(p, K, values, positions, nonconverged, static_cast<cudaStream_t>(stream), T, dvalues, dpositions);
+}
+
+int gcs_b200_program_run_fused_host(gcs_b200_program* p, int64_t K, const double* values, double* positions, uint32_t* nonconverged,
+    int32_t T, const double* dvalues, double* dpositions, float ms[3])
+{
+    RC_TRY(check_fused_run(p, K, values, positions, T, dvalues, dpositions));
+    DeviceScope on(p->device);
+    RC_TRY(on.rc);
+    return run_host(p, K, values, positions, nonconverged, GCS_VARIANT_DEFAULT, ms, T, dvalues, dpositions, RunKind::fused);
 }
 
 int gcs_b200_program_adjoints(gcs_b200_program* p, int32_t T, const double* adj_positions, double* adj_values, void* stream)
@@ -1417,7 +1624,7 @@ void gcs_b200_program_destroy(gcs_b200_program* p)
         if (p->stream) cudaStreamSynchronize(p->stream), cudaStreamDestroy(p->stream);
         for (auto e : p->ev)
             if (e) cudaEventDestroy(e);
-        cudaFree(p->rows), cudaFree(p->initial), cudaFree(p->scratch.ptr);
+        cudaFree(p->rows), cudaFree(p->initial), cudaFree(p->offsets_dev), cudaFree(p->scratch.ptr);
         cudaFree(p->values.ptr), cudaFree(p->positions.ptr), cudaFree(p->counts.ptr);
         cudaFree(p->dvalues.ptr), cudaFree(p->dpositions.ptr);
         cudaFree(p->ent), cudaFree(p->begin), cudaFree(p->readers), cudaFree(p->tape.ptr);

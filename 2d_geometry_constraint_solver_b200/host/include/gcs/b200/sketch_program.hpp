@@ -75,6 +75,14 @@ public:
     ProgramRunStats runTangents(const double* values, std::int64_t K, const double* dvalues, int T, double* positions, double* dpositions,
         std::uint32_t* nonconverged = nullptr, int nDevices = 1);
 
+    // run() (T = 0) or runTangents() (T >= 1) in one kernel launch per device
+    // (gcs_b200_program_run_fused_host): every wave in one cooperative launch, no kind batches.
+    // Positions, dpositions and counts equal run() / runTangents() bit for bit; dvalues in radians for
+    // angles as there (may be null when T = 0).  Instances split over devices as run() splits them.
+    // Leaves a record() alone.  Throws std::invalid_argument for T < 0 before any device call.
+    ProgramRunStats runFused(const double* values, std::int64_t K, const double* dvalues, int T, double* positions, double* dpositions,
+        std::uint32_t* nonconverged = nullptr, int nDevices = 1);
+
     // run(), also recording what adjoints() needs (gcs_b200_program_run_recorded): every wave's
     // batches stay on the device, about n_rows x K x 100 bytes.  Positions and counts are run()'s.
     ProgramRunStats record(const double* values, std::int64_t K, double* positions, std::uint32_t* nonconverged = nullptr,
@@ -123,8 +131,10 @@ private:
     gcs_b200_program* onDevice(int device);
     void release();
     void stage(const double* values, std::int64_t K, const double* dvalues, int T);
+    // how runImpl runs: wave by wave (run, runTangents), recording (record), in one launch (runFused)
+    enum class RunKind { waves, recorded, fused };
     ProgramRunStats runImpl(const double* values, std::int64_t K, const double* dvalues, int T, double* positions, double* dpositions,
-        std::uint32_t* nonconverged, int nDevices, bool recorded = false);
+        std::uint32_t* nonconverged, int nDevices, RunKind how = RunKind::waves);
 
     BatchReport m_report;
     std::vector<gcs_b200_program_row> m_rows;

@@ -221,10 +221,17 @@ ProgramRunStats SketchProgram::runTangents(const double* values, std::int64_t K,
     return runImpl(values, K, dvalues, T, positions, dpositions, nonconverged, nDevices);
 }
 
+ProgramRunStats SketchProgram::runFused(const double* values, std::int64_t K, const double* dvalues, int T, double* positions,
+    double* dpositions, std::uint32_t* nonconverged, int nDevices)
+{
+    if (T < 0) throw std::invalid_argument("SketchProgram::runFused: T must be >= 0 (got " + std::to_string(T) + ")");
+    return runImpl(values, K, dvalues, T, positions, dpositions, nonconverged, nDevices, RunKind::fused);
+}
+
 ProgramRunStats SketchProgram::record(const double* values, std::int64_t K, double* positions, std::uint32_t* nonconverged, int nDevices)
 {
     m_recordedDevices = 0;  // a failed record() leaves nothing to sweep
-    const ProgramRunStats st = runImpl(values, K, nullptr, 0, positions, nullptr, nonconverged, nDevices, true);
+    const ProgramRunStats st = runImpl(values, K, nullptr, 0, positions, nullptr, nonconverged, nDevices, RunKind::recorded);
     m_recordedValues.assign(values, values + static_cast<std::size_t>(K) * nValues());
     m_recordedK = K;
     // runImpl's split: instances in contiguous ranges over the first devicesFor(nDevices, K) devices
@@ -338,9 +345,9 @@ void SketchProgram::stage(const double* values, std::int64_t K, const double* dv
     }
 }
 
-// T = 0: run() or record(); T > 0: runTangents()
+// T = 0: run(), record() or a plain runFused(); T > 0: runTangents() or a tangent runFused()
 ProgramRunStats SketchProgram::runImpl(const double* values, std::int64_t K, const double* dvalues, int T, double* positions,
-    double* dpositions, std::uint32_t* nonconverged, int nDevices, bool recorded)
+    double* dpositions, std::uint32_t* nonconverged, int nDevices, RunKind how)
 {
     const auto t0 = Clock::now();
     if (K < 1) throw std::invalid_argument("SketchProgram::run: K must be >= 1");
@@ -350,12 +357,18 @@ ProgramRunStats SketchProgram::runImpl(const double* values, std::int64_t K, con
     for (int g = 0; g < nDevices; ++g) onDevice(g);
 
     const int variant = kernelVariant();
-    const char* entry = recorded ? "gcs_b200_program_run_recorded_host" : T == 0 ? "gcs_b200_program_run_host" : "gcs_b200_program_run_tangents_host";
+    const char* entry = how == RunKind::fused ? "gcs_b200_program_run_fused_host"
+        : how == RunKind::recorded            ? "gcs_b200_program_run_recorded_host"
+        : T == 0                              ? "gcs_b200_program_run_host"
+                                              : "gcs_b200_program_run_tangents_host";
     ProgramRunStats st = fanOut(K, nDevices, entry, [&](int g, std::int64_t lo, std::int64_t hi, float* ms) {
         gcs_b200_program* p = m_device[static_cast<std::size_t>(g)];
         const std::int64_t vo = lo * static_cast<std::int64_t>(nv), po = lo * static_cast<std::int64_t>(table);
         std::uint32_t* counts = nonconverged ? m_stageCounts + lo : nullptr;
-        return recorded ? gcs_b200_program_run_recorded_host(p, hi - lo, m_stageValues + vo, m_stagePositions + po, counts, variant, ms)
+        if (how == RunKind::fused)
+            return gcs_b200_program_run_fused_host(p, hi - lo, m_stageValues + vo, m_stagePositions + po, counts, T, m_stageDValues + vo * T,
+                m_stageDPositions + po * T, ms);
+        return how == RunKind::recorded ? gcs_b200_program_run_recorded_host(p, hi - lo, m_stageValues + vo, m_stagePositions + po, counts, variant, ms)
             : T == 0 ? gcs_b200_program_run_host(p, hi - lo, m_stageValues + vo, m_stagePositions + po, counts, variant, ms)
             : gcs_b200_program_run_tangents_host(p, hi - lo, m_stageValues + vo, m_stagePositions + po, counts, T, m_stageDValues + vo * T,
                 m_stageDPositions + po * T, variant, ms);

@@ -927,6 +927,20 @@ GCS_API int gcs_host_program_run_tangents(gcs_host_program* h, int64_t K, const 
     }
 }
 
+// run() or run_tangents() in one kernel launch per device (SketchProgram::runFused): T = 0 is a plain
+// run (dvalues, dpositions may be NULL), T > 0 a tangent run; the results equal those entry points'
+// bit for bit.  Returns 0 or -1.
+GCS_API int gcs_host_program_run_fused(gcs_host_program* h, int64_t K, const double* values, int T, const double* dvalues,
+    double* positions, double* dpositions, uint32_t* nonconverged, int n_devices, int64_t* stats)
+{
+    try {
+        programStats(h, h->prog->runFused(values, K, dvalues, T, positions, dpositions, nonconverged, n_devices), n_devices, stats);
+        return 0;
+    } catch (const std::exception& ex) {
+        return fail(ex);
+    }
+}
+
 // run(), recording what gcs_host_program_adjoints needs (SketchProgram::record).  Returns 0 or -1.
 GCS_API int gcs_host_program_run_recorded(gcs_host_program* h, int64_t K, const double* values, double* positions, uint32_t* nonconverged,
     int n_devices, int64_t* stats)

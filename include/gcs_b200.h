@@ -394,6 +394,31 @@ GCS_B200_API int gcs_b200_program_run_recorded(gcs_b200_program* prog, int64_t n
 /* The same with host buffers, as gcs_b200_program_run_host. */
 GCS_B200_API int gcs_b200_program_run_recorded_host(gcs_b200_program* prog, int64_t n_instances, const double* values,
     double* positions, uint32_t* nonconverged, int variant, float ms[3]);
+/* Fused runs: every wave of a run in exactly one kernel launch.  One cooperative launch
+ * (cudaLaunchCooperativeKernel) of a persistent grid does the whole run: it writes the initial
+ * positions into every instance, zeroes nonconverged (and, with n_tangents = T > 0, dpositions), then
+ * for each non-empty wave one thread per (row, instance) gathers the row's columns into registers,
+ * solves both seeds, writes the row's output and count and, for T > 0, its tangents along every
+ * direction; a grid barrier separates the waves.  No copy, no memset, no other launch.
+ * Equality: positions, nonconverged and dpositions are those of gcs_b200_program_run (T = 0) and
+ * gcs_b200_program_run_tangents (T > 0) with any bit-identical variant, bit for bit, NaN for NaN: the
+ * thread runs the same device functions in the same order as the gather, the 2-seed kernels, the
+ * scatter and the tangent kernel.  There is no variant argument: the contracted class is not offered.
+ * Memory: no kind batches.  The only device memory a fused run uses beyond the caller's tables is the
+ * copy of `offsets` uploaded at create.  It leaves the tape of a recorded run alone, so it may come
+ * between a recorded run and its adjoint sweep.  Runs of one program still must not overlap: order
+ * them, fused or not, on one stream.
+ * The grid has as many blocks of 128 threads as the largest wave's rows x K sub-systems fill, at
+ * most as many as can be co-resident on the device: any K works, larger waves are grid-strided.
+ * Stream-ordered on `cuda_stream`, device pointers, layouts as gcs_b200_program_run_tangents; does not
+ * synchronise.  Checked before any device call: n_tangents >= 0, then what gcs_b200_program_run
+ * (T = 0) or gcs_b200_program_run_tangents (T > 0) checks. */
+GCS_B200_API int gcs_b200_program_run_fused(gcs_b200_program* prog, int64_t n_instances, const double* values, double* positions,
+    uint32_t* nonconverged, int32_t n_tangents, const double* dvalues, double* dpositions, void* cuda_stream);
+/* The same with host buffers, as gcs_b200_program_run_tangents_host (values and dvalues up, the one
+ * launch, positions, dpositions and counts down on the program's own stream, then a synchronise). */
+GCS_B200_API int gcs_b200_program_run_fused_host(gcs_b200_program* prog, int64_t n_instances, const double* values,
+    double* positions, uint32_t* nonconverged, int32_t n_tangents, const double* dvalues, double* dpositions, float ms[3]);
 /* Adjoints (reverse mode) of the program's last recorded run, with that run's K: for each instance k
  * and T = n_cotangents >= 1 cotangents adj_positions[k][:][:][t] (a weight on every position
  * coordinate),
